@@ -2,6 +2,7 @@
 """Benchmark of the ChunkyCL render path on B200 (contract: see the task statement / DESIGN.md "Measurement").
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload config1|indoor|entities|large]
+                  [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A step = one window of SPP_PER_STEP path-tracing passes over the full canvas of the BASELINE config-1 scene (synthetic 256^3
@@ -27,6 +28,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 SPP_PER_STEP = 16
+DUMP_LIMIT_BYTES = 64 << 20
 METRIC = "path samples/sec"
 UNIT = "samples/s"
 # The contract line is config1 (the configuration the metric is quoted on that fits one GPU).  --workload selects one of the
@@ -262,6 +264,16 @@ def measure_workload(workload: str, ctx, loader, steps: int, warmup: int, flush,
             "steps": steps, "warmup": warmup, "scene_commit_ms": commit_ms, "scene_device_bytes": ctx.scene_device_bytes()}
 
 
+def dump_window(ctx, out_dir: str, width: int, height: int):
+    """What a caller of the timed path receives after the last step: the window's mean RGB (ccu_render_read), float32
+    [rows, width, 3].  Frames above DUMP_LIMIT_BYTES keep every k-th row (the smallest k that fits)."""
+    img, _ = ctx.render_read()
+    img = img.reshape(height, width, 3)
+    k = -(-img.nbytes // DUMP_LIMIT_BYTES)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "window_rgb.npy"), np.ascontiguousarray(img[::k]))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -273,6 +285,7 @@ def main():
     ap.add_argument("--spp-total", type=int, default=0, help="strong scaling: render this many passes in 1024-pass windows split over the GPUs")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-workloads", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's output to DIR/window_rgb.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
@@ -289,6 +302,9 @@ def main():
     rank, world, local_rank = d.rank, d.world, d.local_rank
     if world != args.gpus and world == 1 and args.gpus > 1:
         print(f"bench.py: --gpus {args.gpus} needs torchrun with {args.gpus} ranks", file=sys.stderr)
+        return 2
+    if args.dump_outputs and world > 1:
+        print("bench.py: --dump-outputs needs a single-GPU run (each rank holds only its share of the reduced window)", file=sys.stderr)
         return 2
     torch.cuda.set_device(local_rank)
 
@@ -336,6 +352,8 @@ def main():
     sampler.stop_flag = True
     sampler.join()
     launches = ctx.launch_count() - launches_w
+    if args.dump_outputs:
+        dump_window(ctx, args.dump_outputs, WIDTH, HEIGHT)
     total_ms = d.max(float(sum(dev_ms)))
     samples_per_step = WIDTH * HEIGHT * window
     value = samples_per_step * args.steps / (total_ms * 1e-3)
@@ -364,7 +382,7 @@ def main():
                   "how": "ccu_bench_gather: random 16-byte ld.global.cg per 32-byte sector over a 4 MiB / 1 GiB array, all SMs"}
 
     # ---- end to end through the public API: seeds H2D + read-back + merge into the host double buffer, every step -----
-    e_steps = max(10, args.steps) if not strong else args.steps
+    e_steps = args.steps
     n_floats = WIDTH * HEIGHT * 3
     if world == 1:
         # CudaPathTracingRenderer.render() exactly as Chunky drives it: ONE render of e_steps windows; every window = 16

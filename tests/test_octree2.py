@@ -1,4 +1,4 @@
-"""`.octree2` loader (SURVEY 8f #4): round trip on a synthetic file, the reference's benchmark scene where it exists."""
+"""`.octree2` loader (SURVEY 8f #4): round trip on a synthetic file, a crop of the reference's benchmark scene."""
 import os
 
 import numpy as np
@@ -7,7 +7,7 @@ import pytest
 from chunkyclplugin_b200 import native, octree2
 from chunkyclplugin_b200.javarandom import pass_seeds
 
-REF_DIR = "/root/reference/benchmark/OpenCL_test"
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def _synthetic_file(tmp_path, scenes):
@@ -63,21 +63,22 @@ def test_bad_files(tmp_path):
         octree2.pack_preorder(np.array([-1, 0, 0], dtype=np.int32))     # branch with missing children
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REF_DIR, "OpenCL_test.octree2")), reason="reference benchmark scene not present")
 def test_reference_benchmark_scene():
-    """The reference's own fixture: numbers as recorded in SURVEY.md section 4."""
+    """The reference's own fixture (benchmark/OpenCL_test), cropped by scripts/make_octree2_fixture.py to one 128^3 cell:
+    its header and 3091 palette NBT compounds verbatim, world and water trees of depth 10 with air outside the cell."""
     import oracle
-    o = octree2.load(os.path.join(REF_DIR, "OpenCL_test.octree2"))
+    path = os.path.join(GOLD, "opencl_test_crop.octree2")
+    o = octree2.load(path)
     st = o.stats()
     assert (o.version, o.palette_version, len(o.blocks)) == (6, 4, 3091)
-    assert st == {"nodes": 2764457, "branches": 345557, "any_type_leaves": 312369, "leaf_types": 2320, "depth": 10,
-                  "water_nodes": 356329, "water_depth": 10}
+    assert st == {"nodes": 255249, "branches": 31906, "any_type_leaves": 23887, "leaf_types": 817, "depth": 10,
+                  "water_nodes": 6177, "water_depth": 10}
     assert 1 + 8 * st["branches"] == st["nodes"]
-    s = octree2.load_scene(os.path.join(REF_DIR, "OpenCL_test.octree2"), os.path.join(REF_DIR, "OpenCL_test.json"), 160, 90)
-    # commit-time layouts against the root descent on the real scene (depth 10, ANY_TYPE leaves)
+    s = octree2.load_scene(path, os.path.join(GOLD, "opencl_test_camera.json"), 160, 90)
+    # commit-time layouts against the root descent on the real scene (depth 10, ANY_TYPE leaves), in and around the cell
     from test_layouts import root_descent
     rng = np.random.default_rng(2)
-    xyz = np.stack([rng.integers(0, 672, 100000), rng.integers(0, 140, 100000), rng.integers(0, 496, 100000)], -1)
+    xyz = np.stack([rng.integers(448, 704, 100000), rng.integers(0, 192, 100000), rng.integers(320, 576, 100000)], -1)
     tree = np.asarray(s.octree, dtype=np.int32)
     want_value, want_level = root_descent(tree, 10, xyz)
     got = native.layout_lookup(tree, 10, xyz)
