@@ -5,20 +5,6 @@
 #pragma once
 #include "ccu_math.cuh"
 
-// march_begin_core is kept out of line (one copy instead of one per ray kind: measured -4 % on the wavefront kernel, whose
-// shading stages are limited by instruction fetch); -DCCU_INLINE_MARCH_BEGIN restores the inlined form.  CCU_NI_MATERIAL /
-// CCU_NI_MATH do the same for the material evaluation / math helpers (measured: no gain, off by default).
-#ifndef CCU_INLINE_MARCH_BEGIN
-#define CCU_MARCH_BEGIN_INLINE static __device__ __noinline__
-#else
-#define CCU_MARCH_BEGIN_INLINE __device__ __forceinline__
-#endif
-#ifdef CCU_NI_MATERIAL
-#define CCU_MATERIAL_INLINE static __device__ __noinline__
-#else
-#define CCU_MATERIAL_INLINE __device__ __forceinline__
-#endif
-
 namespace ccu {
 
 #define CCU_ANY_TYPE 0x7FFFFFFE   // block.h:32
@@ -211,11 +197,10 @@ __device__ __forceinline__ float4 sky_read(const DScene &s, float cs, float ct) 
 // ------------------------------------------------------------------------------------------------------
 // material.h:31-82
 // ------------------------------------------------------------------------------------------------------
-// the material words {flags, tint, texSize, texLocation / ARGB, emittance} evaluated at (u, v); returned by value so that an
-// out-of-line copy (CCU_NI_MATERIAL) hands the result back in registers
+// the material words {flags, tint, texSize, texLocation / ARGB, emittance} evaluated at (u, v)
 struct MatOut { float4 color; float emittance; int ok; };
-CCU_MATERIAL_INLINE MatOut material_eval_core(const DScene &s, uint32_t flags, uint32_t tint, uint32_t tex_size, uint32_t col, uint32_t normal_emittance,
-                                              float u, float v) {
+__device__ __forceinline__ MatOut material_eval_core(const DScene &s, uint32_t flags, uint32_t tint, uint32_t tex_size, uint32_t col, uint32_t normal_emittance,
+                                                     float u, float v) {
     MatOut out;
     out.emittance = 0.0f;
     out.ok = 0;
@@ -516,9 +501,10 @@ struct March {
 };
 
 // octree.h:43-64: 1 / d, the distance to the octree cube for a ray that starts outside of it, and whether it enters at all.
-// Returned by value so that an out-of-line copy (CCU_NI_MARCH_BEGIN) hands the result back in registers.
+// Kept out of line (one copy instead of one per ray kind: measured -4 % on the wavefront kernel, whose shading stages are
+// limited by instruction fetch); the result is returned by value, so the copy hands it back in registers.
 struct MarchStart { float3 inv; float t; int entered; };
-CCU_MARCH_BEGIN_INLINE MarchStart march_begin_core(int depth, float3 origin, float3 direction) {
+static __device__ __noinline__ MarchStart march_begin_core(int depth, float3 origin, float3 direction) {
     MarchStart ms;
     ms.inv = f3(1.0f / direction.x, 1.0f / direction.y, 1.0f / direction.z);
     ms.t = 0;

@@ -84,14 +84,6 @@ struct MergeJob {
 
 }  // namespace ccu_host
 
-// BVH stage of the wavefront kernel: with walks that can be handed from warp to warp (CCU_BVH_PARK, ccu_queue.cuh) every warp may
-// walk; the round-1 form needed service warps that never do (23 of 28 walk)
-#if !defined(CCU_BVH_PARK) || CCU_BVH_PARK
-#define CCU_BVH_PARK_DEFAULT_WARPS 64
-#else
-#define CCU_BVH_PARK_DEFAULT_WARPS 23
-#endif
-
 struct ccu_ctx {
     int device = 0;
     cudaStream_t stream = nullptr;        // render stream
@@ -156,8 +148,6 @@ struct ccu_ctx {
     int q_march_bias = 4;
     int q_shade_min = 0;
     int q_sticky_min = 0;      // 0 = default by kernel (CCU_Q_STICKY)
-    int q_leaf_min = 12;
-    int q_bvh_warps = CCU_BVH_PARK_DEFAULT_WARPS;
     int q_march_warps = 18;
     int window_spp = 0;
     int closed_spp = 0;          // passes of the window closed by ccu_render_window_close, read-back in flight, not merged yet

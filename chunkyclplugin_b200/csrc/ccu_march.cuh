@@ -97,10 +97,7 @@ __device__ __forceinline__ int lean_probe(const DScene &s, const unsigned *__res
 // commit nothing.  No branch inside the step means no divergence stacks, no fetch redirects and one load latency per iteration
 // for the whole warp; the lanes whose cell is a single leaf read brick word 0 (one broadcast sector) instead of skipping the load.
 // `done`: the lane's state before the step (only read when !active); returns the state after it.
-// WARP_SKIP (thread-per-ray kernels, whose warps march bundles of neighbouring rays): when no lane of the warp needs a brick -
-// every ray in flight crosses a cell that is one air leaf, the common case high above the terrain - the brick part is skipped
-// for the whole warp (one vote instead of the address arithmetic, the load and the decode).
-template <bool TOPS, bool WARP_SKIP = false>
+template <bool TOPS>
 __device__ __forceinline__ int lean_step_flat(const DScene &s, const unsigned *__restrict__ top, LeanRay &r, bool active, int done) {
     const bool fin0 = r.steps >= s.draw_depth || r.t > r.limit;
     const float3 pos = r.o + r.d * r.t;
@@ -112,13 +109,10 @@ __device__ __forceinline__ int lean_step_flat(const DScene &s, const unsigned *_
     const unsigned ti = (((((unsigned)(bx >> 4) << tl) + (unsigned)(by >> 4)) << tl) + (unsigned)(bz >> 4)) & ((1u << (3 * tl)) - 1u);
     const unsigned e = TOPS ? top[ti] : __ldg(top + ti);
     const bool leaf = (e & CCU_WIDE_LEAF) != 0;
-    int lvl_brick = -1;
-    if (!WARP_SKIP || __any_sync(0xffffffffu, active && !fin && !leaf)) {
-        const unsigned wi = (unsigned)(((bx & 12) << 4) | ((by & 12) << 2) | (bz & 12) | (bx & 3));
-        const unsigned w = __ldg(s.air_bricks + (leaf ? 0u : e * 256u + wi));
-        const int code = (int)((w >> ((((by & 3) << 2) | (bz & 3)) * 2)) & 3u);
-        lvl_brick = w >= CCU_BRICK_UNIFORM ? (int)(w & 31u) : code - 1;
-    }
+    const unsigned wi = (unsigned)(((bx & 12) << 4) | ((by & 12) << 2) | (bz & 12) | (bx & 3));
+    const unsigned w = __ldg(s.air_bricks + (leaf ? 0u : e * 256u + wi));
+    const int code = (int)((w >> ((((by & 3) << 2) | (bz & 3)) * 2)) & 3u);
+    const int lvl_brick = w >= CCU_BRICK_UNIFORM ? (int)(w & 31u) : code - 1;
     const int level = leaf ? ((int)(e << 1)) >> 27 : lvl_brick;       // -1 = not air
     const int low = (1 << (level & 31)) - 1;
     const float ex = lean_exit_axis(bx, low, r.fmx, q.x, r.inv.x);

@@ -11,14 +11,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-// Tuning: CCU_NI_MATH keeps one out-of-line copy of the larger math helpers instead of inlining them at every use (the
-// wavefront kernel's shading stages are instruction-fetch bound; same arithmetic either way).
-#ifdef CCU_NI_MATH
-#define CCU_MATH_INLINE static __device__ __noinline__
-#else
-#define CCU_MATH_INLINE __device__ __forceinline__
-#endif
-
 namespace ccu {
 
 #define CCU_EPS 0.000005f    // constants.h:4
@@ -41,7 +33,7 @@ __device__ __forceinline__ float3 cross3(float3 a, float3 b) {
 // One division site per role (scale, divide, second divide) instead of one per return path: the operations a given input goes
 // through are the same ones in the same order (v / inf for an infinite component; v / (m * r) normally; (v / r) / m when m * r
 // overflows), the quotients of the paths not taken are computed on the side and dropped.
-CCU_MATH_INLINE float3 normalize3(float3 v) {
+__device__ __forceinline__ float3 normalize3(float3 v) {
     const float inf = __int_as_float(0x7f800000), qnan = __int_as_float(0x7fc00000);
     float ax = fabsf(v.x), ay = fabsf(v.y), az = fabsf(v.z);
     if (ax != ax || ay != ay || az != az) return f3(qnan, qnan, qnan);
@@ -65,8 +57,8 @@ __device__ __forceinline__ bool is_nan(float f) { return f != f; }
 __device__ __forceinline__ float nanf_() { return __int_as_float(0x7fc00000); }
 __device__ __forceinline__ float inff_() { return __int_as_float(0x7f800000); }
 
-// (sin x, cos x) returned by value: an out-of-line copy then hands both back in registers
-CCU_MATH_INLINE float2 dm_sincos2(float x) {
+// (sin x, cos x) in one evaluation
+__device__ __forceinline__ float2 dm_sincos2(float x) {
     float s, c;
     float kf = floorf(x * 0.636619772f + 0.5f);
     float r = x - kf * 1.5703125f;
@@ -100,14 +92,14 @@ __device__ __forceinline__ float dm_atan(float t) {
     return sign * (y0 + p);
 }
 // one dm_atan site: the quadrant offset is added afterwards (x > 0: none; x < 0: +pi for y >= 0, -pi for y < 0)
-CCU_MATH_INLINE float dm_atan2(float y, float x) {
+__device__ __forceinline__ float dm_atan2(float y, float x) {
     if (x != x || y != y) return nanf_();
     if (x == 0.0f) return y > 0.0f ? 1.5707963267948966f : (y < 0.0f ? -1.5707963267948966f : 0.0f);
     const float a = dm_atan(y / x);
     if (x > 0.0f) return a;
     return (y >= 0.0f) ? a + 3.14159265358979f : a - 3.14159265358979f;
 }
-CCU_MATH_INLINE float dm_asin(float x) {
+__device__ __forceinline__ float dm_asin(float x) {
     float a = fabsf(x);
     if (a > 1.0f) return nanf_();
     bool big = a > 0.5f;

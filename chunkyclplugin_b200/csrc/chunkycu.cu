@@ -82,9 +82,6 @@ __device__ __forceinline__ int face_of(float3 n) {
 // together (the block test is ~3x the instructions of a march step; run per lane as each ray arrives it executed at 6 of 32
 // lanes), and repeats for the lanes whose block test missed.  The treeData index of the hit leaf (reference numbering,
 // ClSceneLoader.java:56-59) is found by one root descent for the hit voxel only.  HAS_BVH = false compiles the entity BVHs out.
-#ifndef CCU_FH_WARP_SKIP
-#define CCU_FH_WARP_SKIP 0
-#endif
 // threads per block of the first-hit kernel and resident blocks per SM (the warps of a block do not depend on each other, so
 // the block size only decides how many warps wait for the slowest one before their registers are handed on)
 #ifndef CCU_FH_THREADS
@@ -116,11 +113,8 @@ template <bool DEEP>
 static __device__ __noinline__ int first_hit_march(const DScene &s, LeanRay *ray, int st) {
     LeanRay r = *ray;
     while (__any_sync(0xffffffffu, st == 0)) {
-#if CCU_FLAT_MARCH
-        if (!DEEP) st = lean_step_flat<false, CCU_FH_WARP_SKIP != 0>(s, s.air_top, r, st == 0, st);
-        else
-#endif
-        if (st == 0) st = lean_probe<DEEP, false>(s, s.air_top, r);
+        if (!DEEP) st = lean_step_flat<false>(s, s.air_top, r, st == 0, st);
+        else if (st == 0) st = lean_probe<DEEP, false>(s, s.air_top, r);
     }
     ray->t = r.t;
     ray->steps = r.steps;
@@ -614,8 +608,6 @@ int ccu_ctx_create(int device_index, ccu_ctx **out) {
     c->device = device_index;
     c->sm_count = p.multiProcessorCount;
     if (const char *e = getenv("CCU_Q_MARCH_WARPS")) c->q_march_warps = std::max(1, std::min(64, atoi(e)));
-    if (const char *e = getenv("CCU_Q_BVH_WARPS")) c->q_bvh_warps = std::max(1, std::min(64, atoi(e)));
-    if (const char *e = getenv("CCU_Q_LEAF_MIN")) c->q_leaf_min = std::max(1, std::min(32, atoi(e)));
     if (const char *e = getenv("CCU_Q_MARCH_BIAS")) c->q_march_bias = std::max(-32, std::min(32, atoi(e)));
     if (const char *e = getenv("CCU_Q_REFILL_MIN")) c->q_refill_min = std::max(1, std::min(32, atoi(e)));
     if (const char *e = getenv("CCU_Q_STICKY")) c->q_sticky_min = std::max(1, std::min(33, atoi(e)));
@@ -1034,9 +1026,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
         qp.march_bias = c->q_march_bias;
         qp.shade_min = c->q_shade_min;
         qp.sticky_min = c->q_sticky_min > 0 ? c->q_sticky_min : (bvh ? 16 : 33);   // measured: -3 % with BVH stages, +5 % without
-        qp.leaf_min = c->q_leaf_min;
-        qp.bvh_warps = c->q_bvh_warps;
-        qp.march_warps = bvh ? 64 : c->q_march_warps;   // with BVHs the service warps are the ones that do not walk
+        qp.march_warps = bvh ? 64 : c->q_march_warps;   // the cap applies to the BVH-less kernels; with BVH stages every warp may march
         const int lay = air_layout_id(c);
         const int grid = c->sm_count, block = Q_WARPS * 32;
         // The sky table is staged in shared memory when it is small: shared memory and L1 are one array on this chip, and a
@@ -1049,13 +1039,11 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
         const bool sky_smem = sky_texels * 4 <= sky_max && base_smem + sky_texels * 4 <= Q_SMEM_LIMIT;
         qp.sky_texels = sky_smem ? sky_texels : 0;
         qp.bvh_deep = nullptr;
-#if CCU_BVH_PARK
         if (bvh) {
             // scratch for traversal-stack entries beyond the shared-memory part (bvh.h:38 allows 64 pending nodes)
             if (!c->bvh_deep) CU(cudaMalloc(&c->bvh_deep, (size_t)c->sm_count * Q_SLOTS * Q_DEEP * sizeof(int)));
             qp.bvh_deep = c->bvh_deep;
         }
-#endif
         const int smem = base_smem + qp.sky_texels * 4;
         if (bvh) {
             if (lay == 0) k_render_queue<true, 0><<<grid, block, smem, c->stream>>>(c->scene, qp);
