@@ -64,18 +64,13 @@ NcclApi *nccl() {
         if (r_ != ncclSuccess) return fail(CCU_ECUDA, "%s: %s", #call, nccl()->GetErrorString ? nccl()->GetErrorString(r_) : "NCCL error"); \
     } while (0)
 
-__global__ void k_scale_window(float *buf, float factor, size_t n) {
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) buf[i] *= factor;
-}
-
 struct Member {
     ccu_ctx *ctx = nullptr;
     bool owned = false;
     ncclComm_t comm = nullptr;
-    int rank = 0;                 // global rank: which passes (p mod world) and which share of the buffer this GPU owns
-    float *share = nullptr;       // reduce-scatter result: floats [rank * share_n, (rank + 1) * share_n) of the window sum
-    size_t share_n = 0;
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+    int rank = 0;                      // global rank: which passes (p mod world) and which share of the buffer this GPU owns
+    ccu_host::DevBuf<float> share;     // reduce-scatter result: floats [rank * share.n, (rank + 1) * share.n) of the window sum
+    ccu_host::Event ev0, ev1;
 };
 
 }  // namespace
@@ -91,10 +86,7 @@ struct ccu_group {
     float render_ms = 0, reduce_ms = 0;
     // asynchronous share merge (ccu_group_render_merge_async): the reduce-scatter result sits in the share buffers, so the next
     // window may render while the shares travel to the host and are merged
-    std::thread merge_worker;
-    bool merge_active = false;
-    int merge_status = CCU_OK;
-    std::string merge_error;
+    ccu_host::MergeJob merge;
 };
 
 namespace {
@@ -108,21 +100,16 @@ int passes_of_rank(int n_total_before, int n_new, int rank, int world) {
 
 void free_member(Member &m) {
     if (!m.ctx) return;
-    {
-        DeviceGuard g(m.ctx->device);
-        if (m.share) cudaFree(m.share);
-        if (m.ev0) cudaEventDestroy(m.ev0);
-        if (m.ev1) cudaEventDestroy(m.ev1);
-        if (m.comm && nccl()->CommDestroy) nccl()->CommDestroy(m.comm);
-    }
+    DeviceGuard g(m.ctx->device);
+    if (m.comm && nccl()->CommDestroy) nccl()->CommDestroy(m.comm);
     if (m.owned) ccu_ctx_destroy(m.ctx);
     m = Member();
 }
 
 int init_member_events(Member &m) {
     DeviceGuard g(m.ctx->device);
-    CU(cudaEventCreate(&m.ev0));
-    CU(cudaEventCreate(&m.ev1));
+    CU(m.ev0.create(cudaEventDefault));
+    CU(m.ev1.create(cudaEventDefault));
     return CCU_OK;
 }
 
@@ -284,13 +271,9 @@ int ccu_group_render_begin(ccu_group *g, int32_t width, int32_t height) {
             total = m.ctx->accum_floats;
         }
         const size_t share = total / (size_t)g->world;
-        if (m.share_n != share) {
+        if (m.share.n != share) {
             DeviceGuard dg(m.ctx->device);
-            if (m.share) cudaFree(m.share);
-            m.share = nullptr;
-            m.share_n = 0;
-            CU(cudaMalloc(&m.share, share * sizeof(float)));
-            m.share_n = share;
+            CU(m.share.alloc(share));
         }
     }
     g->width = width;
@@ -333,8 +316,6 @@ int ccu_group_render_sync(ccu_group *g) {
     return CCU_OK;
 }
 
-static int join_group_merge(ccu_group *g, std::unique_lock<std::mutex> &lk);
-
 // window means -> (sum over GPUs) in the share buffers; closes the window.  Caller holds g->mu.
 static int reduce_window_locked(ccu_group *g) {
     const int total = g->window_total;
@@ -348,8 +329,7 @@ static int reduce_window_locked(ccu_group *g) {
             const int mine = passes_of_rank(0, total, m.rank, world);
             std::lock_guard<std::mutex> cl(m.ctx->mu);
             DeviceGuard dg(m.ctx->device);
-            k_scale_window<<<m.ctx->sm_count * 4, 256, 0, m.ctx->stream>>>(m.ctx->accum[m.ctx->accum_active], (float)mine, m.ctx->accum_floats);
-            m.ctx->launches++;
+            ccu_host::scale_window(m.ctx, (float)mine, m.ctx->accum_floats);
             CU(cudaGetLastError());
         }
     }
@@ -360,7 +340,7 @@ static int reduce_window_locked(ccu_group *g) {
             std::lock_guard<std::mutex> cl(m.ctx->mu);
             DeviceGuard dg(m.ctx->device);
             cudaEventRecord(m.ev0, m.ctx->stream);
-            ncclResult_t r = api->ReduceScatter(m.ctx->accum[m.ctx->accum_active], m.share, m.share_n, ncclFloat, ncclSum, m.comm, m.ctx->stream);
+            ncclResult_t r = api->ReduceScatter(m.ctx->accum[m.ctx->accum_active].p, m.share.p, m.share.n, ncclFloat, ncclSum, m.comm, m.ctx->stream);
             if (r != ncclSuccess) { api->GroupEnd(); return fail(CCU_ECUDA, "ncclReduceScatter: %s", api->GetErrorString(r)); }
         }
         NC(api->GroupEnd());
@@ -374,7 +354,7 @@ static int reduce_window_locked(ccu_group *g) {
         Member &m = g->local[0];
         std::lock_guard<std::mutex> cl(m.ctx->mu);
         DeviceGuard dg(m.ctx->device);
-        CU(cudaMemcpyAsync(m.share, m.ctx->accum[m.ctx->accum_active], m.share_n * sizeof(float), cudaMemcpyDeviceToDevice, m.ctx->stream));
+        CU(cudaMemcpyAsync(m.share.p, m.ctx->accum[m.ctx->accum_active].p, m.share.n * sizeof(float), cudaMemcpyDeviceToDevice, m.ctx->stream));
     }
     g->reduced_total = total;
     g->reduced_equal = equal;
@@ -399,38 +379,23 @@ int ccu_group_render_reduce(ccu_group *g, int32_t *window_spp) {
     if (!g) return fail(CCU_EINVAL, "ccu_group_render_reduce: null group");
     std::unique_lock<std::mutex> lk(g->mu);
     if (window_spp) *window_spp = g->window_total;
-    int rc = join_group_merge(g, lk);
+    int rc = g->merge.join(lk);
     if (rc != CCU_OK) return rc;
     rc = reduce_window_locked(g);
     if (rc != CCU_OK) return rc;
     return finish_reduce_timing(g);
 }
 
-static int join_group_merge(ccu_group *g, std::unique_lock<std::mutex> &lk) {
-    if (!g->merge_active) return CCU_OK;
-    std::thread t = std::move(g->merge_worker);
-    lk.unlock();
-    if (t.joinable()) t.join();
-    lk.lock();
-    g->merge_active = false;
-    if (g->merge_status != CCU_OK) {
-        const int rc = g->merge_status;
-        g->merge_status = CCU_OK;
-        return fail(rc, "%s", g->merge_error.c_str());
-    }
-    return CCU_OK;
-}
-
 int ccu_group_render_merge_wait(ccu_group *g) {
     if (!g) return fail(CCU_EINVAL, "ccu_group_render_merge_wait: null group");
     std::unique_lock<std::mutex> lk(g->mu);
-    return join_group_merge(g, lk);
+    return g->merge.join(lk);
 }
 
 // reduce (if the window is still open), then start the read-back of every local share on its GPU's copy stream and hand the merge
 // to a worker; returns at once.  Caller holds g->mu through `lk`.
 static int group_merge_start(ccu_group *g, std::unique_lock<std::mutex> &lk, double *sample_buffer, int32_t sample_spp, int32_t *merged_spp) {
-    int rc = join_group_merge(g, lk);          // one merge at a time: the share / staging buffers are about to be reused
+    int rc = g->merge.join(lk);          // one merge at a time: the share / staging buffers are about to be reused
     if (rc != CCU_OK) return rc;
     if (g->window_total > 0) {
         rc = reduce_window_locked(g);
@@ -445,11 +410,11 @@ static int group_merge_start(ccu_group *g, std::unique_lock<std::mutex> &lk, dou
     for (auto &m : g->local) {
         ccu_ctx *c = m.ctx;
         DeviceGuard dg(c->device);
-        const size_t lo = (size_t)m.rank * m.share_n, hi = std::min(n_img, lo + m.share_n);
+        const size_t lo = (size_t)m.rank * m.share.n, hi = std::min(n_img, lo + m.share.n);
         CU(cudaEventRecord(c->window_ev, c->stream));
         CU(cudaStreamWaitEvent(c->copy_stream, c->window_ev, 0));
         if (lo < hi) {
-            rc = ccu_host::start_readback(c, m.share - lo, lo, hi, c->copy_stream);    // indexed by absolute float offset
+            rc = ccu_host::start_readback(c, m.share.p - lo, lo, hi, c->copy_stream);    // indexed by absolute float offset
             if (rc != CCU_OK) return rc;
         }
     }
@@ -457,16 +422,14 @@ static int group_merge_start(ccu_group *g, std::unique_lock<std::mutex> &lk, dou
     const double ds = (double)sample_spp, sinv = 1.0 / (double)(sample_spp + total);
     const double dp = g->reduced_equal ? (double)total / (double)world : 1.0;
     g->reduced_total = 0;
-    g->merge_active = true;
-    g->merge_status = CCU_OK;
-    g->merge_worker = std::thread([=] {
+    g->merge.start([=] {
         const unsigned hw = std::max(1u, std::thread::hardware_concurrency());
         const unsigned merge_threads = std::max(2u, hw / (unsigned)g->local.size());
         std::vector<int> status(g->local.size(), CCU_OK);
         std::vector<std::string> errors(g->local.size());
         auto merge_one = [&](size_t i) {
             Member &m = g->local[i];
-            const size_t lo = (size_t)m.rank * m.share_n, hi = std::min(n_img, lo + m.share_n);
+            const size_t lo = (size_t)m.rank * m.share.n, hi = std::min(n_img, lo + m.share.n);
             const int st = ccu_host::merge_readback(m.ctx, lo, hi, sample_buffer, ds, dp, sinv, merge_threads);
             if (st != CCU_OK) { status[i] = st; errors[i] = ccu_host::last_error(); }
         };
@@ -478,7 +441,8 @@ static int group_merge_start(ccu_group *g, std::unique_lock<std::mutex> &lk, dou
             for (auto &t : th) t.join();
         }
         for (size_t i = 0; i < status.size(); i++)
-            if (status[i] != CCU_OK) { g->merge_status = status[i]; g->merge_error = errors[i]; break; }
+            if (status[i] != CCU_OK) return fail(status[i], "%s", errors[i].c_str());
+        return CCU_OK;
     });
     return CCU_OK;
 }
@@ -496,7 +460,7 @@ int ccu_group_render_merge(ccu_group *g, double *sample_buffer, int32_t sample_s
     std::unique_lock<std::mutex> lk(g->mu);
     int rc = group_merge_start(g, lk, sample_buffer, sample_spp, merged_spp);
     if (rc != CCU_OK) return rc;
-    rc = join_group_merge(g, lk);
+    rc = g->merge.join(lk);
     if (rc != CCU_OK) return rc;
     return finish_reduce_timing(g);
 }

@@ -9,6 +9,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <utility>
 #include <vector>
 
 #include "../../include/chunkycu.h"
@@ -27,6 +28,7 @@ const char *last_error();
                                   cudaGetErrorString(e_), __FILE__, __LINE__);                                            \
     } while (0)
 
+// Owning holders of CUDA resources: move-only, released by their destructor.  Nothing outside them frees a resource.
 template <class T>
 struct DevBuf {
     // never smaller than one 64-byte record: the straight-line kernels read element 0 of an empty array on lanes that have no
@@ -34,6 +36,10 @@ struct DevBuf {
     static constexpr size_t MIN_ELEMS = 64 / sizeof(T) > 4 ? 64 / sizeof(T) : 4;
     T *p = nullptr;
     size_t n = 0;
+    DevBuf() = default;
+    DevBuf(DevBuf &&o) noexcept : p(std::exchange(o.p, nullptr)), n(std::exchange(o.n, 0)) {}
+    DevBuf &operator=(DevBuf &&o) noexcept { std::swap(p, o.p); std::swap(n, o.n); return *this; }
+    ~DevBuf() { release(); }
     cudaError_t alloc(size_t count) {
         release();
         n = count;
@@ -59,7 +65,48 @@ struct DevBuf {
     size_t bytes() const { return p ? std::max<size_t>(n, MIN_ELEMS) * sizeof(T) : 0; }
 };
 
+// an event, a stream or pinned host memory; converts to the raw handle / pointer
+template <class H, auto Destroy>
+struct Handle {
+    H h = nullptr;
+    Handle() = default;
+    Handle(Handle &&o) noexcept : h(std::exchange(o.h, nullptr)) {}
+    Handle &operator=(Handle &&o) noexcept { std::swap(h, o.h); return *this; }
+    ~Handle() { reset(); }
+    operator H() const { return h; }
+    void reset() {
+        if (h) Destroy(h);
+        h = nullptr;
+    }
+};
+struct Event : Handle<cudaEvent_t, cudaEventDestroy> {
+    cudaError_t create(unsigned flags) { reset(); return cudaEventCreateWithFlags(&h, flags); }
+};
+struct Stream : Handle<cudaStream_t, cudaStreamDestroy> {
+    cudaError_t create() { reset(); return cudaStreamCreateWithFlags(&h, cudaStreamNonBlocking); }
+};
+template <class T>
+struct HostBuf : Handle<T *, cudaFreeHost> {
+    cudaError_t alloc(size_t count) {
+        this->reset();
+        cudaError_t e = cudaMallocHost(&this->h, count * sizeof(T));
+        if (e != cudaSuccess) this->h = nullptr;
+        return e;
+    }
+};
+
 constexpr int SEED_SLOTS = 4, SEED_SLOT_INTS = 32768;   // one launch covers at most 32768 passes (16-bit pass index in the wavefront kernel)
+constexpr int MERGE_CHUNKS = 8;                         // read-back chunks of a window merge, one event each
+
+// The seed words of the passes in flight (the only per-pass host->device traffic, OpenClPathTracingRenderer.java:106-109),
+// staged in a small ring of pinned slots so that a render call neither retains the caller's array nor waits for the passes
+// in flight.  Allocated whole or not at all.
+struct SeedRing {
+    DevBuf<int> dev;
+    HostBuf<int> pinned;
+    Event ev[SEED_SLOTS];   // last launch that read each slot
+    int slot = 0;
+};
 
 struct DeviceGuard {
     int prev = -1;
@@ -74,23 +121,63 @@ struct DeviceGuard {
     }
 };
 
-// one asynchronous read-back + merge of a finished window into the host sample buffer (ccu_render_merge_async)
+// One asynchronous read-back + merge into the host sample buffer (ccu_render_merge_async, ccu_group_render_merge_async).
+// The owner's lock guards the fields; the worker writes status / error only, and only before it ends.
 struct MergeJob {
     std::thread worker;
     bool active = false;
     int status = CCU_OK;
     std::string error;
+
+    // runs `body` on the worker; body returns a CCU_* code and sets the thread's error text when it fails
+    template <class F>
+    void start(F body) {
+        active = true;
+        status = CCU_OK;
+        worker = std::thread([this, body] {
+            const int rc = body();
+            if (rc != CCU_OK) { status = rc; error = last_error(); }
+        });
+    }
+    // waits for the worker with `lk` (the owner's lock) released; returns the worker's status and clears it
+    int join(std::unique_lock<std::mutex> &lk) {
+        if (!active) return CCU_OK;
+        std::thread t = std::move(worker);
+        lk.unlock();
+        if (t.joinable()) t.join();
+        lk.lock();
+        active = false;
+        if (status == CCU_OK) return CCU_OK;
+        const int rc = status;
+        status = CCU_OK;
+        return fail(rc, "%s", error.c_str());
+    }
+};
+
+// The scalar state of a committed scene: what commit derived from the uploads, and what the uploads set besides arrays.
+struct SceneInfo {
+    int depth = 0, sky_res = 0;
+    int world_root = 0, actor_root = 0, use_bvh2 = 0, use_air = 0, air_deep = 0;
+    int cell_level = 0, top_log2 = 0, use_wide = 0, air_cell_level = 4, air_top_log2 = 0;
+    int atlas_w = 0, atlas_h = 0, atlas_layers = 0;
+    float sky_intensity = 0;
+    int sun_host[6] = {0, 0, 0, 0, 0, 0};
+    bool have_sun = false, have_octree = false, have_blocks = false, have_mats = false, have_atlas = false, have_sky = false;
+    float3 su{}, sv{}, sw{};   // sun basis (k_sun_setup)
+    float sun_radius_cos = 0;
 };
 
 }  // namespace ccu_host
 
+// Members are destroyed in reverse order of declaration: the streams are declared first so that they outlive every buffer and
+// event used on them.  ccu_ctx_destroy joins the merge worker and synchronises both streams before the delete.
 struct ccu_ctx {
     int device = 0;
-    cudaStream_t stream = nullptr;        // render stream
-    cudaStream_t copy_stream = nullptr;   // read-back of finished windows, camera-ray uploads
-    cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-    cudaEvent_t chunk_ev[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // read-back chunks of a merge
-    cudaEvent_t window_ev = nullptr;      // the window being merged is complete on the render stream
+    ccu_host::Stream stream;        // render stream
+    ccu_host::Stream copy_stream;   // read-back of finished windows, camera-ray uploads
+    ccu_host::Event ev0, ev1;
+    ccu_host::Event chunk_ev[ccu_host::MERGE_CHUNKS];   // read-back chunks of a merge
+    ccu_host::Event window_ev;      // the window being merged is complete on the render stream
     // Locking: `mu` guards every field below and is never held across a wait for rendering work (ccu_render_sync waits on an
     // event outside the lock), so preview / tonemap / camera calls from other threads are not blocked by a long batch;
     // `cam_mu` serialises camera updates.
@@ -106,43 +193,44 @@ struct ccu_ctx {
     ccu_host::DevBuf<int> world_rec, actor_rec, tris2;          // BVH stage layout (ccu_queue.cuh)
     ccu_host::DevBuf<int> block_rec, mat_rec, quad_rec, aabb_rec;   // 16-byte-vectorised palettes (DScene::block_rec ...)
     std::vector<int> quad_host, aabb_host;
-    int world_root = 0, actor_root = 0, use_bvh2 = 0, use_air = 0, air_deep = 0;
-    int cell_level = 0, top_log2 = 0, use_wide = 0, air_cell_level = 4, air_top_log2 = 0;
     double commit_ms = 0;                                       // host time of the last ccu_scene_commit
     ccu_host::DevBuf<uchar4> atlas, sky;
-    int atlas_w = 0, atlas_h = 0, atlas_layers = 0;
-    int depth = 0, sky_res = 0;
-    float sky_intensity = 0;
-    int sun_host[6] = {0, 0, 0, 0, 0, 0};
-    bool have_sun = false, have_octree = false, have_blocks = false, have_mats = false, have_atlas = false, have_sky = false;
+    ccu_host::SceneInfo info;
     bool committed = false;
     ccu_host::DevBuf<float> sun_basis;
-    float *unorm = nullptr;
+    ccu_host::DevBuf<float> unorm;
+
+    // Every device array of the scene, each passed to f as a pointer to member (replicate_scene, ccu_scene_device_bytes).
+    template <class F>
+    static void each_scene_buf(F f) {
+        f(&ccu_ctx::tree); f(&ccu_ctx::block_palette); f(&ccu_ctx::quad_models); f(&ccu_ctx::aabb_models); f(&ccu_ctx::mat_palette);
+        f(&ccu_ctx::trigs); f(&ccu_ctx::world_bvh); f(&ccu_ctx::actor_bvh); f(&ccu_ctx::sun_words); f(&ccu_ctx::top); f(&ccu_ctx::wide);
+        f(&ccu_ctx::air_top); f(&ccu_ctx::air_wide); f(&ccu_ctx::air_bricks); f(&ccu_ctx::world_rec); f(&ccu_ctx::actor_rec);
+        f(&ccu_ctx::tris2); f(&ccu_ctx::block_rec); f(&ccu_ctx::mat_rec); f(&ccu_ctx::quad_rec); f(&ccu_ctx::aabb_rec); f(&ccu_ctx::atlas);
+        f(&ccu_ctx::sky); f(&ccu_ctx::sun_basis);
+    }
 
     // camera: pre-generated rays are double buffered so that an upload overlaps the passes in flight
     int projector_type = 0;
     float cam[15] = {0};
     ccu_host::DevBuf<float> rays[2];
-    cudaEvent_t rays_used[2] = {nullptr, nullptr};   // last launch that read rays[i]
+    ccu_host::Event rays_used[2];   // last launch that read rays[i]
     int rays_active = 0;
     bool have_camera = false;
 
     // render target: the accumulation window is double buffered so that the read-back / merge of a finished window
     // overlaps the rendering of the next one (OpenClPathTracingRenderer.java:150-151,172-177)
     int width = 0, height = 0;
-    float *accum[2] = {nullptr, nullptr};   // running mean float[accum_floats] each
+    ccu_host::DevBuf<float> accum[2];       // running mean float[accum_floats] each
     size_t accum_floats = 0;                // 3*W*H rounded up (ccu_group needs equal reduce-scatter shares)
     size_t accum_align = 256;               // accum_floats is a multiple of this (set by the group before ccu_render_begin)
     int accum_active = 0;
     const float *window_base = nullptr;     // the buffer that holds what the reference's single buffer would hold right now
-    float *pinned = nullptr;                // host staging float[accum_floats]
-    int *seeds_dev = nullptr, *seeds_pinned = nullptr;   // ring of seed slots (device / pinned host)
-    cudaEvent_t seeds_ev[4] = {nullptr, nullptr, nullptr, nullptr};
-    int seeds_slot = 0;
-    int *fh_scratch = nullptr;              // first-hit planes (kept between calls)
-    size_t fh_scratch_pixels = 0;
-    unsigned int *work_counter = nullptr;
-    int *bvh_deep = nullptr;                // wavefront kernel, BVH scenes: traversal-stack entries beyond the shared-memory part
+    ccu_host::HostBuf<float> pinned;        // host staging float[accum_floats]
+    ccu_host::SeedRing seeds;
+    ccu_host::DevBuf<int> fh_scratch;       // first-hit planes (kept between calls)
+    ccu_host::DevBuf<unsigned> work_counter;
+    ccu_host::DevBuf<int> bvh_deep;         // wavefront kernel, BVH scenes: traversal-stack entries beyond the shared-memory part
     int yield_below = 20;
     int q_refill_min = 8;
     int q_march_bias = 4;
@@ -169,4 +257,7 @@ int merge_readback(ccu_ctx *c, size_t lo, size_t hi, double *sample_buffer, doub
 int merge_window_range(ccu_ctx *c, const float *src_dev, size_t lo, size_t hi, double *sample_buffer, double ds, double dp, double sinv,
                        cudaStream_t stream, unsigned max_threads);
 int replicate_scene(ccu_ctx *src, ccu_ctx *dst);
+// multiplies the first n floats of the active accumulation window by `factor` on the render stream and counts the launch
+// (caller holds c->mu, c->device is current); the launch error is left for cudaGetLastError
+void scale_window(ccu_ctx *c, float factor, size_t n);
 }  // namespace ccu_host
