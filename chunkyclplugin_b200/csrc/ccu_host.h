@@ -6,6 +6,7 @@
 #include <algorithm>
 #include <cstdint>
 #include <cstring>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -158,13 +159,53 @@ struct MergeJob {
 struct SceneInfo {
     int depth = 0, sky_res = 0;
     int world_root = 0, actor_root = 0, use_bvh2 = 0, use_air = 0, air_deep = 0;
+    int world_bvh_empty = 1, actor_bvh_empty = 1;   // the bvh.h:23-32 probe of the committed BVHs
     int cell_level = 0, top_log2 = 0, use_wide = 0, air_cell_level = 4, air_top_log2 = 0;
     int atlas_w = 0, atlas_h = 0, atlas_layers = 0;
     float sky_intensity = 0;
     int sun_host[6] = {0, 0, 0, 0, 0, 0};
-    bool have_sun = false, have_octree = false, have_blocks = false, have_mats = false, have_atlas = false, have_sky = false;
+    bool have_sun = false, have_atlas = false, have_sky = false;
     float3 su{}, sv{}, sw{};   // sun basis (k_sun_setup)
     float sun_radius_cos = 0;
+};
+
+// The reference's packed int arrays, one ccu_scene_set_* call each.
+enum SceneArray { OCTREE, BLOCK_PALETTE, QUAD_MODELS, AABB_MODELS, MAT_PALETTE, TRIANGLES, WORLD_BVH, ACTOR_BVH, N_ARRAYS };
+struct ArrayDesc {
+    const char *setter;   // entry point named in error messages
+    bool optional;        // released by ccu_scene_begin; absent at commit, it is one zero word (empty palette / EMPTY_NODE)
+};
+constexpr ArrayDesc ARRAY_DESC[N_ARRAYS] = {
+    {"ccu_scene_set_octree", false},      {"ccu_scene_set_block_palette", false}, {"ccu_scene_set_quad_models", true},
+    {"ccu_scene_set_aabb_models", true},  {"ccu_scene_set_material_palette", false}, {"ccu_scene_set_triangles", true},
+    {"ccu_scene_set_world_bvh", true},    {"ccu_scene_set_actor_bvh", true},
+};
+// The device buffer of one packed array and the host copy commit builds its layouts from.  `host` is set exactly while `dev`
+// holds the array; it never changes once set, so a replica shares it.
+struct PackedArray {
+    DevBuf<int> dev;
+    std::shared_ptr<const std::vector<int>> host;
+};
+
+// Everything a context knows about its scene: the uploads, the layouts commit builds from them, and the launch view.
+struct Scene {
+    PackedArray arrays[N_ARRAYS];
+    DevBuf<unsigned> top, wide;                       // value-carrying octree layout
+    DevBuf<unsigned> air_top, air_wide, air_bricks;   // march layout (ccu_march.cuh)
+    DevBuf<int> world_rec, actor_rec, tris2;          // BVH stage layout (ccu_queue.cuh)
+    DevBuf<int> block_rec, mat_rec, quad_rec, aabb_rec;   // 16-byte-vectorised palettes (DScene::block_rec ...)
+    DevBuf<uchar4> atlas, sky;
+    SceneInfo info;
+    ccu::DScene view{};   // every field that depends on the committed scene alone (commit, replicate_scene)
+
+    // Calls f(a's buffer, b's same buffer) for every device array of a scene (replicate_scene, ccu_scene_device_bytes).
+    template <class F>
+    static void each_buf(Scene &a, Scene &b, F f) {
+        for (int i = 0; i < N_ARRAYS; i++) f(a.arrays[i].dev, b.arrays[i].dev);
+        f(a.top, b.top); f(a.wide, b.wide); f(a.air_top, b.air_top); f(a.air_wide, b.air_wide); f(a.air_bricks, b.air_bricks);
+        f(a.world_rec, b.world_rec); f(a.actor_rec, b.actor_rec); f(a.tris2, b.tris2); f(a.block_rec, b.block_rec);
+        f(a.mat_rec, b.mat_rec); f(a.quad_rec, b.quad_rec); f(a.aabb_rec, b.aabb_rec); f(a.atlas, b.atlas); f(a.sky, b.sky);
+    }
 };
 
 }  // namespace ccu_host
@@ -184,31 +225,10 @@ struct ccu_ctx {
     std::mutex mu, cam_mu;
     int sm_count = 0;
 
-    // scene as uploaded (reference packed layouts)
-    ccu_host::DevBuf<int> tree, block_palette, quad_models, aabb_models, mat_palette, trigs, world_bvh, actor_bvh, sun_words;
-    std::vector<int> tree_host, world_host, actor_host, trigs_host, block_host, mat_host;   // kept for the commit-time layouts
-    // commit-time layouts
-    ccu_host::DevBuf<unsigned> top, wide;                       // value-carrying octree layout
-    ccu_host::DevBuf<unsigned> air_top, air_wide, air_bricks;   // march layout (ccu_march.cuh)
-    ccu_host::DevBuf<int> world_rec, actor_rec, tris2;          // BVH stage layout (ccu_queue.cuh)
-    ccu_host::DevBuf<int> block_rec, mat_rec, quad_rec, aabb_rec;   // 16-byte-vectorised palettes (DScene::block_rec ...)
-    std::vector<int> quad_host, aabb_host;
-    double commit_ms = 0;                                       // host time of the last ccu_scene_commit
-    ccu_host::DevBuf<uchar4> atlas, sky;
-    ccu_host::SceneInfo info;
-    bool committed = false;
-    ccu_host::DevBuf<float> sun_basis;
+    ccu_host::Scene scene;
+    bool committed = false;   // `scene` is complete: render calls launch on it
+    double commit_ms = 0;     // host time of the last ccu_scene_commit
     ccu_host::DevBuf<float> unorm;
-
-    // Every device array of the scene, each passed to f as a pointer to member (replicate_scene, ccu_scene_device_bytes).
-    template <class F>
-    static void each_scene_buf(F f) {
-        f(&ccu_ctx::tree); f(&ccu_ctx::block_palette); f(&ccu_ctx::quad_models); f(&ccu_ctx::aabb_models); f(&ccu_ctx::mat_palette);
-        f(&ccu_ctx::trigs); f(&ccu_ctx::world_bvh); f(&ccu_ctx::actor_bvh); f(&ccu_ctx::sun_words); f(&ccu_ctx::top); f(&ccu_ctx::wide);
-        f(&ccu_ctx::air_top); f(&ccu_ctx::air_wide); f(&ccu_ctx::air_bricks); f(&ccu_ctx::world_rec); f(&ccu_ctx::actor_rec);
-        f(&ccu_ctx::tris2); f(&ccu_ctx::block_rec); f(&ccu_ctx::mat_rec); f(&ccu_ctx::quad_rec); f(&ccu_ctx::aabb_rec); f(&ccu_ctx::atlas);
-        f(&ccu_ctx::sky); f(&ccu_ctx::sun_basis);
-    }
 
     // camera: pre-generated rays are double buffered so that an upload overlaps the passes in flight
     int projector_type = 0;
@@ -246,16 +266,12 @@ struct ccu_ctx {
     float last_ms = 0;
     bool timing_pending = false;
     int64_t launches = 0;
-
-    ccu::DScene scene{};
 };
 
 namespace ccu_host {
 // internal entry points shared with ccu_group.cu (caller holds no lock)
 int start_readback(ccu_ctx *c, const float *src_dev, size_t lo, size_t hi, cudaStream_t stream);
 int merge_readback(ccu_ctx *c, size_t lo, size_t hi, double *sample_buffer, double ds, double dp, double sinv, unsigned max_threads);
-int merge_window_range(ccu_ctx *c, const float *src_dev, size_t lo, size_t hi, double *sample_buffer, double ds, double dp, double sinv,
-                       cudaStream_t stream, unsigned max_threads);
 int replicate_scene(ccu_ctx *src, ccu_ctx *dst);
 // multiplies the first n floats of the active accumulation window by `factor` on the render stream and counts the launch
 // (caller holds c->mu, c->device is current); the launch error is left for cudaGetLastError

@@ -2,14 +2,15 @@
 // the BVH stage layout.  Included by chunkycu.cu only.
 #pragma once
 #include <algorithm>
+#include <cmath>
 #include <cstdlib>
+#include <cstring>
 #include <thread>
 #include <unordered_map>
 #include <vector>
 
 #include "ccu_device.cuh"
 #include "ccu_march.cuh"
-
 
 // ------------------------------------------------------------------------------------------------------
 // commit-time traversal layout (see DScene::top / DScene::wide)
@@ -254,41 +255,36 @@ struct BvhLayout {
     int root = 0;
     bool ok = true;
 };
-struct TriRepack {
+// Both entity BVHs, which share the triangle blocks (build_bvh_stage).
+struct BvhStage {
+    BvhLayout world, actor;
     std::vector<int> tris;                       // per leaf: {count, 0 x 7} + count x (20 words (PackedTriangle.java:46-78) + 4 pad)
-    int add(const std::vector<int> &trigs, int prim, bool &ok) {
-        if (prim < 0 || (size_t)prim >= trigs.size()) { ok = false; return 0; }
+    std::unordered_map<int, int> leaf_at;        // palette offset -> block: a leaf both BVHs reference is stored once
+    bool ok = true;
+    // block of the leaf at triangle-palette offset `prim`, in units of 32 bytes
+    int leaf(const std::vector<int> &trigs, int prim, bool &valid) {
+        auto [at, fresh] = leaf_at.try_emplace(prim, 0);
+        if (!fresh) return at->second;
+        if (prim < 0 || (size_t)prim >= trigs.size()) { valid = false; return 0; }
         const int count = trigs[(size_t)prim];
-        if (count < 0 || (size_t)prim + 1 + (size_t)count * 20 > trigs.size()) { ok = false; return 0; }
-        const int off = (int)(tris.size() / 8);      // in units of 32 bytes
+        if (count < 0 || (size_t)prim + 1 + (size_t)count * 20 > trigs.size()) { valid = false; return 0; }
+        at->second = (int)(tris.size() / 8);
         tris.push_back(count);
         tris.insert(tris.end(), 7, 0);
         for (int i = 0; i < count; i++) {
             tris.insert(tris.end(), trigs.begin() + prim + 1 + (size_t)i * 20, trigs.begin() + prim + 1 + (size_t)(i + 1) * 20);
             tris.insert(tris.end(), 4, 0);
         }
-        return off;
+        return at->second;
     }
 };
 
-int bvh_ref(const std::vector<int> &bvh, const std::vector<int> &trigs, size_t node, int depth, BvhLayout &b, TriRepack &tr,
-            std::unordered_map<int, int> &leaf_map) {
+int bvh_ref(const std::vector<int> &bvh, const std::vector<int> &trigs, size_t node, int depth, BvhLayout &b, BvhStage &s) {
     if (!b.ok) return -1;
     // deeper than the traversal stack of the reference (int nodesToVisit[64], bvh.h:38): undefined there, refused here
     if (node + 6 >= bvh.size() || depth >= 64) { b.ok = false; return -1; }
     const int head = bvh[node];
-    if (head <= 0) {
-        const int prim = -head;
-        auto it = leaf_map.find(prim);   // a leaf block referenced twice (both BVHs share the palette) is stored once
-        int off;
-        if (it != leaf_map.end()) {
-            off = it->second;
-        } else {
-            off = tr.add(trigs, prim, b.ok);
-            leaf_map.emplace(prim, off);
-        }
-        return -(1 + off);
-    }
+    if (head <= 0) return -(1 + s.leaf(trigs, -head, b.ok));
     const size_t left = node + 7, right = (size_t)head;
     if (left + 6 >= bvh.size() || right + 6 >= bvh.size()) { b.ok = false; return -1; }
     const size_t r = b.rec.size() / 16;
@@ -298,11 +294,34 @@ int bvh_ref(const std::vector<int> &bvh, const std::vector<int> &trigs, size_t n
         b.rec[r * 16 + i] = bvh[left + 1 + i];
         b.rec[r * 16 + 8 + i] = bvh[right + 1 + i];
     }
-    const int rl = bvh_ref(bvh, trigs, left, depth + 1, b, tr, leaf_map);
-    const int rr = bvh_ref(bvh, trigs, right, depth + 1, b, tr, leaf_map);
+    const int rl = bvh_ref(bvh, trigs, left, depth + 1, b, s);
+    const int rr = bvh_ref(bvh, trigs, right, depth + 1, b, s);
     b.rec[r * 16 + 6] = rl;
     b.rec[r * 16 + 14] = rr;
     return (int)r;
+}
+
+inline bool bvh_is_empty(const std::vector<int> &bvh) {   // bvh.h:23-32
+    if (bvh.size() < 7) return true;
+    if (bvh[0] != 0) return false;
+    for (int i = 1; i < 7; i++) {
+        float f;
+        memcpy(&f, &bvh[i], 4);
+        if (!std::isnan(f)) return false;
+    }
+    return true;
+}
+
+// The BVH stage layout of the world and actor BVHs.  When either cannot be held (malformed, or deeper than the 64 entries of
+// the reference's traversal stack, bvh.h:38), ok is false and the records and triangle blocks are empty.
+inline BvhStage build_bvh_stage(const std::vector<int> &world, const std::vector<int> &actor, const std::vector<int> &trigs) {
+    BvhStage s;
+    if (!bvh_is_empty(world)) s.world.root = bvh_ref(world, trigs, 0, 0, s.world, s);
+    if (!bvh_is_empty(actor)) s.actor.root = bvh_ref(actor, trigs, 0, 0, s.actor, s);
+    s.ok = s.world.ok && s.actor.ok;
+    if (!s.ok) { s.world.rec.clear(); s.actor.rec.clear(); s.tris.clear(); }
+    s.tris.insert(s.tris.end(), 8, 0);      // the leaf stage reads the 32 bytes behind a count word before it looks at the count
+    return s;
 }
 
 inline void wide_fill_slab(const int *tree, size_t n, int depth, int cl, int dim, int x0, int x1, unsigned *top, WideLayout &b) {
@@ -368,20 +387,20 @@ struct PaletteRecs {
     bool ok = true;
 };
 
-inline PaletteRecs build_palette_recs(const std::vector<int> &bp, const std::vector<int> &mp, const int *quads, size_t n_quads,
-                                      const int *aabbs, size_t n_aabbs) {
+inline PaletteRecs build_palette_recs(const std::vector<int> &bp, const std::vector<int> &mp, const std::vector<int> &quads,
+                                      const std::vector<int> &aabbs) {
     PaletteRecs r;
     const size_t n_mat = mp.size() / 6;
     r.mat.assign(std::max<size_t>(n_mat, 1) * 8, 0);
     for (size_t i = 0; i < n_mat; i++)
         for (int k = 0; k < 6; k++) r.mat[i * 8 + k] = mp[i * 6 + k];
     std::unordered_map<int, int> quad_at, aabb_at;     // model pointer -> offset in units of 16 bytes
-    auto model = [&](const int *src, size_t n, int ptr, int words, std::vector<int> &dst, std::unordered_map<int, int> &at, int &out) {
+    auto model = [&](const std::vector<int> &src, int ptr, int words, std::vector<int> &dst, std::unordered_map<int, int> &at, int &out) {
         auto it = at.find(ptr);
         if (it != at.end()) { out = it->second; return true; }
-        if (ptr < 0 || (size_t)ptr >= n) return false;
+        if (ptr < 0 || (size_t)ptr >= src.size()) return false;
         const int count = src[ptr];
-        if (count < 0 || (size_t)ptr + 1 + (size_t)count * words > n) return false;
+        if (count < 0 || (size_t)ptr + 1 + (size_t)count * words > src.size()) return false;
         out = (int)(dst.size() / 4);
         dst.push_back(count); dst.push_back(0); dst.push_back(0); dst.push_back(0);
         for (int i = 0; i < count; i++) {
@@ -405,9 +424,9 @@ inline PaletteRecs build_palette_recs(const std::vector<int> &bp, const std::vec
                 rec[0] = 0x7FFFFFFF;
             }
         } else if (type == 2) {
-            if (!model(aabbs, n_aabbs, ptr, 13, r.aabb, aabb_at, rec[1])) rec[0] = 0x7FFFFFFF;
+            if (!model(aabbs, ptr, 13, r.aabb, aabb_at, rec[1])) rec[0] = 0x7FFFFFFF;
         } else if (type == 3) {
-            if (!model(quads, n_quads, ptr, 15, r.quad, quad_at, rec[1])) rec[0] = 0x7FFFFFFF;
+            if (!model(quads, ptr, 15, r.quad, quad_at, rec[1])) rec[0] = 0x7FFFFFFF;
         }
     }
     if (r.quad.empty()) r.quad.assign(4, 0);
