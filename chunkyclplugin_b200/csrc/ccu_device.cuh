@@ -503,10 +503,14 @@ struct March {
 // octree.h:43-64: 1 / d, the distance to the octree cube for a ray that starts outside of it, and whether it enters at all.
 // Kept out of line (one copy instead of one per ray kind: measured -4 % on the wavefront kernel, whose shading stages are
 // limited by instruction fetch); the result is returned by value, so the copy hands it back in registers.
+// inv is NaN on an axis whose origin component is NaN.  Every use of inv multiplies it by a coordinate difference that is
+// NaN on that axis anyway (the box tests, AABB_exit, the block test), so no result changes; lean_prepare, which sees inv
+// but not the origin, needs it to give that axis the NaN exit operand (ccu_march.cuh, lean_exit_axis).
 struct MarchStart { float3 inv; float t; int entered; };
 static __device__ __noinline__ MarchStart march_begin_core(int depth, float3 origin, float3 direction) {
     MarchStart ms;
-    ms.inv = f3(1.0f / direction.x, 1.0f / direction.y, 1.0f / direction.z);
+    ms.inv = f3(origin.x == origin.x ? 1.0f / direction.x : nanf_(), origin.y == origin.y ? 1.0f / direction.y : nanf_(),
+                origin.z == origin.z ? 1.0f / direction.z : nanf_());
     ms.t = 0;
     ms.entered = 1;
     int lx = f2i(floorf(origin.x)) >> depth, ly = f2i(floorf(origin.y)) >> depth, lz = f2i(floorf(origin.z)) >> depth;

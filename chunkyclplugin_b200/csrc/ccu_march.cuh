@@ -29,6 +29,7 @@ struct LeanRay {
     float t, limit;
     int steps;
     int fmx, fmy, fmz;        // -1 when the leaf cube is left through its upper plane on that axis, else 0
+    float nmx, nmy, nmz;      // second operand of the exit term's fmaxf: -inf or NaN (lean_exit_axis)
 };
 
 __device__ __forceinline__ void lean_prepare(LeanRay &r) {
@@ -36,16 +37,27 @@ __device__ __forceinline__ void lean_prepare(LeanRay &r) {
     r.fmx = r.inv.x < 0.0f ? 0 : -1;
     r.fmy = r.inv.y < 0.0f ? 0 : -1;
     r.fmz = r.inv.z < 0.0f ? 0 : -1;
+    r.nmx = r.inv.x < 0.0f ? -inff_() : nanf_();
+    r.nmy = r.inv.y < 0.0f ? -inff_() : nanf_();
+    r.nmz = r.inv.z < 0.0f ? -inff_() : nanf_();
 }
 
-// AABB_exit (primitives.h:52-61) along one axis for a point q strictly inside the leaf cube [lo, hi):
-// fmax((lo-q)*inv, (hi-q)*inv).  lo - q <= 0 < hi - q, so the maximum is the (hi-q)*inv term for inv >= 0 and the
-// (lo-q)*inv term for inv < 0; the only case where that term is NaN while the reference's fmax is not is inv = -inf with
-// q == lo, where the reference yields the other term, -inf: fmaxf(x, -inf) maps exactly that NaN to -inf and leaves every
-// other x alone.  The plane is ((b >> level) + far) << level = (b with its low `level` bits cleared / set) + far.
-__device__ __forceinline__ float lean_exit_axis(int b, int low, int fm, float q, float inv) {
+// AABB_exit (primitives.h:52-61) along one axis for the offset position q of a voxel b of the leaf cube [lo, hi):
+// fmax((lo-q)*inv, (hi-q)*inv).  The far-plane term ((hi-q)*inv for inv >= 0, (lo-q)*inv for inv < 0) is that maximum
+// except where it is NaN, and then `nm` (lean_prepare) gives the reference's result:
+//  - q finite (lo <= q < hi): NaN only for inv = -inf and q == lo, where the reference's other term is -inf, so
+//    nm = -inf for inv < 0.  An infinite q never gets here: f2i saturates and the cube test ends the march.
+//  - inv NaN, or q NaN (a NaN origin component, or 0 * inf in o + d * t): both of the reference's terms are NaN, and
+//    its fmin drops the axis; nm = NaN keeps the NaN, which fminf drops too.  nm = NaN for inv >= 0 and inv NaN;
+//    march_begin_core makes inv NaN on an axis whose origin component is NaN, so that case gets NaN too (and costs
+//    nothing per step or per load).  The one case left, q NaN from 0 * inf for d = -0 (t infinite), maps to -inf instead,
+//    but once t is infinite every axis with a finite non-zero d leaves the cube at the next step and every other
+//    axis's q is NaN, so the march only meets voxel (0,0,0) with a NaN position, whose block test misses, until
+//    draw_depth: a miss either way.
+// The plane is ((b >> level) + far) << level = (b with its low `level` bits cleared / set) + far.
+__device__ __forceinline__ float lean_exit_axis(int b, int low, int fm, float q, float inv, float nm) {
     const int plane = ((b & ~low) | (low & fm)) - fm;
-    return fmaxf(((float)plane - q) * inv, -inff_());
+    return fmaxf(((float)plane - q) * inv, nm);
 }
 
 // One iteration of octree.h:66-107.  Returns 0 = air leaf left (keep marching), 1 = non-air leaf reached (ray not
@@ -84,9 +96,9 @@ __device__ __forceinline__ int lean_probe(const DScene &s, const unsigned *__res
     }
     if (level < 0) return 1;
     const int low = (1 << level) - 1;
-    const float ex = lean_exit_axis(bx, low, r.fmx, q.x, r.inv.x);
-    const float ey = lean_exit_axis(by, low, r.fmy, q.y, r.inv.y);
-    const float ez = lean_exit_axis(bz, low, r.fmz, q.z, r.inv.z);
+    const float ex = lean_exit_axis(bx, low, r.fmx, q.x, r.inv.x, r.nmx);
+    const float ey = lean_exit_axis(by, low, r.fmy, q.y, r.inv.y, r.nmy);
+    const float ez = lean_exit_axis(bz, low, r.fmz, q.z, r.inv.z, r.nmz);
     r.t += fminf(ex, fminf(ey, ez)) + CCU_OFFSET;
     r.steps++;
     return 0;
@@ -115,9 +127,9 @@ __device__ __forceinline__ int lean_step_flat(const DScene &s, const unsigned *_
     const int lvl_brick = w >= CCU_BRICK_UNIFORM ? (int)(w & 31u) : code - 1;
     const int level = leaf ? ((int)(e << 1)) >> 27 : lvl_brick;       // -1 = not air
     const int low = (1 << (level & 31)) - 1;
-    const float ex = lean_exit_axis(bx, low, r.fmx, q.x, r.inv.x);
-    const float ey = lean_exit_axis(by, low, r.fmy, q.y, r.inv.y);
-    const float ez = lean_exit_axis(bz, low, r.fmz, q.z, r.inv.z);
+    const float ex = lean_exit_axis(bx, low, r.fmx, q.x, r.inv.x, r.nmx);
+    const float ey = lean_exit_axis(by, low, r.fmy, q.y, r.inv.y, r.nmy);
+    const float ez = lean_exit_axis(bz, low, r.fmz, q.z, r.inv.z, r.nmz);
     const float tn = r.t + (fminf(ex, fminf(ey, ez)) + CCU_OFFSET);
     const bool adv = active && !fin && level >= 0;
     r.t = adv ? tn : r.t;

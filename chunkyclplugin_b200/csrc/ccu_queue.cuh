@@ -234,7 +234,7 @@ __device__ __forceinline__ void q_stage_march(const DScene &s, const unsigned *_
     int cur = -1;   // slot of the ray this lane is marching (row * 32 + column), -1 = none
     LeanRay r;
     r.o = r.d = r.inv = r.doff = f3(0, 0, 0);
-    r.t = 0; r.limit = 0; r.steps = 0; r.fmx = r.fmy = r.fmz = 0;
+    r.t = 0; r.limit = 0; r.steps = 0; r.fmx = r.fmy = r.fmz = 0; r.nmx = r.nmy = r.nmz = 0;
     int done = 0;   // 0 = ray in flight, 1 = reached a non-air leaf, 2 = finished
     int recheck = 0;
     int busy = 0;   // lanes that hold a ray, in flight or finished (warp-uniform, changes only at a refill)

@@ -143,6 +143,12 @@ class Oracle:
         lib().oracle_preview(C.byref(self._s), res.ctypes.data_as(C.c_void_p), C.c_int(threads))
         return res
 
+    def sun_basis(self) -> np.ndarray:
+        """float32[3, 3]: rows sw, su, sv of Sun_new (sky.h:19-40)."""
+        out = np.zeros(9, np.float32)
+        lib().oracle_sun_basis(C.byref(self._s), out.ctypes.data_as(C.c_void_p))
+        return out.reshape(3, 3)
+
     def camera_rays(self, seed: int) -> np.ndarray:
         n = self._s.width * self._s.height
         rays = np.zeros(n * 6, np.float32)

@@ -1010,6 +1010,13 @@ void oracle_math(int fn, int libm, const float *x, const float *y, float *out, i
         }
     }
 }
+/* Sun_new (sky.h:19-40): out = sw, su, sv of the scene's sun */
+void oracle_sun_basis(const OracleScene *s, float *out) {
+    Math m = {s->math_mode == 1};
+    Sun sun = sun_new(s, &m);
+    v3 b[3] = {sun.sw, sun.su, sun.sv};
+    for (int i = 0; i < 3; i++) { out[3 * i] = b[i].x; out[3 * i + 1] = b[i].y; out[3 * i + 2] = b[i].z; }
+}
 void oracle_camera_rays(const OracleScene *s, int32_t seed, float *rays) {
     OracleCounters cn;
     Ctx c;

@@ -8,6 +8,7 @@ import pytest
 
 from chunkyclplugin_b200.javarandom import pass_seeds
 from conftest import load_scene
+from oracle.edge_rays import embed_octree
 
 pytestmark = pytest.mark.gpu
 
@@ -99,21 +100,6 @@ def test_second_scene_does_not_inherit_the_first_scenes_entities(scenes, cuda_ct
 # ---------------------------------------------------------------------------------------------------------
 # deep worlds / deep BVHs
 # ---------------------------------------------------------------------------------------------------------
-def embed_octree(tree: np.ndarray, extra_levels: int) -> np.ndarray:
-    """The same voxels in the low corner of a cube 2^extra_levels times larger (all other octants air)."""
-    tree = np.asarray(tree, np.int32)
-    k = extra_levels
-    shift = 8 * k
-    out = np.zeros(1 + 8 * k + tree.size - 1, np.int32)
-    out[0] = 1
-    for i in range(k):
-        out[1 + 8 * i] = 1 + 8 * (i + 1) if i + 1 < k else (tree[0] + shift if tree[0] > 0 else tree[0])
-    body = tree[1:].copy()
-    body[body > 0] += shift
-    out[1 + 8 * k:] = body
-    return out
-
-
 def test_deep_world_uses_nodes_between_top_table_and_bricks(scenes, cuda_ctx):
     """Octree depth 13: the top table cannot have 16^3 cells any more (air_cell_level 6, 64-ary nodes down to the bricks)."""
     import oracle
