@@ -162,6 +162,7 @@ struct SceneInfo {
     int world_bvh_empty = 1, actor_bvh_empty = 1;   // the bvh.h:23-32 probe of the committed BVHs
     int cell_level = 0, top_log2 = 0, use_wide = 0, air_cell_level = 4, air_top_log2 = 0;
     int atlas_w = 0, atlas_h = 0, atlas_layers = 0;
+    int has_specular = 0;   // a material word 5 is not 0: CCU_RENDER_SPECULAR launches the specular kernels
     float sky_intensity = 0;
     int sun_host[6] = {0, 0, 0, 0, 0, 0};
     bool have_sun = false, have_atlas = false, have_sky = false;

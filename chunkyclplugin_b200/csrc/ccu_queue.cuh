@@ -67,6 +67,8 @@ enum QField : int {
     QF_HNY = QF_COUNT, QF_HNZ, QF_HCX, QF_HCY, QF_HCZ,
     QF_BREF, QF_BSP,        // the walk's next node and (stack entries | phase << 8)
     QF_COUNT_BVH,
+    QF_HSPEC = QF_COUNT_BVH,   // HAS_BVH + SPEC only: word 5 of the closest hit's material
+    QF_COUNT_BVH_SPEC,
     QF_HDIST = QF_LIMIT, QF_HEM = QF_T, QF_HNX = QF_STEPS
 };
 // QF_META: pass (bits 0..15) | ray depth (bits 16..23) | flags
@@ -85,11 +87,14 @@ constexpr int Q_SMEM_LIMIT = 227 * 1024 - 1280;   // dynamic shared memory a CTA
 constexpr int Q_STACK = CCU_Q_STACK;
 constexpr int Q_DEEP = 64 - Q_STACK;          // stack entries beyond the shared-memory part
 constexpr int Q_STACK_WORDS = Q_STACK * Q_SLOTS;
-__host__ __device__ constexpr int q_fields(bool bvh) { return bvh ? (int)QF_COUNT_BVH : (int)QF_COUNT; }
+__host__ __device__ constexpr int q_fields(bool bvh, bool spec) { return bvh ? (spec ? (int)QF_COUNT_BVH_SPEC : (int)QF_COUNT_BVH) : (int)QF_COUNT; }
 __host__ __device__ constexpr int q_stages(bool bvh) { return bvh ? (int)QS_COUNT_BVH : (int)QS_COUNT; }
 __host__ __device__ constexpr int q_mask_words(bool bvh) { return q_stages(bvh) * Q_MW * 32; }
 // slot fields + work masks + control words (live, tile lock / base / used) [+ the staged top table]
-__host__ __device__ constexpr int q_smem_bytes(bool bvh, bool tops) { return (q_fields(bvh) * Q_SLOTS + q_mask_words(bvh) + 32 + (tops ? Q_TOP_WORDS : 0) + (bvh ? Q_STACK_WORDS : 0)) * 4; }
+__host__ __device__ constexpr int q_smem_bytes(bool bvh, bool tops, bool spec) {
+    return (q_fields(bvh, spec) * Q_SLOTS + q_mask_words(bvh) + 32 + (tops ? Q_TOP_WORDS : 0) + (bvh ? Q_STACK_WORDS : 0)) * 4;
+}
+static_assert(q_smem_bytes(true, true, true) + 64 * 64 * 4 <= Q_SMEM_LIMIT, "the largest kernel still stages a 64 x 64 sky table");
 
 #ifdef CCU_Q_STATS
 // debug counters (build with -DCCU_Q_STATS): [2*st] = executions of stage st, [2*st+1] = lanes that had a slot;
@@ -288,8 +293,10 @@ __device__ __forceinline__ void q_stage_march(const DScene &s, const unsigned *_
 // What follows closestIntersect in rayTracer.cl:93-107 for a ray whose closest hit is known: sky for a miss
 // (kernel.h:26-31), otherwise the surface response (kernel.h:33-44) and the sun sampling ray (sky.h:68-93); when the ray
 // was the shadow ray (or sun sampling is off) the diffuse bounce (nextPath, kernel.h:46-98) follows right away.
+// SPEC: a specular event at the hit (DESIGN "Beyond the reference: specular materials") bounces right away, without a sun sample.
+template <bool SPEC>
 __device__ __forceinline__ void q_shade(const DScene &s, uint32_t *F, unsigned *mask, int lane, int row, float3 o, float3 d, float distance,
-                                        bool ray_hit, const Surf &hit) {
+                                        bool ray_hit, const SurfT<SPEC> &hit) {
     const int slot = row * 32 + lane;
     uint32_t meta = QU(QF_META) & ~QM_HIT;
     const bool shadow = (meta & QM_SHADOW) != 0;
@@ -299,6 +306,8 @@ __device__ __forceinline__ void q_shade(const DScene &s, uint32_t *F, unsigned *
     bool sun = false, bounce = false;
     float3 from = o;                 // the shadow ray starts at the surface point, so that is where its bounce starts
     float3 normal = f3(0, 0, 0);     // surface normal for either continuation
+    bool specular = false;           // SPEC: the bounce is a specular event's (mirror direction blended by the roughness ro)
+    float ro = 0;
     if (!ray_hit) {
         // kernel.h:26-31 with emittance 1 (path segment) or |d.n| (shadow ray)
         float3 throughput = f3(QFL(QF_THRX), QFL(QF_THRY), QFL(QF_THRZ));
@@ -310,7 +319,7 @@ __device__ __forceinline__ void q_shade(const DScene &s, uint32_t *F, unsigned *
         else q_push(mask, QS_END, lane, row);
     } else if (shadow) {
         bounce = true;
-    } else {
+    } else if (!SPEC) {
         // kernel.h:20-22 + applyRayColor kernel.h:33-44
         float3 throughput = f3(QFL(QF_THRX), QFL(QF_THRY), QFL(QF_THRZ));
         float3 color = f3(QFL(QF_COLX), QFL(QF_COLY), QFL(QF_COLZ));
@@ -322,6 +331,27 @@ __device__ __forceinline__ void q_shade(const DScene &s, uint32_t *F, unsigned *
         QFL(QF_COLX) = color.x; QFL(QF_COLY) = color.y; QFL(QF_COLZ) = color.z;
         normal = hit.normal;
         if (s.sun_flags & 1) sun = true;
+        else bounce = true;
+    } else {
+        // the event draws come first; then applyRayColor (diffuse event) or its emission with the throughput tinted by a
+        // metal only (specular event)
+        bool metal = false;
+        if constexpr (SPEC) {
+            uint32_t rng = QU(QF_RNG);
+            specular = specular_event(hit.spec, rng, metal, ro);
+            QU(QF_RNG) = rng;
+        }
+        float3 throughput = f3(QFL(QF_THRX), QFL(QF_THRY), QFL(QF_THRZ));
+        float3 color = f3(QFL(QF_COLX), QFL(QF_COLY), QFL(QF_COLZ));
+        from = o + d * (distance - CCU_OFFSET);
+        float3 col = f3(hit.color.x, hit.color.y, hit.color.z);
+        const float3 tinted = throughput * col;
+        color = color + (col * (hit.emittance * s.emitter_scale)) * tinted;
+        if (!specular || metal) throughput = tinted;
+        QFL(QF_THRX) = throughput.x; QFL(QF_THRY) = throughput.y; QFL(QF_THRZ) = throughput.z;
+        QFL(QF_COLX) = color.x; QFL(QF_COLY) = color.y; QFL(QF_COLZ) = color.z;
+        normal = hit.normal;
+        if ((s.sun_flags & 1) && !specular) sun = true;
         else bounce = true;
     }
     if (!(sun || bounce)) return;
@@ -345,6 +375,7 @@ __device__ __forceinline__ void q_shade(const DScene &s, uint32_t *F, unsigned *
         next_limit = distance;
     } else {
         next_d = diffuse_direction_sc(normal, x1, sn, cs);
+        if (SPEC && specular) next_d = specular_direction(d, normal, next_d, ro);
         next_o = from + next_d * CCU_OFFSET;
         next_limit = inff_();
         const int ray_depth = (int)((meta >> 16) & 0xFF) + 1;
@@ -364,7 +395,7 @@ __device__ __forceinline__ void q_shade(const DScene &s, uint32_t *F, unsigned *
 
 // BLOCK (kind_block = true) and EXIT (false): the octree part of closestIntersect (kernel.h:14-16) is finished here;
 // without BVHs the ray is shaded right away, with BVHs it goes to the BVH stage.  kind_block is warp-uniform.
-template <bool HAS_BVH>
+template <bool HAS_BVH, bool SPEC>
 __device__ __forceinline__ bool q_stage_resolve(const DScene &s, uint32_t *F, unsigned *mask, int lane, const bool kind_block, int min_lanes) {
     const int row = q_pop_batch(mask, kind_block ? QS_BLOCK : QS_EXIT, lane, min_lanes);
     if (row == -2) return false;
@@ -379,8 +410,9 @@ __device__ __forceinline__ bool q_stage_resolve(const DScene &s, uint32_t *F, un
     m.steps = QI(QF_STEPS);
     bool ray_hit = false;
     float hit_t = 0;
-    Surf hit;
+    SurfT<SPEC> hit;
     hit.normal = f3(0, 0, 0); hit.color = make_float4(0, 0, 0, 0); hit.emittance = 0;
+    surf_set_spec(hit, 0u);
     if (kind_block) {
         // the leaf under the ray (octree.h:81-88): value and level
         const Cell c = march_cell(m);
@@ -401,6 +433,7 @@ __device__ __forceinline__ bool q_stage_resolve(const DScene &s, uint32_t *F, un
             QFL(QF_HEM) = hit.emittance;
             QFL(QF_HNX) = hit.normal.x; QFL(QF_HNY) = hit.normal.y; QFL(QF_HNZ) = hit.normal.z;
             QFL(QF_HCX) = hit.color.x; QFL(QF_HCY) = hit.color.y; QFL(QF_HCZ) = hit.color.z;
+            if constexpr (SPEC) QU(QF_HSPEC) = hit.spec;
         }
         const uint32_t meta = QU(QF_META);
         QU(QF_META) = ray_hit ? (meta | QM_HIT) : (meta & ~QM_HIT);
@@ -423,6 +456,7 @@ __device__ __forceinline__ bool q_stage_resolve(const DScene &s, uint32_t *F, un
 }
 
 // SHADE (HAS_BVH kernels): closestIntersect is complete (kernel.h:17-22)
+template <bool SPEC>
 __device__ __forceinline__ bool q_stage_shade(const DScene &s, uint32_t *F, unsigned *mask, int lane, int min_lanes) {
     const int row = q_pop_batch(mask, QS_SHADE, lane, min_lanes);
     if (row == -2) return false;
@@ -432,10 +466,11 @@ __device__ __forceinline__ bool q_stage_shade(const DScene &s, uint32_t *F, unsi
     const float3 o = f3(QFL(QF_OX), QFL(QF_OY), QFL(QF_OZ));
     const float3 d = f3(QFL(QF_DX), QFL(QF_DY), QFL(QF_DZ));
     const bool ray_hit = (QU(QF_META) & QM_HIT) != 0;
-    Surf hit;
+    SurfT<SPEC> hit;
     hit.normal = f3(QFL(QF_HNX), QFL(QF_HNY), QFL(QF_HNZ));
     hit.color = make_float4(QFL(QF_HCX), QFL(QF_HCY), QFL(QF_HCZ), 0.0f);
     hit.emittance = QFL(QF_HEM);
+    if constexpr (SPEC) hit.spec = QU(QF_HSPEC);
     q_shade(s, F, mask, lane, row, o, d, QFL(QF_HDIST), ray_hit, hit);
     return true;
 }
@@ -591,6 +626,7 @@ __device__ __forceinline__ void q_stage_bvh(const DScene &s, uint32_t *F, unsign
 }
 
 // QS_LEAF: the triangles of one leaf (bvh.h:52-67) for walks that sit at a leaf, then the walk's next node from its stack
+template <bool SPEC>
 __device__ __forceinline__ bool q_stage_leaf(const DScene &s, uint32_t *F, unsigned *mask, int *stk, int *deep, int lane, int min_lanes) {
     const int row = q_pop_batch(mask, QS_LEAF, lane, min_lanes);
     if (row == -2) return false;
@@ -603,8 +639,9 @@ __device__ __forceinline__ bool q_stage_leaf(const DScene &s, uint32_t *F, unsig
     int ref = QI(QF_BREF);
     const int bsp = QI(QF_BSP);
     int sp = bsp & 0xFF, phase = bsp >> 8;
-    Surf hit;
+    SurfT<SPEC> hit;
     hit.normal = f3(0, 0, 0); hit.color = make_float4(0, 0, 0, 0); hit.emittance = 0;
+    surf_set_spec(hit, 0u);
     bool any = false;
     const int *blk = s.tris2 + (size_t)(-(ref + 1)) * 8;
     const int num = __ldg(blk);
@@ -635,6 +672,7 @@ __device__ __forceinline__ bool q_stage_leaf(const DScene &s, uint32_t *F, unsig
         QFL(QF_HEM) = hit.emittance;
         QFL(QF_HNX) = hit.normal.x; QFL(QF_HNY) = hit.normal.y; QFL(QF_HNZ) = hit.normal.z;
         QFL(QF_HCX) = hit.color.x; QFL(QF_HCY) = hit.color.y; QFL(QF_HCZ) = hit.color.z;
+        if constexpr (SPEC) QU(QF_HSPEC) = hit.spec;
         QU(QF_META) = meta | QM_HIT;
     }
     if (any && first_hit_ends) { phase = 2; ref = 0; }
@@ -789,14 +827,14 @@ __device__ __forceinline__ bool q_stage_end(const DScene &s, const PassParams &w
 }
 
 // LAY 0: the top table of the air layout fits Q_TOP_WORDS and is staged in shared memory; 1: it is read from global memory;
-// 2: deep world (64-ary nodes between the top table and the bricks)
-template <bool HAS_BVH, int LAY>
+// 2: deep world (64-ary nodes between the top table and the bricks).  SPEC: CCU_RENDER_SPECULAR on a scene with specular words.
+template <bool HAS_BVH, int LAY, bool SPEC>
 __global__ void __launch_bounds__(Q_WARPS * 32, 1) k_render_queue(const __grid_constant__ DScene s, const __grid_constant__ QueueParams qp) {
     constexpr int NST = q_stages(HAS_BVH);
     constexpr int MASK_WORDS = q_mask_words(HAS_BVH);
     extern __shared__ uint32_t q_mem[];
     uint32_t *F = q_mem;
-    unsigned *mask = q_mem + q_fields(HAS_BVH) * Q_SLOTS;
+    unsigned *mask = q_mem + q_fields(HAS_BVH, SPEC) * Q_SLOTS;
     int *live = reinterpret_cast<int *>(mask + MASK_WORDS);
     unsigned *top_s = mask + MASK_WORDS + 32;
     int *stk = reinterpret_cast<int *>(top_s + (LAY == 0 ? Q_TOP_WORDS : 0));   // HAS_BVH only: stacks by slot
@@ -870,11 +908,11 @@ __global__ void __launch_bounds__(Q_WARPS * 32, 1) k_render_queue(const __grid_c
         switch (best) {
             case QS_MARCH: QSTAT(0, 1); q_stage_march<NST, LAY>(s, top, F, mask, lane, qp.yield_below, qp.refill_min); break;
             case QS_BLOCK:
-            case QS_EXIT: ran = q_stage_resolve<HAS_BVH>(s, F, mask, lane, best == QS_BLOCK, min_lanes); break;
+            case QS_EXIT: ran = q_stage_resolve<HAS_BVH, SPEC>(s, F, mask, lane, best == QS_BLOCK, min_lanes); break;
             case QS_END: ran = q_stage_end<!HAS_BVH>(s, qp.w, F, mask, live, lane, min_lanes); break;
             case QS_BVH: QSTAT(16, 1); if (HAS_BVH) q_stage_bvh<NST>(s, F, mask, stk, qp.bvh_deep, lane, qp.yield_below, qp.refill_min); break;
-            case QS_LEAF: if (HAS_BVH) ran = q_stage_leaf(s, F, mask, stk, qp.bvh_deep, lane, min_lanes); break;
-            default: if (HAS_BVH) ran = q_stage_shade(s, F, mask, lane, min_lanes); break;
+            case QS_LEAF: if (HAS_BVH) ran = q_stage_leaf<SPEC>(s, F, mask, stk, qp.bvh_deep, lane, min_lanes); break;
+            default: if (HAS_BVH) ran = q_stage_shade<SPEC>(s, F, mask, lane, min_lanes); break;
         }
         sticky = (ran && best != QS_MARCH && best != QS_BVH) ? best : -1;
         if (ran) {

@@ -44,7 +44,8 @@ __global__ void k_sun_setup(const int *sun_words, float *out /* su sv sw radius_
 // Thread-per-pixel path tracer: all passes of the batch in one launch, the running mean of
 // rayTracer.cl:109-112 carried in registers between passes (identical arithmetic, no memory round trip).
 // MODE: 0 = the reference's own node array, 1 = commit-time layouts, 2 = commit-time layouts of a deep world.
-template <int MODE>
+// SPEC: CCU_RENDER_SPECULAR on a scene with specular words (sample_pixel).
+template <int MODE, bool SPEC>
 __global__ void __launch_bounds__(128) k_render_mega(const __grid_constant__ DScene s, const int *__restrict__ seeds, int n_passes,
                                                      int start_spp, float *res, const float *res_prev, int n_pixels) {
     stage_tables(s, nullptr);
@@ -53,7 +54,7 @@ __global__ void __launch_bounds__(128) k_render_mega(const __grid_constant__ DSc
         const float *pp = res_prev + (size_t)gid * 3;    // what the reference's single buffer holds when the window starts
         float3 buf = f3(pp[0], pp[1], pp[2]);
         for (int pass = 0; pass < n_passes; pass++) {
-            float3 col = sample_pixel<MODE>(s, gid, __ldg(seeds + pass));
+            float3 col = sample_pixel<MODE, SPEC>(s, gid, __ldg(seeds + pass));
             int spp = start_spp + pass;
             float fs = (float)spp, fs1 = (float)(spp + 1);
             buf.x = (buf.x * fs + col.x) / fs1;
@@ -425,12 +426,16 @@ void dispatch(bool v, F &&f) {
     else f(std::false_type{});
 }
 
-// the wavefront kernel (ccu_queue.cuh) for the scene's entity BVHs and air layout (air_layout_id)
-auto queue_kernel(bool bvh, int lay) {
-    decltype(&k_render_queue<false, 0>) k = nullptr;
-    dispatch(bvh, [&](auto B) { dispatch<3>(lay, [&](auto L) { k = k_render_queue<B, L>; }); });
+// the wavefront kernel (ccu_queue.cuh) for the scene's entity BVHs and air layout (air_layout_id), with or without specular events
+auto queue_kernel(bool bvh, int lay, bool spec) {
+    decltype(&k_render_queue<false, 0, false>) k = nullptr;
+    dispatch(bvh, [&](auto B) { dispatch<3>(lay, [&](auto L) { dispatch(spec, [&](auto S) { k = k_render_queue<B, L, S>; }); }); });
     return k;
 }
+
+// CCU_RENDER_SPECULAR launches the specular kernels only on a scene that has a specular word: without one they compute exactly
+// what the other kernels compute
+bool specular_launch(const ccu_ctx *c) { return (c->params.flags & CCU_RENDER_SPECULAR) && c->scene.info.has_specular; }
 
 }  // namespace
 
@@ -590,8 +595,9 @@ int ccu_ctx_create(int device_index, ccu_ctx **out) {
     for (Event &ev : c->chunk_ev) if (e == cudaSuccess) e = ev.create(cudaEventDisableTiming);
     for (Event &ev : c->rays_used) if (e == cudaSuccess) e = ev.create(cudaEventDisableTiming);
     for (bool bvh : {false, true})
-        for (int lay = 0; lay < 3 && e == cudaSuccess; lay++)
-            e = cudaFuncSetAttribute(queue_kernel(bvh, lay), cudaFuncAttributeMaxDynamicSharedMemorySize, Q_SMEM_LIMIT);
+        for (bool spec : {false, true})
+            for (int lay = 0; lay < 3 && e == cudaSuccess; lay++)
+                e = cudaFuncSetAttribute(queue_kernel(bvh, lay, spec), cudaFuncAttributeMaxDynamicSharedMemorySize, Q_SMEM_LIMIT);
     if (e == cudaSuccess) e = c->unorm.alloc(256);
     if (e == cudaSuccess) {
         k_unorm_table<<<1, 256, 0, c->stream>>>(c->unorm.p);
@@ -767,6 +773,10 @@ int ccu_scene_commit(ccu_ctx *c) {
         CU(sc.mat_rec.upload(pr.mat.data(), pr.mat.size(), c->stream));
         CU(sc.quad_rec.upload(pr.quad.data(), pr.quad.size(), c->stream));
         CU(sc.aabb_rec.upload(pr.aabb.data(), pr.aabb.size(), c->stream));
+        // word 5 (specular / metalness / roughness) of every material on a record, and of every full cube's material
+        in.has_specular = 0;
+        for (size_t i = 0; i + 7 < pr.mat.size(); i += 8) in.has_specular |= pr.mat[i + 5] != 0;
+        for (size_t i = 0; i + 7 < pr.block.size(); i += 8) in.has_specular |= pr.block[i] == 1 && pr.block[i + 7] != 0;
     }
     // BVH stage layout (pair records + aligned triangle blocks); a scene whose BVHs it cannot hold is rendered by the
     // thread-per-pixel kernel on the reference's own arrays
@@ -892,7 +902,7 @@ int ccu_render_set_params(ccu_ctx *c, const ccu_render_params *p) {
     if (!c || !p) return fail(CCU_EINVAL, "ccu_render_set_params: null argument");
     if (p->draw_depth < 0 || p->draw_depth >= (1 << 24) || p->max_depth < 1 || p->max_depth > 255) return fail(CCU_EINVAL, "bad render params");
     if (p->kernel != 0 && p->kernel != 1 && p->kernel != 4) return fail(CCU_EINVAL, "unknown kernel %d (0 auto, 1 thread-per-pixel, 4 wavefront)", p->kernel);
-    if (p->flags & ~(CCU_RENDER_NO_ENTITIES | CCU_RENDER_NO_SUN)) return fail(CCU_EINVAL, "unknown render flags 0x%x", p->flags);
+    if (p->flags & ~(CCU_RENDER_NO_ENTITIES | CCU_RENDER_NO_SUN | CCU_RENDER_SPECULAR)) return fail(CCU_EINVAL, "unknown render flags 0x%x", p->flags);
     std::lock_guard<std::mutex> lk(c->mu);
     c->params = *p;
     return CCU_OK;
@@ -931,6 +941,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
     if (first_chunk) CU(cudaEventRecord(c->ev0, c->stream));
     const bool bvh = !(s.world_bvh_empty && s.actor_bvh_empty);
     const int mode = layout_mode(c);
+    const bool spec = specular_launch(c);
     float *res = c->accum[c->accum_active].p;
     const float *res_prev = c->window_spp == 0 ? c->window_base : res;
     int kernel = c->params.kernel;
@@ -938,7 +949,9 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
     if (kernel == 1) {
         const int threads = 128, blocks = (n_pixels + threads - 1) / threads;
         dispatch<3>(mode, [&](auto M) {
-            k_render_mega<M><<<blocks, threads, 0, c->stream>>>(s, seeds_dev, n_passes, c->window_spp, res, res_prev, n_pixels);
+            dispatch(spec, [&](auto S) {
+                k_render_mega<M, S><<<blocks, threads, 0, c->stream>>>(s, seeds_dev, n_passes, c->window_spp, res, res_prev, n_pixels);
+            });
         });
     } else {
         // persistent wavefront kernel (ccu_queue.cuh): one CTA per SM, pixels handed out through a counter
@@ -965,7 +978,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
         // 128 x 128 table (64 KiB) taken from L1 costs more brick / atlas hits than the sky lookups gain (measured: +1.8 % per
         // pass on config 1).  CCU_SKY_SMEM_MAX (bytes, default 16 KiB = 64 x 64 texels) moves the threshold.
         const int sky_texels = c->scene.info.sky_res * c->scene.info.sky_res;
-        const int base_smem = q_smem_bytes(bvh, lay == 0);
+        const int base_smem = q_smem_bytes(bvh, lay == 0, spec);
         const char *sky_env = getenv("CCU_SKY_SMEM_MAX");
         const int sky_max = sky_env ? atoi(sky_env) : 16384;
         const bool sky_smem = sky_texels * 4 <= sky_max && base_smem + sky_texels * 4 <= Q_SMEM_LIMIT;
@@ -977,7 +990,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
             qp.bvh_deep = c->bvh_deep.p;
         }
         const int smem = base_smem + qp.sky_texels * 4;
-        queue_kernel(bvh, lay)<<<grid, block, smem, c->stream>>>(s, qp);
+        queue_kernel(bvh, lay, spec)<<<grid, block, smem, c->stream>>>(s, qp);
 #ifdef CCU_Q_STATS
         {
             cudaStreamSynchronize(c->stream);

@@ -14,7 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # CHUNKYCU_LIB: load another build of the same library (kernel tuning sweeps build variants next to each other)
 LIB_PATH = os.environ.get("CHUNKYCU_LIB") or os.path.join(_HERE, "libchunkycu.so")
 
-CCU_RENDER_NO_ENTITIES, CCU_RENDER_NO_SUN = 1, 2
+CCU_RENDER_NO_ENTITIES, CCU_RENDER_NO_SUN, CCU_RENDER_SPECULAR = 1, 2, 4
 CCU_UNIQUE_ID_BYTES = 128
 
 CCU_OK, CCU_ENODEVICE, CCU_EINVAL, CCU_ECUDA, CCU_ENOMEM, CCU_ESTATE = 0, -1, -2, -3, -4, -5

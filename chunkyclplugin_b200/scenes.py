@@ -343,12 +343,17 @@ class AtlasBuilder:
         return np.stack(self.layers, axis=0)
 
 
+def specular_word(specular: float = 0.0, metalness: float = 0.0, roughness: float = 0.0) -> int:
+    """Word 5 of a packed material (PackedMaterial.java:69-71): specular, metalness, roughness bytes."""
+    return int(specular * 255.0) | (int(metalness * 255.0) << 8) | (int(roughness * 255.0) << 16)
+
+
 def pack_material(size: int, loc: int, emittance: float = 0.0, tint: int = 0, textured: bool = True,
-                  argb: int = 0xFFFFFFFF, specular: float = 0.0) -> List[int]:
+                  argb: int = 0xFFFFFFFF, specular: float = 0.0, metalness: float = 0.0, roughness: float = 0.0) -> List[int]:
     """PackedMaterial.pack (PackedMaterial.java:88-100)."""
     flags = 4 if textured else 0
     w2, w3 = (size, loc) if textured else (-1 if argb & 0x80000000 else 0, argb)
-    return [flags, tint, w2, w3, int(emittance * 255.0), int(specular * 255.0)]
+    return [flags, tint, w2, w3, int(emittance * 255.0), specular_word(specular, metalness, roughness)]
 
 
 def _i32(words) -> np.ndarray:
@@ -774,6 +779,21 @@ def entity_scene(size: int = 256, width: int = 1920, height: int = 1080, n_world
     return _finish(f"entities{size}", tree, base.octree_depth, pal, base.camera, width, height,
                    world_bvh=wb, actor_bvh=ab, trigs=trigs,
                    meta={"size": size, "world_tris": int(tw.shape[0]), "actor_tris": int(ta.shape[0])})
+
+
+# (specular, metalness, roughness) that glossy() hands out in turn: specular only, metal only, specular + rough, zero,
+# metal + specular + rough
+GLOSS = ((0.8, 0.0, 0.0), (0.0, 0.9, 0.0), (0.7, 0.0, 0.5), (0.0, 0.0, 0.0), (0.3, 0.6, 0.25))
+
+
+def glossy(p: PackedScene) -> PackedScene:
+    """The scene with word 5 of its materials set (CCU_RENDER_SPECULAR): materials take the GLOSS entries in turn, emitters
+    become emissive-specular.  Full cubes, model blocks and entity triangles of the scene thereby get a mix of materials."""
+    mp = p.mat_palette.copy()
+    for i in range(mp.size // 6):
+        emissive = (mp[6 * i] & 2) or (mp[6 * i + 4] & 0xFF)
+        mp[6 * i + 5] = specular_word(0.5) if emissive else specular_word(*GLOSS[i % len(GLOSS)])
+    return dataclasses.replace(p, mat_palette=mp, name=p.name + "_glossy")
 
 
 def mixed_test_scene(size: int = 64, width: int = 96, height: int = 54, seed: int = 99) -> PackedScene:

@@ -51,6 +51,13 @@ typedef struct ccu_render_params {
 /* Sunlight disabled (indoor scenes): bit 0 of the sun flags (PackedSun.java:16, tested at sky.h:45,69) reads as 0 - no sun
  * sampling, no sun disc - without re-uploading sunData. */
 #define CCU_RENDER_NO_SUN 2
+/* Specular, metallic and rough materials (beyond the reference, which shades every surface diffuse): word 5 of a material
+ * (specular bits 0-7, metalness 8-15, roughness 16-23, each byte / 255) picks at every path-segment hit a metal event with
+ * probability metalness, else a specular one with probability specular.  Such an event reflects the ray about the normal,
+ * blended towards a diffuse direction by the roughness, takes no sun sample and tints the throughput by the surface colour
+ * only for a metal.  A material whose word 5 is 0 shades as without the flag.  DESIGN.md "Beyond the reference: specular
+ * materials" holds the exact contract. */
+#define CCU_RENDER_SPECULAR 4
 
 /* ---- device enumeration: RendererInstance.java:39-75,123-157 (clGetPlatformIDs/clGetDeviceIDs/clGetDeviceInfo),
  *      used by the GPU selector UI (ui/GpuSelector.java:24-87) -------------------------------------------------- */

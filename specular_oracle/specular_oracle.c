@@ -1,0 +1,301 @@
+/*
+ * specular_oracle.c - CPU restatement of CCU_RENDER_SPECULAR (DESIGN.md section 9).  TEST INFRASTRUCTURE ONLY.
+ *
+ * The reference has no specular path, so there is nothing of it to pin this file against: DESIGN.md section 9 is the contract,
+ * this file restates it, and the tests hold this restatement and the CUDA kernels to each other bit for bit (plus analytic and
+ * statistical checks of the restatement alone).
+ *
+ * Everything the reference does is taken unchanged from the parity oracle, whose source is compiled into this library as is
+ * (camera, octree march, primitives, materials, BVHs, sky, sun, applyRayColor, nextPath, RNG, the arithmetic contract).
+ * Restated here are only the functions whose record must also carry word 5 of the material the surface's colour came from
+ * (block test, octree march, BVH walk, closestIntersect: the oracle's IntersectionRecord has no such field) and the path
+ * loop with the specular event.  Each is the oracle function of the same name plus that word, operation for operation.
+ */
+#include "../oracle/chunky_oracle.c"
+
+/* Material_sample (material.h:31-82) through the oracle; on success also word 5 of the material */
+static int material_sample_w5(const Ctx *c, int material, Record *rec, uint32_t *w5, float u, float v) {
+    if (!material_sample(c, material, rec, u, v)) return 0;
+    *w5 = (uint32_t)c->sc->mat_palette[material + 5];
+    return 1;
+}
+
+/* intersect_block (block.h:30-118) */
+static float intersect_block_w5(const Ctx *c, int block, int bx, int by, int bz, Record *rec, uint32_t *w5, v3 origin, v3 direction,
+                                v3 inv) {
+    if (block == ANY_TYPE) return NAN;
+    const OracleScene *s = c->sc;
+    int model_type = s->block_palette[block + 0];
+    int model_ptr = s->block_palette[block + 1];
+    c->cnt->block_tests++;
+    v3 norm_origin = vsub(vsub(origin, vscale(direction, OFFSET)), V((float)bx, (float)by, (float)bz));
+    v3 normal = V(0, 0, 0);
+    float u = 0, v = 0;
+    switch (model_type) {
+    default:
+    case 0:
+        return NAN;
+    case 1: {
+        AABB box = {0, 1, 0, 1, 0, 1};
+        float dist = aabb_full(&box, norm_origin, origin, inv, &normal, &u, &v, 0);
+        if (dist != dist) return NAN;
+        rec->normal = normal;
+        if (material_sample_w5(c, model_ptr, rec, w5, u, v)) return dist - OFFSET;
+        return NAN;
+    }
+    case 2: {
+        int hit = 0;
+        float dist = HUGE_VALF;
+        int material = 0;
+        int boxes = s->aabb_models[model_ptr];
+        for (int i = 0; i < boxes; i++) {
+            const int32_t *model = s->aabb_models + model_ptr + 1 + i * 13;
+            c->cnt->aabb_boxes++;
+            float t = textured_aabb(model, dist, norm_origin, direction, inv, &normal, &u, &v, &material);
+            if (t == t) {
+                if (material_sample_w5(c, material, rec, w5, u, v)) { rec->normal = normal; dist = t; hit = 1; }
+            }
+        }
+        return hit ? dist : NAN;
+    }
+    case 3: {
+        int hit = 0;
+        float dist = HUGE_VALF;
+        int quads = s->quad_models[model_ptr];
+        for (int i = 0; i < quads; i++) {
+            const int32_t *q = s->quad_models + model_ptr + 1 + i * 15;
+            c->cnt->quads++;
+            float t = quad_intersect(q, dist, norm_origin, direction, &normal, &u, &v);
+            if (t == t) {
+                if (material_sample_w5(c, q[13], rec, w5, u, v)) { rec->normal = normal; dist = t; hit = 1; }
+            }
+        }
+        return hit ? dist : NAN;
+    }
+    }
+}
+
+/* octree_intersect (octree.h:41-109) */
+static int octree_intersect_w5(const Ctx *c, const Path *ray, Record *rec, uint32_t *w5) {
+    const OracleScene *s = c->sc;
+    const int32_t *tree = s->octree;
+    int depth = s->octree_depth;
+    float dist_march = 0;
+    v3 inv = V(1.0f / ray->direction.x, 1.0f / ray->direction.y, 1.0f / ray->direction.z);
+    v3 offset_d = vscale(ray->direction, OFFSET);
+    int lx, ly, lz;
+    floor3i(ray->origin, &lx, &ly, &lz);
+    if (((lx >> depth) != 0) | ((ly >> depth) != 0) | ((lz >> depth) != 0)) {
+        float size = (float)(1 << depth);
+        AABB box = {0, size, 0, size, 0, size};
+        float dist = aabb_quick(&box, ray->origin, inv);
+        if (dist != dist || dist < 0) return 0;
+        dist_march += dist + OFFSET;
+    }
+    for (int i = 0; i < s->draw_depth; i++) {
+        if (dist_march > rec->distance) return 0;
+        v3 pos = vadd(ray->origin, vscale(ray->direction, dist_march));
+        int bx, by, bz;
+        floor3i(vadd(pos, offset_d), &bx, &by, &bz);
+        if (((bx >> depth) != 0) | ((by >> depth) != 0) | ((bz >> depth) != 0)) return 0;
+        c->cnt->march_steps++;
+        int level = depth;
+        int node = 0;
+        int data = tree[0];
+        c->cnt->descent_loads++;
+        while (data > 0) {
+            level--;
+            node = data + ((((bx >> level) & 1) << 2) | (((by >> level) & 1) << 1) | ((bz >> level) & 1));
+            data = tree[node];
+            c->cnt->descent_loads++;
+        }
+        data = -data;
+        lx = bx >> level; ly = by >> level; lz = bz >> level;
+        if (data != 0) {
+            float dist = intersect_block_w5(c, data, bx, by, bz, rec, w5, pos, ray->direction, inv);
+            if (dist == dist) {
+                rec->distance = dist_march + dist;
+                rec->material = data;
+                rec->hit_node = node;
+                rec->hit_kind = 1;
+                return 1;
+            }
+        }
+        AABB box = {(float)(lx << level), (float)((lx + 1) << level), (float)(ly << level), (float)((ly + 1) << level),
+                    (float)(lz << level), (float)((lz + 1) << level)};
+        dist_march += aabb_exit(&box, vadd(pos, offset_d), inv) + OFFSET;
+    }
+    return 0;
+}
+
+/* bvh_intersect (bvh.h:22-113) */
+static int bvh_intersect_w5(const Ctx *c, const int32_t *bvh, const Path *ray, Record *rec, uint32_t *w5, int kind) {
+    const int32_t *trigs = c->sc->bvh_trigs;
+    c->cnt->bvh_calls++;
+    if (bvh[0] == 0) {
+        int all_nan = 1;
+        for (int i = 1; i < 7; i++) { float f = as_float(bvh[i]); if (f == f) all_nan = 0; }
+        if (all_nan) return 0;
+    }
+    int hit = 0, to_visit = 0, current = 0;
+    int stack[64];
+    v3 inv = V(1.0f / ray->direction.x, 1.0f / ray->direction.y, 1.0f / ray->direction.z);
+    for (;;) {
+        int head = bvh[current];
+        if (head <= 0) {
+            int prim = -head;
+            int num = trigs[prim];
+            c->cnt->bvh_leaf++;
+            for (int i = 0; i < num; i++) {
+                v3 normal; float u, v; int material;
+                c->cnt->triangles++;
+                float dist = triangle_intersect(trigs + prim + 1 + 20 * i, rec->distance, ray->origin, ray->direction, &normal, &u, &v, &material);
+                if (dist == dist) {
+                    if (material_sample_w5(c, material, rec, w5, u, v)) {
+                        rec->normal = normal; rec->distance = dist; hit = 1;
+                        rec->hit_kind = kind; rec->hit_node = -1;
+                    }
+                }
+            }
+            if (to_visit == 0) break;
+            current = stack[--to_visit];
+        } else {
+            int offset = head;
+            c->cnt->bvh_inner++;
+            const int32_t *n1 = bvh + current + 7;
+            AABB b1 = {as_float(n1[1]), as_float(n1[2]), as_float(n1[3]), as_float(n1[4]), as_float(n1[5]), as_float(n1[6])};
+            float t1 = aabb_quick(&b1, ray->origin, inv);
+            const int32_t *n2 = bvh + offset;
+            AABB b2 = {as_float(n2[1]), as_float(n2[2]), as_float(n2[3]), as_float(n2[4]), as_float(n2[5]), as_float(n2[6])};
+            float t2 = aabb_quick(&b2, ray->origin, inv);
+            int miss1 = (t1 != t1) || t1 > rec->distance;
+            int miss2 = (t2 != t2) || t2 > rec->distance;
+            if (miss1) {
+                if (miss2) {
+                    if (to_visit == 0) break;
+                    current = stack[--to_visit];
+                } else {
+                    current = offset;
+                }
+            } else if (miss2) {
+                current += 7;
+            } else if (t1 < t2) {
+                stack[to_visit++] = offset;
+                current += 7;
+            } else {
+                stack[to_visit++] = current + 7;
+                current = offset;
+            }
+        }
+    }
+    return hit;
+}
+
+/* closest_intersect (kernel.h:14-24) */
+static int closest_intersect_w5(const Ctx *c, const Path *ray, Record *rec, uint32_t *w5) {
+    int hit = 0;
+    c->cnt->rays++;
+    hit |= octree_intersect_w5(c, ray, rec, w5);
+    hit |= bvh_intersect_w5(c, c->sc->world_bvh, ray, rec, w5, 2);
+    hit |= bvh_intersect_w5(c, c->sc->actor_bvh, ray, rec, w5, 3);
+    if (hit) rec->point = vadd(ray->origin, vscale(ray->direction, rec->distance - OFFSET));
+    return hit;
+}
+
+/* The specular event of a path-segment hit on a material with word 5 = w (DESIGN.md section 9, steps 1 and 3): the event
+ * draws; on a specular event the emission of applyRayColor, the throughput tinted only by a metal, no sun sample, and the
+ * mirror direction blended towards nextPath's cosine-weighted one by the roughness.  Returns 0 for a diffuse event (nothing
+ * done), else 1 with *more = whether the path continues. */
+static int specular_event(const Ctx *c, Path *p, Record *rec, uint32_t w, uint32_t *state, int *more) {
+    float sp = (float)(w & 0xFF) / 255.0f, me = (float)((w >> 8) & 0xFF) / 255.0f, ro = (float)((w >> 16) & 0xFF) / 255.0f;
+    int metal = 0, spec = 0;
+    if (me > 0) metal = rng_float(state) < me;
+    if (!metal && sp > 0) spec = rng_float(state) < sp;
+    if (!metal && !spec) return 0;
+    v3 col = V(rec->color[0], rec->color[1], rec->color[2]);
+    v3 tinted = vmul(p->throughput, col);
+    p->pix_color = vadd(p->pix_color, vmul(vscale(col, rec->emittance * c->sc->emitter_scale), tinted));
+    if (metal) p->throughput = tinted;
+    v3 d = p->direction, n = rec->normal;
+    v3 r = vnormalize(vsub(d, vscale(n, 2.0f * vdot(d, n))));
+    Path q = *p;
+    next_path(c, &q, rec, state, c->sc->max_depth); /* the two draws and the cosine-weighted direction */
+    p->direction = ro > 0 ? vnormalize(vadd(vscale(r, 1.0f - ro), vscale(q.direction, ro))) : r;
+    p->origin = vadd(rec->point, vscale(p->direction, OFFSET));
+    p->ray_depth += 1;
+    rec->distance = HUGE_VALF;
+    *more = p->ray_depth < c->sc->max_depth;
+    return 1;
+}
+
+/* one path sample: rayTracer.cl:40-107 with the specular events */
+static v3 sample_pixel_specular(const Ctx *c, int gid, int32_t seed) {
+    Path p;
+    Record rec;
+    uint32_t w5 = 0;
+    p.pix_color = V(0, 0, 0);
+    p.throughput = V(1, 1, 1);
+    p.ray_depth = 0;
+    record_new(&rec);
+    uint32_t state = (uint32_t)seed + (uint32_t)gid;
+    rng_next(&state);
+    camera_ray(c, gid, &state, &p, 0);
+    c->cnt->samples++;
+    for (;;) {
+        c->cnt->segments++;
+        if (!closest_intersect_w5(c, &p, &rec, &w5)) {
+            rec.emittance = 1;
+            intersect_sky(c, &p, &rec);
+            break;
+        }
+        int more;
+        if (specular_event(c, &p, &rec, w5, &state, &more)) {
+            if (!more) break;
+            continue;
+        }
+        apply_ray_color(&p, &rec, c->sc->emitter_scale);
+        if (sun_sample_direction(c, &p, &rec, &state)) {
+            Record s = rec; /* IntersectionRecord_copy keeps distance: SURVEY Q4 */
+            s.point = rec.normal;
+            if (!closest_intersect(c, &p, &s)) intersect_sky(c, &p, &s);   /* the shadow ray needs no word 5 */
+        }
+        if (!next_path(c, &p, &rec, &state, c->sc->max_depth)) break;
+    }
+    return p.pix_color;
+}
+
+/* oracle_render with the specular events (same arguments, same running mean) */
+int specular_render(const OracleScene *s, const int32_t *seeds, int n_passes, int start_spp, float *res, const int32_t *gids,
+                    int64_t n_gids, int nthreads, OracleCounters *out_counters) {
+    int64_t n = gids ? n_gids : (int64_t)s->width * s->height;
+    OracleCounters total;
+    memset(&total, 0, sizeof total);
+#ifdef _OPENMP
+    if (nthreads > 0) omp_set_num_threads(nthreads);
+#endif
+#pragma omp parallel
+    {
+        OracleCounters local;
+        memset(&local, 0, sizeof local);
+        Ctx c;
+        ctx_init(&c, s, &local);
+#pragma omp for schedule(dynamic, 64)
+        for (int64_t k = 0; k < n; k++) {
+            int gid = gids ? gids[k] : (int)k;
+            float *px = res + (size_t)gid * 3;
+            v3 buf = V(px[0], px[1], px[2]);
+            for (int pass = 0; pass < n_passes; pass++) {
+                v3 col = sample_pixel_specular(&c, gid, seeds[pass]);
+                int spp = start_spp + pass;
+                buf.x = (buf.x * (float)spp + col.x) / (float)(spp + 1);
+                buf.y = (buf.y * (float)spp + col.y) / (float)(spp + 1);
+                buf.z = (buf.z * (float)spp + col.z) / (float)(spp + 1);
+            }
+            px[0] = buf.x; px[1] = buf.y; px[2] = buf.z;
+        }
+#pragma omp critical
+        counters_add(&total, &local);
+    }
+    if (out_counters) *out_counters = total;
+    return 0;
+}
