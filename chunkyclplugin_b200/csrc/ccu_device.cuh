@@ -78,6 +78,18 @@ struct DScene {   // what a launch reads: commit fills the scene's fields once (
     float emitter_scale;
 };
 
+// The emitter table of CCU_RENDER_EMITTER_SAMPLING (DESIGN §10), built at commit and passed to the thread-per-pixel kernel as
+// an argument of its own (after the others, so that every kernel keeps the parameter offsets it had without it):
+// emit[i] = {x, y, z, block palette position} sorted by (x, y, z); the cell lists in CSR form, L(c) = list[off[c] .. off[c + 1]),
+// cells of 1 << shift voxels, index (cx * dim.y + cy) * dim.z + cz over the cell box whose low voxel corner is g0.
+struct EmitView {
+    const int4 *__restrict__ emit;
+    const int *__restrict__ off;
+    const int *__restrict__ list;
+    int3 g0, dim;
+    int shift;
+};
+
 // What a successful intersection writes into the IntersectionRecord (wavefront.h:37-78).  The specular kernels (SPEC, DESIGN
 // "Beyond the reference: specular materials") also carry word 5 of the material the colour came from: specular, metalness and
 // roughness bytes.  The other kernels keep the reference's record exactly.
@@ -872,6 +884,80 @@ __device__ __forceinline__ bool specular_event(uint32_t w, uint32_t &rng, bool &
 __device__ __forceinline__ float3 specular_direction(float3 d, float3 n, float3 q, float ro) {
     const float3 r = normalize3(d - n * (2.0f * dot3(d, n)));
     return ro > 0 ? normalize3(r * (1.0f - ro) + q * ro) : r;
+}
+
+// ------------------------------------------------------------------------------------------------------
+// beyond the reference: emitter sampling (CCU_RENDER_EMITTER_SAMPLING, DESIGN §10)
+// ------------------------------------------------------------------------------------------------------
+#define CCU_NEE_DELTA (8.0f * CCU_OFFSET)   // the shadow ray stops this far before the sampled point
+
+// The grid cell of voxel (vx, vy, vz); false when the voxel lies outside the grid (always, on a scene without emitters).
+__device__ __forceinline__ bool emitter_voxel_cell(const EmitView &g, int vx, int vy, int vz, int3 &c) {
+    const long long dx = (long long)vx - g.g0.x, dy = (long long)vy - g.g0.y, dz = (long long)vz - g.g0.z;
+    if (dx < 0 || dy < 0 || dz < 0) return false;
+    c = make_int3((int)(dx >> g.shift), (int)(dy >> g.shift), (int)(dz >> g.shift));
+    return c.x < g.dim.x && c.y < g.dim.y && c.z < g.dim.z;
+}
+// The cell of point x: that of voxel floor(x); a NaN component is outside.
+__device__ __forceinline__ bool emitter_cell(const EmitView &g, float3 x, int3 &c) {
+    if (!(x.x == x.x && x.y == x.y && x.z == x.z)) return false;
+    return emitter_voxel_cell(g, f2i(floorf(x.x)), f2i(floorf(x.y)), f2i(floorf(x.z)), c);
+}
+// The list L(c) of cell c: first index into g.list, and its length N.
+__device__ __forceinline__ int emitter_list(const EmitView &g, int3 c, int &N) {
+    const int ci = (c.x * g.dim.y + c.y) * g.dim.z + c.z;
+    const int b = __ldg(g.off + ci);
+    N = __ldg(g.off + ci + 1) - b;
+    return b;
+}
+// The emission rule: an octree hit on voxel (bx, by, bz) of block palette position `block` that the previous hit's sample
+// covered (an emitter whose cell is within Chebyshev distance 1 of that hit's cell c) delivers no emission.
+__device__ __forceinline__ bool emitter_covered(const DScene &s, const EmitView &g, int block, int bx, int by, int bz, int3 c) {
+    const int4 r0 = __ldg(s.block_rec + 2 * block), r1 = __ldg(s.block_rec + 2 * block + 1);
+    if (r0.x != 1 || !((r0.z & 2) || (r1.z & 0xFF))) return false;
+    int3 e;
+    if (!emitter_voxel_cell(g, bx, by, bz, e)) return false;
+    return abs(e.x - c.x) <= 1 && abs(e.y - c.y) <= 1 && abs(e.z - c.z) <= 1;
+}
+// DESIGN §10 steps 2-4 at a hit x with normal n and throughput T, for the non-empty list emit_list[b .. b + N): draws u0..u3
+// and returns whether a shadow ray is traced; if so it runs from x along w up to `limit` and carries the contribution `c`.
+__device__ __forceinline__ bool nee_sample(const DScene &s, const EmitView &g, int b, int N, float3 x, float3 n, float3 T, uint32_t &rng, float3 &c,
+                                           float3 &w, float &limit) {
+    const float u0 = rng_float(rng);
+    const float u1 = rng_float(rng);
+    const float u2 = rng_float(rng);
+    const float u3 = rng_float(rng);
+    const int4 e = __ldg(g.emit + __ldg(g.list + b + min((int)(u0 * (float)N), N - 1)));
+    const float ex = (float)e.x, ey = (float)e.y, ez = (float)e.z;
+    // the faces x lies strictly outside of, in the order -x, +x, -y, +y, -z, +z; 4 bits each: axis * 2 + (1 for the + face)
+    unsigned faces = 0;
+    int f = 0;
+    if (x.x < ex) faces |= 0u << (4 * f++); else if (x.x > (float)(e.x + 1)) faces |= 1u << (4 * f++);
+    if (x.y < ey) faces |= 2u << (4 * f++); else if (x.y > (float)(e.y + 1)) faces |= 3u << (4 * f++);
+    if (x.z < ez) faces |= 4u << (4 * f++); else if (x.z > (float)(e.z + 1)) faces |= 5u << (4 * f++);
+    if (f == 0) return false;
+    const int face = (int)((faces >> (4 * min((int)(u1 * (float)f), f - 1))) & 15u);
+    const int axis = face >> 1, plus = face & 1;
+    // the point and the uv of aabb_full (primitives.h:66-112) at local point (u2, u3) on the face
+    float3 p;
+    float u, v;
+    if (axis == 0) { p = f3((float)(e.x + plus), ey + u2, ez + u3); u = plus ? u3 : 1.0f - u3; v = u2; }
+    else if (axis == 1) { p = f3(ex + u2, (float)(e.y + plus), ez + u3); u = u2; v = plus ? u3 : 1.0f - u3; }
+    else { p = f3(ex + u2, ey + u3, (float)(e.z + plus)); u = plus ? 1.0f - u2 : u2; v = u3; }
+    const int4 r0 = __ldg(s.block_rec + 2 * e.w), r1 = __ldg(s.block_rec + 2 * e.w + 1);
+    const MatOut m = material_eval_core(s, (uint32_t)r0.z, (uint32_t)r0.w, (uint32_t)r1.x, (uint32_t)r1.y, (uint32_t)r1.z, u, v);
+    if (!m.ok) return false;
+    const float3 dv = p - x;
+    const float d2 = dot3(dv, dv);
+    const float dist = sqrtf(d2);
+    w = dv * (1.0f / dist);
+    const float cx = dot3(w, n);
+    if (!(cx > 0.0f)) return false;
+    const float ce = fabsf(axis == 0 ? w.x : (axis == 1 ? w.y : w.z));
+    const float k = ((m.emittance * s.emitter_scale) * ((cx * ce) / d2)) * ((float)(N * f) / CCU_PI_F);
+    c = f3((T.x * (m.color.x * m.color.x)) * k, (T.y * (m.color.y * m.color.y)) * k, (T.z * (m.color.z * m.color.z)) * k);
+    limit = dist - CCU_NEE_DELTA;
+    return true;
 }
 
 }  // namespace ccu

@@ -163,6 +163,8 @@ struct SceneInfo {
     int cell_level = 0, top_log2 = 0, use_wide = 0, air_cell_level = 4, air_top_log2 = 0;
     int atlas_w = 0, atlas_h = 0, atlas_layers = 0;
     int has_specular = 0;   // a material word 5 is not 0: CCU_RENDER_SPECULAR launches the specular kernels
+    int has_emitters = 0;   // the emitter table is not empty: CCU_RENDER_EMITTER_SAMPLING launches the NEE kernels
+    int emit_g0[3] = {0, 0, 0}, emit_dim[3] = {0, 0, 0}, emit_shift = 3;   // emitter grid (EmitView::g0 ...)
     float sky_intensity = 0;
     int sun_host[6] = {0, 0, 0, 0, 0, 0};
     bool have_sun = false, have_atlas = false, have_sky = false;
@@ -195,9 +197,11 @@ struct Scene {
     DevBuf<unsigned> air_top, air_wide, air_bricks;   // march layout (ccu_march.cuh)
     DevBuf<int> world_rec, actor_rec, tris2;          // BVH stage layout (ccu_queue.cuh)
     DevBuf<int> block_rec, mat_rec, quad_rec, aabb_rec;   // 16-byte-vectorised palettes (DScene::block_rec ...)
+    DevBuf<int> emit, emit_off, emit_list;                // emitter table and cell lists (EmitView)
     DevBuf<uchar4> atlas, sky;
     SceneInfo info;
     ccu::DScene view{};   // every field that depends on the committed scene alone (commit, replicate_scene)
+    ccu::EmitView emit_view{};   // the emitter table's launch view (fill_view, with `view`)
 
     // Calls f(a's buffer, b's same buffer) for every device array of a scene (replicate_scene, ccu_scene_device_bytes).
     template <class F>
@@ -206,6 +210,7 @@ struct Scene {
         f(a.top, b.top); f(a.wide, b.wide); f(a.air_top, b.air_top); f(a.air_wide, b.air_wide); f(a.air_bricks, b.air_bricks);
         f(a.world_rec, b.world_rec); f(a.actor_rec, b.actor_rec); f(a.tris2, b.tris2); f(a.block_rec, b.block_rec);
         f(a.mat_rec, b.mat_rec); f(a.quad_rec, b.quad_rec); f(a.aabb_rec, b.aabb_rec); f(a.atlas, b.atlas); f(a.sky, b.sky);
+        f(a.emit, b.emit); f(a.emit_off, b.emit_off); f(a.emit_list, b.emit_list);
     }
 };
 

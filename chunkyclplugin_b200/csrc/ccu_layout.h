@@ -434,4 +434,98 @@ inline PaletteRecs build_palette_recs(const std::vector<int> &bp, const std::vec
     return r;
 }
 
+// ------------------------------------------------------------------------------------------------------
+// emitter table of CCU_RENDER_EMITTER_SAMPLING (DESIGN §10; DScene::emit ...)
+// ------------------------------------------------------------------------------------------------------
+constexpr int EMIT_SHIFT0 = 3;                  // cells of G = 8 voxels to start with
+constexpr long long EMIT_CELL_BUDGET = 1 << 21; // G doubles until the cell box has at most this many cells
+constexpr long long EMIT_MAX = 1 << 18;         // a scene with more emitter voxels gets no table (the flag changes nothing)
+
+struct EmitterGrid {
+    std::vector<int> emit;        // {x, y, z, block} per emitter, sorted by (x, y, z)
+    std::vector<int> off, list;   // CSR cell lists
+    int g0[3] = {0, 0, 0}, dim[3] = {0, 0, 0}, shift = EMIT_SHIFT0;
+};
+
+// An emitter block: a palette position whose fused record (build_palette_recs) is a full cube whose material has textured
+// emittance (flag bit 1) or a non-zero emittance byte.
+inline bool block_emits(const std::vector<int> &block_rec, int b) {
+    if (b < 0 || (size_t)b * 8 + 7 >= block_rec.size()) return false;
+    const int *r = &block_rec[(size_t)b * 8];
+    return r[0] == 1 && ((r[2] & 2) || (r[6] & 0xFF));
+}
+
+inline EmitterGrid build_emitter_grid(const int *tree, size_t n, int depth, const std::vector<int> &block_rec) {
+    EmitterGrid g;
+    if (n == 0 || depth < 0 || depth > 30) return g;
+    struct Leaf { int x, y, z, level, block; };
+    std::vector<Leaf> leaves;
+    long long count = 0;
+    // depth-first over the reference's node array (ClSceneLoader.java:56-59); a malformed pointer ends its branch
+    struct Item { size_t node; int x, y, z, level; };
+    std::vector<Item> stack{{0, 0, 0, 0, depth}};
+    while (!stack.empty()) {
+        const Item it = stack.back();
+        stack.pop_back();
+        const int data = tree[it.node];
+        if (data > 0) {
+            if (it.level == 0 || (size_t)data + 7 >= n) continue;
+            for (int k = 7; k >= 0; k--)
+                stack.push_back({(size_t)data + k, (it.x << 1) | (k >> 2), (it.y << 1) | ((k >> 1) & 1), (it.z << 1) | (k & 1), it.level - 1});
+            continue;
+        }
+        if (data == INT32_MIN || !block_emits(block_rec, -data)) continue;
+        if (it.level > 6) return EmitterGrid{};   // 8^7 voxels alone exceed EMIT_MAX
+        count += 1ll << (3 * it.level);
+        if (count > EMIT_MAX) return EmitterGrid{};
+        leaves.push_back({it.x << it.level, it.y << it.level, it.z << it.level, it.level, -data});
+    }
+    if (leaves.empty()) return g;
+    std::vector<int4> e;
+    e.reserve((size_t)count);
+    for (const Leaf &l : leaves) {
+        const int s = 1 << l.level;
+        for (int x = 0; x < s; x++)
+            for (int y = 0; y < s; y++)
+                for (int z = 0; z < s; z++) e.push_back(make_int4(l.x + x, l.y + y, l.z + z, l.block));
+    }
+    std::sort(e.begin(), e.end(), [](const int4 &a, const int4 &b) {
+        return a.x != b.x ? a.x < b.x : (a.y != b.y ? a.y < b.y : a.z < b.z);
+    });
+    int lo[3] = {INT32_MAX, INT32_MAX, INT32_MAX}, hi[3] = {0, 0, 0};
+    for (const int4 &v : e) {
+        const int c[3] = {v.x, v.y, v.z};
+        for (int a = 0; a < 3; a++) { lo[a] = std::min(lo[a], c[a]); hi[a] = std::max(hi[a], c[a]); }
+    }
+    // the cell box: the emitters' cells and one more cell on every side
+    for (;; g.shift++) {
+        long long cells = 1;
+        for (int a = 0; a < 3; a++) {
+            const int c0 = (lo[a] >> g.shift) - 1, c1 = (hi[a] >> g.shift) + 1;
+            g.g0[a] = c0 * (1 << g.shift);
+            g.dim[a] = c1 - c0 + 1;
+            cells *= g.dim[a];
+        }
+        if (cells <= EMIT_CELL_BUDGET) break;
+    }
+    const size_t n_cells = (size_t)g.dim[0] * g.dim[1] * g.dim[2];
+    g.off.assign(n_cells + 1, 0);
+    auto each_cell = [&](const int4 &v, auto f) {
+        const int cx = (v.x - g.g0[0]) >> g.shift, cy = (v.y - g.g0[1]) >> g.shift, cz = (v.z - g.g0[2]) >> g.shift;
+        for (int dx = -1; dx <= 1; dx++)
+            for (int dy = -1; dy <= 1; dy++)
+                for (int dz = -1; dz <= 1; dz++) f(((size_t)(cx + dx) * g.dim[1] + (size_t)(cy + dy)) * g.dim[2] + (size_t)(cz + dz));
+    };
+    for (const int4 &v : e) each_cell(v, [&](size_t c) { g.off[c + 1]++; });
+    for (size_t c = 0; c < n_cells; c++) g.off[c + 1] += g.off[c];
+    g.list.resize((size_t)g.off[n_cells]);
+    std::vector<int> fill(g.off.begin(), g.off.end() - 1);
+    for (size_t i = 0; i < e.size(); i++) each_cell(e[i], [&](size_t c) { g.list[(size_t)fill[c]++] = (int)i; });
+    g.emit.resize(e.size() * 4);
+    for (size_t i = 0; i < e.size(); i++) {
+        g.emit[4 * i] = e[i].x; g.emit[4 * i + 1] = e[i].y; g.emit[4 * i + 2] = e[i].z; g.emit[4 * i + 3] = e[i].w;
+    }
+    return g;
+}
+
 }  // namespace

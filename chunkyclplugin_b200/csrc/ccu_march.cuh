@@ -190,9 +190,10 @@ __device__ __forceinline__ bool closest_intersect_mode(const DScene &s, float3 o
 }
 
 // one path sample for pixel gid, thread-sequential: rayTracer.cl:40-107 (+ kernel.h:33-98, sky.h:68-93); SPEC adds the specular
-// events of CCU_RENDER_SPECULAR (DESIGN "Beyond the reference: specular materials")
-template <int MODE, bool SPEC>
-__device__ __forceinline__ float3 sample_pixel(const DScene &s, int gid, int seed) {
+// events of CCU_RENDER_SPECULAR (DESIGN "Beyond the reference: specular materials"), NEE the emitter sampling of
+// CCU_RENDER_EMITTER_SAMPLING (DESIGN §10)
+template <int MODE, bool SPEC, bool NEE>
+__device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &g, int gid, int seed) {
     float3 color = f3(0, 0, 0), throughput = f3(1, 1, 1);
     int ray_depth = 0;
     uint32_t rng = (uint32_t)seed + (uint32_t)gid;
@@ -208,12 +209,19 @@ __device__ __forceinline__ float3 sample_pixel(const DScene &s, int gid, int see
     rec.surf.emittance = 0;
     surf_set_spec(rec.surf, 0u);
     HitInfo hi = {-1, 0, 0, 0, 0};
+    bool nee_prev = false;   // NEE: the hit this segment left sampled the list of cell nee_cell
+    int3 nee_cell = make_int3(0, 0, 0);
     for (;;) {
         if (!closest_intersect_mode<MODE>(s, origin, direction, rec, hi)) {
             // miss: emittance = 1, sky (+ sun disc) added through the throughput (rayTracer.cl:95-97, kernel.h:26-31)
             float3 sky = sky_radiance(s, direction);
             color = color + (sky * throughput) * 1.0f;
             break;
+        }
+        bool emits = true;   // NEE: an emitter the previous hit's sample covered delivers no emission here
+        if constexpr (NEE) {
+            emits = !(nee_prev && hi.kind == 1 && emitter_covered(s, g, rec.material, hi.bx, hi.by, hi.bz, nee_cell));
+            nee_prev = false;
         }
         bool specular = false, metal = false;
         float ro = 0;
@@ -222,7 +230,7 @@ __device__ __forceinline__ float3 sample_pixel(const DScene &s, int gid, int see
             // specular event: the emission of applyRayColor, the throughput tinted by a metal only, no sun sample
             const float3 col = f3(rec.surf.color.x, rec.surf.color.y, rec.surf.color.z);
             const float3 tinted = throughput * col;
-            color = color + (col * (rec.surf.emittance * s.emitter_scale)) * tinted;
+            if (emits) color = color + (col * (rec.surf.emittance * s.emitter_scale)) * tinted;
             if (metal) throughput = tinted;
             const float x1 = rng_float(rng);
             const float x2 = rng_float(rng);
@@ -237,7 +245,7 @@ __device__ __forceinline__ float3 sample_pixel(const DScene &s, int gid, int see
         origin = rec.point;
         float3 col = f3(rec.surf.color.x, rec.surf.color.y, rec.surf.color.z);
         throughput = throughput * col;
-        color = color + (col * (rec.surf.emittance * s.emitter_scale)) * throughput;
+        if (emits) color = color + (col * (rec.surf.emittance * s.emitter_scale)) * throughput;
         // sun sampling + shadow ray (sky.h:68-93, rayTracer.cl:101-106)
         if (s.sun_flags & 1) {
             float x1 = rng_float(rng);
@@ -249,6 +257,24 @@ __device__ __forceinline__ float3 sample_pixel(const DScene &s, int gid, int see
             if (!closest_intersect_mode<MODE>(s, origin, d, sh, shi)) {
                 float3 sky = sky_radiance(s, d);
                 color = color + (sky * throughput) * shadow_emittance;
+            }
+        }
+        // emitter sampling (DESIGN §10): only where the bounce below will be traced, and without a draw where L(cell) is empty
+        if constexpr (NEE) {
+            int3 cell;
+            int n_list = 0, first = 0;
+            if (ray_depth + 1 < s.max_depth && emitter_cell(g, origin, cell)) first = emitter_list(g, cell, n_list);
+            if (n_list > 0) {
+                nee_prev = true;
+                nee_cell = cell;
+                float3 c, w;
+                float limit;
+                if (nee_sample(s, g, first, n_list, origin, rec.surf.normal, throughput, rng, c, w, limit)) {
+                    RecordT<SPEC> sh = rec;
+                    sh.distance = limit;
+                    HitInfo shi;
+                    if (!closest_intersect_mode<MODE>(s, origin, w, sh, shi)) color = color + c;
+                }
             }
         }
         // kernel.h:46-98 diffuse bounce

@@ -44,17 +44,18 @@ __global__ void k_sun_setup(const int *sun_words, float *out /* su sv sw radius_
 // Thread-per-pixel path tracer: all passes of the batch in one launch, the running mean of
 // rayTracer.cl:109-112 carried in registers between passes (identical arithmetic, no memory round trip).
 // MODE: 0 = the reference's own node array, 1 = commit-time layouts, 2 = commit-time layouts of a deep world.
-// SPEC: CCU_RENDER_SPECULAR on a scene with specular words (sample_pixel).
-template <int MODE, bool SPEC>
+// SPEC: CCU_RENDER_SPECULAR on a scene with specular words; NEE: CCU_RENDER_EMITTER_SAMPLING on a scene with emitters (sample_pixel).
+template <int MODE, bool SPEC, bool NEE>
 __global__ void __launch_bounds__(128) k_render_mega(const __grid_constant__ DScene s, const int *__restrict__ seeds, int n_passes,
-                                                     int start_spp, float *res, const float *res_prev, int n_pixels) {
+                                                     int start_spp, float *res, const float *res_prev, int n_pixels,
+                                                     const __grid_constant__ EmitView g) {
     stage_tables(s, nullptr);
     for (int gid = blockIdx.x * blockDim.x + threadIdx.x; gid < n_pixels; gid += gridDim.x * blockDim.x) {
         float *px = res + (size_t)gid * 3;
         const float *pp = res_prev + (size_t)gid * 3;    // what the reference's single buffer holds when the window starts
         float3 buf = f3(pp[0], pp[1], pp[2]);
         for (int pass = 0; pass < n_passes; pass++) {
-            float3 col = sample_pixel<MODE, SPEC>(s, gid, __ldg(seeds + pass));
+            float3 col = sample_pixel<MODE, SPEC, NEE>(s, g, gid, __ldg(seeds + pass));
             int spp = start_spp + pass;
             float fs = (float)spp, fs1 = (float)(spp + 1);
             buf.x = (buf.x * fs + col.x) / fs1;
@@ -346,6 +347,11 @@ void fill_view(ccu_host::Scene &sc) {
     s.su = in.su; s.sv = in.sv; s.sw = in.sw; s.sun_radius_cos = in.sun_radius_cos;
     s.sun_flags = in.sun_host[0]; s.sun_tex_size = in.sun_host[1]; s.sun_tex = in.sun_host[2];
     memcpy(&s.sun_intensity, &in.sun_host[3], 4);
+    EmitView &g = sc.emit_view;
+    g.emit = reinterpret_cast<const int4 *>(sc.emit.p); g.off = sc.emit_off.p; g.list = sc.emit_list.p;
+    g.g0 = make_int3(in.emit_g0[0], in.emit_g0[1], in.emit_g0[2]);
+    g.dim = make_int3(in.emit_dim[0], in.emit_dim[1], in.emit_dim[2]);
+    g.shift = in.emit_shift;
 }
 
 // The launch view with this launch's camera, rays, canvas and render params (caller holds c->mu, the scene is committed).
@@ -427,15 +433,21 @@ void dispatch(bool v, F &&f) {
 }
 
 // the wavefront kernel (ccu_queue.cuh) for the scene's entity BVHs and air layout (air_layout_id), with or without specular events
-auto queue_kernel(bool bvh, int lay, bool spec) {
-    decltype(&k_render_queue<false, 0, false>) k = nullptr;
-    dispatch(bvh, [&](auto B) { dispatch<3>(lay, [&](auto L) { dispatch(spec, [&](auto S) { k = k_render_queue<B, L, S>; }); }); });
+auto queue_kernel(bool bvh, int lay, bool spec, bool nee) {
+    decltype(&k_render_queue<false, 0, false, false>) k = nullptr;
+    dispatch(bvh, [&](auto B) {
+        dispatch<3>(lay, [&](auto L) { dispatch(spec, [&](auto S) { dispatch(nee, [&](auto N) { k = k_render_queue<B, L, S, N>; }); }); });
+    });
     return k;
 }
 
 // CCU_RENDER_SPECULAR launches the specular kernels only on a scene that has a specular word: without one they compute exactly
 // what the other kernels compute
 bool specular_launch(const ccu_ctx *c) { return (c->params.flags & CCU_RENDER_SPECULAR) && c->scene.info.has_specular; }
+
+// CCU_RENDER_EMITTER_SAMPLING launches the NEE kernels only on a scene with emitters: without one they draw nothing and compute
+// exactly what the other kernels compute
+bool nee_launch(const ccu_ctx *c) { return (c->params.flags & CCU_RENDER_EMITTER_SAMPLING) && c->scene.info.has_emitters; }
 
 }  // namespace
 
@@ -596,8 +608,9 @@ int ccu_ctx_create(int device_index, ccu_ctx **out) {
     for (Event &ev : c->rays_used) if (e == cudaSuccess) e = ev.create(cudaEventDisableTiming);
     for (bool bvh : {false, true})
         for (bool spec : {false, true})
-            for (int lay = 0; lay < 3 && e == cudaSuccess; lay++)
-                e = cudaFuncSetAttribute(queue_kernel(bvh, lay, spec), cudaFuncAttributeMaxDynamicSharedMemorySize, Q_SMEM_LIMIT);
+            for (bool nee : {false, true})
+                for (int lay = 0; lay < 3 && e == cudaSuccess; lay++)
+                    e = cudaFuncSetAttribute(queue_kernel(bvh, lay, spec, nee), cudaFuncAttributeMaxDynamicSharedMemorySize, Q_SMEM_LIMIT);
     if (e == cudaSuccess) e = c->unorm.alloc(256);
     if (e == cudaSuccess) {
         k_unorm_table<<<1, 256, 0, c->stream>>>(c->unorm.p);
@@ -777,6 +790,20 @@ int ccu_scene_commit(ccu_ctx *c) {
         in.has_specular = 0;
         for (size_t i = 0; i + 7 < pr.mat.size(); i += 8) in.has_specular |= pr.mat[i + 5] != 0;
         for (size_t i = 0; i + 7 < pr.block.size(); i += 8) in.has_specular |= pr.block[i] == 1 && pr.block[i + 7] != 0;
+        // emitter table and cell lists, only when a full cube emits (a scene without one uploads three empty arrays)
+        EmitterGrid eg;
+        bool any = false;
+        for (int b = 0; (size_t)b * 8 < pr.block.size() && !any; b++) any = block_emits(pr.block, b);
+        if (any) {
+            const std::vector<int> &tree = host(ccu_host::OCTREE);
+            eg = build_emitter_grid(tree.data(), tree.size(), in.depth, pr.block);
+        }
+        in.has_emitters = eg.emit.empty() ? 0 : 1;
+        for (int a = 0; a < 3; a++) { in.emit_g0[a] = eg.g0[a]; in.emit_dim[a] = eg.dim[a]; }
+        in.emit_shift = eg.shift;
+        CU(sc.emit.upload(eg.emit.data(), eg.emit.size(), c->stream));
+        CU(sc.emit_off.upload(eg.off.data(), eg.off.size(), c->stream));
+        CU(sc.emit_list.upload(eg.list.data(), eg.list.size(), c->stream));
     }
     // BVH stage layout (pair records + aligned triangle blocks); a scene whose BVHs it cannot hold is rendered by the
     // thread-per-pixel kernel on the reference's own arrays
@@ -899,10 +926,12 @@ int ccu_render_begin(ccu_ctx *c, int32_t width, int32_t height) {
 }
 
 int ccu_render_set_params(ccu_ctx *c, const ccu_render_params *p) {
-    if (!c || !p) return fail(CCU_EINVAL, "ccu_render_set_params: null argument");
+    // the parameters are checked before the context, so that a host can validate them without a device
+    if (!p) return fail(CCU_EINVAL, "ccu_render_set_params: null argument");
     if (p->draw_depth < 0 || p->draw_depth >= (1 << 24) || p->max_depth < 1 || p->max_depth > 255) return fail(CCU_EINVAL, "bad render params");
     if (p->kernel != 0 && p->kernel != 1 && p->kernel != 4) return fail(CCU_EINVAL, "unknown kernel %d (0 auto, 1 thread-per-pixel, 4 wavefront)", p->kernel);
-    if (p->flags & ~(CCU_RENDER_NO_ENTITIES | CCU_RENDER_NO_SUN | CCU_RENDER_SPECULAR)) return fail(CCU_EINVAL, "unknown render flags 0x%x", p->flags);
+    if (p->flags & ~(CCU_RENDER_NO_ENTITIES | CCU_RENDER_NO_SUN | CCU_RENDER_SPECULAR | CCU_RENDER_EMITTER_SAMPLING)) return fail(CCU_EINVAL, "unknown render flags 0x%x", p->flags);
+    if (!c) return fail(CCU_EINVAL, "ccu_render_set_params: null argument");
     std::lock_guard<std::mutex> lk(c->mu);
     c->params = *p;
     return CCU_OK;
@@ -942,6 +971,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
     const bool bvh = !(s.world_bvh_empty && s.actor_bvh_empty);
     const int mode = layout_mode(c);
     const bool spec = specular_launch(c);
+    const bool nee = nee_launch(c);
     float *res = c->accum[c->accum_active].p;
     const float *res_prev = c->window_spp == 0 ? c->window_base : res;
     int kernel = c->params.kernel;
@@ -950,7 +980,10 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
         const int threads = 128, blocks = (n_pixels + threads - 1) / threads;
         dispatch<3>(mode, [&](auto M) {
             dispatch(spec, [&](auto S) {
-                k_render_mega<M, S><<<blocks, threads, 0, c->stream>>>(s, seeds_dev, n_passes, c->window_spp, res, res_prev, n_pixels);
+                dispatch(nee, [&](auto N) {
+                    k_render_mega<M, S, N><<<blocks, threads, 0, c->stream>>>(s, seeds_dev, n_passes, c->window_spp, res, res_prev, n_pixels,
+                                                                        c->scene.emit_view);
+                });
             });
         });
     } else {
@@ -978,7 +1011,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
         // 128 x 128 table (64 KiB) taken from L1 costs more brick / atlas hits than the sky lookups gain (measured: +1.8 % per
         // pass on config 1).  CCU_SKY_SMEM_MAX (bytes, default 16 KiB = 64 x 64 texels) moves the threshold.
         const int sky_texels = c->scene.info.sky_res * c->scene.info.sky_res;
-        const int base_smem = q_smem_bytes(bvh, lay == 0, spec);
+        const int base_smem = q_smem_bytes(bvh, lay == 0, spec, nee);
         const char *sky_env = getenv("CCU_SKY_SMEM_MAX");
         const int sky_max = sky_env ? atoi(sky_env) : 16384;
         const bool sky_smem = sky_texels * 4 <= sky_max && base_smem + sky_texels * 4 <= Q_SMEM_LIMIT;
@@ -990,7 +1023,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
             qp.bvh_deep = c->bvh_deep.p;
         }
         const int smem = base_smem + qp.sky_texels * 4;
-        queue_kernel(bvh, lay, spec)<<<grid, block, smem, c->stream>>>(s, qp);
+        queue_kernel(bvh, lay, spec, nee)<<<grid, block, smem, c->stream>>>(s, qp, c->scene.emit_view);
 #ifdef CCU_Q_STATS
         {
             cudaStreamSynchronize(c->stream);
@@ -1383,6 +1416,27 @@ int ccu_debug_bvh_layout(const int32_t *bvh, int64_t n_bvh, const int32_t *trigs
         if (tris_cap < (int64_t)t.size()) return fail(CCU_EINVAL, "ccu_debug_bvh_layout: tris buffer too small");
         std::copy(t.begin(), t.end(), tris);
     }
+    return CCU_OK;
+}
+
+// Host-only check of the emitter table (no CUDA call): what ccu_scene_commit builds for this octree and these palettes.  info =
+// {has_emitters, g0 x y z, dim x y z, shift, emitters, list words}; emit (4 ints per emitter), off (cells + 1) and list are
+// filled when given, and must then hold what a call without them reported.
+int ccu_debug_emitter_grid(const int32_t *tree, int64_t n_tree, int32_t depth, const int32_t *block_palette, int64_t n_block,
+                           const int32_t *mat_palette, int64_t n_mat, int32_t info[10], int32_t *emit, int32_t *off, int32_t *list) {
+    if (!tree || n_tree < 1 || depth < 0 || depth > 30 || !block_palette || n_block < 0 || !mat_palette || n_mat < 0 || !info)
+        return fail(CCU_EINVAL, "ccu_debug_emitter_grid: bad argument");
+    const PaletteRecs pr = build_palette_recs(std::vector<int>(block_palette, block_palette + n_block),
+                                              std::vector<int>(mat_palette, mat_palette + n_mat), {}, {});
+    const EmitterGrid g = build_emitter_grid(tree, (size_t)n_tree, depth, pr.block);
+    info[0] = g.emit.empty() ? 0 : 1;
+    for (int a = 0; a < 3; a++) { info[1 + a] = g.g0[a]; info[4 + a] = g.dim[a]; }
+    info[7] = g.shift;
+    info[8] = (int)(g.emit.size() / 4);
+    info[9] = (int)g.list.size();
+    if (emit) std::copy(g.emit.begin(), g.emit.end(), emit);
+    if (off) std::copy(g.off.begin(), g.off.end(), off);
+    if (list) std::copy(g.list.begin(), g.list.end(), list);
     return CCU_OK;
 }
 

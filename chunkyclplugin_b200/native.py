@@ -14,7 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 # CHUNKYCU_LIB: load another build of the same library (kernel tuning sweeps build variants next to each other)
 LIB_PATH = os.environ.get("CHUNKYCU_LIB") or os.path.join(_HERE, "libchunkycu.so")
 
-CCU_RENDER_NO_ENTITIES, CCU_RENDER_NO_SUN, CCU_RENDER_SPECULAR = 1, 2, 4
+CCU_RENDER_NO_ENTITIES, CCU_RENDER_NO_SUN, CCU_RENDER_SPECULAR, CCU_RENDER_EMITTER_SAMPLING = 1, 2, 4, 8
 CCU_UNIQUE_ID_BYTES = 128
 
 CCU_OK, CCU_ENODEVICE, CCU_EINVAL, CCU_ECUDA, CCU_ENOMEM, CCU_ESTATE = 0, -1, -2, -3, -4, -5
@@ -85,6 +85,7 @@ SYMBOLS = {
     "ccu_bench_gather": (C.c_int, [_vp, _i64, _i32, C.POINTER(_f), C.POINTER(_f)]),
     "ccu_debug_layout_lookup": (C.c_int, [_vp, _i64, _i32, _vp, _i64, _vp, _vp, _vp, _vp]),
     "ccu_debug_bvh_layout": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _i64, _vp, _i64, C.POINTER(_i64), C.POINTER(_i64), _pi32, _pi32]),
+    "ccu_debug_emitter_grid": (C.c_int, [_vp, _i64, _i32, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp]),
     # multi-GPU
     "ccu_group_create": (C.c_int, [_vp, _i32, C.POINTER(_vp)]),
     "ccu_group_unique_id": (C.c_int, [_vp]),
@@ -176,6 +177,24 @@ def debug_bvh_layout(bvh: np.ndarray, trigs: np.ndarray):
     check(lib.ccu_debug_bvh_layout(_ptr(bvh), bvh.size, _ptr(trigs), trigs.size, _ptr(rec), rec.size, _ptr(tris), tris.size,
                                    C.byref(nr), C.byref(nt), C.byref(root), C.byref(ok)))
     return rec[:nr.value].reshape(-1, 16), tris[:nt.value], root.value, bool(ok.value)
+
+
+def debug_emitter_grid(tree: np.ndarray, depth: int, block_palette: np.ndarray, mat_palette: np.ndarray):
+    """The emitter table of CCU_RENDER_EMITTER_SAMPLING the library builds at commit (host only).  Returns a dict:
+    has_emitters, g0 / dim (int[3]: grid origin in voxels, size in cells), shift (log2 of the cell edge), emit (int32[n, 4]:
+    x, y, z, block palette position), off (int32[cells + 1]) and list (int32[...])."""
+    tree, bp, mp = (np.ascontiguousarray(a, dtype=np.int32) for a in (tree, block_palette, mat_palette))
+    info = np.zeros(10, dtype=np.int32)
+    lib = load()
+    args = (_ptr(tree), tree.size, depth, _ptr(bp), bp.size, _ptr(mp), mp.size, _ptr(info))
+    check(lib.ccu_debug_emitter_grid(*args, None, None, None))
+    cells = int(np.prod(info[4:7].astype(np.int64)))
+    emit = np.zeros(max(int(info[8]) * 4, 1), dtype=np.int32)
+    off = np.zeros(cells + 1, dtype=np.int32)
+    lst = np.zeros(max(int(info[9]), 1), dtype=np.int32)
+    check(lib.ccu_debug_emitter_grid(*args, _ptr(emit), _ptr(off), _ptr(lst)))
+    return {"has_emitters": bool(info[0]), "g0": info[1:4].copy(), "dim": info[4:7].copy(), "shift": int(info[7]),
+            "emit": emit[:info[8] * 4].reshape(-1, 4), "off": off if info[0] else off[:0], "list": lst[:info[9]]}
 
 
 def device_count() -> int:

@@ -58,6 +58,16 @@ typedef struct ccu_render_params {
  * only for a metal.  A material whose word 5 is 0 shades as without the flag.  DESIGN.md "Beyond the reference: specular
  * materials" holds the exact contract. */
 #define CCU_RENDER_SPECULAR 4
+/* Emitter sampling (next-event estimation; beyond the reference, which finds a block emitter only when a diffuse bounce hits
+ * it): at every diffuse path-segment hit whose bounce will be traced, one full-cube emitter voxel near the hit (the emitter
+ * list of its grid cell) is sampled with a point on one of its faces facing the hit, and a shadow ray delivers its light;
+ * the bounce then leaves out the emission of an emitter that list covered.  On flat-coloured emitters the image's
+ * expectation is unchanged.  On textured ones (colour or emittance from the atlas) it is not exactly: the sample reads the
+ * texel at the sampled point, while the reference's full-cube block test reads a texel shifted by its marched-position quirk
+ * (SURVEY Q2), so the two weight the texture differently.  Quads, AABB models and triangles keep the reference's behaviour.
+ * A scene without full-cube emitters renders exactly as without the flag.  Both render kernels implement it.  DESIGN.md §10
+ * holds the exact contract. */
+#define CCU_RENDER_EMITTER_SAMPLING 8
 
 /* ---- device enumeration: RendererInstance.java:39-75,123-157 (clGetPlatformIDs/clGetDeviceIDs/clGetDeviceInfo),
  *      used by the GPU selector UI (ui/GpuSelector.java:24-87) -------------------------------------------------- */
@@ -174,6 +184,14 @@ int ccu_debug_layout_lookup(const int32_t *tree, int64_t n, int32_t depth, const
  * the reference's traversal stack, bvh.h:38).  Used by the CPU test-suite. */
 int ccu_debug_bvh_layout(const int32_t *bvh, int64_t n_bvh, const int32_t *trigs, int64_t n_trigs, int32_t *rec, int64_t rec_cap,
                          int32_t *tris, int64_t tris_cap, int64_t *rec_words, int64_t *tris_words, int32_t *root, int32_t *ok);
+
+/* Test support, host only: the emitter table of CCU_RENDER_EMITTER_SAMPLING that ccu_scene_commit builds from the reference's
+ * octree node array and the block / material palettes (DESIGN.md §10).  info = {has_emitters, grid origin x y z (voxels), grid
+ * size x y z (cells), log2 of the cell edge, emitters, list words}; emit (4 ints per emitter: x, y, z, block palette position,
+ * sorted by x, y, z), off (cells + 1 offsets into list) and list may be NULL (sizes only) and must otherwise hold those sizes.
+ * Used by the CPU test-suite. */
+int ccu_debug_emitter_grid(const int32_t *tree, int64_t n_tree, int32_t depth, const int32_t *block_palette, int64_t n_block,
+                           const int32_t *mat_palette, int64_t n_mat, int32_t info[10], int32_t *emit, int32_t *off, int32_t *list);
 
 /* ---- multi-GPU: samples-per-pixel split over the GPUs of one box (SURVEY.md 8e) -------------------------------------------
  * The reference is one JVM and one device (RendererInstance.java:81-101).  A group is N contexts, each holding a full scene

@@ -1,5 +1,6 @@
 /*
- * specular_oracle.c - CPU restatement of CCU_RENDER_SPECULAR (DESIGN.md section 9).  TEST INFRASTRUCTURE ONLY.
+ * specular_oracle.c - CPU restatement of CCU_RENDER_SPECULAR (DESIGN.md section 9) and CCU_RENDER_EMITTER_SAMPLING
+ * (section 10).  TEST INFRASTRUCTURE ONLY.
  *
  * The reference has no specular path, so there is nothing of it to pin this file against: DESIGN.md section 9 is the contract,
  * this file restates it, and the tests hold this restatement and the CUDA kernels to each other bit for bit (plus analytic and
@@ -10,6 +11,8 @@
  * Restated here are only the functions whose record must also carry word 5 of the material the surface's colour came from
  * (block test, octree march, BVH walk, closestIntersect: the oracle's IntersectionRecord has no such field) and the path
  * loop with the specular event.  Each is the oracle function of the same name plus that word, operation for operation.
+ * The octree march also reports the hit voxel, which the emission rule of emitter sampling needs.  The path loop knows
+ * both flags; the emitter table it samples is built by the Python side of this package from the packed arrays.
  */
 #include "../oracle/chunky_oracle.c"
 
@@ -76,7 +79,7 @@ static float intersect_block_w5(const Ctx *c, int block, int bx, int by, int bz,
 }
 
 /* octree_intersect (octree.h:41-109) */
-static int octree_intersect_w5(const Ctx *c, const Path *ray, Record *rec, uint32_t *w5) {
+static int octree_intersect_w5(const Ctx *c, const Path *ray, Record *rec, uint32_t *w5, int vox[3]) {
     const OracleScene *s = c->sc;
     const int32_t *tree = s->octree;
     int depth = s->octree_depth;
@@ -118,6 +121,7 @@ static int octree_intersect_w5(const Ctx *c, const Path *ray, Record *rec, uint3
                 rec->material = data;
                 rec->hit_node = node;
                 rec->hit_kind = 1;
+                vox[0] = bx; vox[1] = by; vox[2] = bz;
                 return 1;
             }
         }
@@ -192,10 +196,10 @@ static int bvh_intersect_w5(const Ctx *c, const int32_t *bvh, const Path *ray, R
 }
 
 /* closest_intersect (kernel.h:14-24) */
-static int closest_intersect_w5(const Ctx *c, const Path *ray, Record *rec, uint32_t *w5) {
+static int closest_intersect_w5(const Ctx *c, const Path *ray, Record *rec, uint32_t *w5, int vox[3]) {
     int hit = 0;
     c->cnt->rays++;
-    hit |= octree_intersect_w5(c, ray, rec, w5);
+    hit |= octree_intersect_w5(c, ray, rec, w5, vox);
     hit |= bvh_intersect_w5(c, c->sc->world_bvh, ray, rec, w5, 2);
     hit |= bvh_intersect_w5(c, c->sc->actor_bvh, ray, rec, w5, 3);
     if (hit) rec->point = vadd(ray->origin, vscale(ray->direction, rec->distance - OFFSET));
@@ -206,7 +210,7 @@ static int closest_intersect_w5(const Ctx *c, const Path *ray, Record *rec, uint
  * draws; on a specular event the emission of applyRayColor, the throughput tinted only by a metal, no sun sample, and the
  * mirror direction blended towards nextPath's cosine-weighted one by the roughness.  Returns 0 for a diffuse event (nothing
  * done), else 1 with *more = whether the path continues. */
-static int specular_event(const Ctx *c, Path *p, Record *rec, uint32_t w, uint32_t *state, int *more) {
+static int specular_event(const Ctx *c, Path *p, Record *rec, uint32_t w, uint32_t *state, int *more, int emits) {
     float sp = (float)(w & 0xFF) / 255.0f, me = (float)((w >> 8) & 0xFF) / 255.0f, ro = (float)((w >> 16) & 0xFF) / 255.0f;
     int metal = 0, spec = 0;
     if (me > 0) metal = rng_float(state) < me;
@@ -214,7 +218,7 @@ static int specular_event(const Ctx *c, Path *p, Record *rec, uint32_t w, uint32
     if (!metal && !spec) return 0;
     v3 col = V(rec->color[0], rec->color[1], rec->color[2]);
     v3 tinted = vmul(p->throughput, col);
-    p->pix_color = vadd(p->pix_color, vmul(vscale(col, rec->emittance * c->sc->emitter_scale), tinted));
+    if (emits) p->pix_color = vadd(p->pix_color, vmul(vscale(col, rec->emittance * c->sc->emitter_scale), tinted));
     if (metal) p->throughput = tinted;
     v3 d = p->direction, n = rec->normal;
     v3 r = vnormalize(vsub(d, vscale(n, 2.0f * vdot(d, n))));
@@ -228,11 +232,91 @@ static int specular_event(const Ctx *c, Path *p, Record *rec, uint32_t w, uint32
     return 1;
 }
 
-/* one path sample: rayTracer.cl:40-107 with the specular events */
-static v3 sample_pixel_specular(const Ctx *c, int gid, int32_t seed) {
+/* ---- emitter sampling (DESIGN.md section 10) ---- */
+#define NEE_DELTA (8.0f * OFFSET)
+
+typedef struct {
+    const int32_t *emit;   /* {x, y, z, block} per emitter, sorted by (x, y, z) */
+    const int32_t *off;    /* cell lists in CSR form */
+    const int32_t *list;
+    int32_t g0[3], dim[3], shift;
+} EmitterGrid;
+
+static int voxel_cell(const EmitterGrid *g, int vx, int vy, int vz, int cl[3]) {
+    int64_t d[3] = {(int64_t)vx - g->g0[0], (int64_t)vy - g->g0[1], (int64_t)vz - g->g0[2]};
+    for (int a = 0; a < 3; a++) {
+        if (d[a] < 0) return 0;
+        cl[a] = (int)(d[a] >> g->shift);
+    }
+    return cl[0] < g->dim[0] && cl[1] < g->dim[1] && cl[2] < g->dim[2];
+}
+
+static int point_cell(const EmitterGrid *g, v3 x, int cl[3]) {
+    if (x.x != x.x || x.y != x.y || x.z != x.z) return 0;
+    int vx, vy, vz;
+    floor3i(x, &vx, &vy, &vz);
+    return voxel_cell(g, vx, vy, vz, cl);
+}
+
+/* the emission rule: an octree hit on an emitter voxel whose cell is within Chebyshev distance 1 of the sampled cell */
+static int emitter_covered(const Ctx *c, const EmitterGrid *g, int block, const int vox[3], const int cell[3]) {
+    const int32_t *bp = c->sc->block_palette, *mp = c->sc->mat_palette;
+    if (bp[block] != 1) return 0;
+    int ptr = bp[block + 1];
+    if (!((mp[ptr] & 2) || (mp[ptr + 4] & 0xFF))) return 0;
+    int e[3];
+    if (!voxel_cell(g, vox[0], vox[1], vox[2], e)) return 0;
+    return abs(e[0] - cell[0]) <= 1 && abs(e[1] - cell[1]) <= 1 && abs(e[2] - cell[2]) <= 1;
+}
+
+/* steps 2-4: the four draws, the emitter, face and point, the material at the point and the contribution; returns 0 when
+ * no shadow ray is traced */
+static int nee_sample(const Ctx *c, const EmitterGrid *g, int b, int n, v3 x, v3 normal, v3 T, uint32_t *state, v3 *out, v3 *w,
+                      float *limit) {
+    float u0 = rng_float(state);
+    float u1 = rng_float(state);
+    float u2 = rng_float(state);
+    float u3 = rng_float(state);
+    int i = (int)(u0 * (float)n);
+    if (i > n - 1) i = n - 1;
+    const int32_t *e = g->emit + 4 * (size_t)g->list[b + i];
+    float ex = (float)e[0], ey = (float)e[1], ez = (float)e[2];
+    int faces[3], f = 0;
+    if (x.x < ex) faces[f++] = 0; else if (x.x > (float)(e[0] + 1)) faces[f++] = 1;
+    if (x.y < ey) faces[f++] = 2; else if (x.y > (float)(e[1] + 1)) faces[f++] = 3;
+    if (x.z < ez) faces[f++] = 4; else if (x.z > (float)(e[2] + 1)) faces[f++] = 5;
+    if (f == 0) return 0;
+    int k = (int)(u1 * (float)f);
+    if (k > f - 1) k = f - 1;
+    int axis = faces[k] >> 1, plus = faces[k] & 1;
+    v3 p;
+    float u, v;
+    if (axis == 0) { p = V((float)(e[0] + plus), ey + u2, ez + u3); u = plus ? u3 : 1.0f - u3; v = u2; }
+    else if (axis == 1) { p = V(ex + u2, (float)(e[1] + plus), ez + u3); u = u2; v = plus ? u3 : 1.0f - u3; }
+    else { p = V(ex + u2, ey + u3, (float)(e[2] + plus)); u = plus ? 1.0f - u2 : u2; v = u3; }
+    Record m;
+    record_new(&m);
+    if (!material_sample(c, c->sc->block_palette[e[3] + 1], &m, u, v)) return 0;
+    v3 dv = vsub(p, x);
+    float d2 = vdot(dv, dv);
+    float dist = sqrtf(d2);
+    *w = vscale(dv, 1.0f / dist);
+    float cx = vdot(*w, normal);
+    if (!(cx > 0.0f)) return 0;
+    float ce = fabsf(axis == 0 ? w->x : (axis == 1 ? w->y : w->z));
+    float kk = ((m.emittance * c->sc->emitter_scale) * ((cx * ce) / d2)) * ((float)(n * f) / PI_F);
+    *out = V((T.x * (m.color[0] * m.color[0])) * kk, (T.y * (m.color[1] * m.color[1])) * kk, (T.z * (m.color[2] * m.color[2])) * kk);
+    *limit = dist - NEE_DELTA;
+    return 1;
+}
+
+/* one path sample: rayTracer.cl:40-107 with the specular events (spec) and emitter sampling (g != NULL) */
+static v3 sample_pixel_ext(const Ctx *c, int gid, int32_t seed, int spec, const EmitterGrid *g) {
     Path p;
     Record rec;
     uint32_t w5 = 0;
+    int vox[3] = {0, 0, 0};
+    int nee_prev = 0, nee_cell[3] = {0, 0, 0};
     p.pix_color = V(0, 0, 0);
     p.throughput = V(1, 1, 1);
     p.ray_depth = 0;
@@ -243,30 +327,57 @@ static v3 sample_pixel_specular(const Ctx *c, int gid, int32_t seed) {
     c->cnt->samples++;
     for (;;) {
         c->cnt->segments++;
-        if (!closest_intersect_w5(c, &p, &rec, &w5)) {
+        if (!closest_intersect_w5(c, &p, &rec, &w5, vox)) {
             rec.emittance = 1;
             intersect_sky(c, &p, &rec);
             break;
         }
+        int emits = 1;
+        if (g) {
+            emits = !(nee_prev && rec.hit_kind == 1 && emitter_covered(c, g, rec.material, vox, nee_cell));
+            nee_prev = 0;
+        }
         int more;
-        if (specular_event(c, &p, &rec, w5, &state, &more)) {
+        if (spec && specular_event(c, &p, &rec, w5, &state, &more, emits)) {
             if (!more) break;
             continue;
         }
-        apply_ray_color(&p, &rec, c->sc->emitter_scale);
+        if (emits) {
+            apply_ray_color(&p, &rec, c->sc->emitter_scale);
+        } else {   /* applyRayColor without its emission term */
+            p.origin = rec.point;
+            p.throughput = vmul(p.throughput, V(rec.color[0], rec.color[1], rec.color[2]));
+        }
         if (sun_sample_direction(c, &p, &rec, &state)) {
             Record s = rec; /* IntersectionRecord_copy keeps distance: SURVEY Q4 */
             s.point = rec.normal;
             if (!closest_intersect(c, &p, &s)) intersect_sky(c, &p, &s);   /* the shadow ray needs no word 5 */
+        }
+        int cell[3];
+        if (g && p.ray_depth + 1 < c->sc->max_depth && point_cell(g, p.origin, cell)) {
+            int ci = (cell[0] * g->dim[1] + cell[1]) * g->dim[2] + cell[2];
+            int b = g->off[ci], n = g->off[ci + 1] - b;
+            if (n > 0) {
+                v3 contrib, w;
+                float limit;
+                nee_prev = 1;
+                memcpy(nee_cell, cell, sizeof cell);
+                if (nee_sample(c, g, b, n, p.origin, rec.normal, p.throughput, &state, &contrib, &w, &limit)) {
+                    Path q = p;
+                    q.direction = w;
+                    Record s = rec;
+                    s.distance = limit;
+                    if (!closest_intersect(c, &q, &s)) p.pix_color = vadd(p.pix_color, contrib);
+                }
+            }
         }
         if (!next_path(c, &p, &rec, &state, c->sc->max_depth)) break;
     }
     return p.pix_color;
 }
 
-/* oracle_render with the specular events (same arguments, same running mean) */
-int specular_render(const OracleScene *s, const int32_t *seeds, int n_passes, int start_spp, float *res, const int32_t *gids,
-                    int64_t n_gids, int nthreads, OracleCounters *out_counters) {
+static int render_ext(const OracleScene *s, const int32_t *seeds, int n_passes, int start_spp, float *res, const int32_t *gids,
+                      int64_t n_gids, int nthreads, OracleCounters *out_counters, int spec, const EmitterGrid *g) {
     int64_t n = gids ? n_gids : (int64_t)s->width * s->height;
     OracleCounters total;
     memset(&total, 0, sizeof total);
@@ -285,7 +396,7 @@ int specular_render(const OracleScene *s, const int32_t *seeds, int n_passes, in
             float *px = res + (size_t)gid * 3;
             v3 buf = V(px[0], px[1], px[2]);
             for (int pass = 0; pass < n_passes; pass++) {
-                v3 col = sample_pixel_specular(&c, gid, seeds[pass]);
+                v3 col = sample_pixel_ext(&c, gid, seeds[pass], spec, g);
                 int spp = start_spp + pass;
                 buf.x = (buf.x * (float)spp + col.x) / (float)(spp + 1);
                 buf.y = (buf.y * (float)spp + col.y) / (float)(spp + 1);
@@ -299,3 +410,17 @@ int specular_render(const OracleScene *s, const int32_t *seeds, int n_passes, in
     if (out_counters) *out_counters = total;
     return 0;
 }
+
+/* oracle_render with the specular events (same arguments, same running mean) */
+int specular_render(const OracleScene *s, const int32_t *seeds, int n_passes, int start_spp, float *res, const int32_t *gids,
+                    int64_t n_gids, int nthreads, OracleCounters *out_counters) {
+    return render_ext(s, seeds, n_passes, start_spp, res, gids, n_gids, nthreads, out_counters, 1, NULL);
+}
+
+/* oracle_render with CCU_RENDER_SPECULAR (spec) and CCU_RENDER_EMITTER_SAMPLING (g != NULL) */
+int flags_render(const OracleScene *s, const int32_t *seeds, int n_passes, int start_spp, float *res, const int32_t *gids,
+                 int64_t n_gids, int nthreads, OracleCounters *out_counters, int spec, const EmitterGrid *g) {
+    return render_ext(s, seeds, n_passes, start_spp, res, gids, n_gids, nthreads, out_counters, spec, g);
+}
+
+int emitter_grid_struct_size(void) { return (int)sizeof(EmitterGrid); }
