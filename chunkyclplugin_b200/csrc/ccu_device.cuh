@@ -919,8 +919,59 @@ __device__ __forceinline__ bool emitter_covered(const DScene &s, const EmitView 
     if (!emitter_voxel_cell(g, bx, by, bz, e)) return false;
     return abs(e.x - c.x) <= 1 && abs(e.y - c.y) <= 1 && abs(e.z - c.z) <= 1;
 }
+// The emitter sampler a kernel is built with: none, the area sampler of CCU_RENDER_EMITTER_SAMPLING (DESIGN §10), or that
+// sampler with the near field of CCU_RENDER_EMITTER_NEAR_FIELD (DESIGN §11).
+enum NeeKind : int { NEE_NONE = 0, NEE_AREA = 1, NEE_NEAR = 2 };
+#define CCU_NEE_RHO2 0.015625f   // DESIGN §11: an emitter is near when its box distance² is below rho² = (1/8)²
+
+// DESIGN §11 step 4 at a hit x with normal n for emitter e (palette position e.w) from a list of N, whose box distance² is
+// below rho²: a cosine-weighted direction (nextPath's, from u2 and u3), scored when it enters the emitter's box through a face
+// x lies outside of.
+__device__ __forceinline__ bool nee_near(const DScene &s, int4 e, int N, float3 x, float3 n, float3 T, float u2, float u3, float3 &c,
+                                         float3 &w, float &limit) {
+    w = diffuse_direction(n, u2, u3);
+    const float3 inv = f3(1.0f / w.x, 1.0f / w.y, 1.0f / w.z);
+    const float ex = (float)e.x, ey = (float)e.y, ez = (float)e.z;
+    const float ax0 = (ex - x.x) * inv.x, ax1 = ((float)(e.x + 1) - x.x) * inv.x;
+    const float ay0 = (ey - x.y) * inv.y, ay1 = ((float)(e.y + 1) - x.y) * inv.y;
+    const float az0 = (ez - x.z) * inv.z, az1 = ((float)(e.z + 1) - x.z) * inv.z;
+    if (!(ax0 == ax0 && ax1 == ax1 && ay0 == ay0 && ay1 == ay1 && az0 == az0 && az1 == az1)) return false;
+    // entry: the largest of the near ends (lowest axis on a tie); exit: the smallest of the far ends
+    float tn = ax0 < ax1 ? ax0 : ax1, tf = ax0 < ax1 ? ax1 : ax0;
+    int axis = 0;
+    const float ly = ay0 < ay1 ? ay0 : ay1, hy = ay0 < ay1 ? ay1 : ay0;
+    const float lz = az0 < az1 ? az0 : az1, hz = az0 < az1 ? az1 : az0;
+    if (ly > tn) { tn = ly; axis = 1; }
+    if (lz > tn) { tn = lz; axis = 2; }
+    if (hy < tf) tf = hy;
+    if (hz < tf) tf = hz;
+    if (!(tn <= tf && tn > 0.0f)) return false;
+    // the entry face must be one x lies strictly outside of
+    const float xa = axis == 0 ? x.x : (axis == 1 ? x.y : x.z), wa = axis == 0 ? w.x : (axis == 1 ? w.y : w.z);
+    const int ea = axis == 0 ? e.x : (axis == 1 ? e.y : e.z);
+    const int plus = wa < 0.0f ? 1 : 0;
+    if (!(plus ? xa > (float)(ea + 1) : xa < (float)ea)) return false;
+    // the entry point's in-face coordinates take the places of (u2, u3) in the uv of aabb_full (DESIGN §10 step 3)
+    const float3 p = x + w * tn;
+    const float px = fminf(fmaxf(p.x - ex, 0.0f), 1.0f), py = fminf(fmaxf(p.y - ey, 0.0f), 1.0f), pz = fminf(fmaxf(p.z - ez, 0.0f), 1.0f);
+    float u, v;
+    if (axis == 0) { u = plus ? pz : 1.0f - pz; v = py; }
+    else if (axis == 1) { u = px; v = plus ? pz : 1.0f - pz; }
+    else { u = plus ? 1.0f - px : px; v = py; }
+    const int4 r0 = __ldg(s.block_rec + 2 * e.w), r1 = __ldg(s.block_rec + 2 * e.w + 1);
+    const MatOut m = material_eval_core(s, (uint32_t)r0.z, (uint32_t)r0.w, (uint32_t)r1.x, (uint32_t)r1.y, (uint32_t)r1.z, u, v);
+    if (!m.ok) return false;
+    // the cosine and 1/pi of the estimator cancel against the direction's density cx / pi
+    const float k = (m.emittance * s.emitter_scale) * (float)N;
+    c = f3((T.x * (m.color.x * m.color.x)) * k, (T.y * (m.color.y * m.color.y)) * k, (T.z * (m.color.z * m.color.z)) * k);
+    limit = tn - CCU_NEE_DELTA;
+    return true;
+}
+
 // DESIGN §10 steps 2-4 at a hit x with normal n and throughput T, for the non-empty list emit_list[b .. b + N): draws u0..u3
 // and returns whether a shadow ray is traced; if so it runs from x along w up to `limit` and carries the contribution `c`.
+// KIND == NEE_NEAR: an emitter nearer than rho is sampled by direction instead (DESIGN §11).
+template <int KIND>
 __device__ __forceinline__ bool nee_sample(const DScene &s, const EmitView &g, int b, int N, float3 x, float3 n, float3 T, uint32_t &rng, float3 &c,
                                            float3 &w, float &limit) {
     const float u0 = rng_float(rng);
@@ -936,6 +987,13 @@ __device__ __forceinline__ bool nee_sample(const DScene &s, const EmitView &g, i
     if (x.y < ey) faces |= 2u << (4 * f++); else if (x.y > (float)(e.y + 1)) faces |= 3u << (4 * f++);
     if (x.z < ez) faces |= 4u << (4 * f++); else if (x.z > (float)(e.z + 1)) faces |= 5u << (4 * f++);
     if (f == 0) return false;
+    if constexpr (KIND == NEE_NEAR) {
+        // box distance² of x to the emitter: o_a is x's distance to the slab [e_a, e_a + 1] on axis a
+        const float ox = x.x < ex ? ex - x.x : (x.x > (float)(e.x + 1) ? x.x - (float)(e.x + 1) : 0.0f);
+        const float oy = x.y < ey ? ey - x.y : (x.y > (float)(e.y + 1) ? x.y - (float)(e.y + 1) : 0.0f);
+        const float oz = x.z < ez ? ez - x.z : (x.z > (float)(e.z + 1) ? x.z - (float)(e.z + 1) : 0.0f);
+        if ((ox * ox + oy * oy) + oz * oz < CCU_NEE_RHO2) return nee_near(s, e, N, x, n, T, u2, u3, c, w, limit);
+    }
     const int face = (int)((faces >> (4 * min((int)(u1 * (float)f), f - 1))) & 15u);
     const int axis = face >> 1, plus = face & 1;
     // the point and the uv of aabb_full (primitives.h:66-112) at local point (u2, u3) on the face

@@ -190,9 +190,9 @@ __device__ __forceinline__ bool closest_intersect_mode(const DScene &s, float3 o
 }
 
 // one path sample for pixel gid, thread-sequential: rayTracer.cl:40-107 (+ kernel.h:33-98, sky.h:68-93); SPEC adds the specular
-// events of CCU_RENDER_SPECULAR (DESIGN "Beyond the reference: specular materials"), NEE the emitter sampling of
-// CCU_RENDER_EMITTER_SAMPLING (DESIGN §10)
-template <int MODE, bool SPEC, bool NEE>
+// events of CCU_RENDER_SPECULAR (DESIGN "Beyond the reference: specular materials"), NEE the emitter sampler (NeeKind) of
+// CCU_RENDER_EMITTER_SAMPLING (DESIGN §10) and CCU_RENDER_EMITTER_NEAR_FIELD (§11)
+template <int MODE, bool SPEC, int NEE>
 __device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &g, int gid, int seed) {
     float3 color = f3(0, 0, 0), throughput = f3(1, 1, 1);
     int ray_depth = 0;
@@ -269,7 +269,7 @@ __device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &
                 nee_cell = cell;
                 float3 c, w;
                 float limit;
-                if (nee_sample(s, g, first, n_list, origin, rec.surf.normal, throughput, rng, c, w, limit)) {
+                if (nee_sample<NEE>(s, g, first, n_list, origin, rec.surf.normal, throughput, rng, c, w, limit)) {
                     RecordT<SPEC> sh = rec;
                     sh.distance = limit;
                     HitInfo shi;

@@ -303,10 +303,10 @@ __device__ __forceinline__ void q_stage_march(const DScene &s, const unsigned *_
 // (kernel.h:26-31), otherwise the surface response (kernel.h:33-44) and the sun sampling ray (sky.h:68-93); when the ray
 // was the shadow ray (or sun sampling is off) the diffuse bounce (nextPath, kernel.h:46-98) follows right away.
 // SPEC: a specular event at the hit (DESIGN "Beyond the reference: specular materials") bounces right away, without a sun sample.
-// NEE: after the sun sample (or in its place) and before the bounce, the emitter sample of DESIGN §10 with its own shadow ray
-// (NFI: index of the two NEE fields); `covered`: the hit is an emitter the previous hit's sample covered, whose emission is
+// NEE (a NeeKind): after the sun sample (or in its place) and before the bounce, the emitter sample of DESIGN §10 (§11 for
+// NEE_NEAR) with its own shadow ray (NFI: index of the two NEE fields); `covered`: the hit is an emitter the previous hit's sample covered, whose emission is
 // left out.
-template <bool SPEC, bool NEE, int NFI>
+template <bool SPEC, int NEE, int NFI>
 __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint32_t *F, unsigned *mask, int lane, int row, float3 o,
                                         float3 d, float distance, bool ray_hit, const SurfT<SPEC> &hit, bool covered) {
     const int slot = row * 32 + lane;
@@ -395,7 +395,7 @@ __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint
                 uint32_t rng = QU(QF_RNG);
                 float3 c, w;
                 float limit;
-                const bool ray = nee_sample(s, g, first, n_list, from, normal, f3(QFL(QF_THRX), QFL(QF_THRY), QFL(QF_THRZ)), rng, c, w, limit);
+                const bool ray = nee_sample<NEE>(s, g, first, n_list, from, normal, f3(QFL(QF_THRX), QFL(QF_THRY), QFL(QF_THRZ)), rng, c, w, limit);
                 QU(QF_RNG) = rng;
                 if (ray) {
                     QFL(QF_SNX) = normal.x; QFL(QF_SNY) = normal.y; QFL(QF_SNZ) = normal.z;
@@ -460,7 +460,7 @@ __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint
 
 // NEE: whether an octree hit on voxel c of block `data` is an emitter the sample of the previous hit covered (a path-segment
 // ray whose meta carries QM_NEE_PREV; the cell waits in QF_SN*)
-template <bool NEE>
+template <int NEE>
 __device__ __forceinline__ bool q_covered(const DScene &s, const EmitView &g, const uint32_t *F, int slot, uint32_t meta, int data, const Cell &c) {
     if (!NEE || (meta & (QM_SHADOW | QM_NEE_RAY)) || !(meta & QM_NEE_PREV)) return false;
     const int3 cell = make_int3((int)F[QF_SNX * Q_SLOTS + slot], (int)F[QF_SNY * Q_SLOTS + slot], (int)F[QF_SNZ * Q_SLOTS + slot]);
@@ -469,7 +469,7 @@ __device__ __forceinline__ bool q_covered(const DScene &s, const EmitView &g, co
 
 // BLOCK (kind_block = true) and EXIT (false): the octree part of closestIntersect (kernel.h:14-16) is finished here;
 // without BVHs the ray is shaded right away, with BVHs it goes to the BVH stage.  kind_block is warp-uniform.
-template <bool HAS_BVH, bool SPEC, bool NEE>
+template <bool HAS_BVH, bool SPEC, int NEE>
 __device__ __forceinline__ bool q_stage_resolve(const DScene &s, const EmitView &g, uint32_t *F, unsigned *mask, int lane, const bool kind_block,
                                                 int min_lanes) {
     const int row = q_pop_batch(mask, kind_block ? QS_BLOCK : QS_EXIT, lane, min_lanes);
@@ -535,7 +535,7 @@ __device__ __forceinline__ bool q_stage_resolve(const DScene &s, const EmitView 
 }
 
 // SHADE (HAS_BVH kernels): closestIntersect is complete (kernel.h:17-22)
-template <bool SPEC, bool NEE>
+template <bool SPEC, int NEE>
 __device__ __forceinline__ bool q_stage_shade(const DScene &s, const EmitView &g, uint32_t *F, unsigned *mask, int lane, int min_lanes) {
     const int row = q_pop_batch(mask, QS_SHADE, lane, min_lanes);
     if (row == -2) return false;
@@ -706,7 +706,7 @@ __device__ __forceinline__ void q_stage_bvh(const DScene &s, uint32_t *F, unsign
 }
 
 // QS_LEAF: the triangles of one leaf (bvh.h:52-67) for walks that sit at a leaf, then the walk's next node from its stack
-template <bool SPEC, bool NEE>
+template <bool SPEC, int NEE>
 __device__ __forceinline__ bool q_stage_leaf(const DScene &s, uint32_t *F, unsigned *mask, int *stk, int *deep, int lane, int min_lanes) {
     const int row = q_pop_batch(mask, QS_LEAF, lane, min_lanes);
     if (row == -2) return false;
@@ -908,9 +908,9 @@ __device__ __forceinline__ bool q_stage_end(const DScene &s, const PassParams &w
 
 // LAY 0: the top table of the air layout fits Q_TOP_WORDS and is staged in shared memory; 1: it is read from global memory;
 // 2: deep world (64-ary nodes between the top table and the bricks).  SPEC: CCU_RENDER_SPECULAR on a scene with specular words.
-// NEE: CCU_RENDER_EMITTER_SAMPLING on a scene with emitters (table `g`, an argument after the others so that the kernels without
-// it keep their parameter offsets).
-template <bool HAS_BVH, int LAY, bool SPEC, bool NEE>
+// NEE: the emitter sampler (NeeKind) of CCU_RENDER_EMITTER_SAMPLING, with CCU_RENDER_EMITTER_NEAR_FIELD for NEE_NEAR, on a scene
+// with emitters (table `g`, an argument after the others so that the kernels without it keep their parameter offsets).
+template <bool HAS_BVH, int LAY, bool SPEC, int NEE>
 __global__ void __launch_bounds__(Q_WARPS * 32, 1) k_render_queue(const __grid_constant__ DScene s, const __grid_constant__ QueueParams qp,
                                                                  const __grid_constant__ EmitView g) {
     constexpr int NST = q_stages(HAS_BVH);

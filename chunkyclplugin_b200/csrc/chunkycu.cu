@@ -44,8 +44,9 @@ __global__ void k_sun_setup(const int *sun_words, float *out /* su sv sw radius_
 // Thread-per-pixel path tracer: all passes of the batch in one launch, the running mean of
 // rayTracer.cl:109-112 carried in registers between passes (identical arithmetic, no memory round trip).
 // MODE: 0 = the reference's own node array, 1 = commit-time layouts, 2 = commit-time layouts of a deep world.
-// SPEC: CCU_RENDER_SPECULAR on a scene with specular words; NEE: CCU_RENDER_EMITTER_SAMPLING on a scene with emitters (sample_pixel).
-template <int MODE, bool SPEC, bool NEE>
+// SPEC: CCU_RENDER_SPECULAR on a scene with specular words; NEE: the emitter sampler (NeeKind) of CCU_RENDER_EMITTER_SAMPLING and
+// CCU_RENDER_EMITTER_NEAR_FIELD on a scene with emitters (sample_pixel).
+template <int MODE, bool SPEC, int NEE>
 __global__ void __launch_bounds__(128) k_render_mega(const __grid_constant__ DScene s, const int *__restrict__ seeds, int n_passes,
                                                      int start_spp, float *res, const float *res_prev, int n_pixels,
                                                      const __grid_constant__ EmitView g) {
@@ -433,10 +434,10 @@ void dispatch(bool v, F &&f) {
 }
 
 // the wavefront kernel (ccu_queue.cuh) for the scene's entity BVHs and air layout (air_layout_id), with or without specular events
-auto queue_kernel(bool bvh, int lay, bool spec, bool nee) {
-    decltype(&k_render_queue<false, 0, false, false>) k = nullptr;
+auto queue_kernel(bool bvh, int lay, bool spec, int nee) {
+    decltype(&k_render_queue<false, 0, false, NEE_NONE>) k = nullptr;
     dispatch(bvh, [&](auto B) {
-        dispatch<3>(lay, [&](auto L) { dispatch(spec, [&](auto S) { dispatch(nee, [&](auto N) { k = k_render_queue<B, L, S, N>; }); }); });
+        dispatch<3>(lay, [&](auto L) { dispatch(spec, [&](auto S) { dispatch<3>(nee, [&](auto N) { k = k_render_queue<B, L, S, N>; }); }); });
     });
     return k;
 }
@@ -446,8 +447,11 @@ auto queue_kernel(bool bvh, int lay, bool spec, bool nee) {
 bool specular_launch(const ccu_ctx *c) { return (c->params.flags & CCU_RENDER_SPECULAR) && c->scene.info.has_specular; }
 
 // CCU_RENDER_EMITTER_SAMPLING launches the NEE kernels only on a scene with emitters: without one they draw nothing and compute
-// exactly what the other kernels compute
-bool nee_launch(const ccu_ctx *c) { return (c->params.flags & CCU_RENDER_EMITTER_SAMPLING) && c->scene.info.has_emitters; }
+// exactly what the other kernels compute.  CCU_RENDER_EMITTER_NEAR_FIELD picks the near-field sampler (NEE_NEAR) among them.
+int nee_launch(const ccu_ctx *c) {
+    if (!((c->params.flags & CCU_RENDER_EMITTER_SAMPLING) && c->scene.info.has_emitters)) return NEE_NONE;
+    return (c->params.flags & CCU_RENDER_EMITTER_NEAR_FIELD) ? NEE_NEAR : NEE_AREA;
+}
 
 }  // namespace
 
@@ -608,7 +612,7 @@ int ccu_ctx_create(int device_index, ccu_ctx **out) {
     for (Event &ev : c->rays_used) if (e == cudaSuccess) e = ev.create(cudaEventDisableTiming);
     for (bool bvh : {false, true})
         for (bool spec : {false, true})
-            for (bool nee : {false, true})
+            for (int nee : {NEE_NONE, NEE_AREA, NEE_NEAR})
                 for (int lay = 0; lay < 3 && e == cudaSuccess; lay++)
                     e = cudaFuncSetAttribute(queue_kernel(bvh, lay, spec, nee), cudaFuncAttributeMaxDynamicSharedMemorySize, Q_SMEM_LIMIT);
     if (e == cudaSuccess) e = c->unorm.alloc(256);
@@ -930,7 +934,10 @@ int ccu_render_set_params(ccu_ctx *c, const ccu_render_params *p) {
     if (!p) return fail(CCU_EINVAL, "ccu_render_set_params: null argument");
     if (p->draw_depth < 0 || p->draw_depth >= (1 << 24) || p->max_depth < 1 || p->max_depth > 255) return fail(CCU_EINVAL, "bad render params");
     if (p->kernel != 0 && p->kernel != 1 && p->kernel != 4) return fail(CCU_EINVAL, "unknown kernel %d (0 auto, 1 thread-per-pixel, 4 wavefront)", p->kernel);
-    if (p->flags & ~(CCU_RENDER_NO_ENTITIES | CCU_RENDER_NO_SUN | CCU_RENDER_SPECULAR | CCU_RENDER_EMITTER_SAMPLING)) return fail(CCU_EINVAL, "unknown render flags 0x%x", p->flags);
+    if (p->flags & ~(CCU_RENDER_NO_ENTITIES | CCU_RENDER_NO_SUN | CCU_RENDER_SPECULAR | CCU_RENDER_EMITTER_SAMPLING | CCU_RENDER_EMITTER_NEAR_FIELD))
+        return fail(CCU_EINVAL, "unknown render flags 0x%x", p->flags);
+    if ((p->flags & CCU_RENDER_EMITTER_NEAR_FIELD) && !(p->flags & CCU_RENDER_EMITTER_SAMPLING))
+        return fail(CCU_EINVAL, "CCU_RENDER_EMITTER_NEAR_FIELD needs CCU_RENDER_EMITTER_SAMPLING");
     if (!c) return fail(CCU_EINVAL, "ccu_render_set_params: null argument");
     std::lock_guard<std::mutex> lk(c->mu);
     c->params = *p;
@@ -971,7 +978,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
     const bool bvh = !(s.world_bvh_empty && s.actor_bvh_empty);
     const int mode = layout_mode(c);
     const bool spec = specular_launch(c);
-    const bool nee = nee_launch(c);
+    const int nee = nee_launch(c);
     float *res = c->accum[c->accum_active].p;
     const float *res_prev = c->window_spp == 0 ? c->window_base : res;
     int kernel = c->params.kernel;
@@ -980,7 +987,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
         const int threads = 128, blocks = (n_pixels + threads - 1) / threads;
         dispatch<3>(mode, [&](auto M) {
             dispatch(spec, [&](auto S) {
-                dispatch(nee, [&](auto N) {
+                dispatch<3>(nee, [&](auto N) {
                     k_render_mega<M, S, N><<<blocks, threads, 0, c->stream>>>(s, seeds_dev, n_passes, c->window_spp, res, res_prev, n_pixels,
                                                                         c->scene.emit_view);
                 });
@@ -1011,7 +1018,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
         // 128 x 128 table (64 KiB) taken from L1 costs more brick / atlas hits than the sky lookups gain (measured: +1.8 % per
         // pass on config 1).  CCU_SKY_SMEM_MAX (bytes, default 16 KiB = 64 x 64 texels) moves the threshold.
         const int sky_texels = c->scene.info.sky_res * c->scene.info.sky_res;
-        const int base_smem = q_smem_bytes(bvh, lay == 0, spec, nee);
+        const int base_smem = q_smem_bytes(bvh, lay == 0, spec, nee != NEE_NONE);
         const char *sky_env = getenv("CCU_SKY_SMEM_MAX");
         const int sky_max = sky_env ? atoi(sky_env) : 16384;
         const bool sky_smem = sky_texels * 4 <= sky_max && base_smem + sky_texels * 4 <= Q_SMEM_LIMIT;

@@ -15,6 +15,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("CHUNKYCU_LIB") or os.path.join(_HERE, "libchunkycu.so")
 
 CCU_RENDER_NO_ENTITIES, CCU_RENDER_NO_SUN, CCU_RENDER_SPECULAR, CCU_RENDER_EMITTER_SAMPLING = 1, 2, 4, 8
+CCU_RENDER_EMITTER_NEAR_FIELD = 128
 CCU_UNIQUE_ID_BYTES = 128
 
 CCU_OK, CCU_ENODEVICE, CCU_EINVAL, CCU_ECUDA, CCU_ENOMEM, CCU_ESTATE = 0, -1, -2, -3, -4, -5

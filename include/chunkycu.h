@@ -68,6 +68,13 @@ typedef struct ccu_render_params {
  * A scene without full-cube emitters renders exactly as without the flag.  Both render kernels implement it.  DESIGN.md §10
  * holds the exact contract. */
 #define CCU_RENDER_EMITTER_SAMPLING 8
+/* Near-field emitter sampling, valid only together with CCU_RENDER_EMITTER_SAMPLING (ccu_render_set_params refuses it alone):
+ * when the sampled emitter voxel lies within 1/8 of the hit (distance to its box), the sample is a cosine-weighted direction
+ * scored when it enters the voxel, instead of a point on a face.  The area sampler's weight grows without bound as a hit
+ * approaches an emitter face, which shows as fireflies where a surface meets an emitter; with this flag every sample's
+ * contribution is bounded.  Farther emitters are sampled exactly as without it, and the image's expectation is that of
+ * CCU_RENDER_EMITTER_SAMPLING.  DESIGN.md §11 holds the exact contract. */
+#define CCU_RENDER_EMITTER_NEAR_FIELD 128
 
 /* ---- device enumeration: RendererInstance.java:39-75,123-157 (clGetPlatformIDs/clGetDeviceIDs/clGetDeviceInfo),
  *      used by the GPU selector UI (ui/GpuSelector.java:24-87) -------------------------------------------------- */

@@ -78,6 +78,8 @@ public final class ChunkyCu {
     /** ccu_render_params.flags: Chunky's "draw entities" / sunlight toggles as launch parameters (reference README.md:31-35), and
      *  specular / metallic / rough materials from material word 5 (beyond the reference, DESIGN "Beyond the reference: specular materials"). */
     public static final int RENDER_NO_ENTITIES = 1, RENDER_NO_SUN = 2, RENDER_SPECULAR = 4, RENDER_EMITTER_SAMPLING = 8;
+    /** ccu_render_params.flags: near-field emitter sampling (DESIGN §11), valid only together with RENDER_EMITTER_SAMPLING. */
+    public static final int RENDER_EMITTER_NEAR_FIELD = 128;
     private static final StructLayout RENDER_PARAMS = MemoryLayout.structLayout(JAVA_INT.withName("draw_depth"), JAVA_INT.withName("max_depth"),
             JAVA_FLOAT.withName("emitter_scale"), JAVA_INT.withName("kernel"), JAVA_INT.withName("flags"));
 

@@ -1,12 +1,14 @@
-"""Cost and gain of CCU_RENDER_EMITTER_SAMPLING on BASELINE config 3 (indoor256: glowstone-lit rooms, sun off) and config 1
+"""Cost and gain of CCU_RENDER_EMITTER_SAMPLING, alone and with CCU_RENDER_EMITTER_NEAR_FIELD, on BASELINE config 3 (indoor256: glowstone-lit rooms, sun off) and config 1
 with decorations (256^3 terrain with scattered glowstone, sun on), both at 1920 x 1080.
 
-Per config, two legs on kernel 0 (the wavefront kernel, what bench.py times) alternated window by window in one process
-(16-pass windows, L2 flushed before each): `off` with the flag off and `on` with it on.  Then the gain: RMSE of a K-pass
+Per config, three legs on kernel 0 (the wavefront kernel, what bench.py times) alternated window by window in one process
+(16-pass windows, L2 flushed before each): `off` with the flags off, `on` with CCU_RENDER_EMITTER_SAMPLING (DESIGN §10) and
+`near` with it and CCU_RENDER_EMITTER_NEAR_FIELD (§11).  Then the gain: RMSE of a K-pass
 render of each leg against a --ref-spp flag-off render on a disjoint seed stream, for each K of --spp.  For an unbiased
 estimator the RMSE falls as 1 / sqrt(K) (variance, not bias): `rmse_ratio_hi_lo` compares the RMSE at the largest K with the
 RMSE at the smallest, against the 1 / sqrt ratio.  At equal device time the flag-off kernel renders t_on / t_off times the
-passes, so its RMSE becomes rmse(off) * sqrt(t_off / t_on); `equal_time_ratio` divides the flag-on RMSE by that.  The
+passes, so its RMSE becomes rmse(off) * sqrt(t_off / t_on); `equal_time_ratio` divides the `on` RMSE by that, and
+`equal_time_ratio_near` the `near` RMSE by the same with t_near.  The
 per-pixel median absolute error is reported beside the RMSE (robust to a few very bright pixels).  Also the commit time of
 config 5 (depth-11 world without emitters: the table is not built).  Prints one JSON line with the GPU's name, power limit
 and SM clock.
@@ -64,7 +66,7 @@ def main():
     from conftest import load_scene
 
     NEE = native.CCU_RENDER_EMITTER_SAMPLING
-    legs = {"off": (0, 0), "on": (0, NEE)}
+    legs = {"off": (0, 0), "on": (0, NEE), "near": (0, NEE | native.CCU_RENDER_EMITTER_NEAR_FIELD)}
     configs = {"config3_indoor256": S.indoor_scene(256, 1920, 1080),
                "config1_decorated": S.terrain_scene(256, 1920, 1080, decorate=True)}
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")      # > 126 MB L2
@@ -107,6 +109,8 @@ def main():
                      for k, v in ms.items()},
             "equal_time_ratio": {str(n): err["on"][n]["rmse"] / (err["off"][n]["rmse"] * float(np.sqrt(per_pass["off"] / per_pass["on"])))
                                  for n in args.spp},
+            "equal_time_ratio_near": {str(n): err["near"][n]["rmse"] / (err["off"][n]["rmse"] * float(np.sqrt(per_pass["off"] / per_pass["near"])))
+                                      for n in args.spp},
         }
     ctx = native.Context(0)
     load_scene(ctx, S.large_world_scene())

@@ -1,8 +1,8 @@
-"""ctypes binding of the CPU restatement of CCU_RENDER_SPECULAR and CCU_RENDER_EMITTER_SAMPLING (specular_oracle.c).
-TEST INFRASTRUCTURE ONLY.
+"""ctypes binding of the CPU restatement of CCU_RENDER_SPECULAR, CCU_RENDER_EMITTER_SAMPLING and CCU_RENDER_EMITTER_NEAR_FIELD
+(specular_oracle.c).  TEST INFRASTRUCTURE ONLY.
 
 ``SpecularOracle`` is the parity oracle (``oracle.Oracle``) with the specular events of DESIGN.md section 9 in its path
-loop; ``FlagsOracle`` takes the render flags and adds the emitter sampling of section 10, with the emitter table that
+loop; ``FlagsOracle`` takes the render flags and adds the emitter sampling of sections 10 and 11, with the emitter table that
 ``emitter_grid`` builds from the packed arrays.  Everything else - first hit, preview, counters - is the oracle's.  Like the
 oracle, only tests/ and scripts use it.
 """
@@ -44,7 +44,7 @@ class _Grid(C.Structure):
                 ("g0", C.c_int32 * 3), ("dim", C.c_int32 * 3), ("shift", C.c_int32)]
 
 
-CCU_RENDER_SPECULAR, CCU_RENDER_EMITTER_SAMPLING = 4, 8
+CCU_RENDER_SPECULAR, CCU_RENDER_EMITTER_SAMPLING, CCU_RENDER_EMITTER_NEAR_FIELD = 4, 8, 128
 EMIT_SHIFT0, EMIT_CELL_BUDGET, EMIT_MAX = 3, 1 << 21, 1 << 18      # DESIGN.md section 10
 
 
@@ -141,8 +141,9 @@ class SpecularOracle(oracle.Oracle):
 
 
 class FlagsOracle(oracle.Oracle):
-    """oracle.Oracle whose render() runs the path loop with the given CCU_RENDER_SPECULAR / CCU_RENDER_EMITTER_SAMPLING bits
-    (the other flags act on the scene: oracle.edge_rays.without_sun, or empty BVHs for CCU_RENDER_NO_ENTITIES)."""
+    """oracle.Oracle whose render() runs the path loop with the given CCU_RENDER_SPECULAR / CCU_RENDER_EMITTER_SAMPLING /
+    CCU_RENDER_EMITTER_NEAR_FIELD bits (the other flags act on the scene: oracle.edge_rays.without_sun, or empty BVHs for
+    CCU_RENDER_NO_ENTITIES)."""
 
     def __init__(self, scene, flags: int = 0, **kw):
         super().__init__(scene, **kw)
@@ -173,6 +174,7 @@ class FlagsOracle(oracle.Oracle):
         nee = (self.flags & CCU_RENDER_EMITTER_SAMPLING) and self.grid["has_emitters"]
         lib().flags_render(C.byref(self._s), sd.ctypes.data_as(C.c_void_p), C.c_int(sd.size), C.c_int(start_spp),
                            res.ctypes.data_as(C.c_void_p), gp, C.c_int64(gn), C.c_int(threads), C.byref(cnt),
-                           C.c_int(1 if self.flags & CCU_RENDER_SPECULAR else 0), C.byref(self._grid) if nee else None)
+                           C.c_int(1 if self.flags & CCU_RENDER_SPECULAR else 0), C.byref(self._grid) if nee else None,
+                           C.c_int(1 if self.flags & CCU_RENDER_EMITTER_NEAR_FIELD else 0))
         self._counters(cnt)
         return res

@@ -269,10 +269,73 @@ static int emitter_covered(const Ctx *c, const EmitterGrid *g, int block, const 
     return abs(e[0] - cell[0]) <= 1 && abs(e[1] - cell[1]) <= 1 && abs(e[2] - cell[2]) <= 1;
 }
 
+/* ---- near-field emitter sampling (DESIGN.md section 11) ---- */
+#define NEE_RHO2 0.015625f   /* an emitter is near when its box distance^2 is below rho^2 = (1/8)^2 */
+
+/* next_path's cosine-weighted direction about n for the draws x1, x2 (kernel.h:50-92) */
+static v3 diffuse_direction(const Ctx *c, v3 n, float x1, float x2) {
+    float r = sqrtf(x1);
+    float theta = 2 * PI_F * x2;
+    float tx = r * m_cos(&c->math, theta);
+    float ty = r * m_sin(&c->math, theta);
+    float tz = sqrtf(1 - x1);
+    float xx, xy, xz;
+    if ((double)fabsf(n.x) > 0.1) { xx = 0; xy = 1; } else { xx = 1; xy = 0; }
+    xz = 0;
+    float ux = xy * n.z - xz * n.y;
+    float uy = xz * n.x - xx * n.z;
+    float uz = xx * n.y - xy * n.x;
+    r = 1 / sqrtf((ux * ux + uy * uy) + uz * uz);
+    ux *= r; uy *= r; uz *= r;
+    float vx = uy * n.z - uz * n.y;
+    float vy = uz * n.x - ux * n.z;
+    float vz = ux * n.y - uy * n.x;
+    return V((ux * tx + vx * ty) + n.x * tz, (uy * tx + vy * ty) + n.y * tz, (uz * tx + vz * ty) + n.z * tz);
+}
+
+static float vget(v3 a, int i) { return i == 0 ? a.x : (i == 1 ? a.y : a.z); }
+static float clamp01(float a) { return a < 0.0f ? 0.0f : (a > 1.0f ? 1.0f : a); }
+
+/* section 11 step 4: the direction from u2, u3, the slab test against emitter e, the material at the entry point and the
+ * contribution; returns 0 when no shadow ray is traced */
+static int nee_near(const Ctx *c, const int32_t *e, int n, v3 x, v3 normal, v3 T, float u2, float u3, v3 *out, v3 *w, float *limit) {
+    *w = diffuse_direction(c, normal, u2, u3);
+    float lo[3], hi[3];
+    for (int a = 0; a < 3; a++) {
+        float inv = 1.0f / vget(*w, a);
+        float t0 = ((float)e[a] - vget(x, a)) * inv, t1 = ((float)(e[a] + 1) - vget(x, a)) * inv;
+        if (t0 != t0 || t1 != t1) return 0;
+        lo[a] = t0 < t1 ? t0 : t1;
+        hi[a] = t0 < t1 ? t1 : t0;
+    }
+    float tn = lo[0], tf = hi[0];
+    int axis = 0;
+    for (int a = 1; a < 3; a++) {
+        if (lo[a] > tn) { tn = lo[a]; axis = a; }
+        if (hi[a] < tf) tf = hi[a];
+    }
+    if (!(tn <= tf && tn > 0.0f)) return 0;
+    int plus = vget(*w, axis) < 0.0f;
+    if (!(plus ? vget(x, axis) > (float)(e[axis] + 1) : vget(x, axis) < (float)e[axis])) return 0;
+    v3 p = vadd(x, vscale(*w, tn));
+    float px = clamp01(p.x - (float)e[0]), py = clamp01(p.y - (float)e[1]), pz = clamp01(p.z - (float)e[2]);
+    float u, v;
+    if (axis == 0) { u = plus ? pz : 1.0f - pz; v = py; }
+    else if (axis == 1) { u = px; v = plus ? pz : 1.0f - pz; }
+    else { u = plus ? 1.0f - px : px; v = py; }
+    Record m;
+    record_new(&m);
+    if (!material_sample(c, c->sc->block_palette[e[3] + 1], &m, u, v)) return 0;
+    float kk = (m.emittance * c->sc->emitter_scale) * (float)n;
+    *out = V((T.x * (m.color[0] * m.color[0])) * kk, (T.y * (m.color[1] * m.color[1])) * kk, (T.z * (m.color[2] * m.color[2])) * kk);
+    *limit = tn - NEE_DELTA;
+    return 1;
+}
+
 /* steps 2-4: the four draws, the emitter, face and point, the material at the point and the contribution; returns 0 when
- * no shadow ray is traced */
-static int nee_sample(const Ctx *c, const EmitterGrid *g, int b, int n, v3 x, v3 normal, v3 T, uint32_t *state, v3 *out, v3 *w,
-                      float *limit) {
+ * no shadow ray is traced.  near: an emitter whose box distance^2 is below rho^2 is sampled by nee_near (section 11). */
+static int nee_sample(const Ctx *c, const EmitterGrid *g, int near, int b, int n, v3 x, v3 normal, v3 T, uint32_t *state, v3 *out,
+                      v3 *w, float *limit) {
     float u0 = rng_float(state);
     float u1 = rng_float(state);
     float u2 = rng_float(state);
@@ -286,6 +349,14 @@ static int nee_sample(const Ctx *c, const EmitterGrid *g, int b, int n, v3 x, v3
     if (x.y < ey) faces[f++] = 2; else if (x.y > (float)(e[1] + 1)) faces[f++] = 3;
     if (x.z < ez) faces[f++] = 4; else if (x.z > (float)(e[2] + 1)) faces[f++] = 5;
     if (f == 0) return 0;
+    if (near) {
+        float o[3];
+        for (int a = 0; a < 3; a++) {
+            float xa = vget(x, a), lo = (float)e[a], hi = (float)(e[a] + 1);
+            o[a] = xa < lo ? lo - xa : (xa > hi ? xa - hi : 0.0f);
+        }
+        if ((o[0] * o[0] + o[1] * o[1]) + o[2] * o[2] < NEE_RHO2) return nee_near(c, e, n, x, normal, T, u2, u3, out, w, limit);
+    }
     int k = (int)(u1 * (float)f);
     if (k > f - 1) k = f - 1;
     int axis = faces[k] >> 1, plus = faces[k] & 1;
@@ -310,8 +381,8 @@ static int nee_sample(const Ctx *c, const EmitterGrid *g, int b, int n, v3 x, v3
     return 1;
 }
 
-/* one path sample: rayTracer.cl:40-107 with the specular events (spec) and emitter sampling (g != NULL) */
-static v3 sample_pixel_ext(const Ctx *c, int gid, int32_t seed, int spec, const EmitterGrid *g) {
+/* one path sample: rayTracer.cl:40-107 with the specular events (spec) and emitter sampling (g != NULL; near: section 11) */
+static v3 sample_pixel_ext(const Ctx *c, int gid, int32_t seed, int spec, const EmitterGrid *g, int near) {
     Path p;
     Record rec;
     uint32_t w5 = 0;
@@ -362,7 +433,7 @@ static v3 sample_pixel_ext(const Ctx *c, int gid, int32_t seed, int spec, const 
                 float limit;
                 nee_prev = 1;
                 memcpy(nee_cell, cell, sizeof cell);
-                if (nee_sample(c, g, b, n, p.origin, rec.normal, p.throughput, &state, &contrib, &w, &limit)) {
+                if (nee_sample(c, g, near, b, n, p.origin, rec.normal, p.throughput, &state, &contrib, &w, &limit)) {
                     Path q = p;
                     q.direction = w;
                     Record s = rec;
@@ -377,7 +448,7 @@ static v3 sample_pixel_ext(const Ctx *c, int gid, int32_t seed, int spec, const 
 }
 
 static int render_ext(const OracleScene *s, const int32_t *seeds, int n_passes, int start_spp, float *res, const int32_t *gids,
-                      int64_t n_gids, int nthreads, OracleCounters *out_counters, int spec, const EmitterGrid *g) {
+                      int64_t n_gids, int nthreads, OracleCounters *out_counters, int spec, const EmitterGrid *g, int near) {
     int64_t n = gids ? n_gids : (int64_t)s->width * s->height;
     OracleCounters total;
     memset(&total, 0, sizeof total);
@@ -396,7 +467,7 @@ static int render_ext(const OracleScene *s, const int32_t *seeds, int n_passes, 
             float *px = res + (size_t)gid * 3;
             v3 buf = V(px[0], px[1], px[2]);
             for (int pass = 0; pass < n_passes; pass++) {
-                v3 col = sample_pixel_ext(&c, gid, seeds[pass], spec, g);
+                v3 col = sample_pixel_ext(&c, gid, seeds[pass], spec, g, near);
                 int spp = start_spp + pass;
                 buf.x = (buf.x * (float)spp + col.x) / (float)(spp + 1);
                 buf.y = (buf.y * (float)spp + col.y) / (float)(spp + 1);
@@ -414,13 +485,14 @@ static int render_ext(const OracleScene *s, const int32_t *seeds, int n_passes, 
 /* oracle_render with the specular events (same arguments, same running mean) */
 int specular_render(const OracleScene *s, const int32_t *seeds, int n_passes, int start_spp, float *res, const int32_t *gids,
                     int64_t n_gids, int nthreads, OracleCounters *out_counters) {
-    return render_ext(s, seeds, n_passes, start_spp, res, gids, n_gids, nthreads, out_counters, 1, NULL);
+    return render_ext(s, seeds, n_passes, start_spp, res, gids, n_gids, nthreads, out_counters, 1, NULL, 0);
 }
 
-/* oracle_render with CCU_RENDER_SPECULAR (spec) and CCU_RENDER_EMITTER_SAMPLING (g != NULL) */
+/* oracle_render with CCU_RENDER_SPECULAR (spec), CCU_RENDER_EMITTER_SAMPLING (g != NULL) and CCU_RENDER_EMITTER_NEAR_FIELD
+ * (near, with g) */
 int flags_render(const OracleScene *s, const int32_t *seeds, int n_passes, int start_spp, float *res, const int32_t *gids,
-                 int64_t n_gids, int nthreads, OracleCounters *out_counters, int spec, const EmitterGrid *g) {
-    return render_ext(s, seeds, n_passes, start_spp, res, gids, n_gids, nthreads, out_counters, spec, g);
+                 int64_t n_gids, int nthreads, OracleCounters *out_counters, int spec, const EmitterGrid *g, int near) {
+    return render_ext(s, seeds, n_passes, start_spp, res, gids, n_gids, nthreads, out_counters, spec, g, near);
 }
 
 int emitter_grid_struct_size(void) { return (int)sizeof(EmitterGrid); }
