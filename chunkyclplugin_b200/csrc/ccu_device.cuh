@@ -82,12 +82,18 @@ struct DScene {   // what a launch reads: commit fills the scene's fields once (
 // an argument of its own (after the others, so that every kernel keeps the parameter offsets it had without it):
 // emit[i] = {x, y, z, block palette position} sorted by (x, y, z); the cell lists in CSR form, L(c) = list[off[c] .. off[c + 1]),
 // cells of 1 << shift voxels, index (cx * dim.y + cy) * dim.z + cz over the cell box whose low voxel corner is g0.
+// The wider table of CCU_RENDER_EMITTER_MODELS (DESIGN §12) also lists model emitters: mhead[b] is the int4 index in mprim of
+// palette position b's emitting primitives, -1 when b is no model emitter; there mprim holds {m, bbox xmin, xmax, ymin},
+// {ymax, zmin, zmax, 0} (float bits, block-local) and then m records of four int4 (model_prim_words).  The table of
+// CCU_RENDER_EMITTER_SAMPLING alone leaves both null.
 struct EmitView {
     const int4 *__restrict__ emit;
     const int *__restrict__ off;
     const int *__restrict__ list;
     int3 g0, dim;
     int shift;
+    const int *__restrict__ mhead;
+    const int4 *__restrict__ mprim;
 };
 
 // What a successful intersection writes into the IntersectionRecord (wavefront.h:37-78).  The specular kernels (SPEC, DESIGN
@@ -593,11 +599,13 @@ __device__ __forceinline__ void march_exit(March &m, const Cell &c, int level) {
 }
 // Block test of the non-air leaf under the ray (octree.h:92-106).  Returns true on a hit (surf / hit_t filled);
 // otherwise the ray has been advanced past the leaf.
-template <bool SPEC>
-__device__ __forceinline__ bool march_block(const DScene &s, March &m, int data, int level, SurfT<SPEC> &surf, float &hit_t) {
+// CUT (kernels built with CCU_RENDER_EMITTER_MODELS) and `cut` (the ray is an emitter sample's shadow ray): the hit counts only
+// when it lies before the ray's limit, so that a model's own voxel does not occlude the primitive sampled inside it (DESIGN §12).
+template <bool SPEC, bool CUT = false>
+__device__ __forceinline__ bool march_block(const DScene &s, March &m, int data, int level, SurfT<SPEC> &surf, float &hit_t, bool cut = false) {
     Cell c = march_cell(m);
     float dist = intersect_block(s, data, c.bx, c.by, c.bz, surf, c.pos, m.d, m.inv);
-    if (!is_nan(dist)) {
+    if (!is_nan(dist) && !(CUT && cut && !(m.t + dist < m.limit))) {
         hit_t = m.t + dist;
         return true;
     }
@@ -607,7 +615,7 @@ __device__ __forceinline__ bool march_block(const DScene &s, March &m, int data,
 
 // One whole iteration of octree.h:66-107 on the reference's own node array (root descent per step).
 // Returns 0 = keep marching, 1 = hit (hit_t / surf / block / node filled), 2 = ray left.
-template <bool SPEC>
+template <bool SPEC, bool CUT = false>
 __device__ __forceinline__ int march_step_ref(const DScene &s, March &m, SurfT<SPEC> &surf, float &hit_t, int &hit_block, int &hit_node, Cell &hit_cell) {
     if (m.steps >= s.draw_depth || m.t > m.limit) return 2;
     const int depth = s.depth;
@@ -619,7 +627,7 @@ __device__ __forceinline__ int march_step_ref(const DScene &s, March &m, SurfT<S
         march_exit(m, c, level);
         return 0;
     }
-    if (march_block(s, m, data, level, surf, hit_t)) {
+    if (march_block<SPEC, CUT>(s, m, data, level, surf, hit_t, CUT)) {
         hit_block = data;
         hit_node = node;
         hit_cell = c;
@@ -628,7 +636,7 @@ __device__ __forceinline__ int march_step_ref(const DScene &s, March &m, SurfT<S
     return 0;
 }
 
-template <bool SPEC>
+template <bool SPEC, bool CUT = false>
 __device__ __forceinline__ bool octree_intersect_ref(const DScene &s, float3 origin, float3 direction, RecordT<SPEC> &rec, HitInfo &hi) {
     March m;
     if (!march_begin(s, m, origin, direction, rec.distance)) return false;
@@ -636,7 +644,7 @@ __device__ __forceinline__ bool octree_intersect_ref(const DScene &s, float3 ori
         float t;
         int block, node;
         Cell cell;
-        int r = march_step_ref(s, m, rec.surf, t, block, node, cell);
+        int r = march_step_ref<SPEC, CUT>(s, m, rec.surf, t, block, node, cell);
         if (r == 1) {
             rec.distance = t;
             rec.material = block;
@@ -735,9 +743,9 @@ __device__ __forceinline__ bool bvh_pair(const DScene &s, float3 origin, float3 
 }
 
 // kernel.h:14-24 on the reference's own node array
-template <bool SPEC>
+template <bool SPEC, bool CUT = false>
 __device__ __forceinline__ bool closest_intersect_ref(const DScene &s, float3 origin, float3 direction, RecordT<SPEC> &rec, HitInfo &hi) {
-    bool hit = octree_intersect_ref(s, origin, direction, rec, hi);
+    bool hit = octree_intersect_ref<SPEC, CUT>(s, origin, direction, rec, hi);
     int kind = 0;
     if (bvh_pair(s, origin, direction, rec.distance, rec.surf, kind)) {
         hit = true;
@@ -910,19 +918,29 @@ __device__ __forceinline__ int emitter_list(const EmitView &g, int3 c, int &N) {
     N = __ldg(g.off + ci + 1) - b;
     return b;
 }
+// The emitter sampler a kernel is built with: none, the area sampler of CCU_RENDER_EMITTER_SAMPLING (DESIGN §10), that
+// sampler with the near field of CCU_RENDER_EMITTER_NEAR_FIELD (DESIGN §11), or either of the two over the wider table of
+// CCU_RENDER_EMITTER_MODELS, which also samples quad and AABB models (DESIGN §12).
+enum NeeKind : int { NEE_NONE = 0, NEE_AREA = 1, NEE_NEAR = 2, NEE_AREA_MODELS = 3, NEE_NEAR_MODELS = 4 };
+__host__ __device__ constexpr bool nee_near_field(int kind) { return kind == NEE_NEAR || kind == NEE_NEAR_MODELS; }
+__host__ __device__ constexpr bool nee_models(int kind) { return kind == NEE_AREA_MODELS || kind == NEE_NEAR_MODELS; }
+#define CCU_NEE_RHO2 0.015625f   // DESIGN §11: an emitter is near when its box distance² is below rho² = (1/8)²
+
 // The emission rule: an octree hit on voxel (bx, by, bz) of block palette position `block` that the previous hit's sample
-// covered (an emitter whose cell is within Chebyshev distance 1 of that hit's cell c) delivers no emission.
+// covered (an emitter whose cell is within Chebyshev distance 1 of that hit's cell c) delivers no emission.  With the model
+// table a model emitter (mhead >= 0) counts as well.
+template <int KIND = NEE_AREA>
 __device__ __forceinline__ bool emitter_covered(const DScene &s, const EmitView &g, int block, int bx, int by, int bz, int3 c) {
     const int4 r0 = __ldg(s.block_rec + 2 * block), r1 = __ldg(s.block_rec + 2 * block + 1);
-    if (r0.x != 1 || !((r0.z & 2) || (r1.z & 0xFF))) return false;
+    if constexpr (nee_models(KIND)) {
+        if (!(r0.x == 1 && ((r0.z & 2) || (r1.z & 0xFF))) && __ldg(g.mhead + block) < 0) return false;
+    } else {
+        if (r0.x != 1 || !((r0.z & 2) || (r1.z & 0xFF))) return false;
+    }
     int3 e;
     if (!emitter_voxel_cell(g, bx, by, bz, e)) return false;
     return abs(e.x - c.x) <= 1 && abs(e.y - c.y) <= 1 && abs(e.z - c.z) <= 1;
 }
-// The emitter sampler a kernel is built with: none, the area sampler of CCU_RENDER_EMITTER_SAMPLING (DESIGN §10), or that
-// sampler with the near field of CCU_RENDER_EMITTER_NEAR_FIELD (DESIGN §11).
-enum NeeKind : int { NEE_NONE = 0, NEE_AREA = 1, NEE_NEAR = 2 };
-#define CCU_NEE_RHO2 0.015625f   // DESIGN §11: an emitter is near when its box distance² is below rho² = (1/8)²
 
 // DESIGN §11 step 4 at a hit x with normal n for emitter e (palette position e.w) from a list of N, whose box distance² is
 // below rho²: a cosine-weighted direction (nextPath's, from u2 and u3), scored when it enters the emitter's box through a face
@@ -968,9 +986,113 @@ __device__ __forceinline__ bool nee_near(const DScene &s, int4 e, int N, float3 
     return true;
 }
 
+// Material_get + Material_sample of material pointer `material` (material_sample's two paths) as a MatOut
+__device__ __forceinline__ MatOut material_at(const DScene &s, int material, float u, float v) {
+    const int idx = material / 6;
+    if (material >= 0 && idx * 6 == material) {
+        const int4 a = __ldg(s.mat_rec + 2 * idx), b = __ldg(s.mat_rec + 2 * idx + 1);
+        return material_eval_core(s, (uint32_t)a.x, (uint32_t)a.y, (uint32_t)a.z, (uint32_t)a.w, (uint32_t)b.x, u, v);
+    }
+    const int *m = s.mat_palette + material;
+    return material_eval_core(s, __ldg(m), __ldg(m + 1), __ldg(m + 2), __ldg(m + 3), __ldg(m + 4), u, v);
+}
+
+// DESIGN §12 step 3 for a model entry e (palette position e.w, primitives at g.mprim + h) from a list of N: the near branch
+// (NEAR, x within rho of the primitives' bounding box) runs the voxel's block test along a cosine-weighted direction; the far
+// branch samples a point on primitive P[min((int)(u1 m), m - 1)].  A primitive record is {kind, material, face flags, w0},
+// {w1..w4}, {w5..w8}, {w9..w12}: kind 6 a quad (w0..w12 its 13 words), kind 0..5 the box face axis * 2 + (1 for +) of the box
+// w0..w5 (xmin, xmax, ymin, ymax, zmin, zmax).
+template <bool NEAR>
+__device__ __forceinline__ bool nee_model(const DScene &s, const EmitView &g, int h, int4 e, int N, float3 x, float3 n, float3 T, float u1,
+                                          float u2, float u3, float3 &c, float3 &w, float &limit) {
+    const int4 h0 = __ldg(g.mprim + h), h1 = __ldg(g.mprim + h + 1);
+    const int m = h0.x;
+    const float ex = (float)e.x, ey = (float)e.y, ez = (float)e.z;
+    if constexpr (NEAR) {
+        const float lx = ex + i2f(h0.y), hx = ex + i2f(h0.z), ly = ey + i2f(h0.w), hy = ey + i2f(h1.x), lz = ez + i2f(h1.y), hz = ez + i2f(h1.z);
+        const float ox = x.x < lx ? lx - x.x : (x.x > hx ? x.x - hx : 0.0f);
+        const float oy = x.y < ly ? ly - x.y : (x.y > hy ? x.y - hy : 0.0f);
+        const float oz = x.z < lz ? lz - x.z : (x.z > hz ? x.z - hz : 0.0f);
+        if ((ox * ox + oy * oy) + oz * oz < CCU_NEE_RHO2) {
+            w = diffuse_direction(n, u2, u3);
+            const float3 inv = f3(1.0f / w.x, 1.0f / w.y, 1.0f / w.z);
+            Surf hit;
+            hit.emittance = 0.0f;
+            const float t = intersect_block<false>(s, e.w, e.x, e.y, e.z, hit, x, w, inv);
+            if (is_nan(t) || !(hit.emittance > 0.0f)) return false;
+            const float k = (hit.emittance * s.emitter_scale) * (float)N;
+            c = f3((T.x * (hit.color.x * hit.color.x)) * k, (T.y * (hit.color.y * hit.color.y)) * k, (T.z * (hit.color.z * hit.color.z)) * k);
+            limit = t - CCU_NEE_DELTA;
+            return true;
+        }
+    }
+    const int4 *r = g.mprim + h + 2 + 4 * min((int)(u1 * (float)m), m - 1);
+    const int4 q0 = __ldg(r), q1 = __ldg(r + 1), q2 = __ldg(r + 2), q3 = __ldg(r + 3);
+    const bool quad = q0.x == 6;
+    const int axis = q0.x >> 1, plus = q0.x & 1;   // box face
+    float3 l, nq;        // the sampled point (block-local); the quad's normal
+    float u, v, area;
+    if (quad) {
+        const float3 qo = f3(i2f(q0.w), i2f(q1.x), i2f(q1.y));
+        const float3 xv = f3(i2f(q1.z), i2f(q1.w), i2f(q2.x));
+        const float3 yv = f3(i2f(q2.y), i2f(q2.z), i2f(q2.w));
+        l = (qo + xv * u2) + yv * u3;
+        // Quad_intersect's uv at that point
+        u = i2f(q3.x) + u2 * i2f(q3.y);
+        v = i2f(q3.z) + u3 * i2f(q3.w);
+        const float3 cr = cross3(xv, yv);
+        nq = normalize3(cr);
+        area = sqrtf(dot3(cr, cr));
+    } else {
+        const float b[6] = {i2f(q0.w), i2f(q1.x), i2f(q1.y), i2f(q1.z), i2f(q1.w), i2f(q2.x)};
+        const int a1 = axis == 0 ? 1 : 0, a2 = axis == 2 ? 1 : 2;   // the in-face axes, in increasing order
+        const float s1 = b[2 * a1 + 1] - b[2 * a1], s2 = b[2 * a2 + 1] - b[2 * a2];
+        float lv[3];
+        lv[axis] = b[2 * axis + plus];
+        lv[a1] = b[2 * a1] + u2 * s1;
+        lv[a2] = b[2 * a2] + u3 * s2;
+        l = f3(lv[0], lv[1], lv[2]);
+        nq = f3(0, 0, 0);
+        area = s1 * s2;
+        // AABB_full_intersect_map_2 at l, then the face's flip and swap bits (textured_box)
+        if (axis == 0) { u = plus ? 1.0f - l.z : l.z; v = l.y; }
+        else if (axis == 1) { u = l.x; v = plus ? 1.0f - l.z : l.z; }
+        else { u = plus ? l.x : 1.0f - l.x; v = l.y; }
+        const int fl = q0.z;
+        if (fl & 4) u = 1.0f - u;
+        if (fl & 2) v = 1.0f - v;
+        if (fl & 1) { const float t = u; u = v; v = t; }
+    }
+    const MatOut mo = material_at(s, q0.y, u, v);
+    if (!mo.ok) return false;
+    const float3 dv = f3(ex + l.x, ey + l.y, ez + l.z) - x;
+    const float d2 = dot3(dv, dv);
+    const float dist = sqrtf(d2);
+    w = dv * (1.0f / dist);
+    const float cx = dot3(w, n);
+    if (!(cx > 0.0f)) return false;
+    // the front side: Quad_intersect's test, or x strictly outside the face's plane
+    float ce;
+    if (quad) {
+        const float dn = dot3(w, nq);
+        if (!(dn < -CCU_EPS)) return false;
+        ce = -dn;
+    } else {
+        const float xa = axis == 0 ? x.x : (axis == 1 ? x.y : x.z);
+        const float pw = (axis == 0 ? ex : (axis == 1 ? ey : ez)) + (axis == 0 ? l.x : (axis == 1 ? l.y : l.z));
+        if (!(plus ? xa > pw : xa < pw)) return false;
+        ce = fabsf(axis == 0 ? w.x : (axis == 1 ? w.y : w.z));
+    }
+    const float k = ((mo.emittance * s.emitter_scale) * ((cx * ce) / d2)) * (((float)(N * m) * area) / CCU_PI_F);
+    c = f3((T.x * (mo.color.x * mo.color.x)) * k, (T.y * (mo.color.y * mo.color.y)) * k, (T.z * (mo.color.z * mo.color.z)) * k);
+    limit = dist - CCU_NEE_DELTA;
+    return true;
+}
+
 // DESIGN §10 steps 2-4 at a hit x with normal n and throughput T, for the non-empty list emit_list[b .. b + N): draws u0..u3
 // and returns whether a shadow ray is traced; if so it runs from x along w up to `limit` and carries the contribution `c`.
-// KIND == NEE_NEAR: an emitter nearer than rho is sampled by direction instead (DESIGN §11).
+// NEE_NEAR(_MODELS): an emitter nearer than rho is sampled by direction instead (DESIGN §11).  NEE_*_MODELS: a model entry
+// is sampled by nee_model (DESIGN §12).
 template <int KIND>
 __device__ __forceinline__ bool nee_sample(const DScene &s, const EmitView &g, int b, int N, float3 x, float3 n, float3 T, uint32_t &rng, float3 &c,
                                            float3 &w, float &limit) {
@@ -979,6 +1101,10 @@ __device__ __forceinline__ bool nee_sample(const DScene &s, const EmitView &g, i
     const float u2 = rng_float(rng);
     const float u3 = rng_float(rng);
     const int4 e = __ldg(g.emit + __ldg(g.list + b + min((int)(u0 * (float)N), N - 1)));
+    if constexpr (nee_models(KIND)) {
+        const int h = __ldg(g.mhead + e.w);
+        if (h >= 0) return nee_model<nee_near_field(KIND)>(s, g, h, e, N, x, n, T, u1, u2, u3, c, w, limit);
+    }
     const float ex = (float)e.x, ey = (float)e.y, ez = (float)e.z;
     // the faces x lies strictly outside of, in the order -x, +x, -y, +y, -z, +z; 4 bits each: axis * 2 + (1 for the + face)
     unsigned faces = 0;
@@ -987,7 +1113,7 @@ __device__ __forceinline__ bool nee_sample(const DScene &s, const EmitView &g, i
     if (x.y < ey) faces |= 2u << (4 * f++); else if (x.y > (float)(e.y + 1)) faces |= 3u << (4 * f++);
     if (x.z < ez) faces |= 4u << (4 * f++); else if (x.z > (float)(e.z + 1)) faces |= 5u << (4 * f++);
     if (f == 0) return false;
-    if constexpr (KIND == NEE_NEAR) {
+    if constexpr (nee_near_field(KIND)) {
         // box distance² of x to the emitter: o_a is x's distance to the slab [e_a, e_a + 1] on axis a
         const float ox = x.x < ex ? ex - x.x : (x.x > (float)(e.x + 1) ? x.x - (float)(e.x + 1) : 0.0f);
         const float oy = x.y < ey ? ey - x.y : (x.y > (float)(e.y + 1) ? x.y - (float)(e.y + 1) : 0.0f);

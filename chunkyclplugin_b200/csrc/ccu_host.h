@@ -165,6 +165,8 @@ struct SceneInfo {
     int has_specular = 0;   // a material word 5 is not 0: CCU_RENDER_SPECULAR launches the specular kernels
     int has_emitters = 0;   // the emitter table is not empty: CCU_RENDER_EMITTER_SAMPLING launches the NEE kernels
     int emit_g0[3] = {0, 0, 0}, emit_dim[3] = {0, 0, 0}, emit_shift = 3;   // emitter grid (EmitView::g0 ...)
+    int has_model_emitters = 0;   // the wider table of CCU_RENDER_EMITTER_MODELS exists: a model emitter is in the octree
+    int memit_g0[3] = {0, 0, 0}, memit_dim[3] = {0, 0, 0}, memit_shift = 3;   // its grid
     float sky_intensity = 0;
     int sun_host[6] = {0, 0, 0, 0, 0, 0};
     bool have_sun = false, have_atlas = false, have_sky = false;
@@ -198,10 +200,12 @@ struct Scene {
     DevBuf<int> world_rec, actor_rec, tris2;          // BVH stage layout (ccu_queue.cuh)
     DevBuf<int> block_rec, mat_rec, quad_rec, aabb_rec;   // 16-byte-vectorised palettes (DScene::block_rec ...)
     DevBuf<int> emit, emit_off, emit_list;                // emitter table and cell lists (EmitView)
+    DevBuf<int> memit, memit_off, memit_list, memit_head, memit_prim;   // the wider table with model emitters (EmitView)
     DevBuf<uchar4> atlas, sky;
     SceneInfo info;
     ccu::DScene view{};   // every field that depends on the committed scene alone (commit, replicate_scene)
     ccu::EmitView emit_view{};   // the emitter table's launch view (fill_view, with `view`)
+    ccu::EmitView memit_view{};  // the wider table's launch view (CCU_RENDER_EMITTER_MODELS)
 
     // Calls f(a's buffer, b's same buffer) for every device array of a scene (replicate_scene, ccu_scene_device_bytes).
     template <class F>
@@ -211,6 +215,8 @@ struct Scene {
         f(a.world_rec, b.world_rec); f(a.actor_rec, b.actor_rec); f(a.tris2, b.tris2); f(a.block_rec, b.block_rec);
         f(a.mat_rec, b.mat_rec); f(a.quad_rec, b.quad_rec); f(a.aabb_rec, b.aabb_rec); f(a.atlas, b.atlas); f(a.sky, b.sky);
         f(a.emit, b.emit); f(a.emit_off, b.emit_off); f(a.emit_list, b.emit_list);
+        f(a.memit, b.memit); f(a.memit_off, b.memit_off); f(a.memit_list, b.memit_list); f(a.memit_head, b.memit_head);
+        f(a.memit_prim, b.memit_prim);
     }
 };
 

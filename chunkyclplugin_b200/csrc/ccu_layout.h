@@ -455,7 +455,80 @@ inline bool block_emits(const std::vector<int> &block_rec, int b) {
     return r[0] == 1 && ((r[2] & 2) || (r[6] & 0xFF));
 }
 
-inline EmitterGrid build_emitter_grid(const int *tree, size_t n, int depth, const std::vector<int> &block_rec) {
+// The emitter primitives of CCU_RENDER_EMITTER_MODELS (DESIGN §12; EmitView::mhead / mprim): per block palette position the
+// int4 index of its header in `prim`, or -1 when it is no model emitter.  A model emitter is a quad model with a quad whose
+// material emits, or an AABB model with an emitting box face (the material and flags textured_box assigns to it; +z: material
+// 0, flags 0; a face with the no-hit bit never emits).  Header {m, bbox (6 float bits: xmin, xmax, ymin, ymax, zmin, zmax of
+// the emitting primitives, block-local), 0}, then per primitive, in model order (boxes: faces -x, +x, -y, +y, -z, +z),
+// {kind, material, face flags, 13 words}: kind 6 a quad with its 13 geometry / uv words, kind axis * 2 + (1 for +) a box face
+// with the box's 6 words.
+struct ModelEmitters {
+    std::vector<int> head, prim;
+    bool any = false;
+};
+
+// Whether material pointer p of the raw material palette emits: textured emittance (flag bit 1) or an emittance byte.
+inline bool material_emits(const std::vector<int> &mp, int p) {
+    return p >= 0 && (size_t)p + 5 < mp.size() && ((mp[(size_t)p] & 2) || (mp[(size_t)p + 4] & 0xFF));
+}
+
+inline ModelEmitters build_model_emitters(const PaletteRecs &pr, const std::vector<int> &mp) {
+    ModelEmitters me;
+    const size_t n_pos = pr.block.size() / 8;
+    me.head.assign(n_pos, -1);
+    auto as_f = [](int w) { float f; memcpy(&f, &w, 4); return f; };
+    auto as_i = [](float f) { int w; memcpy(&w, &f, 4); return w; };
+    for (size_t b = 0; b < n_pos; b++) {
+        const int type = pr.block[b * 8], ref = pr.block[b * 8 + 1];
+        if (type != 2 && type != 3) continue;
+        std::vector<int> recs;
+        float lo[3] = {INFINITY, INFINITY, INFINITY}, hi[3] = {-INFINITY, -INFINITY, -INFINITY};
+        auto grow = [&](const float *p) {
+            for (int a = 0; a < 3; a++) { lo[a] = std::min(lo[a], p[a]); hi[a] = std::max(hi[a], p[a]); }
+        };
+        const std::vector<int> &src = type == 2 ? pr.aabb : pr.quad;
+        const int count = src[(size_t)ref * 4];
+        for (int i = 0; i < count; i++) {
+            const int *w = &src[(size_t)(ref + 1 + 4 * i) * 4];
+            if (type == 3) {
+                if (!material_emits(mp, w[13])) continue;
+                recs.push_back(6); recs.push_back(w[13]); recs.push_back(0);
+                for (int k = 0; k < 13; k++) recs.push_back(w[k]);
+                const float o[3] = {as_f(w[0]), as_f(w[1]), as_f(w[2])}, x[3] = {as_f(w[3]), as_f(w[4]), as_f(w[5])},
+                            y[3] = {as_f(w[6]), as_f(w[7]), as_f(w[8])};
+                const float ox[3] = {o[0] + x[0], o[1] + x[1], o[2] + x[2]}, oy[3] = {o[0] + y[0], o[1] + y[1], o[2] + y[2]};
+                const float oxy[3] = {ox[0] + y[0], ox[1] + y[1], ox[2] + y[2]};
+                grow(o); grow(ox); grow(oy); grow(oxy);
+                continue;
+            }
+            const float bx[6] = {as_f(w[0]), as_f(w[1]), as_f(w[2]), as_f(w[3]), as_f(w[4]), as_f(w[5])};
+            // faces -x, +x, -y, +y, -z, +z: material word and flag shift of textured_box
+            const int mat[6] = {w[10], w[8], w[12], w[11], w[9], 0}, shift[6] = {12, 4, 20, 16, 8, -1};
+            for (int f = 0; f < 6; f++) {
+                const int fl = shift[f] < 0 ? 0 : (w[6] >> shift[f]) & 15;
+                if ((fl & 8) || !material_emits(mp, mat[f])) continue;
+                recs.push_back(f); recs.push_back(mat[f]); recs.push_back(fl);
+                for (int k = 0; k < 13; k++) recs.push_back(k < 6 ? w[k] : 0);
+                const int axis = f >> 1;
+                float c0[3] = {bx[0], bx[2], bx[4]}, c1[3] = {bx[1], bx[3], bx[5]};
+                c0[axis] = c1[axis] = bx[2 * axis + (f & 1)];
+                grow(c0); grow(c1);
+            }
+        }
+        if (recs.empty()) continue;
+        me.any = true;
+        me.head[b] = (int)(me.prim.size() / 4);
+        const int m = (int)(recs.size() / 16);
+        const int hd[8] = {m, as_i(lo[0]), as_i(hi[0]), as_i(lo[1]), as_i(hi[1]), as_i(lo[2]), as_i(hi[2]), 0};
+        me.prim.insert(me.prim.end(), hd, hd + 8);
+        me.prim.insert(me.prim.end(), recs.begin(), recs.end());
+    }
+    return me;
+}
+
+// The table over the voxels whose leaf value b satisfies emits(b) (block_emits for DESIGN §10; with model emitters for §12).
+template <class Emits>
+inline EmitterGrid build_emitter_grid(const int *tree, size_t n, int depth, Emits emits) {
     EmitterGrid g;
     if (n == 0 || depth < 0 || depth > 30) return g;
     struct Leaf { int x, y, z, level, block; };
@@ -474,7 +547,7 @@ inline EmitterGrid build_emitter_grid(const int *tree, size_t n, int depth, cons
                 stack.push_back({(size_t)data + k, (it.x << 1) | (k >> 2), (it.y << 1) | ((k >> 1) & 1), (it.z << 1) | (k & 1), it.level - 1});
             continue;
         }
-        if (data == INT32_MIN || !block_emits(block_rec, -data)) continue;
+        if (data == INT32_MIN || !emits(-data)) continue;
         if (it.level > 6) return EmitterGrid{};   // 8^7 voxels alone exceed EMIT_MAX
         count += 1ll << (3 * it.level);
         if (count > EMIT_MAX) return EmitterGrid{};
@@ -526,6 +599,17 @@ inline EmitterGrid build_emitter_grid(const int *tree, size_t n, int depth, cons
         g.emit[4 * i] = e[i].x; g.emit[4 * i + 1] = e[i].y; g.emit[4 * i + 2] = e[i].z; g.emit[4 * i + 3] = e[i].w;
     }
     return g;
+}
+
+// The wider table of DESIGN §12: the full-cube emitters and the model emitters of `me`; empty when no model emitter is in it
+// (or it exceeds the limits of build_emitter_grid).
+inline EmitterGrid build_model_grid(const int *tree, size_t n, int depth, const PaletteRecs &pr, const ModelEmitters &me) {
+    if (!me.any) return EmitterGrid{};
+    const auto is_model = [&](int b) { return b >= 0 && (size_t)b < me.head.size() && me.head[(size_t)b] >= 0; };
+    EmitterGrid g = build_emitter_grid(tree, n, depth, [&](int b) { return block_emits(pr.block, b) || is_model(b); });
+    for (size_t i = 3; i < g.emit.size(); i += 4)
+        if (is_model(g.emit[i])) return g;
+    return EmitterGrid{};
 }
 
 }  // namespace

@@ -140,7 +140,7 @@ __device__ __forceinline__ int lean_step_flat(const DScene &s, const unsigned *_
 // Octree_octreeIntersect (octree.h:41-109) for the thread-per-ray kernels (first-hit, preview, thread-per-pixel render):
 // the air steps run on the march layout, the leaf value / block test of a non-air leaf on the value-carrying layout.
 // hi.node is left at -1 (the first-hit kernel finds the treeData index of the hit voxel by one root descent).
-template <bool DEEP, bool SPEC>
+template <bool DEEP, bool SPEC, bool CUT = false>
 __device__ __forceinline__ bool octree_intersect_lean(const DScene &s, float3 origin, float3 direction, RecordT<SPEC> &rec, HitInfo &hi) {
     March m;
     if (!march_begin(s, m, origin, direction, rec.distance)) return false;
@@ -156,7 +156,7 @@ __device__ __forceinline__ bool octree_intersect_lean(const DScene &s, float3 or
         int level;
         const int data = find_leaf_wide(s, c.bx, c.by, c.bz, level);
         float t;
-        if (march_block(s, m, data, level, rec.surf, t)) {
+        if (march_block<SPEC, CUT>(s, m, data, level, rec.surf, t, CUT)) {
             rec.distance = t;
             rec.material = data;
             hi.node = -1;
@@ -169,9 +169,9 @@ __device__ __forceinline__ bool octree_intersect_lean(const DScene &s, float3 or
 }
 
 // kernel.h:14-24 on the commit-time layouts
-template <bool DEEP, bool SPEC>
+template <bool DEEP, bool SPEC, bool CUT = false>
 __device__ __forceinline__ bool closest_intersect_lean(const DScene &s, float3 origin, float3 direction, RecordT<SPEC> &rec, HitInfo &hi) {
-    bool hit = octree_intersect_lean<DEEP>(s, origin, direction, rec, hi);
+    bool hit = octree_intersect_lean<DEEP, SPEC, CUT>(s, origin, direction, rec, hi);
     int kind = 0;
     if (bvh_pair(s, origin, direction, rec.distance, rec.surf, kind)) {
         hit = true;
@@ -182,16 +182,17 @@ __device__ __forceinline__ bool closest_intersect_lean(const DScene &s, float3 o
     return hit;
 }
 
-// MODE 0: the reference's own node array (root descent per step); 1: commit-time layouts; 2: commit-time layouts, deep world
-template <int MODE, bool SPEC>
+// MODE 0: the reference's own node array (root descent per step); 1: commit-time layouts; 2: commit-time layouts, deep world.
+// CUT: an octree hit counts only before rec.distance (march_block; emitter-sample shadow rays of CCU_RENDER_EMITTER_MODELS).
+template <int MODE, bool SPEC, bool CUT = false>
 __device__ __forceinline__ bool closest_intersect_mode(const DScene &s, float3 origin, float3 direction, RecordT<SPEC> &rec, HitInfo &hi) {
-    if (MODE == 0) return closest_intersect_ref(s, origin, direction, rec, hi);
-    return closest_intersect_lean<MODE == 2>(s, origin, direction, rec, hi);
+    if (MODE == 0) return closest_intersect_ref<SPEC, CUT>(s, origin, direction, rec, hi);
+    return closest_intersect_lean<MODE == 2, SPEC, CUT>(s, origin, direction, rec, hi);
 }
 
 // one path sample for pixel gid, thread-sequential: rayTracer.cl:40-107 (+ kernel.h:33-98, sky.h:68-93); SPEC adds the specular
 // events of CCU_RENDER_SPECULAR (DESIGN "Beyond the reference: specular materials"), NEE the emitter sampler (NeeKind) of
-// CCU_RENDER_EMITTER_SAMPLING (DESIGN §10) and CCU_RENDER_EMITTER_NEAR_FIELD (§11)
+// CCU_RENDER_EMITTER_SAMPLING (DESIGN §10), CCU_RENDER_EMITTER_NEAR_FIELD (§11) and CCU_RENDER_EMITTER_MODELS (§12)
 template <int MODE, bool SPEC, int NEE>
 __device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &g, int gid, int seed) {
     float3 color = f3(0, 0, 0), throughput = f3(1, 1, 1);
@@ -220,7 +221,7 @@ __device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &
         }
         bool emits = true;   // NEE: an emitter the previous hit's sample covered delivers no emission here
         if constexpr (NEE) {
-            emits = !(nee_prev && hi.kind == 1 && emitter_covered(s, g, rec.material, hi.bx, hi.by, hi.bz, nee_cell));
+            emits = !(nee_prev && hi.kind == 1 && emitter_covered<NEE>(s, g, rec.material, hi.bx, hi.by, hi.bz, nee_cell));
             nee_prev = false;
         }
         bool specular = false, metal = false;
@@ -273,7 +274,7 @@ __device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &
                     RecordT<SPEC> sh = rec;
                     sh.distance = limit;
                     HitInfo shi;
-                    if (!closest_intersect_mode<MODE>(s, origin, w, sh, shi)) color = color + c;
+                    if (!closest_intersect_mode<MODE, SPEC, nee_models(NEE)>(s, origin, w, sh, shi)) color = color + c;
                 }
             }
         }

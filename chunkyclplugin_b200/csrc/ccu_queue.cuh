@@ -464,7 +464,7 @@ template <int NEE>
 __device__ __forceinline__ bool q_covered(const DScene &s, const EmitView &g, const uint32_t *F, int slot, uint32_t meta, int data, const Cell &c) {
     if (!NEE || (meta & (QM_SHADOW | QM_NEE_RAY)) || !(meta & QM_NEE_PREV)) return false;
     const int3 cell = make_int3((int)F[QF_SNX * Q_SLOTS + slot], (int)F[QF_SNY * Q_SLOTS + slot], (int)F[QF_SNZ * Q_SLOTS + slot]);
-    return emitter_covered(s, g, data, c.bx, c.by, c.bz, cell);
+    return emitter_covered<NEE>(s, g, data, c.bx, c.by, c.bz, cell);
 }
 
 // BLOCK (kind_block = true) and EXIT (false): the octree part of closestIntersect (kernel.h:14-16) is finished here;
@@ -494,7 +494,9 @@ __device__ __forceinline__ bool q_stage_resolve(const DScene &s, const EmitView 
         const Cell c = march_cell(m);
         int level;
         const int data = find_leaf_wide(s, c.bx, c.by, c.bz, level);   // the kernel is only launched on the commit-time layouts
-        if (!march_block(s, m, data, level, hit, hit_t)) {
+        // NEE_*_MODELS: an emitter sample's shadow ray counts a block hit only before its limit (march_block)
+        const bool cut = nee_models(NEE) ? (QU(QF_META) & QM_NEE_RAY) != 0 : false;
+        if (!march_block<SPEC, nee_models(NEE)>(s, m, data, level, hit, hit_t, cut)) {
             QFL(QF_T) = m.t; QI(QF_STEPS) = m.steps;
             q_push(mask, QS_MARCH, lane, row);
             return true;
@@ -908,7 +910,8 @@ __device__ __forceinline__ bool q_stage_end(const DScene &s, const PassParams &w
 
 // LAY 0: the top table of the air layout fits Q_TOP_WORDS and is staged in shared memory; 1: it is read from global memory;
 // 2: deep world (64-ary nodes between the top table and the bricks).  SPEC: CCU_RENDER_SPECULAR on a scene with specular words.
-// NEE: the emitter sampler (NeeKind) of CCU_RENDER_EMITTER_SAMPLING, with CCU_RENDER_EMITTER_NEAR_FIELD for NEE_NEAR, on a scene
+// NEE: the emitter sampler (NeeKind) of CCU_RENDER_EMITTER_SAMPLING, with CCU_RENDER_EMITTER_NEAR_FIELD for NEE_NEAR(_MODELS) and
+// CCU_RENDER_EMITTER_MODELS for NEE_*_MODELS (the table `g` is then the wider one, DESIGN §12), on a scene
 // with emitters (table `g`, an argument after the others so that the kernels without it keep their parameter offsets).
 template <bool HAS_BVH, int LAY, bool SPEC, int NEE>
 __global__ void __launch_bounds__(Q_WARPS * 32, 1) k_render_queue(const __grid_constant__ DScene s, const __grid_constant__ QueueParams qp,

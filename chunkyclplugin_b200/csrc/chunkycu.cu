@@ -45,7 +45,7 @@ __global__ void k_sun_setup(const int *sun_words, float *out /* su sv sw radius_
 // rayTracer.cl:109-112 carried in registers between passes (identical arithmetic, no memory round trip).
 // MODE: 0 = the reference's own node array, 1 = commit-time layouts, 2 = commit-time layouts of a deep world.
 // SPEC: CCU_RENDER_SPECULAR on a scene with specular words; NEE: the emitter sampler (NeeKind) of CCU_RENDER_EMITTER_SAMPLING and
-// CCU_RENDER_EMITTER_NEAR_FIELD on a scene with emitters (sample_pixel).
+// CCU_RENDER_EMITTER_NEAR_FIELD / CCU_RENDER_EMITTER_MODELS on a scene with emitters (sample_pixel).
 template <int MODE, bool SPEC, int NEE>
 __global__ void __launch_bounds__(128) k_render_mega(const __grid_constant__ DScene s, const int *__restrict__ seeds, int n_passes,
                                                      int start_spp, float *res, const float *res_prev, int n_pixels,
@@ -353,6 +353,12 @@ void fill_view(ccu_host::Scene &sc) {
     g.g0 = make_int3(in.emit_g0[0], in.emit_g0[1], in.emit_g0[2]);
     g.dim = make_int3(in.emit_dim[0], in.emit_dim[1], in.emit_dim[2]);
     g.shift = in.emit_shift;
+    EmitView &mg = sc.memit_view;
+    mg.emit = reinterpret_cast<const int4 *>(sc.memit.p); mg.off = sc.memit_off.p; mg.list = sc.memit_list.p;
+    mg.g0 = make_int3(in.memit_g0[0], in.memit_g0[1], in.memit_g0[2]);
+    mg.dim = make_int3(in.memit_dim[0], in.memit_dim[1], in.memit_dim[2]);
+    mg.shift = in.memit_shift;
+    mg.mhead = sc.memit_head.p; mg.mprim = reinterpret_cast<const int4 *>(sc.memit_prim.p);
 }
 
 // The launch view with this launch's camera, rays, canvas and render params (caller holds c->mu, the scene is committed).
@@ -437,7 +443,7 @@ void dispatch(bool v, F &&f) {
 auto queue_kernel(bool bvh, int lay, bool spec, int nee) {
     decltype(&k_render_queue<false, 0, false, NEE_NONE>) k = nullptr;
     dispatch(bvh, [&](auto B) {
-        dispatch<3>(lay, [&](auto L) { dispatch(spec, [&](auto S) { dispatch<3>(nee, [&](auto N) { k = k_render_queue<B, L, S, N>; }); }); });
+        dispatch<3>(lay, [&](auto L) { dispatch(spec, [&](auto S) { dispatch<5>(nee, [&](auto N) { k = k_render_queue<B, L, S, N>; }); }); });
     });
     return k;
 }
@@ -448,9 +454,15 @@ bool specular_launch(const ccu_ctx *c) { return (c->params.flags & CCU_RENDER_SP
 
 // CCU_RENDER_EMITTER_SAMPLING launches the NEE kernels only on a scene with emitters: without one they draw nothing and compute
 // exactly what the other kernels compute.  CCU_RENDER_EMITTER_NEAR_FIELD picks the near-field sampler (NEE_NEAR) among them.
+// CCU_RENDER_EMITTER_MODELS picks the samplers of the wider table (NEE_*_MODELS, EmitView memit_view) when the scene has one;
+// without a model emitter it changes nothing.
 int nee_launch(const ccu_ctx *c) {
-    if (!((c->params.flags & CCU_RENDER_EMITTER_SAMPLING) && c->scene.info.has_emitters)) return NEE_NONE;
-    return (c->params.flags & CCU_RENDER_EMITTER_NEAR_FIELD) ? NEE_NEAR : NEE_AREA;
+    const int f = c->params.flags;
+    if (!(f & CCU_RENDER_EMITTER_SAMPLING)) return NEE_NONE;
+    if ((f & CCU_RENDER_EMITTER_MODELS) && c->scene.info.has_model_emitters)
+        return (f & CCU_RENDER_EMITTER_NEAR_FIELD) ? NEE_NEAR_MODELS : NEE_AREA_MODELS;
+    if (!c->scene.info.has_emitters) return NEE_NONE;
+    return (f & CCU_RENDER_EMITTER_NEAR_FIELD) ? NEE_NEAR : NEE_AREA;
 }
 
 }  // namespace
@@ -612,7 +624,7 @@ int ccu_ctx_create(int device_index, ccu_ctx **out) {
     for (Event &ev : c->rays_used) if (e == cudaSuccess) e = ev.create(cudaEventDisableTiming);
     for (bool bvh : {false, true})
         for (bool spec : {false, true})
-            for (int nee : {NEE_NONE, NEE_AREA, NEE_NEAR})
+            for (int nee : {NEE_NONE, NEE_AREA, NEE_NEAR, NEE_AREA_MODELS, NEE_NEAR_MODELS})
                 for (int lay = 0; lay < 3 && e == cudaSuccess; lay++)
                     e = cudaFuncSetAttribute(queue_kernel(bvh, lay, spec, nee), cudaFuncAttributeMaxDynamicSharedMemorySize, Q_SMEM_LIMIT);
     if (e == cudaSuccess) e = c->unorm.alloc(256);
@@ -800,7 +812,7 @@ int ccu_scene_commit(ccu_ctx *c) {
         for (int b = 0; (size_t)b * 8 < pr.block.size() && !any; b++) any = block_emits(pr.block, b);
         if (any) {
             const std::vector<int> &tree = host(ccu_host::OCTREE);
-            eg = build_emitter_grid(tree.data(), tree.size(), in.depth, pr.block);
+            eg = build_emitter_grid(tree.data(), tree.size(), in.depth, [&](int b) { return block_emits(pr.block, b); });
         }
         in.has_emitters = eg.emit.empty() ? 0 : 1;
         for (int a = 0; a < 3; a++) { in.emit_g0[a] = eg.g0[a]; in.emit_dim[a] = eg.dim[a]; }
@@ -808,6 +820,18 @@ int ccu_scene_commit(ccu_ctx *c) {
         CU(sc.emit.upload(eg.emit.data(), eg.emit.size(), c->stream));
         CU(sc.emit_off.upload(eg.off.data(), eg.off.size(), c->stream));
         CU(sc.emit_list.upload(eg.list.data(), eg.list.size(), c->stream));
+        // the wider table of CCU_RENDER_EMITTER_MODELS, only when a model emits (otherwise five empty arrays)
+        const ModelEmitters me = build_model_emitters(pr, host(ccu_host::MAT_PALETTE));
+        const std::vector<int> &mtree = host(ccu_host::OCTREE);
+        const EmitterGrid mg = build_model_grid(mtree.data(), mtree.size(), in.depth, pr, me);
+        in.has_model_emitters = mg.emit.empty() ? 0 : 1;
+        for (int a = 0; a < 3; a++) { in.memit_g0[a] = mg.g0[a]; in.memit_dim[a] = mg.dim[a]; }
+        in.memit_shift = mg.shift;
+        CU(sc.memit.upload(mg.emit.data(), mg.emit.size(), c->stream));
+        CU(sc.memit_off.upload(mg.off.data(), mg.off.size(), c->stream));
+        CU(sc.memit_list.upload(mg.list.data(), mg.list.size(), c->stream));
+        CU(sc.memit_head.upload(in.has_model_emitters ? me.head.data() : nullptr, in.has_model_emitters ? me.head.size() : 0, c->stream));
+        CU(sc.memit_prim.upload(in.has_model_emitters ? me.prim.data() : nullptr, in.has_model_emitters ? me.prim.size() : 0, c->stream));
     }
     // BVH stage layout (pair records + aligned triangle blocks); a scene whose BVHs it cannot hold is rendered by the
     // thread-per-pixel kernel on the reference's own arrays
@@ -934,10 +958,13 @@ int ccu_render_set_params(ccu_ctx *c, const ccu_render_params *p) {
     if (!p) return fail(CCU_EINVAL, "ccu_render_set_params: null argument");
     if (p->draw_depth < 0 || p->draw_depth >= (1 << 24) || p->max_depth < 1 || p->max_depth > 255) return fail(CCU_EINVAL, "bad render params");
     if (p->kernel != 0 && p->kernel != 1 && p->kernel != 4) return fail(CCU_EINVAL, "unknown kernel %d (0 auto, 1 thread-per-pixel, 4 wavefront)", p->kernel);
-    if (p->flags & ~(CCU_RENDER_NO_ENTITIES | CCU_RENDER_NO_SUN | CCU_RENDER_SPECULAR | CCU_RENDER_EMITTER_SAMPLING | CCU_RENDER_EMITTER_NEAR_FIELD))
+    if (p->flags & ~(CCU_RENDER_NO_ENTITIES | CCU_RENDER_NO_SUN | CCU_RENDER_SPECULAR | CCU_RENDER_EMITTER_SAMPLING | CCU_RENDER_EMITTER_NEAR_FIELD |
+                     CCU_RENDER_EMITTER_MODELS))
         return fail(CCU_EINVAL, "unknown render flags 0x%x", p->flags);
     if ((p->flags & CCU_RENDER_EMITTER_NEAR_FIELD) && !(p->flags & CCU_RENDER_EMITTER_SAMPLING))
         return fail(CCU_EINVAL, "CCU_RENDER_EMITTER_NEAR_FIELD needs CCU_RENDER_EMITTER_SAMPLING");
+    if ((p->flags & CCU_RENDER_EMITTER_MODELS) && !(p->flags & CCU_RENDER_EMITTER_SAMPLING))
+        return fail(CCU_EINVAL, "CCU_RENDER_EMITTER_MODELS needs CCU_RENDER_EMITTER_SAMPLING");
     if (!c) return fail(CCU_EINVAL, "ccu_render_set_params: null argument");
     std::lock_guard<std::mutex> lk(c->mu);
     c->params = *p;
@@ -979,6 +1006,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
     const int mode = layout_mode(c);
     const bool spec = specular_launch(c);
     const int nee = nee_launch(c);
+    const EmitView &emit_view = nee_models(nee) ? c->scene.memit_view : c->scene.emit_view;
     float *res = c->accum[c->accum_active].p;
     const float *res_prev = c->window_spp == 0 ? c->window_base : res;
     int kernel = c->params.kernel;
@@ -987,9 +1015,9 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
         const int threads = 128, blocks = (n_pixels + threads - 1) / threads;
         dispatch<3>(mode, [&](auto M) {
             dispatch(spec, [&](auto S) {
-                dispatch<3>(nee, [&](auto N) {
+                dispatch<5>(nee, [&](auto N) {
                     k_render_mega<M, S, N><<<blocks, threads, 0, c->stream>>>(s, seeds_dev, n_passes, c->window_spp, res, res_prev, n_pixels,
-                                                                        c->scene.emit_view);
+                                                                        emit_view);
                 });
             });
         });
@@ -1030,7 +1058,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
             qp.bvh_deep = c->bvh_deep.p;
         }
         const int smem = base_smem + qp.sky_texels * 4;
-        queue_kernel(bvh, lay, spec, nee)<<<grid, block, smem, c->stream>>>(s, qp, c->scene.emit_view);
+        queue_kernel(bvh, lay, spec, nee)<<<grid, block, smem, c->stream>>>(s, qp, emit_view);
 #ifdef CCU_Q_STATS
         {
             cudaStreamSynchronize(c->stream);
@@ -1435,7 +1463,7 @@ int ccu_debug_emitter_grid(const int32_t *tree, int64_t n_tree, int32_t depth, c
         return fail(CCU_EINVAL, "ccu_debug_emitter_grid: bad argument");
     const PaletteRecs pr = build_palette_recs(std::vector<int>(block_palette, block_palette + n_block),
                                               std::vector<int>(mat_palette, mat_palette + n_mat), {}, {});
-    const EmitterGrid g = build_emitter_grid(tree, (size_t)n_tree, depth, pr.block);
+    const EmitterGrid g = build_emitter_grid(tree, (size_t)n_tree, depth, [&](int b) { return block_emits(pr.block, b); });
     info[0] = g.emit.empty() ? 0 : 1;
     for (int a = 0; a < 3; a++) { info[1 + a] = g.g0[a]; info[4 + a] = g.dim[a]; }
     info[7] = g.shift;
@@ -1444,6 +1472,37 @@ int ccu_debug_emitter_grid(const int32_t *tree, int64_t n_tree, int32_t depth, c
     if (emit) std::copy(g.emit.begin(), g.emit.end(), emit);
     if (off) std::copy(g.off.begin(), g.off.end(), off);
     if (list) std::copy(g.list.begin(), g.list.end(), list);
+    return CCU_OK;
+}
+
+// Host-only check of the wider emitter table of CCU_RENDER_EMITTER_MODELS (no CUDA call): what ccu_scene_commit builds.  info =
+// {has_model_emitters, g0 x y z, dim x y z, shift, emitters, list words, head entries, prim words}.
+int ccu_debug_emitter_models(const int32_t *tree, int64_t n_tree, int32_t depth, const int32_t *block_palette, int64_t n_block,
+                             const int32_t *mat_palette, int64_t n_mat, const int32_t *quad_models, int64_t n_quad,
+                             const int32_t *aabb_models, int64_t n_aabb, int32_t info[12], int32_t *emit, int32_t *off,
+                             int32_t *list, int32_t *head, int32_t *prim) {
+    if (!tree || n_tree < 1 || depth < 0 || depth > 30 || !block_palette || n_block < 0 || !mat_palette || n_mat < 0 || !quad_models ||
+        n_quad < 0 || !aabb_models || n_aabb < 0 || !info)
+        return fail(CCU_EINVAL, "ccu_debug_emitter_models: bad argument");
+    const std::vector<int> mp(mat_palette, mat_palette + n_mat);
+    const PaletteRecs pr = build_palette_recs(std::vector<int>(block_palette, block_palette + n_block), mp,
+                                              std::vector<int>(quad_models, quad_models + n_quad),
+                                              std::vector<int>(aabb_models, aabb_models + n_aabb));
+    const ModelEmitters me = build_model_emitters(pr, mp);
+    const EmitterGrid g = build_model_grid(tree, (size_t)n_tree, depth, pr, me);
+    const bool has = !g.emit.empty();
+    info[0] = has ? 1 : 0;
+    for (int a = 0; a < 3; a++) { info[1 + a] = g.g0[a]; info[4 + a] = g.dim[a]; }
+    info[7] = g.shift;
+    info[8] = (int)(g.emit.size() / 4);
+    info[9] = (int)g.list.size();
+    info[10] = has ? (int)me.head.size() : 0;
+    info[11] = has ? (int)me.prim.size() : 0;
+    if (emit) std::copy(g.emit.begin(), g.emit.end(), emit);
+    if (off) std::copy(g.off.begin(), g.off.end(), off);
+    if (list) std::copy(g.list.begin(), g.list.end(), list);
+    if (head && has) std::copy(me.head.begin(), me.head.end(), head);
+    if (prim && has) std::copy(me.prim.begin(), me.prim.end(), prim);
     return CCU_OK;
 }
 

@@ -16,6 +16,7 @@ LIB_PATH = os.environ.get("CHUNKYCU_LIB") or os.path.join(_HERE, "libchunkycu.so
 
 CCU_RENDER_NO_ENTITIES, CCU_RENDER_NO_SUN, CCU_RENDER_SPECULAR, CCU_RENDER_EMITTER_SAMPLING = 1, 2, 4, 8
 CCU_RENDER_EMITTER_NEAR_FIELD = 128
+CCU_RENDER_EMITTER_MODELS = 256
 CCU_UNIQUE_ID_BYTES = 128
 
 CCU_OK, CCU_ENODEVICE, CCU_EINVAL, CCU_ECUDA, CCU_ENOMEM, CCU_ESTATE = 0, -1, -2, -3, -4, -5
@@ -87,6 +88,7 @@ SYMBOLS = {
     "ccu_debug_layout_lookup": (C.c_int, [_vp, _i64, _i32, _vp, _i64, _vp, _vp, _vp, _vp]),
     "ccu_debug_bvh_layout": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _i64, _vp, _i64, C.POINTER(_i64), C.POINTER(_i64), _pi32, _pi32]),
     "ccu_debug_emitter_grid": (C.c_int, [_vp, _i64, _i32, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp]),
+    "ccu_debug_emitter_models": (C.c_int, [_vp, _i64, _i32, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
     # multi-GPU
     "ccu_group_create": (C.c_int, [_vp, _i32, C.POINTER(_vp)]),
     "ccu_group_unique_id": (C.c_int, [_vp]),
@@ -196,6 +198,28 @@ def debug_emitter_grid(tree: np.ndarray, depth: int, block_palette: np.ndarray, 
     check(lib.ccu_debug_emitter_grid(*args, _ptr(emit), _ptr(off), _ptr(lst)))
     return {"has_emitters": bool(info[0]), "g0": info[1:4].copy(), "dim": info[4:7].copy(), "shift": int(info[7]),
             "emit": emit[:info[8] * 4].reshape(-1, 4), "off": off if info[0] else off[:0], "list": lst[:info[9]]}
+
+
+def debug_emitter_models(p):
+    """The wider emitter table of CCU_RENDER_EMITTER_MODELS the library builds at commit for the packed scene p (host only):
+    the keys of debug_emitter_grid plus head (int32 per block palette position: int4 index of its primitive list in prim, -1
+    for no model emitter) and prim (int32 headers and primitive records, DESIGN.md §12); all empty without a model emitter."""
+    arrs = [np.ascontiguousarray(a, dtype=np.int32) for a in (p.octree, p.block_palette, p.mat_palette, p.quad_models, p.aabb_models)]
+    tree, bp, mp, qm, am = arrs
+    info = np.zeros(12, dtype=np.int32)
+    lib = load()
+    args = (_ptr(tree), tree.size, p.octree_depth, _ptr(bp), bp.size, _ptr(mp), mp.size, _ptr(qm), qm.size, _ptr(am), am.size, _ptr(info))
+    check(lib.ccu_debug_emitter_models(*args, None, None, None, None, None))
+    cells = int(np.prod(info[4:7].astype(np.int64)))
+    emit = np.zeros(max(int(info[8]) * 4, 1), dtype=np.int32)
+    off = np.zeros(cells + 1, dtype=np.int32)
+    lst = np.zeros(max(int(info[9]), 1), dtype=np.int32)
+    head = np.zeros(max(int(info[10]), 1), dtype=np.int32)
+    prim = np.zeros(max(int(info[11]), 1), dtype=np.int32)
+    check(lib.ccu_debug_emitter_models(*args, _ptr(emit), _ptr(off), _ptr(lst), _ptr(head), _ptr(prim)))
+    return {"has_emitters": bool(info[0]), "g0": info[1:4].copy(), "dim": info[4:7].copy(), "shift": int(info[7]),
+            "emit": emit[:info[8] * 4].reshape(-1, 4), "off": off if info[0] else off[:0], "list": lst[:info[9]],
+            "head": head[:info[10]], "prim": prim[:info[11]]}
 
 
 def device_count() -> int:

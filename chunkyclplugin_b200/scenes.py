@@ -554,6 +554,14 @@ def terrain_scene(size: int = 256, width: int = 1920, height: int = 1080, seed: 
 def indoor_scene(size: int = 256, width: int = 1920, height: int = 1080, seed: int = 4242) -> PackedScene:
     """BASELINE config 3: solid stone with carved rooms/corridors, glowstone on ceilings, sun flag off."""
     pal = Palettes()
+    vox, cam = _indoor_voxels(size, seed)
+    tree, depth = build_octree(vox, pal.block_mapping)
+    return _finish(f"indoor{size}", tree, depth, pal, cam, width, height, sun_draw=False,
+                   meta={"size": size, "seed": seed})
+
+
+def _indoor_voxels(size: int, seed: int):
+    """indoor_scene's types[x, y, z] and camera"""
     vox = np.full((size, size, size), STONE, dtype=np.int32)
     cell = 16
     n = size // cell
@@ -582,7 +590,6 @@ def indoor_scene(size: int = 256, width: int = 1920, height: int = 1080, seed: i
     sel = np.zeros_like(vox, dtype=bool)
     sel[:, 1:, :] = ceil & pick
     vox[sel] = GLOWSTONE
-    tree, depth = build_octree(vox, pal.block_mapping)
     # camera inside a room near the centre
     ix = iy = iz = n // 2
     found = None
@@ -595,8 +602,7 @@ def indoor_scene(size: int = 256, width: int = 1920, height: int = 1080, seed: i
             break
     a, b, c = found
     cam = pinhole_camera((a * cell + 3.3, b * cell + 4.2, c * cell + 2.6), 35.0, -8.0, 90.0)
-    return _finish(f"indoor{size}", tree, depth, pal, cam, width, height, sun_draw=False,
-                   meta={"size": size, "seed": seed})
+    return vox, cam
 
 
 def large_world_scene(sx: int = 2048, sy: int = 256, sz: int = 2048, width: int = 3840, height: int = 2160,
@@ -819,3 +825,106 @@ def mixed_test_scene(size: int = 64, width: int = 96, height: int = 54, seed: in
     s = _finish(f"mixed{size}", base.octree, base.octree_depth, pal, cam, width, height,
                 world_bvh=wb, actor_bvh=ab, trigs=trigs, meta={"size": size})
     return s
+
+
+# --------------------------------------------------------------------------------------
+# model-block lights (CCU_RENDER_EMITTER_MODELS, DESIGN.md §12): torches and lanterns
+# --------------------------------------------------------------------------------------
+TORCH, LANTERN = 9, 10          # type indices of Palettes.block_mapping after add_model_lights
+
+
+def torch_texture(size: int = 16, seed: int = 7) -> np.ndarray:
+    """A 2-texel-wide stick (columns 7, 8) with a flame in its top three rows; every other texel, and two texels of the flame
+    tip, are alpha 0 (the alpha test cuts them)."""
+    y, x = np.mgrid[0:size, 0:size]
+    h = hash_u32(x, y, 101, seed)
+    tex = np.zeros((size, size, 4), np.uint8)
+    stick = (x >= 7) & (x <= 8)
+    flame = stick & (y < 3)
+    tex[stick] = [120, 85, 45, 255]
+    tex[flame] = [255, 210, 90, 255]
+    tex[..., 0] = np.clip(tex[..., 0].astype(np.int32) + ((h & 15).astype(np.int32) - 8) * stick, 0, 255).astype(np.uint8)
+    tex[0, 7, 3] = tex[0, 8, 3] = 0
+    return tex
+
+
+def _torch_quads(mat: int) -> List[int]:
+    """Four one-sided outward quads around the stick [7/16, 9/16] x [0, 10/16] x [7/16, 9/16] and one on its top, the sides
+    mapped to the stick's texels and the top to the flame; packed as PackedQuad words (PackedQuad.java:41-66)."""
+    a, b, t = 7 / 16, 9 / 16, 10 / 16
+    w = b - a
+    quads = []
+    for o, xv, yv in (((a, 0, a), (0, 0, w), (0, t, 0)),      # -x
+                      ((b, 0, b), (0, 0, -w), (0, t, 0)),     # +x
+                      ((b, 0, a), (-w, 0, 0), (0, t, 0)),     # -z
+                      ((a, 0, b), (w, 0, 0), (0, t, 0)),      # +z
+                      ((a, t, a), (0, 0, w), (w, 0, 0))):     # +y
+        uv = [a, w, 0.0, t] if yv[1] else [a, w, 1 - 3 / 16, 2 / 16]
+        quads += list(f2i(list(o) + list(xv) + list(yv) + uv)) + [mat, 0]
+    return [len(quads) // 15] + quads
+
+
+def _lantern_boxes(body: int, cap: int) -> List[int]:
+    """An emitting body box whose bottom (-y) face is disabled and whose +x face is flipped in u (its +z face reads material
+    0, SURVEY Q10), under a non-emitting cap box; packed as PackedAabb words (PackedAabb.java:75-102)."""
+    flags = (0b1000 << 20) | (0b0100 << 4)
+    out = [2]
+    for box, m, fl in (((5 / 16, 11 / 16, 1 / 16, 8 / 16, 5 / 16, 11 / 16), body, flags), ((6 / 16, 10 / 16, 8 / 16, 10 / 16, 6 / 16, 10 / 16), cap, 0)):
+        out += list(f2i(list(box))) + [fl] + [m] * 6
+    return out
+
+
+def add_model_lights(pal: Palettes, emittance: float = 1.0) -> Tuple[int, int]:
+    """Appends a torch (quad model, alpha-tested textured emitter) and a lantern (AABB model mixing emitting and non-emitting
+    faces) to the palettes; returns their block palette positions (type indices TORCH, LANTERN)."""
+    assert len(pal.blocks) == 2 * TORCH
+    torch = pal.put_material(pack_material(*pal.atlas.add(torch_texture()), emittance=emittance))
+    body = pal.put_material(pack_material(*pal.atlas.add(block_texture(GLOWSTONE, seed=11)), emittance=emittance))
+    cap = pal.put_material(pack_material(0, 0, textured=False, argb=_s32(0xFF404048)))
+    qptr = len(pal.quad)
+    pal.quad += _torch_quads(torch)
+    aptr = len(pal.aabb)
+    pal.aabb += _lantern_boxes(body, cap)
+    b_torch = len(pal.blocks)
+    pal.blocks += [3, qptr]
+    b_lantern = len(pal.blocks)
+    pal.blocks += [2, aptr]
+    return b_torch, b_lantern
+
+
+def indoor_models_scene(size: int = 256, width: int = 1920, height: int = 1080, seed: int = 4242) -> PackedScene:
+    """BASELINE config 3 lit only by model blocks: the rooms, corridors and camera of indoor_scene, no glowstone; a lantern
+    hangs under each ceiling voxel that indoor_scene turns into glowstone, and torches stand on 1 in 64 floor voxels."""
+    pal = Palettes()
+    add_model_lights(pal)
+    vox, cam = _indoor_voxels(size, seed)
+    X, Y, Z = np.mgrid[0:size, 0:size, 0:size]
+    lamp = vox == GLOWSTONE
+    vox[lamp] = STONE
+    below = np.zeros_like(lamp)
+    below[:, :-1, :] = lamp[:, 1:, :]
+    vox[below & (vox == AIR)] = LANTERN
+    floor = np.zeros_like(lamp)
+    floor[:, 1:, :] = (vox[:, :-1, :] == STONE) & (vox[:, 1:, :] == AIR)
+    vox[floor & ((hash_u32(X, Y, Z, seed + 2) % 64) == 0)] = TORCH
+    tree, depth = build_octree(vox, pal.block_mapping)
+    return _finish(f"indoor_models{size}", tree, depth, pal, cam, width, height, sun_draw=False,
+                   meta={"size": size, "seed": seed})
+
+
+def emissive_models(p: PackedScene, emittance: float = 1.0) -> PackedScene:
+    """p with every material that a quad or AABB model of its block palette references made emissive (emittance byte), the
+    rest unchanged: config 1 decorated with its CROSS and SLAB blocks lit."""
+    bp = np.asarray(p.block_palette, np.int64)
+    mp = np.array(p.mat_palette, np.int32)
+    mats = set()
+    for b in range(0, bp.size - 1, 2):
+        if bp[b] == 3:
+            q = int(bp[b + 1])
+            mats.update(int(p.quad_models[q + 1 + 15 * i + 13]) for i in range(int(p.quad_models[q])))
+        elif bp[b] == 2:
+            a = int(bp[b + 1])
+            mats.update(int(p.aabb_models[a + 1 + 13 * i + k]) for i in range(int(p.aabb_models[a])) for k in range(7, 13))
+    for m in mats:
+        mp[m + 4] = int(emittance * 255.0)
+    return dataclasses.replace(p, mat_palette=mp, name=p.name + "_litmodels")

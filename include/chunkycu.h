@@ -64,7 +64,8 @@ typedef struct ccu_render_params {
  * the bounce then leaves out the emission of an emitter that list covered.  On flat-coloured emitters the image's
  * expectation is unchanged.  On textured ones (colour or emittance from the atlas) it is not exactly: the sample reads the
  * texel at the sampled point, while the reference's full-cube block test reads a texel shifted by its marched-position quirk
- * (SURVEY Q2), so the two weight the texture differently.  Quads, AABB models and triangles keep the reference's behaviour.
+ * (SURVEY Q2), so the two weight the texture differently.  Quads, AABB models (see CCU_RENDER_EMITTER_MODELS) and triangles
+ * keep the reference's behaviour.
  * A scene without full-cube emitters renders exactly as without the flag.  Both render kernels implement it.  DESIGN.md §10
  * holds the exact contract. */
 #define CCU_RENDER_EMITTER_SAMPLING 8
@@ -75,6 +76,14 @@ typedef struct ccu_render_params {
  * contribution is bounded.  Farther emitters are sampled exactly as without it, and the image's expectation is that of
  * CCU_RENDER_EMITTER_SAMPLING.  DESIGN.md §11 holds the exact contract. */
 #define CCU_RENDER_EMITTER_NEAR_FIELD 128
+/* Model emitters, valid only together with CCU_RENDER_EMITTER_SAMPLING (ccu_render_set_params refuses it alone): emitter
+ * sampling also samples quad models (torches, candles, end rods) and AABB models (lanterns, campfires) with an emitting quad or
+ * box face, by a point on one of those primitives (with CCU_RENDER_EMITTER_NEAR_FIELD, by direction when the hit lies within
+ * 1/8 of them), and the bounce leaves out their emission where the list covered them.  The image's expectation is that of
+ * the flags without it, with the textured full-cube caveat above for full cubes only.  A scene without model emitters renders
+ * exactly as with CCU_RENDER_EMITTER_SAMPLING alone.  Triangles keep the reference's behaviour.  DESIGN.md §12 holds the
+ * exact contract. */
+#define CCU_RENDER_EMITTER_MODELS 256
 
 /* ---- device enumeration: RendererInstance.java:39-75,123-157 (clGetPlatformIDs/clGetDeviceIDs/clGetDeviceInfo),
  *      used by the GPU selector UI (ui/GpuSelector.java:24-87) -------------------------------------------------- */
@@ -199,6 +208,16 @@ int ccu_debug_bvh_layout(const int32_t *bvh, int64_t n_bvh, const int32_t *trigs
  * Used by the CPU test-suite. */
 int ccu_debug_emitter_grid(const int32_t *tree, int64_t n_tree, int32_t depth, const int32_t *block_palette, int64_t n_block,
                            const int32_t *mat_palette, int64_t n_mat, int32_t info[10], int32_t *emit, int32_t *off, int32_t *list);
+/* Test support, host only: the wider emitter table of CCU_RENDER_EMITTER_MODELS (DESIGN.md §12) that ccu_scene_commit builds
+ * from the octree node array and the block / material / quad / AABB palettes.  info = {has_model_emitters, grid origin x y z,
+ * grid size x y z, log2 of the cell edge, emitters, list words, head entries, primitive words}; emit, off and list as in
+ * ccu_debug_emitter_grid; head (one int per block palette position: the int4 index of its primitive list in prim, -1 for no
+ * model emitter) and prim (the headers {m, bounding box as 6 float bits, 0} and the 16-word primitive records) may be NULL
+ * (sizes only) and must otherwise hold those sizes.  Used by the CPU test-suite. */
+int ccu_debug_emitter_models(const int32_t *tree, int64_t n_tree, int32_t depth, const int32_t *block_palette, int64_t n_block,
+                             const int32_t *mat_palette, int64_t n_mat, const int32_t *quad_models, int64_t n_quad,
+                             const int32_t *aabb_models, int64_t n_aabb, int32_t info[12], int32_t *emit, int32_t *off,
+                             int32_t *list, int32_t *head, int32_t *prim);
 
 /* ---- multi-GPU: samples-per-pixel split over the GPUs of one box (SURVEY.md 8e) -------------------------------------------
  * The reference is one JVM and one device (RendererInstance.java:81-101).  A group is N contexts, each holding a full scene

@@ -80,6 +80,9 @@ public final class ChunkyCu {
     public static final int RENDER_NO_ENTITIES = 1, RENDER_NO_SUN = 2, RENDER_SPECULAR = 4, RENDER_EMITTER_SAMPLING = 8;
     /** ccu_render_params.flags: near-field emitter sampling (DESIGN §11), valid only together with RENDER_EMITTER_SAMPLING. */
     public static final int RENDER_EMITTER_NEAR_FIELD = 128;
+    /** ccu_render_params.flags: emitter sampling also samples quad and AABB model emitters (DESIGN §12), valid only together
+     *  with RENDER_EMITTER_SAMPLING. */
+    public static final int RENDER_EMITTER_MODELS = 256;
     private static final StructLayout RENDER_PARAMS = MemoryLayout.structLayout(JAVA_INT.withName("draw_depth"), JAVA_INT.withName("max_depth"),
             JAVA_FLOAT.withName("emitter_scale"), JAVA_INT.withName("kernel"), JAVA_INT.withName("flags"));
 

@@ -1,9 +1,9 @@
-"""ctypes binding of the CPU restatement of CCU_RENDER_SPECULAR, CCU_RENDER_EMITTER_SAMPLING and CCU_RENDER_EMITTER_NEAR_FIELD
-(specular_oracle.c).  TEST INFRASTRUCTURE ONLY.
+"""ctypes binding of the CPU restatement of CCU_RENDER_SPECULAR, CCU_RENDER_EMITTER_SAMPLING, CCU_RENDER_EMITTER_NEAR_FIELD
+and CCU_RENDER_EMITTER_MODELS (specular_oracle.c).  TEST INFRASTRUCTURE ONLY.
 
 ``SpecularOracle`` is the parity oracle (``oracle.Oracle``) with the specular events of DESIGN.md section 9 in its path
-loop; ``FlagsOracle`` takes the render flags and adds the emitter sampling of sections 10 and 11, with the emitter table that
-``emitter_grid`` builds from the packed arrays.  Everything else - first hit, preview, counters - is the oracle's.  Like the
+loop; ``FlagsOracle`` takes the render flags and adds the emitter sampling of sections 10 to 12, with the emitter table that
+``emitter_grid`` builds from the packed arrays (``model_emitters`` adds the model emitters of section 12).  Everything else - first hit, preview, counters - is the oracle's.  Like the
 oracle, only tests/ and scripts use it.
 """
 from __future__ import annotations
@@ -41,10 +41,10 @@ def lib():
 
 class _Grid(C.Structure):
     _fields_ = [("emit", C.c_void_p), ("off", C.c_void_p), ("list", C.c_void_p),
-                ("g0", C.c_int32 * 3), ("dim", C.c_int32 * 3), ("shift", C.c_int32)]
+                ("g0", C.c_int32 * 3), ("dim", C.c_int32 * 3), ("shift", C.c_int32), ("mhead", C.c_void_p), ("mprim", C.c_void_p)]
 
 
-CCU_RENDER_SPECULAR, CCU_RENDER_EMITTER_SAMPLING, CCU_RENDER_EMITTER_NEAR_FIELD = 4, 8, 128
+CCU_RENDER_SPECULAR, CCU_RENDER_EMITTER_SAMPLING, CCU_RENDER_EMITTER_NEAR_FIELD, CCU_RENDER_EMITTER_MODELS = 4, 8, 128, 256
 EMIT_SHIFT0, EMIT_CELL_BUDGET, EMIT_MAX = 3, 1 << 21, 1 << 18      # DESIGN.md section 10
 
 
@@ -80,11 +80,74 @@ def emitter_blocks(block_palette: np.ndarray, mat_palette: np.ndarray) -> np.nda
     return out
 
 
-def emitter_grid(p) -> dict:
-    """The emitter table and cell lists of DESIGN.md section 10 for a packed scene (same keys as native.debug_emitter_grid)."""
+def _f32(words) -> np.ndarray:
+    return np.asarray(words, np.int32).view(np.float32)
+
+
+def _material_emits(mp: np.ndarray, ptr: int) -> bool:
+    return 0 <= ptr and ptr + 5 < mp.size and bool((mp[ptr] & 2) or (mp[ptr + 4] & 0xFF))
+
+
+def model_emitters(p):
+    """DESIGN.md section 12: (head, prim) of the model emitters, as native.debug_emitter_models returns them.  head[b] is the
+    int4 index in prim of palette position b's emitting primitives, -1 for no model emitter; prim holds per model emitter the
+    header {m, bounding box (float32 bits: xmin, xmax, ymin, ymax, zmin, zmax), 0} and m records of 16 words {kind, material,
+    face flags, 13 words}: kind 6 a quad and its 13 words, kind axis * 2 + (1 for +) a box face and the box's 6 words."""
+    bp = np.asarray(p.block_palette, np.int64)
+    mp = np.asarray(p.mat_palette, np.int64)
+    quads, aabbs = np.asarray(p.quad_models, np.int32), np.asarray(p.aabb_models, np.int32)
+    n_pos = max(bp.size - 1, 1)
+    head = np.full(n_pos, -1, np.int32)
+    prim = []
+    for b in range(bp.size - 1):
+        typ, ptr = int(bp[b]), int(bp[b + 1])
+        if typ not in (2, 3):
+            continue
+        src, words = (aabbs, 13) if typ == 2 else (quads, 15)
+        if ptr < 0 or ptr >= src.size or src[ptr] < 0 or ptr + 1 + int(src[ptr]) * words > src.size:
+            continue
+        recs, pts = [], []
+        for i in range(int(src[ptr])):
+            w = src[ptr + 1 + i * words:ptr + 1 + (i + 1) * words]
+            if typ == 3:
+                if not _material_emits(mp, int(w[13])):
+                    continue
+                recs.append([6, int(w[13]), 0] + [int(v) for v in w[:13]])
+                o, x, y = _f32(w[0:3]), _f32(w[3:6]), _f32(w[6:9])
+                pts += [o, o + x, o + y, (o + x) + y]
+                continue
+            box = _f32(w[0:6])
+            for f, (mat, sh) in enumerate(((w[10], 12), (w[8], 4), (w[12], 20), (w[11], 16), (w[9], 8), (0, None))):
+                fl = 0 if sh is None else (int(w[6]) >> sh) & 15
+                if fl & 8 or not _material_emits(mp, int(mat)):
+                    continue
+                recs.append([f, int(mat), fl] + [int(v) for v in w[:6]] + [0] * 7)
+                axis = f >> 1
+                lo, hi = box[0::2].copy(), box[1::2].copy()
+                lo[axis] = hi[axis] = box[2 * axis + (f & 1)]
+                pts += [lo, hi]
+        if not recs:
+            continue
+        pts = np.stack(pts).astype(np.float32)
+        bb = np.stack([pts.min(0), pts.max(0)], 1).reshape(-1).astype(np.float32).view(np.int32)
+        head[b] = sum(len(r) for r in prim) // 4
+        prim.append([len(recs)] + [int(v) for v in bb] + [0])
+        prim += recs
+    return head, np.array([v for r in prim for v in r], np.int32)
+
+
+def emitter_grid(p, models: bool = False) -> dict:
+    """The emitter table and cell lists of DESIGN.md section 10 for a packed scene (same keys as native.debug_emitter_grid).
+    models: the wider table of section 12, with "head" / "prim" (model_emitters); it is empty unless it holds a model emitter."""
     empty = {"has_emitters": False, "g0": np.zeros(3, np.int32), "dim": np.zeros(3, np.int32), "shift": EMIT_SHIFT0,
              "emit": np.zeros((0, 4), np.int32), "off": np.zeros(0, np.int32), "list": np.zeros(0, np.int32)}
     emits = emitter_blocks(p.block_palette, p.mat_palette)
+    if models:
+        head, prim = model_emitters(p)
+        empty.update(head=np.zeros(0, np.int32), prim=np.zeros(0, np.int32))
+        emits = emits | (head[:emits.size] >= 0)
+        if not (head >= 0).any():
+            return empty
     corner, level, value = _leaves(p.octree, p.octree_depth)
     sel = (value >= 0) & (value < emits.size)
     sel[sel] = emits[value[sel]]
@@ -115,8 +178,13 @@ def emitter_grid(p) -> dict:
     order = np.lexsort((idx, lin))
     off = np.zeros(int(np.prod(dim)) + 1, np.int64)
     np.add.at(off, lin + 1, 1)
-    return {"has_emitters": True, "g0": g0.astype(np.int32), "dim": dim.astype(np.int32), "shift": shift,
-            "emit": e.astype(np.int32), "off": np.cumsum(off).astype(np.int32), "list": idx[order].astype(np.int32)}
+    out = {"has_emitters": True, "g0": g0.astype(np.int32), "dim": dim.astype(np.int32), "shift": shift,
+           "emit": e.astype(np.int32), "off": np.cumsum(off).astype(np.int32), "list": idx[order].astype(np.int32)}
+    if models:
+        if not (head[e[:, 3]] >= 0).any():
+            return empty
+        out.update(head=head, prim=prim)
+    return out
 
 
 class SpecularOracle(oracle.Oracle):
@@ -142,18 +210,23 @@ class SpecularOracle(oracle.Oracle):
 
 class FlagsOracle(oracle.Oracle):
     """oracle.Oracle whose render() runs the path loop with the given CCU_RENDER_SPECULAR / CCU_RENDER_EMITTER_SAMPLING /
-    CCU_RENDER_EMITTER_NEAR_FIELD bits (the other flags act on the scene: oracle.edge_rays.without_sun, or empty BVHs for
-    CCU_RENDER_NO_ENTITIES)."""
+    CCU_RENDER_EMITTER_NEAR_FIELD / CCU_RENDER_EMITTER_MODELS bits (the other flags act on the scene:
+    oracle.edge_rays.without_sun, or empty BVHs for CCU_RENDER_NO_ENTITIES).  With CCU_RENDER_EMITTER_MODELS the wider table
+    of section 12 is sampled when the scene has one, else the table of section 10."""
 
     def __init__(self, scene, flags: int = 0, **kw):
         super().__init__(scene, **kw)
         self.flags = flags
-        self.grid = emitter_grid(scene)
+        self.grid = emitter_grid(scene, models=True) if flags & CCU_RENDER_EMITTER_MODELS else None
+        if not (self.grid and self.grid["has_emitters"]):
+            self.grid = emitter_grid(scene)
         g = _Grid()
-        for k in ("emit", "off", "list"):
+        for k in ("emit", "off", "list", "head", "prim"):
+            if k not in self.grid:
+                continue
             a = np.ascontiguousarray(self.grid[k], dtype=np.int32)
             self._keep["grid_" + k] = a
-            setattr(g, k, a.ctypes.data)
+            setattr(g, {"head": "mhead", "prim": "mprim"}.get(k, k), a.ctypes.data)
         g.g0[:] = [int(v) for v in self.grid["g0"]]
         g.dim[:] = [int(v) for v in self.grid["dim"]]
         g.shift = self.grid["shift"]

@@ -1,6 +1,6 @@
 /*
  * specular_oracle.c - CPU restatement of CCU_RENDER_SPECULAR (DESIGN.md section 9) and CCU_RENDER_EMITTER_SAMPLING
- * (section 10).  TEST INFRASTRUCTURE ONLY.
+ * (sections 10-12).  TEST INFRASTRUCTURE ONLY.
  *
  * The reference has no specular path, so there is nothing of it to pin this file against: DESIGN.md section 9 is the contract,
  * this file restates it, and the tests hold this restatement and the CUDA kernels to each other bit for bit (plus analytic and
@@ -79,7 +79,7 @@ static float intersect_block_w5(const Ctx *c, int block, int bx, int by, int bz,
 }
 
 /* octree_intersect (octree.h:41-109) */
-static int octree_intersect_w5(const Ctx *c, const Path *ray, Record *rec, uint32_t *w5, int vox[3]) {
+static int octree_intersect_w5(const Ctx *c, const Path *ray, Record *rec, uint32_t *w5, int vox[3], int cut) {
     const OracleScene *s = c->sc;
     const int32_t *tree = s->octree;
     int depth = s->octree_depth;
@@ -116,7 +116,8 @@ static int octree_intersect_w5(const Ctx *c, const Path *ray, Record *rec, uint3
         lx = bx >> level; ly = by >> level; lz = bz >> level;
         if (data != 0) {
             float dist = intersect_block_w5(c, data, bx, by, bz, rec, w5, pos, ray->direction, inv);
-            if (dist == dist) {
+            /* cut (section 12): an emitter sample's shadow ray counts a block hit only before its limit */
+            if (dist == dist && !(cut && !(dist_march + dist < rec->distance))) {
                 rec->distance = dist_march + dist;
                 rec->material = data;
                 rec->hit_node = node;
@@ -196,10 +197,10 @@ static int bvh_intersect_w5(const Ctx *c, const int32_t *bvh, const Path *ray, R
 }
 
 /* closest_intersect (kernel.h:14-24) */
-static int closest_intersect_w5(const Ctx *c, const Path *ray, Record *rec, uint32_t *w5, int vox[3]) {
+static int closest_intersect_w5(const Ctx *c, const Path *ray, Record *rec, uint32_t *w5, int vox[3], int cut) {
     int hit = 0;
     c->cnt->rays++;
-    hit |= octree_intersect_w5(c, ray, rec, w5, vox);
+    hit |= octree_intersect_w5(c, ray, rec, w5, vox, cut);
     hit |= bvh_intersect_w5(c, c->sc->world_bvh, ray, rec, w5, 2);
     hit |= bvh_intersect_w5(c, c->sc->actor_bvh, ray, rec, w5, 3);
     if (hit) rec->point = vadd(ray->origin, vscale(ray->direction, rec->distance - OFFSET));
@@ -240,6 +241,9 @@ typedef struct {
     const int32_t *off;    /* cell lists in CSR form */
     const int32_t *list;
     int32_t g0[3], dim[3], shift;
+    const int32_t *mhead;  /* section 12: per block palette position the int4 index of its primitives in mprim, or -1; NULL
+                              for the table of section 10 */
+    const int32_t *mprim;
 } EmitterGrid;
 
 static int voxel_cell(const EmitterGrid *g, int vx, int vy, int vz, int cl[3]) {
@@ -261,9 +265,8 @@ static int point_cell(const EmitterGrid *g, v3 x, int cl[3]) {
 /* the emission rule: an octree hit on an emitter voxel whose cell is within Chebyshev distance 1 of the sampled cell */
 static int emitter_covered(const Ctx *c, const EmitterGrid *g, int block, const int vox[3], const int cell[3]) {
     const int32_t *bp = c->sc->block_palette, *mp = c->sc->mat_palette;
-    if (bp[block] != 1) return 0;
-    int ptr = bp[block + 1];
-    if (!((mp[ptr] & 2) || (mp[ptr + 4] & 0xFF))) return 0;
+    int cube = bp[block] == 1 && ((mp[bp[block + 1]] & 2) || (mp[bp[block + 1] + 4] & 0xFF));
+    if (!cube && !(g->mhead && g->mhead[block] >= 0)) return 0;
     int e[3];
     if (!voxel_cell(g, vox[0], vox[1], vox[2], e)) return 0;
     return abs(e[0] - cell[0]) <= 1 && abs(e[1] - cell[1]) <= 1 && abs(e[2] - cell[2]) <= 1;
@@ -332,8 +335,100 @@ static int nee_near(const Ctx *c, const int32_t *e, int n, v3 x, v3 normal, v3 T
     return 1;
 }
 
+/* ---- model emitters (DESIGN.md section 12) ---- */
+/* step 3 for a model entry e whose primitives start at int4 index h of g->mprim: the near branch (the voxel's block test along a
+ * cosine-weighted direction) or a point on primitive min((int)(u1 m), m - 1) */
+static int nee_model(const Ctx *c, const EmitterGrid *g, int h, const int32_t *e, int n, int near, v3 x, v3 normal, v3 T, float u1,
+                     float u2, float u3, v3 *out, v3 *w, float *limit) {
+    const int32_t *hd = g->mprim + 4 * (size_t)h;
+    int m = hd[0];
+    float ex = (float)e[0], ey = (float)e[1], ez = (float)e[2];
+    if (near) {
+        float lo[3] = {ex + as_float(hd[1]), ey + as_float(hd[3]), ez + as_float(hd[5])};
+        float hi[3] = {ex + as_float(hd[2]), ey + as_float(hd[4]), ez + as_float(hd[6])};
+        float o[3];
+        for (int a = 0; a < 3; a++) {
+            float xa = vget(x, a);
+            o[a] = xa < lo[a] ? lo[a] - xa : (xa > hi[a] ? xa - hi[a] : 0.0f);
+        }
+        if ((o[0] * o[0] + o[1] * o[1]) + o[2] * o[2] < NEE_RHO2) {
+            *w = diffuse_direction(c, normal, u2, u3);
+            v3 inv = V(1.0f / w->x, 1.0f / w->y, 1.0f / w->z);
+            Record r;
+            record_new(&r);
+            r.emittance = 0;
+            float t = intersect_block(c, e[3], e[0], e[1], e[2], &r, x, *w, inv);
+            if (t != t || !(r.emittance > 0.0f)) return 0;
+            float kk = (r.emittance * c->sc->emitter_scale) * (float)n;
+            *out = V((T.x * (r.color[0] * r.color[0])) * kk, (T.y * (r.color[1] * r.color[1])) * kk, (T.z * (r.color[2] * r.color[2])) * kk);
+            *limit = t - NEE_DELTA;
+            return 1;
+        }
+    }
+    int j = (int)(u1 * (float)m);
+    if (j > m - 1) j = m - 1;
+    const int32_t *r = hd + 8 + 16 * (size_t)j;
+    const int32_t *q = r + 3;    /* the 13 words */
+    int quad = r[0] == 6, axis = r[0] >> 1, plus = r[0] & 1;
+    v3 l, nq = V(0, 0, 0);
+    float u, v, area;
+    if (quad) {
+        v3 qo = V(as_float(q[0]), as_float(q[1]), as_float(q[2]));
+        v3 xv = V(as_float(q[3]), as_float(q[4]), as_float(q[5]));
+        v3 yv = V(as_float(q[6]), as_float(q[7]), as_float(q[8]));
+        l = vadd(vadd(qo, vscale(xv, u2)), vscale(yv, u3));
+        u = as_float(q[9]) + u2 * as_float(q[10]);
+        v = as_float(q[11]) + u3 * as_float(q[12]);
+        v3 cr = vcross(xv, yv);
+        nq = vnormalize(cr);
+        area = sqrtf(vdot(cr, cr));
+    } else {
+        float b[6];
+        for (int k = 0; k < 6; k++) b[k] = as_float(q[k]);
+        int a1 = axis == 0 ? 1 : 0, a2 = axis == 2 ? 1 : 2;
+        float s1 = b[2 * a1 + 1] - b[2 * a1], s2 = b[2 * a2 + 1] - b[2 * a2];
+        float lv[3];
+        lv[axis] = b[2 * axis + plus];
+        lv[a1] = b[2 * a1] + u2 * s1;
+        lv[a2] = b[2 * a2] + u3 * s2;
+        l = V(lv[0], lv[1], lv[2]);
+        area = s1 * s2;
+        if (axis == 0) { u = plus ? 1.0f - l.z : l.z; v = l.y; }
+        else if (axis == 1) { u = l.x; v = plus ? 1.0f - l.z : l.z; }
+        else { u = plus ? l.x : 1.0f - l.x; v = l.y; }
+        int fl = r[2];
+        if (fl & 4) u = 1.0f - u;
+        if (fl & 2) v = 1.0f - v;
+        if (fl & 1) { float t = u; u = v; v = t; }
+    }
+    Record mr;
+    record_new(&mr);
+    if (!material_sample(c, r[1], &mr, u, v)) return 0;
+    v3 dv = vsub(V(ex + l.x, ey + l.y, ez + l.z), x);
+    float d2 = vdot(dv, dv);
+    float dist = sqrtf(d2);
+    *w = vscale(dv, 1.0f / dist);
+    float cx = vdot(*w, normal);
+    if (!(cx > 0.0f)) return 0;
+    float ce;
+    if (quad) {
+        float dn = vdot(*w, nq);
+        if (!(dn < -EPS)) return 0;
+        ce = -dn;
+    } else {
+        float pw = vget(V(ex, ey, ez), axis) + vget(l, axis);
+        if (!(plus ? vget(x, axis) > pw : vget(x, axis) < pw)) return 0;
+        ce = fabsf(vget(*w, axis));
+    }
+    float kk = ((mr.emittance * c->sc->emitter_scale) * ((cx * ce) / d2)) * (((float)(n * m) * area) / PI_F);
+    *out = V((T.x * (mr.color[0] * mr.color[0])) * kk, (T.y * (mr.color[1] * mr.color[1])) * kk, (T.z * (mr.color[2] * mr.color[2])) * kk);
+    *limit = dist - NEE_DELTA;
+    return 1;
+}
+
 /* steps 2-4: the four draws, the emitter, face and point, the material at the point and the contribution; returns 0 when
- * no shadow ray is traced.  near: an emitter whose box distance^2 is below rho^2 is sampled by nee_near (section 11). */
+ * no shadow ray is traced.  near: an emitter whose box distance^2 is below rho^2 is sampled by nee_near (section 11).  With
+ * the table of section 12 a model entry is sampled by nee_model. */
 static int nee_sample(const Ctx *c, const EmitterGrid *g, int near, int b, int n, v3 x, v3 normal, v3 T, uint32_t *state, v3 *out,
                       v3 *w, float *limit) {
     float u0 = rng_float(state);
@@ -343,6 +438,7 @@ static int nee_sample(const Ctx *c, const EmitterGrid *g, int near, int b, int n
     int i = (int)(u0 * (float)n);
     if (i > n - 1) i = n - 1;
     const int32_t *e = g->emit + 4 * (size_t)g->list[b + i];
+    if (g->mhead && g->mhead[e[3]] >= 0) return nee_model(c, g, g->mhead[e[3]], e, n, near, x, normal, T, u1, u2, u3, out, w, limit);
     float ex = (float)e[0], ey = (float)e[1], ez = (float)e[2];
     int faces[3], f = 0;
     if (x.x < ex) faces[f++] = 0; else if (x.x > (float)(e[0] + 1)) faces[f++] = 1;
@@ -398,7 +494,7 @@ static v3 sample_pixel_ext(const Ctx *c, int gid, int32_t seed, int spec, const 
     c->cnt->samples++;
     for (;;) {
         c->cnt->segments++;
-        if (!closest_intersect_w5(c, &p, &rec, &w5, vox)) {
+        if (!closest_intersect_w5(c, &p, &rec, &w5, vox, 0)) {
             rec.emittance = 1;
             intersect_sky(c, &p, &rec);
             break;
@@ -438,7 +534,13 @@ static v3 sample_pixel_ext(const Ctx *c, int gid, int32_t seed, int spec, const 
                     q.direction = w;
                     Record s = rec;
                     s.distance = limit;
-                    if (!closest_intersect(c, &q, &s)) p.pix_color = vadd(p.pix_color, contrib);
+                    if (g->mhead) {   /* section 12: the shadow ray counts a block hit only before its limit */
+                        uint32_t sw5;
+                        int svox[3];
+                        if (!closest_intersect_w5(c, &q, &s, &sw5, svox, 1)) p.pix_color = vadd(p.pix_color, contrib);
+                    } else if (!closest_intersect(c, &q, &s)) {
+                        p.pix_color = vadd(p.pix_color, contrib);
+                    }
                 }
             }
         }
