@@ -167,6 +167,8 @@ struct SceneInfo {
     int emit_g0[3] = {0, 0, 0}, emit_dim[3] = {0, 0, 0}, emit_shift = 3;   // emitter grid (EmitView::g0 ...)
     int has_model_emitters = 0;   // the wider table of CCU_RENDER_EMITTER_MODELS exists: a model emitter is in the octree
     int memit_g0[3] = {0, 0, 0}, memit_dim[3] = {0, 0, 0}, memit_shift = 3;   // its grid
+    int has_biome = 0;      // biome colours were set: CCU_RENDER_BIOME_TINT launches the biome kernels
+    int biome_box[4] = {0, 0, 0, 0};   // the biome grid's chunk box (BiomeView::x0, z0, gx, gz)
     float sky_intensity = 0;
     int sun_host[6] = {0, 0, 0, 0, 0, 0};
     bool have_sun = false, have_atlas = false, have_sky = false;
@@ -192,6 +194,12 @@ struct PackedArray {
     std::shared_ptr<const std::vector<int>> host;
 };
 
+// The biome colours of ccu_scene_set_biome_colors as given (n chunks); commit lays them out (build_biome_layout).
+struct BiomeColors {
+    std::vector<int32_t> chunks;   // n x {cx, cz}
+    std::vector<float> rgb;        // n x 3 planes x 256 texels x 3
+};
+
 // Everything a context knows about its scene: the uploads, the layouts commit builds from them, and the launch view.
 struct Scene {
     PackedArray arrays[N_ARRAYS];
@@ -201,11 +209,15 @@ struct Scene {
     DevBuf<int> block_rec, mat_rec, quad_rec, aabb_rec;   // 16-byte-vectorised palettes (DScene::block_rec ...)
     DevBuf<int> emit, emit_off, emit_list;                // emitter table and cell lists (EmitView)
     DevBuf<int> memit, memit_off, memit_list, memit_head, memit_prim;   // the wider table with model emitters (EmitView)
+    DevBuf<int> biome_grid;                               // biome colours (BiomeView), only when set
+    DevBuf<float4> biome_tiles;
+    std::shared_ptr<const BiomeColors> biome;             // set while the scene has biome colours; shared by a replica
     DevBuf<uchar4> atlas, sky;
     SceneInfo info;
     ccu::DScene view{};   // every field that depends on the committed scene alone (commit, replicate_scene)
     ccu::EmitView emit_view{};   // the emitter table's launch view (fill_view, with `view`)
     ccu::EmitView memit_view{};  // the wider table's launch view (CCU_RENDER_EMITTER_MODELS)
+    ccu::BiomeView biome_view{};  // the biome colours' launch view (CCU_RENDER_BIOME_TINT)
 
     // Calls f(a's buffer, b's same buffer) for every device array of a scene (replicate_scene, ccu_scene_device_bytes).
     template <class F>
@@ -216,7 +228,7 @@ struct Scene {
         f(a.mat_rec, b.mat_rec); f(a.quad_rec, b.quad_rec); f(a.aabb_rec, b.aabb_rec); f(a.atlas, b.atlas); f(a.sky, b.sky);
         f(a.emit, b.emit); f(a.emit_off, b.emit_off); f(a.emit_list, b.emit_list);
         f(a.memit, b.memit); f(a.memit_off, b.memit_off); f(a.memit_list, b.memit_list); f(a.memit_head, b.memit_head);
-        f(a.memit_prim, b.memit_prim);
+        f(a.memit_prim, b.memit_prim); f(a.biome_grid, b.biome_grid); f(a.biome_tiles, b.biome_tiles);
     }
 };
 

@@ -3,6 +3,7 @@
 #pragma once
 #include <algorithm>
 #include <cmath>
+#include <cstdint>
 #include <cstdlib>
 #include <cstring>
 #include <thread>
@@ -610,6 +611,52 @@ inline EmitterGrid build_model_grid(const int *tree, size_t n, int depth, const 
     for (size_t i = 3; i < g.emit.size(); i += 4)
         if (is_model(g.emit[i])) return g;
     return EmitterGrid{};
+}
+
+// ------------------------------------------------------------------------------------------------------
+// biome colours of CCU_RENDER_BIOME_TINT (BiomeView, DESIGN §13)
+// ------------------------------------------------------------------------------------------------------
+// chunks: n x {cx, cz}; rgb: n x 3 planes x 256 texels x 3 floats, as ccu_scene_set_biome_colors takes them (already checked
+// there).  The grid covers the chunks' bounding box: gx x gz chunk indices from chunk (x0, z0), index (cx - x0) * gz + (cz - z0),
+// -1 = no tile; tiles: the same texels as {r, g, b, 0}.  status: 0 built; 1 chunk `bad` lies outside the octree's `extent` x
+// `extent` chunks (extent = max(1, 2^depth / 16)); 2 the bounding box has more than CCU_BIOME_GRID_MAX cells (nothing built).
+#define CCU_BIOME_GRID_MAX (1ll << 24)   // grid cells (64 MiB): every chunk of a depth-16 octree
+struct BiomeLayout {
+    int x0 = 0, z0 = 0, gx = 0, gz = 0;
+    int64_t extent = 1;
+    std::vector<int> grid;
+    std::vector<float> tiles;   // float4 per texel
+    int status = 0;
+    int64_t bad = -1;
+};
+inline BiomeLayout build_biome_layout(const int32_t *chunks, const float *rgb, int64_t n, int depth) {
+    BiomeLayout b;
+    b.extent = depth > 4 ? 1ll << (depth - 4) : 1;
+    if (n == 0) return b;
+    int64_t lx = INT64_MAX, lz = INT64_MAX, hx = -1, hz = -1;
+    for (int64_t i = 0; i < n; i++) {
+        const int64_t cx = chunks[2 * i], cz = chunks[2 * i + 1];
+        if (cx >= b.extent || cz >= b.extent) {
+            b.status = 1;
+            b.bad = i;
+            return b;
+        }
+        lx = std::min(lx, cx); hx = std::max(hx, cx);
+        lz = std::min(lz, cz); hz = std::max(hz, cz);
+    }
+    if ((hx - lx + 1) * (hz - lz + 1) > CCU_BIOME_GRID_MAX) {
+        b.status = 2;
+        return b;
+    }
+    b.x0 = (int)lx; b.z0 = (int)lz; b.gx = (int)(hx - lx + 1); b.gz = (int)(hz - lz + 1);
+    b.grid.assign((size_t)b.gx * b.gz, -1);
+    b.tiles.assign((size_t)n * 3 * 256 * 4, 0.0f);
+    for (int64_t i = 0; i < n; i++) {
+        b.grid[(size_t)(chunks[2 * i] - b.x0) * b.gz + (size_t)(chunks[2 * i + 1] - b.z0)] = (int)i;
+        for (size_t t = 0; t < 3 * 256; t++)
+            for (int c = 0; c < 3; c++) b.tiles[((size_t)i * 3 * 256 + t) * 4 + c] = rgb[((size_t)i * 3 * 256 + t) * 3 + c];
+    }
+    return b;
 }
 
 }  // namespace

@@ -140,7 +140,7 @@ __device__ __forceinline__ int lean_step_flat(const DScene &s, const unsigned *_
 // Octree_octreeIntersect (octree.h:41-109) for the thread-per-ray kernels (first-hit, preview, thread-per-pixel render):
 // the air steps run on the march layout, the leaf value / block test of a non-air leaf on the value-carrying layout.
 // hi.node is left at -1 (the first-hit kernel finds the treeData index of the hit voxel by one root descent).
-template <bool DEEP, bool SPEC, bool CUT = false>
+template <bool DEEP, bool SPEC, bool CUT = false, bool BIOME = false>
 __device__ __forceinline__ bool octree_intersect_lean(const DScene &s, float3 origin, float3 direction, RecordT<SPEC> &rec, HitInfo &hi) {
     March m;
     if (!march_begin(s, m, origin, direction, rec.distance)) return false;
@@ -156,7 +156,7 @@ __device__ __forceinline__ bool octree_intersect_lean(const DScene &s, float3 or
         int level;
         const int data = find_leaf_wide(s, c.bx, c.by, c.bz, level);
         float t;
-        if (march_block<SPEC, CUT>(s, m, data, level, rec.surf, t, CUT)) {
+        if (march_block<SPEC, CUT, BIOME>(s, m, data, level, rec.surf, t, CUT)) {
             rec.distance = t;
             rec.material = data;
             hi.node = -1;
@@ -169,9 +169,9 @@ __device__ __forceinline__ bool octree_intersect_lean(const DScene &s, float3 or
 }
 
 // kernel.h:14-24 on the commit-time layouts
-template <bool DEEP, bool SPEC, bool CUT = false>
+template <bool DEEP, bool SPEC, bool CUT = false, bool BIOME = false>
 __device__ __forceinline__ bool closest_intersect_lean(const DScene &s, float3 origin, float3 direction, RecordT<SPEC> &rec, HitInfo &hi) {
-    bool hit = octree_intersect_lean<DEEP, SPEC, CUT>(s, origin, direction, rec, hi);
+    bool hit = octree_intersect_lean<DEEP, SPEC, CUT, BIOME>(s, origin, direction, rec, hi);
     int kind = 0;
     if (bvh_pair(s, origin, direction, rec.distance, rec.surf, kind)) {
         hit = true;
@@ -184,16 +184,18 @@ __device__ __forceinline__ bool closest_intersect_lean(const DScene &s, float3 o
 
 // MODE 0: the reference's own node array (root descent per step); 1: commit-time layouts; 2: commit-time layouts, deep world.
 // CUT: an octree hit counts only before rec.distance (march_block; emitter-sample shadow rays of CCU_RENDER_EMITTER_MODELS).
-template <int MODE, bool SPEC, bool CUT = false>
+// BIOME: octree hits are tinted by the biome colours of CCU_RENDER_BIOME_TINT (intersect_block).
+template <int MODE, bool SPEC, bool CUT = false, bool BIOME = false>
 __device__ __forceinline__ bool closest_intersect_mode(const DScene &s, float3 origin, float3 direction, RecordT<SPEC> &rec, HitInfo &hi) {
-    if (MODE == 0) return closest_intersect_ref<SPEC, CUT>(s, origin, direction, rec, hi);
-    return closest_intersect_lean<MODE == 2, SPEC, CUT>(s, origin, direction, rec, hi);
+    if (MODE == 0) return closest_intersect_ref<SPEC, CUT, BIOME>(s, origin, direction, rec, hi);
+    return closest_intersect_lean<MODE == 2, SPEC, CUT, BIOME>(s, origin, direction, rec, hi);
 }
 
 // one path sample for pixel gid, thread-sequential: rayTracer.cl:40-107 (+ kernel.h:33-98, sky.h:68-93); SPEC adds the specular
 // events of CCU_RENDER_SPECULAR (DESIGN "Beyond the reference: specular materials"), NEE the emitter sampler (NeeKind) of
-// CCU_RENDER_EMITTER_SAMPLING (DESIGN §10), CCU_RENDER_EMITTER_NEAR_FIELD (§11) and CCU_RENDER_EMITTER_MODELS (§12)
-template <int MODE, bool SPEC, int NEE>
+// CCU_RENDER_EMITTER_SAMPLING (DESIGN §10), CCU_RENDER_EMITTER_NEAR_FIELD (§11) and CCU_RENDER_EMITTER_MODELS (§12), BIOME the
+// biome colours of CCU_RENDER_BIOME_TINT (§13)
+template <int MODE, bool SPEC, int NEE, bool BIOME>
 __device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &g, int gid, int seed) {
     float3 color = f3(0, 0, 0), throughput = f3(1, 1, 1);
     int ray_depth = 0;
@@ -213,7 +215,7 @@ __device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &
     bool nee_prev = false;   // NEE: the hit this segment left sampled the list of cell nee_cell
     int3 nee_cell = make_int3(0, 0, 0);
     for (;;) {
-        if (!closest_intersect_mode<MODE>(s, origin, direction, rec, hi)) {
+        if (!closest_intersect_mode<MODE, SPEC, false, BIOME>(s, origin, direction, rec, hi)) {
             // miss: emittance = 1, sky (+ sun disc) added through the throughput (rayTracer.cl:95-97, kernel.h:26-31)
             float3 sky = sky_radiance(s, direction);
             color = color + (sky * throughput) * 1.0f;
@@ -255,7 +257,7 @@ __device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &
             float shadow_emittance = fabsf(dot3(d, rec.surf.normal));
             RecordT<SPEC> sh = rec;                   // keeps the surface hit's distance as the ray limit (SURVEY Q4)
             HitInfo shi;
-            if (!closest_intersect_mode<MODE>(s, origin, d, sh, shi)) {
+            if (!closest_intersect_mode<MODE, SPEC, false, BIOME>(s, origin, d, sh, shi)) {
                 float3 sky = sky_radiance(s, d);
                 color = color + (sky * throughput) * shadow_emittance;
             }
@@ -270,11 +272,11 @@ __device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &
                 nee_cell = cell;
                 float3 c, w;
                 float limit;
-                if (nee_sample<NEE>(s, g, first, n_list, origin, rec.surf.normal, throughput, rng, c, w, limit)) {
+                if (nee_sample<NEE, BIOME>(s, g, first, n_list, origin, rec.surf.normal, throughput, rng, c, w, limit)) {
                     RecordT<SPEC> sh = rec;
                     sh.distance = limit;
                     HitInfo shi;
-                    if (!closest_intersect_mode<MODE, SPEC, nee_models(NEE)>(s, origin, w, sh, shi)) color = color + c;
+                    if (!closest_intersect_mode<MODE, SPEC, nee_models(NEE), BIOME>(s, origin, w, sh, shi)) color = color + c;
                 }
             }
         }

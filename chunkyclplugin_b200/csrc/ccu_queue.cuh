@@ -90,7 +90,7 @@ constexpr int Q_TOP_WORDS = 4096;            // top tables up to 16^3 cells are 
 #ifndef CCU_Q_STACK
 #define CCU_Q_STACK 12
 #endif
-constexpr int Q_SMEM_LIMIT = 227 * 1024 - 1280;   // dynamic shared memory a CTA may ask for, less the kernel's static tables (SmemTables)
+constexpr int Q_SMEM_LIMIT = 227 * 1024 - 1280;   // dynamic shared memory a CTA may ask for, less the kernel's static tables (SmemTables, BiomeView)
 constexpr int Q_STACK = CCU_Q_STACK;
 constexpr int Q_DEEP = 64 - Q_STACK;          // stack entries beyond the shared-memory part
 constexpr int Q_STACK_WORDS = Q_STACK * Q_SLOTS;
@@ -305,8 +305,8 @@ __device__ __forceinline__ void q_stage_march(const DScene &s, const unsigned *_
 // SPEC: a specular event at the hit (DESIGN "Beyond the reference: specular materials") bounces right away, without a sun sample.
 // NEE (a NeeKind): after the sun sample (or in its place) and before the bounce, the emitter sample of DESIGN §10 (§11 for
 // NEE_NEAR) with its own shadow ray (NFI: index of the two NEE fields); `covered`: the hit is an emitter the previous hit's sample covered, whose emission is
-// left out.
-template <bool SPEC, int NEE, int NFI>
+// left out.  BIOME: the emitter sample reads the biome colours of CCU_RENDER_BIOME_TINT (DESIGN §13).
+template <bool SPEC, int NEE, int NFI, bool BIOME>
 __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint32_t *F, unsigned *mask, int lane, int row, float3 o,
                                         float3 d, float distance, bool ray_hit, const SurfT<SPEC> &hit, bool covered) {
     const int slot = row * 32 + lane;
@@ -395,7 +395,7 @@ __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint
                 uint32_t rng = QU(QF_RNG);
                 float3 c, w;
                 float limit;
-                const bool ray = nee_sample<NEE>(s, g, first, n_list, from, normal, f3(QFL(QF_THRX), QFL(QF_THRY), QFL(QF_THRZ)), rng, c, w, limit);
+                const bool ray = nee_sample<NEE, BIOME>(s, g, first, n_list, from, normal, f3(QFL(QF_THRX), QFL(QF_THRY), QFL(QF_THRZ)), rng, c, w, limit);
                 QU(QF_RNG) = rng;
                 if (ray) {
                     QFL(QF_SNX) = normal.x; QFL(QF_SNY) = normal.y; QFL(QF_SNZ) = normal.z;
@@ -469,7 +469,8 @@ __device__ __forceinline__ bool q_covered(const DScene &s, const EmitView &g, co
 
 // BLOCK (kind_block = true) and EXIT (false): the octree part of closestIntersect (kernel.h:14-16) is finished here;
 // without BVHs the ray is shaded right away, with BVHs it goes to the BVH stage.  kind_block is warp-uniform.
-template <bool HAS_BVH, bool SPEC, int NEE>
+// BIOME: block hits are tinted by the biome colours of CCU_RENDER_BIOME_TINT (DESIGN §13).
+template <bool HAS_BVH, bool SPEC, int NEE, bool BIOME>
 __device__ __forceinline__ bool q_stage_resolve(const DScene &s, const EmitView &g, uint32_t *F, unsigned *mask, int lane, const bool kind_block,
                                                 int min_lanes) {
     const int row = q_pop_batch(mask, kind_block ? QS_BLOCK : QS_EXIT, lane, min_lanes);
@@ -496,7 +497,7 @@ __device__ __forceinline__ bool q_stage_resolve(const DScene &s, const EmitView 
         const int data = find_leaf_wide(s, c.bx, c.by, c.bz, level);   // the kernel is only launched on the commit-time layouts
         // NEE_*_MODELS: an emitter sample's shadow ray counts a block hit only before its limit (march_block)
         const bool cut = nee_models(NEE) ? (QU(QF_META) & QM_NEE_RAY) != 0 : false;
-        if (!march_block<SPEC, nee_models(NEE)>(s, m, data, level, hit, hit_t, cut)) {
+        if (!march_block<SPEC, nee_models(NEE), BIOME>(s, m, data, level, hit, hit_t, cut)) {
             QFL(QF_T) = m.t; QI(QF_STEPS) = m.steps;
             q_push(mask, QS_MARCH, lane, row);
             return true;
@@ -531,13 +532,13 @@ __device__ __forceinline__ bool q_stage_resolve(const DScene &s, const EmitView 
         QI(QF_BSP) = phase << 8;
         q_push(mask, ref < 0 ? QS_LEAF : QS_BVH, lane, row);
     } else {
-        q_shade<SPEC, NEE, q_nee_field(HAS_BVH, SPEC)>(s, g, F, mask, lane, row, m.o, m.d, distance, ray_hit, hit, covered);
+        q_shade<SPEC, NEE, q_nee_field(HAS_BVH, SPEC), BIOME>(s, g, F, mask, lane, row, m.o, m.d, distance, ray_hit, hit, covered);
     }
     return true;
 }
 
 // SHADE (HAS_BVH kernels): closestIntersect is complete (kernel.h:17-22)
-template <bool SPEC, int NEE>
+template <bool SPEC, int NEE, bool BIOME>
 __device__ __forceinline__ bool q_stage_shade(const DScene &s, const EmitView &g, uint32_t *F, unsigned *mask, int lane, int min_lanes) {
     const int row = q_pop_batch(mask, QS_SHADE, lane, min_lanes);
     if (row == -2) return false;
@@ -552,8 +553,8 @@ __device__ __forceinline__ bool q_stage_shade(const DScene &s, const EmitView &g
     hit.color = make_float4(QFL(QF_HCX), QFL(QF_HCY), QFL(QF_HCZ), 0.0f);
     hit.emittance = QFL(QF_HEM);
     if constexpr (SPEC) hit.spec = QU(QF_HSPEC);
-    q_shade<SPEC, NEE, q_nee_field(true, SPEC)>(s, g, F, mask, lane, row, o, d, QFL(QF_HDIST), ray_hit, hit,
-                                                NEE && (QU(QF_META) & QM_COVERED) != 0);
+    q_shade<SPEC, NEE, q_nee_field(true, SPEC), BIOME>(s, g, F, mask, lane, row, o, d, QFL(QF_HDIST), ray_hit, hit,
+                                                       NEE && (QU(QF_META) & QM_COVERED) != 0);
     return true;
 }
 
@@ -913,9 +914,10 @@ __device__ __forceinline__ bool q_stage_end(const DScene &s, const PassParams &w
 // NEE: the emitter sampler (NeeKind) of CCU_RENDER_EMITTER_SAMPLING, with CCU_RENDER_EMITTER_NEAR_FIELD for NEE_NEAR(_MODELS) and
 // CCU_RENDER_EMITTER_MODELS for NEE_*_MODELS (the table `g` is then the wider one, DESIGN §12), on a scene
 // with emitters (table `g`, an argument after the others so that the kernels without it keep their parameter offsets).
-template <bool HAS_BVH, int LAY, bool SPEC, int NEE>
+// BIOME: CCU_RENDER_BIOME_TINT on a scene with biome colours (`bv`, the last argument for the same reason; DESIGN §13).
+template <bool HAS_BVH, int LAY, bool SPEC, int NEE, bool BIOME>
 __global__ void __launch_bounds__(Q_WARPS * 32, 1) k_render_queue(const __grid_constant__ DScene s, const __grid_constant__ QueueParams qp,
-                                                                 const __grid_constant__ EmitView g) {
+                                                                 const __grid_constant__ EmitView g, const __grid_constant__ BiomeView bv) {
     constexpr int NST = q_stages(HAS_BVH);
     constexpr int MASK_WORDS = q_mask_words(HAS_BVH);
     extern __shared__ uint32_t q_mem[];
@@ -943,6 +945,9 @@ __global__ void __launch_bounds__(Q_WARPS * 32, 1) k_render_queue(const __grid_c
     if (qp.sky_texels > 0) {
         sky_s = reinterpret_cast<uchar4 *>(top_s + (LAY == 0 ? Q_TOP_WORDS : 0) + (HAS_BVH ? Q_STACK_WORDS : 0));
         for (int i = threadIdx.x; i < qp.sky_texels; i += blockDim.x) sky_s[i] = __ldg(s.sky + i);
+    }
+    if constexpr (BIOME) {
+        if (threadIdx.x == 0) biome_smem() = bv;   // read after the barrier of stage_tables
     }
     stage_tables(s, sky_s);
     if (threadIdx.x == 0) {
@@ -994,11 +999,11 @@ __global__ void __launch_bounds__(Q_WARPS * 32, 1) k_render_queue(const __grid_c
         switch (best) {
             case QS_MARCH: QSTAT(0, 1); q_stage_march<NST, LAY>(s, top, F, mask, lane, qp.yield_below, qp.refill_min); break;
             case QS_BLOCK:
-            case QS_EXIT: ran = q_stage_resolve<HAS_BVH, SPEC, NEE>(s, g, F, mask, lane, best == QS_BLOCK, min_lanes); break;
+            case QS_EXIT: ran = q_stage_resolve<HAS_BVH, SPEC, NEE, BIOME>(s, g, F, mask, lane, best == QS_BLOCK, min_lanes); break;
             case QS_END: ran = q_stage_end<!HAS_BVH>(s, qp.w, F, mask, live, lane, min_lanes); break;
             case QS_BVH: QSTAT(16, 1); if (HAS_BVH) q_stage_bvh<NST>(s, F, mask, stk, qp.bvh_deep, lane, qp.yield_below, qp.refill_min); break;
             case QS_LEAF: if (HAS_BVH) ran = q_stage_leaf<SPEC, NEE>(s, F, mask, stk, qp.bvh_deep, lane, min_lanes); break;
-            default: if (HAS_BVH) ran = q_stage_shade<SPEC, NEE>(s, g, F, mask, lane, min_lanes); break;
+            default: if (HAS_BVH) ran = q_stage_shade<SPEC, NEE, BIOME>(s, g, F, mask, lane, min_lanes); break;
         }
         sticky = (ran && best != QS_MARCH && best != QS_BVH) ? best : -1;
         if (ran) {

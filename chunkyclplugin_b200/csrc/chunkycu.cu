@@ -9,6 +9,7 @@
 #include <cstring>
 #include <climits>
 #include <mutex>
+#include <new>
 #include <string>
 #include <thread>
 #include <vector>
@@ -45,18 +46,22 @@ __global__ void k_sun_setup(const int *sun_words, float *out /* su sv sw radius_
 // rayTracer.cl:109-112 carried in registers between passes (identical arithmetic, no memory round trip).
 // MODE: 0 = the reference's own node array, 1 = commit-time layouts, 2 = commit-time layouts of a deep world.
 // SPEC: CCU_RENDER_SPECULAR on a scene with specular words; NEE: the emitter sampler (NeeKind) of CCU_RENDER_EMITTER_SAMPLING and
-// CCU_RENDER_EMITTER_NEAR_FIELD / CCU_RENDER_EMITTER_MODELS on a scene with emitters (sample_pixel).
-template <int MODE, bool SPEC, int NEE>
+// CCU_RENDER_EMITTER_NEAR_FIELD / CCU_RENDER_EMITTER_MODELS on a scene with emitters (sample_pixel).  BIOME: CCU_RENDER_BIOME_TINT
+// on a scene with biome colours (`bv`, after the others so that the other kernels keep their parameter offsets).
+template <int MODE, bool SPEC, int NEE, bool BIOME>
 __global__ void __launch_bounds__(128) k_render_mega(const __grid_constant__ DScene s, const int *__restrict__ seeds, int n_passes,
                                                      int start_spp, float *res, const float *res_prev, int n_pixels,
-                                                     const __grid_constant__ EmitView g) {
+                                                     const __grid_constant__ EmitView g, const __grid_constant__ BiomeView bv) {
+    if constexpr (BIOME) {
+        if (threadIdx.x == 0) biome_smem() = bv;   // read after the barrier of stage_tables
+    }
     stage_tables(s, nullptr);
     for (int gid = blockIdx.x * blockDim.x + threadIdx.x; gid < n_pixels; gid += gridDim.x * blockDim.x) {
         float *px = res + (size_t)gid * 3;
         const float *pp = res_prev + (size_t)gid * 3;    // what the reference's single buffer holds when the window starts
         float3 buf = f3(pp[0], pp[1], pp[2]);
         for (int pass = 0; pass < n_passes; pass++) {
-            float3 col = sample_pixel<MODE, SPEC, NEE>(s, g, gid, __ldg(seeds + pass));
+            float3 col = sample_pixel<MODE, SPEC, NEE, BIOME>(s, g, gid, __ldg(seeds + pass));
             int spp = start_spp + pass;
             float fs = (float)spp, fs1 = (float)(spp + 1);
             buf.x = (buf.x * fs + col.x) / fs1;
@@ -359,6 +364,45 @@ void fill_view(ccu_host::Scene &sc) {
     mg.dim = make_int3(in.memit_dim[0], in.memit_dim[1], in.memit_dim[2]);
     mg.shift = in.memit_shift;
     mg.mhead = sc.memit_head.p; mg.mprim = reinterpret_cast<const int4 *>(sc.memit_prim.p);
+    BiomeView &bv = sc.biome_view;
+    bv.grid = sc.biome_grid.p; bv.tiles = sc.biome_tiles.p;
+    bv.x0 = in.biome_box[0]; bv.z0 = in.biome_box[1]; bv.gx = in.biome_box[2]; bv.gz = in.biome_box[3];
+}
+
+// build_biome_layout with its failures as CCU_* codes; `what` names the entry point
+int biome_layout(const int32_t *chunks, const float *rgb, int64_t n, int depth, BiomeLayout &bl, const char *what) {
+    try {
+        bl = build_biome_layout(chunks, rgb, n, depth);
+    } catch (const std::bad_alloc &) {
+        return fail(CCU_ENOMEM, "%s: no host memory for the biome layout of %lld chunks", what, (long long)n);
+    }
+    if (bl.status == 1)
+        return fail(CCU_EINVAL, "%s: biome chunk %lld (%d, %d) lies outside the octree's %lld x %lld chunks", what, (long long)bl.bad,
+                    chunks[2 * bl.bad], chunks[2 * bl.bad + 1], (long long)bl.extent, (long long)bl.extent);
+    if (bl.status == 2)
+        return fail(CCU_EINVAL, "%s: the biome chunks span more than %lld chunks (bounding box); the grid holds at most that many", what,
+                    (long long)CCU_BIOME_GRID_MAX);
+    return CCU_OK;
+}
+
+// The checks of ccu_scene_set_biome_colors (also applied by ccu_debug_biome_layout); `what` names the entry point.
+int check_biome_colors(const int32_t *chunks, const float *rgb, int64_t n, const char *what) {
+    if (n < 0 || (n > 0 && (!chunks || !rgb))) return fail(CCU_EINVAL, "%s: bad arrays (n=%lld)", what, (long long)n);
+    std::vector<std::pair<int, int>> seen;
+    seen.reserve((size_t)n);
+    for (int64_t i = 0; i < n; i++) {
+        if (chunks[2 * i] < 0 || chunks[2 * i + 1] < 0)
+            return fail(CCU_EINVAL, "%s: chunk %lld (%d, %d) has a negative coordinate", what, (long long)i, chunks[2 * i], chunks[2 * i + 1]);
+        seen.emplace_back(chunks[2 * i], chunks[2 * i + 1]);
+    }
+    std::sort(seen.begin(), seen.end());
+    for (size_t i = 1; i < seen.size(); i++)
+        if (seen[i] == seen[i - 1]) return fail(CCU_EINVAL, "%s: chunk (%d, %d) is given twice", what, seen[i].first, seen[i].second);
+    for (int64_t i = 0; i < n * 3 * 256 * 3; i++)
+        if (!std::isfinite(rgb[i]) || rgb[i] < 0.0f)
+            return fail(CCU_EINVAL, "%s: colour component %lld of chunk %lld is negative or not finite", what, (long long)i,
+                        (long long)(i / (3 * 256 * 3)));
+    return CCU_OK;
 }
 
 // The launch view with this launch's camera, rays, canvas and render params (caller holds c->mu, the scene is committed).
@@ -439,11 +483,16 @@ void dispatch(bool v, F &&f) {
     else f(std::false_type{});
 }
 
-// the wavefront kernel (ccu_queue.cuh) for the scene's entity BVHs and air layout (air_layout_id), with or without specular events
-auto queue_kernel(bool bvh, int lay, bool spec, int nee) {
-    decltype(&k_render_queue<false, 0, false, NEE_NONE>) k = nullptr;
+// the wavefront kernel (ccu_queue.cuh) for the scene's entity BVHs and air layout (air_layout_id), with or without specular events,
+// emitter sampler and biome colours
+auto queue_kernel(bool bvh, int lay, bool spec, int nee, bool biome) {
+    decltype(&k_render_queue<false, 0, false, NEE_NONE, false>) k = nullptr;
     dispatch(bvh, [&](auto B) {
-        dispatch<3>(lay, [&](auto L) { dispatch(spec, [&](auto S) { dispatch<5>(nee, [&](auto N) { k = k_render_queue<B, L, S, N>; }); }); });
+        dispatch<3>(lay, [&](auto L) {
+            dispatch(spec, [&](auto S) {
+                dispatch<5>(nee, [&](auto N) { dispatch(biome, [&](auto T) { k = k_render_queue<B, L, S, N, T>; }); });
+            });
+        });
     });
     return k;
 }
@@ -464,6 +513,10 @@ int nee_launch(const ccu_ctx *c) {
     if (!c->scene.info.has_emitters) return NEE_NONE;
     return (f & CCU_RENDER_EMITTER_NEAR_FIELD) ? NEE_NEAR : NEE_AREA;
 }
+
+// CCU_RENDER_BIOME_TINT launches the biome kernels only on a scene with biome colours: without them they compute exactly what the
+// other kernels compute
+bool biome_launch(const ccu_ctx *c) { return (c->params.flags & CCU_RENDER_BIOME_TINT) && c->scene.info.has_biome; }
 
 }  // namespace
 
@@ -541,11 +594,13 @@ int replicate_scene(ccu_ctx *src, ccu_ctx *dst) {
     dst->committed = false;
     b.info = SceneInfo();
     for (PackedArray &p : b.arrays) p.host.reset();
+    b.biome.reset();
     int rc = CCU_OK;
     Scene::each_buf(a, b, [&](auto &x, auto &y) { if (rc == CCU_OK) rc = copy_buf(src, dst, x, y); });
     if (rc != CCU_OK) return rc;
     CU(cudaStreamSynchronize(dst->stream));
     for (int i = 0; i < N_ARRAYS; i++) b.arrays[i].host = a.arrays[i].host;
+    b.biome = a.biome;
     b.info = a.info;
     fill_view(b);
     dst->committed = true;
@@ -625,8 +680,9 @@ int ccu_ctx_create(int device_index, ccu_ctx **out) {
     for (bool bvh : {false, true})
         for (bool spec : {false, true})
             for (int nee : {NEE_NONE, NEE_AREA, NEE_NEAR, NEE_AREA_MODELS, NEE_NEAR_MODELS})
-                for (int lay = 0; lay < 3 && e == cudaSuccess; lay++)
-                    e = cudaFuncSetAttribute(queue_kernel(bvh, lay, spec, nee), cudaFuncAttributeMaxDynamicSharedMemorySize, Q_SMEM_LIMIT);
+                for (bool biome : {false, true})
+                    for (int lay = 0; lay < 3 && e == cudaSuccess; lay++)
+                        e = cudaFuncSetAttribute(queue_kernel(bvh, lay, spec, nee, biome), cudaFuncAttributeMaxDynamicSharedMemorySize, Q_SMEM_LIMIT);
     if (e == cudaSuccess) e = c->unorm.alloc(256);
     if (e == cudaSuccess) {
         k_unorm_table<<<1, 256, 0, c->stream>>>(c->unorm.p);
@@ -667,6 +723,9 @@ int ccu_scene_begin(ccu_ctx *c) {
         if (ccu_host::ARRAY_DESC[i].optional) c->scene.arrays[i].dev.release();
     }
     c->scene.info.have_atlas = c->scene.info.have_sky = c->scene.info.have_sun = false;
+    c->scene.biome.reset();
+    c->scene.biome_grid.release();
+    c->scene.biome_tiles.release();
     return CCU_OK;
 }
 
@@ -682,6 +741,27 @@ int ccu_scene_set_material_palette(ccu_ctx *c, const int32_t *w, int64_t n) { re
 int ccu_scene_set_triangles(ccu_ctx *c, const int32_t *w, int64_t n) { return set_array(c, ccu_host::TRIANGLES, w, n); }
 int ccu_scene_set_world_bvh(ccu_ctx *c, const int32_t *w, int64_t n) { return set_array(c, ccu_host::WORLD_BVH, w, n); }
 int ccu_scene_set_actor_bvh(ccu_ctx *c, const int32_t *w, int64_t n) { return set_array(c, ccu_host::ACTOR_BVH, w, n); }
+
+// Kept on the host until commit, which lays the colours out for the octree's extent.
+int ccu_scene_set_biome_colors(ccu_ctx *c, const int32_t *chunks, const float *rgb, int64_t n) {
+    if (!c) return fail(CCU_EINVAL, "ccu_scene_set_biome_colors: null context");
+    std::shared_ptr<ccu_host::BiomeColors> b;
+    try {
+        const int rc = check_biome_colors(chunks, rgb, n, "ccu_scene_set_biome_colors");
+        if (rc != CCU_OK) return rc;
+        if (n > 0) {
+            b = std::make_shared<ccu_host::BiomeColors>();
+            b->chunks.assign(chunks, chunks + 2 * n);
+            b->rgb.assign(rgb, rgb + n * 3 * 256 * 3);
+        }
+    } catch (const std::bad_alloc &) {
+        return fail(CCU_ENOMEM, "ccu_scene_set_biome_colors: no host memory for %lld chunks", (long long)n);
+    }
+    std::lock_guard<std::mutex> lk(c->mu);
+    c->committed = false;
+    c->scene.biome = std::move(b);
+    return CCU_OK;
+}
 
 int ccu_scene_atlas_create(ccu_ctx *c, int32_t width, int32_t height, int32_t layers) {
     if (!c) return fail(CCU_EINVAL, "ccu_scene_atlas_create: null context");
@@ -847,6 +927,21 @@ int ccu_scene_commit(ccu_ctx *c) {
         CU(sc.actor_rec.upload(bs.actor.rec.data(), bs.actor.rec.size(), c->stream));
         CU(sc.tris2.upload(bs.tris.data(), bs.tris.size(), c->stream));
     }
+    // biome colours (CCU_RENDER_BIOME_TINT), only when set
+    in.has_biome = 0;
+    for (int &v : in.biome_box) v = 0;
+    sc.biome_grid.release();
+    sc.biome_tiles.release();
+    if (sc.biome) {
+        const ccu_host::BiomeColors &bc = *sc.biome;
+        BiomeLayout bl;
+        const int rc = biome_layout(bc.chunks.data(), bc.rgb.data(), (int64_t)bc.chunks.size() / 2, in.depth, bl, "commit");
+        if (rc != CCU_OK) return rc;
+        CU(sc.biome_grid.upload(bl.grid.data(), bl.grid.size(), c->stream));
+        CU(sc.biome_tiles.upload(reinterpret_cast<const float4 *>(bl.tiles.data()), bl.tiles.size() / 4, c->stream));
+        in.has_biome = 1;
+        in.biome_box[0] = bl.x0; in.biome_box[1] = bl.z0; in.biome_box[2] = bl.gx; in.biome_box[3] = bl.gz;
+    }
     // sun basis, computed on the device
     {
         DevBuf<int> words;
@@ -959,7 +1054,7 @@ int ccu_render_set_params(ccu_ctx *c, const ccu_render_params *p) {
     if (p->draw_depth < 0 || p->draw_depth >= (1 << 24) || p->max_depth < 1 || p->max_depth > 255) return fail(CCU_EINVAL, "bad render params");
     if (p->kernel != 0 && p->kernel != 1 && p->kernel != 4) return fail(CCU_EINVAL, "unknown kernel %d (0 auto, 1 thread-per-pixel, 4 wavefront)", p->kernel);
     if (p->flags & ~(CCU_RENDER_NO_ENTITIES | CCU_RENDER_NO_SUN | CCU_RENDER_SPECULAR | CCU_RENDER_EMITTER_SAMPLING | CCU_RENDER_EMITTER_NEAR_FIELD |
-                     CCU_RENDER_EMITTER_MODELS))
+                     CCU_RENDER_EMITTER_MODELS | CCU_RENDER_BIOME_TINT))
         return fail(CCU_EINVAL, "unknown render flags 0x%x", p->flags);
     if ((p->flags & CCU_RENDER_EMITTER_NEAR_FIELD) && !(p->flags & CCU_RENDER_EMITTER_SAMPLING))
         return fail(CCU_EINVAL, "CCU_RENDER_EMITTER_NEAR_FIELD needs CCU_RENDER_EMITTER_SAMPLING");
@@ -1007,6 +1102,8 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
     const bool spec = specular_launch(c);
     const int nee = nee_launch(c);
     const EmitView &emit_view = nee_models(nee) ? c->scene.memit_view : c->scene.emit_view;
+    const bool biome = biome_launch(c);
+    const BiomeView &biome_view = c->scene.biome_view;
     float *res = c->accum[c->accum_active].p;
     const float *res_prev = c->window_spp == 0 ? c->window_base : res;
     int kernel = c->params.kernel;
@@ -1016,8 +1113,10 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
         dispatch<3>(mode, [&](auto M) {
             dispatch(spec, [&](auto S) {
                 dispatch<5>(nee, [&](auto N) {
-                    k_render_mega<M, S, N><<<blocks, threads, 0, c->stream>>>(s, seeds_dev, n_passes, c->window_spp, res, res_prev, n_pixels,
-                                                                        emit_view);
+                    dispatch(biome, [&](auto T) {
+                        k_render_mega<M, S, N, T><<<blocks, threads, 0, c->stream>>>(s, seeds_dev, n_passes, c->window_spp, res, res_prev,
+                                                                                   n_pixels, emit_view, biome_view);
+                    });
                 });
             });
         });
@@ -1058,7 +1157,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
             qp.bvh_deep = c->bvh_deep.p;
         }
         const int smem = base_smem + qp.sky_texels * 4;
-        queue_kernel(bvh, lay, spec, nee)<<<grid, block, smem, c->stream>>>(s, qp, emit_view);
+        queue_kernel(bvh, lay, spec, nee, biome)<<<grid, block, smem, c->stream>>>(s, qp, emit_view, biome_view);
 #ifdef CCU_Q_STATS
         {
             cudaStreamSynchronize(c->stream);
@@ -1503,6 +1602,26 @@ int ccu_debug_emitter_models(const int32_t *tree, int64_t n_tree, int32_t depth,
     if (list) std::copy(g.list.begin(), g.list.end(), list);
     if (head && has) std::copy(me.head.begin(), me.head.end(), head);
     if (prim && has) std::copy(me.prim.begin(), me.prim.end(), prim);
+    return CCU_OK;
+}
+
+// Host-only check of the biome layout (no CUDA call): what ccu_scene_commit builds from these colours for an octree of `depth`.
+int ccu_debug_biome_layout(const int32_t *chunks, const float *rgb, int64_t n, int32_t depth, int32_t info[5], int32_t *grid, float *tiles) {
+    if (depth < 0 || depth > 30 || !info) return fail(CCU_EINVAL, "ccu_debug_biome_layout: bad argument");
+    int rc;
+    try {
+        rc = check_biome_colors(chunks, rgb, n, "ccu_debug_biome_layout");
+    } catch (const std::bad_alloc &) {
+        return fail(CCU_ENOMEM, "ccu_debug_biome_layout: no host memory for %lld chunks", (long long)n);
+    }
+    if (rc != CCU_OK) return rc;
+    BiomeLayout bl;
+    rc = biome_layout(chunks, rgb, n, depth, bl, "ccu_debug_biome_layout");
+    if (rc != CCU_OK) return rc;
+    info[0] = bl.x0; info[1] = bl.z0; info[2] = bl.gx; info[3] = bl.gz;
+    info[4] = (int)n;
+    if (grid) std::copy(bl.grid.begin(), bl.grid.end(), grid);
+    if (tiles) std::copy(bl.tiles.begin(), bl.tiles.end(), tiles);
     return CCU_OK;
 }
 

@@ -17,6 +17,7 @@ LIB_PATH = os.environ.get("CHUNKYCU_LIB") or os.path.join(_HERE, "libchunkycu.so
 CCU_RENDER_NO_ENTITIES, CCU_RENDER_NO_SUN, CCU_RENDER_SPECULAR, CCU_RENDER_EMITTER_SAMPLING = 1, 2, 4, 8
 CCU_RENDER_EMITTER_NEAR_FIELD = 128
 CCU_RENDER_EMITTER_MODELS = 256
+CCU_RENDER_BIOME_TINT = 512
 CCU_UNIQUE_ID_BYTES = 128
 
 CCU_OK, CCU_ENODEVICE, CCU_EINVAL, CCU_ECUDA, CCU_ENOMEM, CCU_ESTATE = 0, -1, -2, -3, -4, -5
@@ -53,6 +54,7 @@ SYMBOLS = {
     "ccu_scene_set_triangles": (C.c_int, [_vp, _vp, _i64]),
     "ccu_scene_set_world_bvh": (C.c_int, [_vp, _vp, _i64]),
     "ccu_scene_set_actor_bvh": (C.c_int, [_vp, _vp, _i64]),
+    "ccu_scene_set_biome_colors": (C.c_int, [_vp, _vp, _vp, _i64]),
     "ccu_scene_atlas_create": (C.c_int, [_vp, _i32, _i32, _i32]),
     "ccu_scene_atlas_write": (C.c_int, [_vp, _i32, _i32, _i32, _i32, _i32, _vp]),
     "ccu_scene_set_atlas": (C.c_int, [_vp, _vp, _i32, _i32, _i32]),
@@ -89,6 +91,7 @@ SYMBOLS = {
     "ccu_debug_bvh_layout": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _i64, _vp, _i64, C.POINTER(_i64), C.POINTER(_i64), _pi32, _pi32]),
     "ccu_debug_emitter_grid": (C.c_int, [_vp, _i64, _i32, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp]),
     "ccu_debug_emitter_models": (C.c_int, [_vp, _i64, _i32, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "ccu_debug_biome_layout": (C.c_int, [_vp, _vp, _i64, _i32, _vp, _vp, _vp]),
     # multi-GPU
     "ccu_group_create": (C.c_int, [_vp, _i32, C.POINTER(_vp)]),
     "ccu_group_unique_id": (C.c_int, [_vp]),
@@ -222,6 +225,29 @@ def debug_emitter_models(p):
             "head": head[:info[10]], "prim": prim[:info[11]]}
 
 
+def _biome_arrays(chunks, rgb):
+    chunks = np.ascontiguousarray(chunks, dtype=np.int32).reshape(-1, 2)
+    rgb = np.ascontiguousarray(rgb, dtype=np.float32).reshape(-1, 3, 256, 3)
+    if rgb.shape[0] != chunks.shape[0]:
+        raise ValueError(f"{chunks.shape[0]} chunks but {rgb.shape[0]} colour tiles")
+    return chunks, rgb
+
+
+def debug_biome_layout(chunks, rgb, depth: int):
+    """The biome layout of CCU_RENDER_BIOME_TINT the library builds at commit for an octree of `depth` (host only): a dict with
+    x0, z0 (the low chunk of the chunks' bounding box), grid (int32[gx, gz], indexed [cx - x0, cz - z0], -1 = no tile) and tiles
+    (float32[n, 3, 256, 4])."""
+    chunks, rgb = _biome_arrays(chunks, rgb)
+    n = chunks.shape[0]
+    info = np.zeros(5, dtype=np.int32)
+    lib = load()
+    check(lib.ccu_debug_biome_layout(_ptr(chunks), _ptr(rgb), n, depth, _ptr(info), None, None))
+    grid = np.zeros((int(info[2]), int(info[3])), dtype=np.int32)
+    tiles = np.zeros((n, 3, 256, 4), dtype=np.float32)
+    check(lib.ccu_debug_biome_layout(_ptr(chunks), _ptr(rgb), n, depth, _ptr(info), _ptr(grid), _ptr(tiles)))
+    return {"x0": int(info[0]), "z0": int(info[1]), "grid": grid, "tiles": tiles}
+
+
 def device_count() -> int:
     n = C.c_int()
     check(load().ccu_device_count(C.byref(n)))
@@ -286,6 +312,11 @@ class Context:
     def set_triangles(self, a): self._words(self._lib.ccu_scene_set_triangles, a)
     def set_world_bvh(self, a): self._words(self._lib.ccu_scene_set_world_bvh, a)
     def set_actor_bvh(self, a): self._words(self._lib.ccu_scene_set_actor_bvh, a)
+
+    def set_biome_colors(self, chunks, rgb):
+        """chunks int[n, 2] {cx, cz}, rgb float[n, 3, 256, 3] (planes foliage, grass, water; texel (z & 15) * 16 + (x & 15))."""
+        chunks, rgb = _biome_arrays(chunks, rgb)
+        check(self._lib.ccu_scene_set_biome_colors(self._h, _ptr(chunks), _ptr(rgb), chunks.shape[0]))
 
     def atlas_create(self, width: int, height: int, layers: int):
         check(self._lib.ccu_scene_atlas_create(self._h, width, height, layers))

@@ -113,6 +113,26 @@ class RendererInstance:
 # ----------------------------------------------------------------------------------------------------
 # ClSceneLoader.java + AbstractSceneLoader.java:42-162
 # ----------------------------------------------------------------------------------------------------
+def upload_scene(ctx, p) -> None:
+    """Upload and commit a PackedScene through the C ABI in the order of the reference's loader (AbstractSceneLoader.java:60-162),
+    with its biome colours when it has them."""
+    ctx.scene_begin()
+    ctx.set_atlas(p.atlas)                      # ClTextureLoader.buildTextures
+    ctx.set_block_palette(p.block_palette)
+    ctx.set_material_palette(p.mat_palette)
+    ctx.set_aabb_models(p.aabb_models)
+    ctx.set_quad_models(p.quad_models)
+    ctx.set_triangles(p.bvh_trigs)
+    ctx.set_world_bvh(p.world_bvh)
+    ctx.set_actor_bvh(p.actor_bvh)
+    ctx.set_sun(p.sun)
+    ctx.set_sky(p.sky, p.sky_intensity)         # ClSky
+    if p.biome is not None:
+        ctx.set_biome_colors(*p.biome)          # CCU_RENDER_BIOME_TINT's colours (beyond the reference)
+    ctx.set_octree(p.octree, p.octree_depth)    # loadOctree, ClSceneLoader.java:52-63
+    ctx.scene_commit()
+
+
 class CudaSceneLoader:
     def __init__(self, instance: Optional[RendererInstance] = None):
         self.instance = instance or RendererInstance.get()
@@ -131,22 +151,9 @@ class CudaSceneLoader:
         if resetReason in ("NONE", "MODE_CHANGE"):
             self.modCount = modCount
             return True
-        p, ctx = scene.packed, self.instance.context
-        ctx.scene_begin()
-        ctx.set_atlas(p.atlas)                      # ClTextureLoader.buildTextures
-        ctx.set_block_palette(p.block_palette)
-        ctx.set_material_palette(p.mat_palette)
-        ctx.set_aabb_models(p.aabb_models)
-        ctx.set_quad_models(p.quad_models)
-        ctx.set_triangles(p.bvh_trigs)
-        ctx.set_world_bvh(p.world_bvh)
-        ctx.set_actor_bvh(p.actor_bvh)
-        ctx.set_sun(p.sun)
-        ctx.set_sky(p.sky, p.sky_intensity)         # ClSky
-        ctx.set_octree(p.octree, p.octree_depth)    # loadOctree, ClSceneLoader.java:52-63
-        ctx.scene_commit()
+        upload_scene(self.instance.context, scene.packed)
         self.modCount = modCount
-        self._loaded_scene_id = id(p)
+        self._loaded_scene_id = id(scene.packed)
         return True
 
 

@@ -67,6 +67,9 @@ class PackedScene:
     height: int
     name: str = "scene"
     meta: dict = dataclasses.field(default_factory=dict)
+    # biome colours for CCU_RENDER_BIOME_TINT: (chunks int32[n, 2] {cx, cz}, rgb float32[n, 3, 256, 3]) as
+    # ccu_scene_set_biome_colors takes them (planes foliage, grass, water; texel (z & 15) * 16 + (x & 15)), or None
+    biome: Optional[Tuple[np.ndarray, np.ndarray]] = None
 
     def arrays(self) -> Dict[str, np.ndarray]:
         return {k: getattr(self, k) for k in (
@@ -928,3 +931,43 @@ def emissive_models(p: PackedScene, emittance: float = 1.0) -> PackedScene:
     for m in mats:
         mp[m + 4] = int(emittance * 255.0)
     return dataclasses.replace(p, mat_palette=mp, name=p.name + "_litmodels")
+
+
+# --------------------------------------------------------------------------------------
+# biome colours (CCU_RENDER_BIOME_TINT, DESIGN.md §13)
+# --------------------------------------------------------------------------------------
+def biome_field(chunks: np.ndarray, seed: int = 1) -> np.ndarray:
+    """float32[n, 3, 256, 3] linear colours of the chunks {cx, cz}: per plane a field that runs at different rates along x and z
+    (so that a swapped axis, a wrong chunk or a wrong texel shows), offset by a hash of the chunk."""
+    chunks = np.asarray(chunks, np.int64).reshape(-1, 2)
+    t = np.arange(256)
+    x = chunks[:, 0:1] * 16 + (t & 15)[None, :]          # [n, 256] voxel x of every texel
+    z = chunks[:, 1:2] * 16 + (t >> 4)[None, :]
+    out = np.empty((chunks.shape[0], 3, 256, 3), np.float32)
+    for plane in range(3):
+        h = hash_u32(chunks[:, 0], chunks[:, 1], seed, plane).astype(np.float64)[:, None] / 2.0 ** 32
+        for c, (fx, fz) in enumerate(((0.031, 0.007), (0.005, 0.043), (0.019, 0.013))):
+            f = (x * fx + z * (fz * (plane + 1)) + h * (c + 1)) % 1.0
+            out[:, plane, :, c] = 0.05 + 0.9 * f
+    return out
+
+
+def with_biomes(p: PackedScene, seed: int = 1, holes: float = 0.125) -> PackedScene:
+    """p with biome colours over the octree's max(1, 2^depth / 16)^2 chunks (biome_field); a hash of the chunk leaves out about
+    the fraction `holes` of them."""
+    g = max(1, (1 << p.octree_depth) // 16)
+    cx, cz = np.meshgrid(np.arange(g), np.arange(g), indexing="ij")
+    chunks = np.stack([cx.reshape(-1), cz.reshape(-1)], 1)
+    keep = hash_u32(chunks[:, 0], chunks[:, 1], seed, 7).astype(np.float64) / 2.0 ** 32 >= holes
+    chunks = chunks[keep].astype(np.int32)
+    return dataclasses.replace(p, biome=(chunks, biome_field(chunks, seed)), name=p.name + "_biomes")
+
+
+def water_tinted(p: PackedScene) -> PackedScene:
+    """p with every second untinted full-cube material given the water tint (tint type 3)."""
+    bp = np.asarray(p.block_palette, np.int64)
+    mp = np.array(p.mat_palette, np.int32)
+    mats = sorted({int(bp[b + 1]) for b in range(0, bp.size - 1, 2) if bp[b] == 1 and mp[int(bp[b + 1]) + 1] == 0})
+    for m in mats[::2]:
+        mp[m + 1] = 3 << 24
+    return dataclasses.replace(p, mat_palette=mp, name=p.name + "_water")

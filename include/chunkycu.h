@@ -84,6 +84,14 @@ typedef struct ccu_render_params {
  * exactly as with CCU_RENDER_EMITTER_SAMPLING alone.  Triangles keep the reference's behaviour.  DESIGN.md §12 holds the
  * exact contract. */
 #define CCU_RENDER_EMITTER_MODELS 256
+/* Biome tints (beyond the reference, which gives every grass, foliage and water surface one fixed colour): on a scene with biome
+ * colours (ccu_scene_set_biome_colors), a material of tint type 1 (foliage), 2 (grass) or 3 (water) on a full cube, an AABB
+ * model face or a quad of octree voxel (x, y, z) is tinted by the colour of its tint type at column (x, z) instead of the fixed
+ * tint, where that column's chunk has colours; the alpha is multiplied by 255/256 as with the fixed tint.  Emitter samples
+ * (CCU_RENDER_EMITTER_SAMPLING) read the colour at the emitter's voxel.  Triangles, tint 0xFF and chunks without colours keep the
+ * reference's behaviour, and a scene without biome colours renders exactly as without the flag.  Valid alone and with every
+ * other flag; both render kernels implement it.  DESIGN.md §13 holds the exact contract. */
+#define CCU_RENDER_BIOME_TINT 512
 
 /* ---- device enumeration: RendererInstance.java:39-75,123-157 (clGetPlatformIDs/clGetDeviceIDs/clGetDeviceInfo),
  *      used by the GPU selector UI (ui/GpuSelector.java:24-87) -------------------------------------------------- */
@@ -109,6 +117,14 @@ int ccu_scene_set_material_palette(ccu_ctx *ctx, const int32_t *words, int64_t n
 int ccu_scene_set_triangles(ccu_ctx *ctx, const int32_t *words, int64_t n);        /* getTrigPalette :130 */
 int ccu_scene_set_world_bvh(ccu_ctx *ctx, const int32_t *words, int64_t n);        /* getWorldBvh :135 */
 int ccu_scene_set_actor_bvh(ccu_ctx *ctx, const int32_t *words, int64_t n);        /* getActorBvh :139 */
+/* Biome colours for CCU_RENDER_BIOME_TINT (optional; beyond the reference).  chunks = n x {cx, cz}: chunk (cx, cz) covers voxels
+ * 16 cx <= x < 16 cx + 16 and 16 cz <= z < 16 cz + 16 at every y; rgb = n x 3 planes x 256 texels x 3 floats, planes in tint-type
+ * order (foliage, grass, water), texel (z & 15) * 16 + (x & 15), linear RGB as Chunky stores it.  CCU_EINVAL for n < 0, a null
+ * array with n > 0, a negative coordinate, a duplicate chunk or a negative or non-finite component; n = 0 removes the colours.
+ * ccu_scene_begin removes them too.  ccu_scene_commit fails with CCU_EINVAL when a chunk lies outside the octree's
+ * max(1, 2^depth / 16) chunks per axis, or when the chunks' bounding box holds more than 2^24 chunks (the lookup grid covers
+ * that box: every chunk of a depth-16 octree fits). */
+int ccu_scene_set_biome_colors(ccu_ctx *ctx, const int32_t *chunks, const float *rgb, int64_t n);
 /* texture atlas: ClTextureLoader.java:46-66 - clCreateImage(8192x8192xlayers RGBA8) then one clEnqueueWriteImage
  * per texture at (16*tileX, 16*tileY, layer) */
 int ccu_scene_atlas_create(ccu_ctx *ctx, int32_t width, int32_t height, int32_t layers);
@@ -218,6 +234,13 @@ int ccu_debug_emitter_models(const int32_t *tree, int64_t n_tree, int32_t depth,
                              const int32_t *mat_palette, int64_t n_mat, const int32_t *quad_models, int64_t n_quad,
                              const int32_t *aabb_models, int64_t n_aabb, int32_t info[12], int32_t *emit, int32_t *off,
                              int32_t *list, int32_t *head, int32_t *prim);
+
+/* Test support, host only: the biome layout ccu_scene_commit builds from ccu_scene_set_biome_colors' arrays for an octree of
+ * `depth` (DESIGN.md §13), with the same checks.  info = {x0, z0, gx, gz, tiles}: the grid covers the chunks' bounding box, gx x gz
+ * chunks from chunk (x0, z0); grid (gx x gz ints, index (cx - x0) * gz + (cz - z0), the tile of the chunk or -1) and tiles (tiles
+ * x 3 planes x 256 texels x 4 floats {r, g, b, 0}) may be NULL (sizes only) and must otherwise hold those sizes.  Used by the CPU
+ * test-suite. */
+int ccu_debug_biome_layout(const int32_t *chunks, const float *rgb, int64_t n, int32_t depth, int32_t info[5], int32_t *grid, float *tiles);
 
 /* ---- multi-GPU: samples-per-pixel split over the GPUs of one box (SURVEY.md 8e) -------------------------------------------
  * The reference is one JVM and one device (RendererInstance.java:81-101).  A group is N contexts, each holding a full scene

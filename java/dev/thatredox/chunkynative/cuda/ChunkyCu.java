@@ -39,6 +39,8 @@ public final class ChunkyCu {
     private static final MethodHandle SET_TRIANGLES = h("ccu_scene_set_triangles", WORDS);
     private static final MethodHandle SET_WORLD_BVH = h("ccu_scene_set_world_bvh", WORDS);
     private static final MethodHandle SET_ACTOR_BVH = h("ccu_scene_set_actor_bvh", WORDS);
+    private static final MethodHandle SET_BIOME_COLORS = h("ccu_scene_set_biome_colors", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG));
+    private static final MethodHandle DEBUG_BIOME_LAYOUT = h("ccu_debug_biome_layout", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, JAVA_INT, ADDRESS, ADDRESS, ADDRESS));
     private static final MethodHandle ATLAS_CREATE = h("ccu_scene_atlas_create", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT, JAVA_INT, JAVA_INT));
     private static final MethodHandle ATLAS_WRITE = h("ccu_scene_atlas_write", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, ADDRESS));
     private static final MethodHandle SET_SKY = h("ccu_scene_set_sky", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, JAVA_FLOAT));
@@ -83,6 +85,8 @@ public final class ChunkyCu {
     /** ccu_render_params.flags: emitter sampling also samples quad and AABB model emitters (DESIGN §12), valid only together
      *  with RENDER_EMITTER_SAMPLING. */
     public static final int RENDER_EMITTER_MODELS = 256;
+    /** ccu_render_params.flags: grass, foliage and water tinted by the biome colours of {@link Context#setBiomeColors} (DESIGN §13). */
+    public static final int RENDER_BIOME_TINT = 512;
     private static final StructLayout RENDER_PARAMS = MemoryLayout.structLayout(JAVA_INT.withName("draw_depth"), JAVA_INT.withName("max_depth"),
             JAVA_FLOAT.withName("emitter_scale"), JAVA_INT.withName("kernel"), JAVA_INT.withName("flags"));
 
@@ -97,6 +101,41 @@ public final class ChunkyCu {
                 msg = "?";
             }
             throw new RuntimeException("chunkycu error " + rc + ": " + msg);
+        }
+    }
+
+    /** Floats per chunk of ccu_scene_set_biome_colors' rgb array: 3 planes x 256 texels x 3. */
+    private static final int BIOME_TILE_FLOATS = 3 * 256 * 3;
+
+    /** The arrays must hold the n chunks they are passed for: 2n ints and 2304n floats (the native side reads that many). */
+    static void checkBiomeArrays(int[] chunks, float[] rgb, int n) {
+        if (n < 0 || (n > 0 && (chunks == null || rgb == null || chunks.length < 2L * n || rgb.length < (long) BIOME_TILE_FLOATS * n)))
+            throw new IllegalArgumentException("biome colours: arrays too short for " + n + " chunks");
+    }
+
+    /** Test support: the biome layout commit builds for an octree of {@code depth}; returns {x0, z0, gx, gz, tiles} and fills grid
+     *  (gx * gz ints) and tiles (tiles * 3 * 256 * 4 floats) when they are large enough (include/chunkycu.h,
+     *  ccu_debug_biome_layout). */
+    public static int[] debugBiomeLayout(int[] chunks, float[] rgb, int n, int depth, int[] grid, float[] tiles) {
+        checkBiomeArrays(chunks, rgb, n);
+        try (Arena a = Arena.ofConfined()) {
+            MemorySegment c = n > 0 ? a.allocateFrom(JAVA_INT, java.util.Arrays.copyOf(chunks, 2 * n)) : MemorySegment.NULL;
+            MemorySegment r = n > 0 ? a.allocateFrom(JAVA_FLOAT, java.util.Arrays.copyOf(rgb, BIOME_TILE_FLOATS * n)) : MemorySegment.NULL;
+            MemorySegment info = a.allocate(JAVA_INT, 5);
+            check((int) DEBUG_BIOME_LAYOUT.invokeExact(c, r, (long) n, depth, info, MemorySegment.NULL, MemorySegment.NULL));
+            int[] out = info.toArray(JAVA_INT);
+            long cells = (long) out[2] * out[3], floats = (long) out[4] * 3 * 256 * 4;
+            if (grid != null && tiles != null && grid.length >= cells && tiles.length >= floats) {
+                MemorySegment gs = a.allocate(JAVA_INT, Math.max(cells, 1)), ts = a.allocate(JAVA_FLOAT, Math.max(floats, 1));
+                check((int) DEBUG_BIOME_LAYOUT.invokeExact(c, r, (long) n, depth, info, gs, ts));
+                MemorySegment.copy(gs, JAVA_INT, 0, grid, 0, (int) cells);
+                MemorySegment.copy(ts, JAVA_FLOAT, 0, tiles, 0, (int) floats);
+            }
+            return out;
+        } catch (RuntimeException e) {
+            throw e;
+        } catch (Throwable t) {
+            throw new RuntimeException(t);
         }
     }
 
@@ -150,6 +189,16 @@ public final class ChunkyCu {
         public void setTriangles(int[] w, int n) { words(SET_TRIANGLES, w, n); }
         public void setWorldBvh(int[] w) { words(SET_WORLD_BVH, w, w.length); }
         public void setActorBvh(int[] w) { words(SET_ACTOR_BVH, w, w.length); }
+        /** Biome colours of n chunks: chunks = n x {cx, cz}, rgb = n x 3 planes (foliage, grass, water) x 256 texels x 3 linear floats,
+         *  texel (z &amp; 15) * 16 + (x &amp; 15).  n = 0 removes them. */
+        public void setBiomeColors(int[] chunks, float[] rgb, int n) {
+            checkBiomeArrays(chunks, rgb, n);
+            try (Arena a = Arena.ofConfined()) {
+                MemorySegment c = n > 0 ? a.allocateFrom(JAVA_INT, java.util.Arrays.copyOf(chunks, 2 * n)) : MemorySegment.NULL;
+                MemorySegment r = n > 0 ? a.allocateFrom(JAVA_FLOAT, java.util.Arrays.copyOf(rgb, BIOME_TILE_FLOATS * n)) : MemorySegment.NULL;
+                check(call(SET_BIOME_COLORS, handle, c, r, (long) n));
+            }
+        }
         public void atlasCreate(int width, int height, int layers) { check(call(ATLAS_CREATE, handle, width, height, layers)); }
         /** One call per texture, as clEnqueueWriteImage in ClTextureLoader.java:60-66. */
         public void atlasWrite(int x, int y, int layer, int w, int h, byte[] rgba) {

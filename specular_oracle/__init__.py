@@ -1,5 +1,5 @@
-"""ctypes binding of the CPU restatement of CCU_RENDER_SPECULAR, CCU_RENDER_EMITTER_SAMPLING, CCU_RENDER_EMITTER_NEAR_FIELD
-and CCU_RENDER_EMITTER_MODELS (specular_oracle.c).  TEST INFRASTRUCTURE ONLY.
+"""ctypes binding of the CPU restatement of CCU_RENDER_SPECULAR, CCU_RENDER_EMITTER_SAMPLING, CCU_RENDER_EMITTER_NEAR_FIELD,
+CCU_RENDER_EMITTER_MODELS and CCU_RENDER_BIOME_TINT (specular_oracle.c).  TEST INFRASTRUCTURE ONLY.
 
 ``SpecularOracle`` is the parity oracle (``oracle.Oracle``) with the specular events of DESIGN.md section 9 in its path
 loop; ``FlagsOracle`` takes the render flags and adds the emitter sampling of sections 10 to 12, with the emitter table that
@@ -36,6 +36,7 @@ def lib():
         _lib = C.CDLL(_LIB_PATH)
         assert _lib.oracle_scene_struct_size() == C.sizeof(oracle._Scene), "OracleScene layout mismatch"
         assert _lib.emitter_grid_struct_size() == C.sizeof(_Grid), "EmitterGrid layout mismatch"
+        assert _lib.biome_tiles_struct_size() == C.sizeof(_Biome), "BiomeTiles layout mismatch"
     return _lib
 
 
@@ -44,7 +45,13 @@ class _Grid(C.Structure):
                 ("g0", C.c_int32 * 3), ("dim", C.c_int32 * 3), ("shift", C.c_int32), ("mhead", C.c_void_p), ("mprim", C.c_void_p)]
 
 
+class _Biome(C.Structure):
+    _fields_ = [("grid", C.c_void_p), ("tiles", C.c_void_p), ("x0", C.c_int32), ("z0", C.c_int32), ("gx", C.c_int32),
+                ("gz", C.c_int32)]
+
+
 CCU_RENDER_SPECULAR, CCU_RENDER_EMITTER_SAMPLING, CCU_RENDER_EMITTER_NEAR_FIELD, CCU_RENDER_EMITTER_MODELS = 4, 8, 128, 256
+CCU_RENDER_BIOME_TINT = 512
 EMIT_SHIFT0, EMIT_CELL_BUDGET, EMIT_MAX = 3, 1 << 21, 1 << 18      # DESIGN.md section 10
 
 
@@ -187,6 +194,30 @@ def emitter_grid(p, models: bool = False) -> dict:
     return out
 
 
+BIOME_GRID_MAX = 1 << 24    # DESIGN.md section 13: cells of the chunk grid
+
+
+def biome_layout(chunks, rgb, depth: int) -> dict:
+    """DESIGN.md section 13: the biome layout commit builds (as native.debug_biome_layout returns it): x0, z0 the low chunk of
+    the chunks' bounding box, grid int32[gx, gz] indexed [cx - x0, cz - z0] holding the chunk's tile or -1, tiles
+    float32[n, 3, 256, 4] with w = 0.  Raises ValueError for a chunk outside the octree's max(1, 2^depth / 16) chunks per axis,
+    or a bounding box of more than BIOME_GRID_MAX chunks."""
+    chunks = np.asarray(chunks, np.int64).reshape(-1, 2)
+    rgb = np.asarray(rgb, np.float32).reshape(-1, 3, 256, 3)
+    extent = 1 << max(depth - 4, 0)
+    if chunks.size and (chunks.min() < 0 or chunks.max() >= extent):
+        raise ValueError(f"a chunk lies outside the octree's {extent} x {extent} chunks")
+    lo = chunks.min(0) if chunks.size else np.zeros(2, np.int64)
+    dim = chunks.max(0) - lo + 1 if chunks.size else np.zeros(2, np.int64)
+    if int(dim[0]) * int(dim[1]) > BIOME_GRID_MAX:
+        raise ValueError(f"the chunks span more than {BIOME_GRID_MAX} chunks")
+    grid = np.full((int(dim[0]), int(dim[1])), -1, np.int32)
+    grid[chunks[:, 0] - lo[0], chunks[:, 1] - lo[1]] = np.arange(chunks.shape[0], dtype=np.int32)
+    tiles = np.zeros((chunks.shape[0], 3, 256, 4), np.float32)
+    tiles[..., :3] = rgb
+    return {"x0": int(lo[0]), "z0": int(lo[1]), "grid": grid, "tiles": tiles}
+
+
 class SpecularOracle(oracle.Oracle):
     """oracle.Oracle whose render() runs the path loop with CCU_RENDER_SPECULAR on."""
 
@@ -210,13 +241,22 @@ class SpecularOracle(oracle.Oracle):
 
 class FlagsOracle(oracle.Oracle):
     """oracle.Oracle whose render() runs the path loop with the given CCU_RENDER_SPECULAR / CCU_RENDER_EMITTER_SAMPLING /
-    CCU_RENDER_EMITTER_NEAR_FIELD / CCU_RENDER_EMITTER_MODELS bits (the other flags act on the scene:
+    CCU_RENDER_EMITTER_NEAR_FIELD / CCU_RENDER_EMITTER_MODELS / CCU_RENDER_BIOME_TINT bits (the other flags act on the scene:
     oracle.edge_rays.without_sun, or empty BVHs for CCU_RENDER_NO_ENTITIES).  With CCU_RENDER_EMITTER_MODELS the wider table
-    of section 12 is sampled when the scene has one, else the table of section 10."""
+    of section 12 is sampled when the scene has one, else the table of section 10.  With CCU_RENDER_BIOME_TINT the biome
+    colours are `biome` = (chunks, rgb) as ccu_scene_set_biome_colors takes them, by default the scene's own (scene.biome)."""
 
-    def __init__(self, scene, flags: int = 0, **kw):
+    def __init__(self, scene, flags: int = 0, biome=None, **kw):
         super().__init__(scene, **kw)
         self.flags = flags
+        if biome is None:
+            biome = getattr(scene, "biome", None)
+        self._biome = None
+        if flags & CCU_RENDER_BIOME_TINT and biome is not None and np.asarray(biome[0]).size > 0:
+            b = biome_layout(biome[0], biome[1], scene.octree_depth)
+            grid, tiles = b["grid"], b["tiles"]
+            self._keep["biome_grid"], self._keep["biome_tiles"] = grid, tiles
+            self._biome = _Biome(grid.ctypes.data, tiles.ctypes.data, b["x0"], b["z0"], grid.shape[0], grid.shape[1])
         self.grid = emitter_grid(scene, models=True) if flags & CCU_RENDER_EMITTER_MODELS else None
         if not (self.grid and self.grid["has_emitters"]):
             self.grid = emitter_grid(scene)
@@ -248,6 +288,7 @@ class FlagsOracle(oracle.Oracle):
         lib().flags_render(C.byref(self._s), sd.ctypes.data_as(C.c_void_p), C.c_int(sd.size), C.c_int(start_spp),
                            res.ctypes.data_as(C.c_void_p), gp, C.c_int64(gn), C.c_int(threads), C.byref(cnt),
                            C.c_int(1 if self.flags & CCU_RENDER_SPECULAR else 0), C.byref(self._grid) if nee else None,
-                           C.c_int(1 if self.flags & CCU_RENDER_EMITTER_NEAR_FIELD else 0))
+                           C.c_int(1 if self.flags & CCU_RENDER_EMITTER_NEAR_FIELD else 0),
+                           C.byref(self._biome) if self._biome is not None else None)
         self._counters(cnt)
         return res
