@@ -4,16 +4,17 @@
 // that air leaf (octree.h:89-106: an air leaf is left through its cube, anything else goes to the block test).  The
 // layout built at commit (chunkycu.cu, build_air_layout) answers that with at most ONE global load below the top table:
 //
-//   air_top[]     dense table over the cells of level air_cell_level (>= 4), index (x*dim + y)*dim + z.  Entry:
+//   air_top[]     dense table over the cells of level air_cell_level (>= 4), index (x*dim + y)*dim + z.
+//                 Shallow worlds (air_cell_level == 4): every entry is the word offset of a brick in air_bricks; a cell that
+//                 is a single leaf refers to the constant brick of that leaf (every voxel = its level, or not air).
+//                 Deep worlds (air_cell_level > 4), and the entries of air_wide[]:
 //                   bit 31 set   leaf  {bits 30..26: level of the air leaf, 31 = not air}
-//                   bit 31 clear index of a brick (air_cell_level == 4) or of a 64-ary node (deeper worlds)
+//                   bit 31 clear word offset of a brick (entries at level 4) or index of a 64-ary node (above)
 //   air_wide[]    64-ary nodes (two octree levels per load), only for worlds whose top table would not fit with 16^3
-//                 cells (octree depth > 11); same entry encoding, entries at level 4 refer to bricks
-//   air_bricks[]  one 1-KiB brick per 16^3 cell that is not a single leaf: 64 blocks of 4^3 voxels, block index
-//                 ((x>>2)&3)<<4 | ((y>>2)&3)<<2 | ((z>>2)&3), 4 words per block (word = x&3), 2 bits per voxel at bit
-//                 position 2*(((y&3)<<2) | (z&3)):  0 = not air, 1 = air leaf of level 0, 2 = air leaf of level 1.
-//                 A 4^3 block that lies inside ONE leaf of level 2 or 3 has all four words = 0 (not air) or
-//                 0xC0000000 | level (air); mixed words never have their top code = 3, so `word >= 0xC0000000` tells.
+//                 cells (octree depth > 11)
+//   air_bricks[]  one 2-KiB brick (CCU_BRICK_WORDS words) per 16^3 cell: 4 bits per voxel, the level of the voxel's air
+//                 leaf (0..14) or CCU_AIR_SOLID (15) = not air.  Voxel (x, y, z) of the cell is the nibble z & 7 of word
+//                 (x << 5) | (y << 1) | (z >> 3) (air_brick_word / air_brick_level): one shift and one mask decode it.
 //
 // The arithmetic of a step is exactly the reference's (same operations on the same values in the same order, so the
 // marched distance is bit-identical); only loop invariants are hoisted and the leaf lookup is replaced.
@@ -22,7 +23,21 @@
 
 namespace ccu {
 
-#define CCU_BRICK_UNIFORM 0xC0000000u
+#define CCU_BRICK_WORDS 512u   // words of a brick: 16^3 voxels x 4 bits
+#define CCU_AIR_SOLID 15        // brick code of a voxel that is not air
+
+// word of a brick that holds voxel (x, y, z) of its cell (only the low 4 bits of each coordinate count)
+__host__ __device__ __forceinline__ unsigned air_brick_word(int x, int y, int z) {
+    return (((unsigned)x & 15u) << 5) | (((unsigned)y & 15u) << 1) | (((unsigned)z >> 3) & 1u);
+}
+// code of voxel z of brick word w: the level of its air leaf, CCU_AIR_SOLID = not air (the rotation takes z << 2 mod 32)
+__host__ __device__ __forceinline__ int air_brick_level(unsigned w, int z) {
+#ifdef __CUDA_ARCH__
+    return (int)(__funnelshift_r(w, w, (unsigned)z << 2) & 15u);
+#else
+    return (int)((w >> ((z & 7) * 4)) & 15u);
+#endif
+}
 
 struct LeanRay {
     float3 o, d, inv, doff;   // doff = d * OFFSET (octree.h:73, loop invariant)
@@ -63,10 +78,10 @@ __device__ __forceinline__ float lean_exit_axis(int b, int low, int fm, float q,
 // One iteration of octree.h:66-107.  Returns 0 = air leaf left (keep marching), 1 = non-air leaf reached (ray not
 // advanced; the block test looks the leaf up), 2 = ray finished without a hit.
 // TOPS: `top` is the air top table staged in shared memory, otherwise it is read from global memory.
-// DEEP: air_cell_level > 4 (64-ary nodes between the top table and the bricks).
+// DEEP: air_cell_level > 4 (64-ary nodes between the top table and the bricks).  draw_depth: as in lean_step_flat.
 template <bool DEEP, bool TOPS>
-__device__ __forceinline__ int lean_probe(const DScene &s, const unsigned *__restrict__ top, LeanRay &r) {
-    if (r.steps >= s.draw_depth || r.t > r.limit) return 2;
+__device__ __forceinline__ int lean_probe(const DScene &s, const unsigned *__restrict__ top, LeanRay &r, int draw_depth) {
+    if (r.steps >= draw_depth || r.t > r.limit) return 2;
     const float3 pos = r.o + r.d * r.t;
     const float3 q = pos + r.doff;
     const int bx = f2i(floorf(q.x)), by = f2i(floorf(q.y)), bz = f2i(floorf(q.z));
@@ -85,16 +100,14 @@ __device__ __forceinline__ int lean_probe(const DScene &s, const unsigned *__res
             e = __ldg(s.air_wide + (e * 64u + (unsigned)((((bx >> lvl) & 3) << 4) | (((by >> lvl) & 3) << 2) | ((bz >> lvl) & 3))));
         }
     }
-    int level;   // level of the air leaf, -1 = not air
-    if (e & CCU_WIDE_LEAF) {
-        level = ((int)(e << 1)) >> 27;       // bits 30..26 as a signed field: 31 = -1 = not air
+    int level;   // level of the air leaf
+    if (DEEP && (e & CCU_WIDE_LEAF)) {
+        level = (int)((e >> 26) & 31u);       // 31 = not air
+        if (level == 31) return 1;
     } else {
-        const unsigned wi = (unsigned)(((bx & 12) << 4) | ((by & 12) << 2) | (bz & 12) | (bx & 3));
-        const unsigned w = __ldg(s.air_bricks + (e * 256u + wi));
-        const int code = (int)((w >> ((((by & 3) << 2) | (bz & 3)) * 2)) & 3u);
-        level = w >= CCU_BRICK_UNIFORM ? (int)(w & 31u) : code - 1;
+        level = air_brick_level(__ldg(s.air_bricks + (e + air_brick_word(bx, by, bz))), bz);
+        if (level == CCU_AIR_SOLID) return 1;
     }
-    if (level < 0) return 1;
     const int low = (1 << level) - 1;
     const float ex = lean_exit_axis(bx, low, r.fmx, q.x, r.inv.x, r.nmx);
     const float ey = lean_exit_axis(by, low, r.fmy, q.y, r.inv.y, r.nmy);
@@ -107,34 +120,41 @@ __device__ __forceinline__ int lean_probe(const DScene &s, const unsigned *__res
 // The same iteration as straight-line code for the shallow layouts (top table over 16^3 cells + bricks): every lane of the warp
 // executes every instruction, lanes without a ray in flight (`active` false) or whose ray ends compute on harmless values and
 // commit nothing.  No branch inside the step means no divergence stacks, no fetch redirects and one load latency per iteration
-// for the whole warp; the lanes whose cell is a single leaf read brick word 0 (one broadcast sector) instead of skipping the load.
+// for the whole warp; the lanes whose cell is a single leaf read the constant brick of that leaf.
 // `done`: the lane's state before the step (only read when !active); returns the state after it.
-template <bool TOPS>
-__device__ __forceinline__ int lean_step_flat(const DScene &s, const unsigned *__restrict__ top, LeanRay &r, bool active, int done) {
-    const bool fin0 = r.steps >= s.draw_depth || r.t > r.limit;
+// The loop invariants come in as values so that a caller's loop keeps them in registers: the step ends once
+// r.steps >= draw_depth (the queue kernel biases steps by -draw_depth and passes 0), and `outside` = ~(2^depth - 1) holds the
+// bits a voxel coordinate inside the octree cube never has.
+// TOP16: the top table has 16^3 cells (s.air_top_log2 == 4) and is staged in shared memory; it is indexed with immediate
+// shifts.  Otherwise it is read from global memory, with s.air_top_log2 cells per axis.
+template <bool TOP16>
+__device__ __forceinline__ int lean_step_flat(const DScene &s, const unsigned *__restrict__ top, LeanRay &r, bool active, int done,
+                                              int draw_depth, unsigned outside) {
+    const bool fin0 = r.steps >= draw_depth || r.t > r.limit;
     const float3 pos = r.o + r.d * r.t;
     const float3 q = pos + r.doff;
     const int bx = f2i(floorf(q.x)), by = f2i(floorf(q.y)), bz = f2i(floorf(q.z));
-    const bool fin = fin0 || (((bx | by | bz) >> s.depth) != 0);
-    const int tl = s.air_top_log2;
+    const bool fin = fin0 || ((unsigned)(bx | by | bz) & outside) != 0;
     // out-of-cube coordinates (finished lanes only) are folded into the table
-    const unsigned ti = (((((unsigned)(bx >> 4) << tl) + (unsigned)(by >> 4)) << tl) + (unsigned)(bz >> 4)) & ((1u << (3 * tl)) - 1u);
-    const unsigned e = TOPS ? top[ti] : __ldg(top + ti);
-    const bool leaf = (e & CCU_WIDE_LEAF) != 0;
-    const unsigned wi = (unsigned)(((bx & 12) << 4) | ((by & 12) << 2) | (bz & 12) | (bx & 3));
-    const unsigned w = __ldg(s.air_bricks + (leaf ? 0u : e * 256u + wi));
-    const int code = (int)((w >> ((((by & 3) << 2) | (bz & 3)) * 2)) & 3u);
-    const int lvl_brick = w >= CCU_BRICK_UNIFORM ? (int)(w & 31u) : code - 1;
-    const int level = leaf ? ((int)(e << 1)) >> 27 : lvl_brick;       // -1 = not air
-    const int low = (1 << (level & 31)) - 1;
+    unsigned ti;
+    if (TOP16) {
+        ti = (((unsigned)bx << 4) & 0xF00u) | ((unsigned)by & 0xF0u) | (((unsigned)bz >> 4) & 0xFu);
+    } else {
+        const int tl = s.air_top_log2;
+        ti = (((((unsigned)(bx >> 4) << tl) + (unsigned)(by >> 4)) << tl) + (unsigned)(bz >> 4)) & ((1u << (3 * tl)) - 1u);
+    }
+    const unsigned e = TOP16 ? top[ti] : __ldg(top + ti);
+    const int level = air_brick_level(__ldg(s.air_bricks + (e + air_brick_word(bx, by, bz))), bz);   // CCU_AIR_SOLID = not air
+    const int low = (1 << level) - 1;
     const float ex = lean_exit_axis(bx, low, r.fmx, q.x, r.inv.x, r.nmx);
     const float ey = lean_exit_axis(by, low, r.fmy, q.y, r.inv.y, r.nmy);
     const float ez = lean_exit_axis(bz, low, r.fmz, q.z, r.inv.z, r.nmz);
     const float tn = r.t + (fminf(ex, fminf(ey, ez)) + CCU_OFFSET);
-    const bool adv = active && !fin && level >= 0;
+    const bool air = level != CCU_AIR_SOLID;
+    const bool adv = active && !fin && air;
     r.t = adv ? tn : r.t;
     r.steps += adv ? 1 : 0;
-    return active ? (fin ? 2 : (level < 0 ? 1 : 0)) : done;
+    return active ? (fin ? 2 : (air ? 0 : 1)) : done;
 }
 
 // Octree_octreeIntersect (octree.h:41-109) for the thread-per-ray kernels (first-hit, preview, thread-per-pixel render):
@@ -148,7 +168,7 @@ __device__ __forceinline__ bool octree_intersect_lean(const DScene &s, float3 or
     r.o = m.o; r.d = m.d; r.inv = m.inv; r.t = m.t; r.limit = m.limit; r.steps = m.steps;
     lean_prepare(r);
     for (;;) {
-        const int st = lean_probe<DEEP, false>(s, s.air_top, r);
+        const int st = lean_probe<DEEP, false>(s, s.air_top, r, s.draw_depth);
         if (st == 0) continue;
         if (st == 2) return false;
         m.t = r.t; m.steps = r.steps;

@@ -230,14 +230,19 @@ __device__ __forceinline__ void q_store_ray(uint32_t *F, unsigned *mask, int lan
 // ------------------------------------------------------------------------------------------------------
 // stages
 // ------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void q_load_lean(const uint32_t *F, int slot, LeanRay &r) {
+// r.steps is loaded as steps - draw_depth (the march loop then ends a ray at r.steps >= 0); q_store_lean_t undoes that.
+__device__ __forceinline__ void q_load_lean(const uint32_t *F, int slot, LeanRay &r, int draw_depth) {
     r.o = f3(__uint_as_float(F[QF_OX * Q_SLOTS + slot]), __uint_as_float(F[QF_OY * Q_SLOTS + slot]), __uint_as_float(F[QF_OZ * Q_SLOTS + slot]));
     r.d = f3(__uint_as_float(F[QF_DX * Q_SLOTS + slot]), __uint_as_float(F[QF_DY * Q_SLOTS + slot]), __uint_as_float(F[QF_DZ * Q_SLOTS + slot]));
     r.inv = f3(__uint_as_float(F[QF_IX * Q_SLOTS + slot]), __uint_as_float(F[QF_IY * Q_SLOTS + slot]), __uint_as_float(F[QF_IZ * Q_SLOTS + slot]));
     r.t = __uint_as_float(F[QF_T * Q_SLOTS + slot]);
     r.limit = __uint_as_float(F[QF_LIMIT * Q_SLOTS + slot]);
-    r.steps = (int)F[QF_STEPS * Q_SLOTS + slot];
+    r.steps = (int)F[QF_STEPS * Q_SLOTS + slot] - draw_depth;
     lean_prepare(r);
+}
+__device__ __forceinline__ void q_store_lean_t(uint32_t *F, int slot, const LeanRay &r, int draw_depth) {
+    F[QF_T * Q_SLOTS + slot] = __float_as_uint(r.t);
+    F[QF_STEPS * Q_SLOTS + slot] = (uint32_t)(r.steps + draw_depth);
 }
 
 // MARCH (NST = number of stages of this kernel; LAY: 0 = top table in shared memory, 1 = in global memory, 2 = deep world)
@@ -245,11 +250,13 @@ template <int NST, int LAY>
 __device__ __forceinline__ void q_stage_march(const DScene &s, const unsigned *__restrict__ top, uint32_t *F, unsigned *mask, int lane,
                                               int yield_below, int refill_min) {
     const unsigned full = 0xffffffffu;
+    const int draw_depth = s.draw_depth;
+    const unsigned outside = ~0u << s.depth;
     int cur = -1;   // slot of the ray this lane is marching (row * 32 + column), -1 = none
     LeanRay r;
     r.o = r.d = r.inv = r.doff = f3(0, 0, 0);
     r.t = 0; r.limit = 0; r.steps = 0; r.fmx = r.fmy = r.fmz = 0; r.nmx = r.nmy = r.nmz = 0;
-    int done = 0;   // 0 = ray in flight, 1 = reached a non-air leaf, 2 = finished
+    int done = 2;   // 0 = ray in flight, 1 = reached a non-air leaf, 2 = finished or no ray (cur < 0)
     int recheck = 0;
     int busy = 0;   // lanes that hold a ray, in flight or finished (warp-uniform, changes only at a refill)
     int n_fly = 0;  // lanes whose ray is in flight (warp-uniform)
@@ -257,16 +264,17 @@ __device__ __forceinline__ void q_stage_march(const DScene &s, const unsigned *_
         // Finished rays are handed over and idle lanes re-filled in batches: once refill_min lanes hold a finished
         // ray, or nothing is in flight.
         {
-            if (cur < 0 || done != 0) {
+            if (done != 0) {
                 if (cur >= 0) {
-                    F[QF_T * Q_SLOTS + cur] = __float_as_uint(r.t);
-                    F[QF_STEPS * Q_SLOTS + cur] = (uint32_t)r.steps;
+                    q_store_lean_t(F, cur, r, draw_depth);
                     q_push(mask, done == 1 ? QS_BLOCK : QS_EXIT, cur & 31, cur >> 5);
-                    done = 0;
                 }
                 const int row = q_pop(mask, QS_MARCH, lane);
                 cur = row < 0 ? -1 : row * 32 + lane;
-                if (cur >= 0) q_load_lean(F, cur, r);
+                done = cur < 0 ? 2 : 0;
+                if (cur >= 0) q_load_lean(F, cur, r, draw_depth);
+                else r.steps = 0;   // an idle lane's march step finds its (biased) step budget spent
+
             }
             busy = __popc(__ballot_sync(full, cur >= 0));
             QSTAT(24, 1);
@@ -283,18 +291,22 @@ __device__ __forceinline__ void q_stage_march(const DScene &s, const unsigned *_
                 recheck--;
             }
         }
-        // march until enough lanes hold a finished ray (or nothing is in flight): a tight inner loop with one backward branch
+        // march until enough lanes hold a finished ray (busy - n_fly >= refill_min) or nothing is in flight: a tight inner loop
+        // with one backward branch
+        // The flat step needs no per-lane state besides the ray: a lane whose ray reached a non-air leaf or finished keeps its
+        // t and steps, so every further step looks up the same voxel, finds the same answer and commits nothing, and an idle
+        // lane has r.steps = 0.
+        const int fly_min = max(busy - refill_min, 0);
         do {
-            if (LAY != 2) done = lean_step_flat<LAY == 0>(s, top, r, cur >= 0 && done == 0, done);
-            else if (cur >= 0 && done == 0) done = lean_probe<LAY == 2, LAY == 0>(s, top, r);
-            n_fly = __popc(__ballot_sync(full, cur >= 0 && done == 0));
+            if (LAY != 2) done = lean_step_flat<LAY == 0>(s, top, r, true, 0, 0, outside);
+            else if (done == 0) done = lean_probe<LAY == 2, LAY == 0>(s, top, r, 0);
+            n_fly = __popc(__ballot_sync(full, done == 0));
             QSTAT(10, 1); QSTAT(11, n_fly);
-        } while (busy - n_fly < refill_min && n_fly != 0);
+        } while (n_fly > fly_min);
     }
     // park the rays still in flight, hand over the finished ones
     if (cur >= 0) {
-        F[QF_T * Q_SLOTS + cur] = __float_as_uint(r.t);
-        F[QF_STEPS * Q_SLOTS + cur] = (uint32_t)r.steps;
+        q_store_lean_t(F, cur, r, draw_depth);
         q_push(mask, done == 0 ? QS_MARCH : (done == 1 ? QS_BLOCK : QS_EXIT), cur & 31, cur >> 5);
     }
 }
@@ -936,10 +948,8 @@ __global__ void __launch_bounds__(Q_WARPS * 32, 1) k_render_queue(const __grid_c
         const int rows_here = min(32, Q_ROWS - 32 * w);
         mask[i] = st == QS_END ? (rows_here >= 32 ? 0xffffffffu : ((1u << rows_here) - 1u)) : 0u;
     }
-    if (LAY == 0) {
-        const int n = 1 << (3 * s.air_top_log2);
-        for (int i = threadIdx.x; i < n; i += blockDim.x) top_s[i] = __ldg(s.air_top + i);
-    }
+    // LAY 0: the top table of a shallow world always has 16^3 cells (build_air_layout pads smaller worlds)
+    if (LAY == 0) for (int i = threadIdx.x; i < Q_TOP_WORDS; i += blockDim.x) top_s[i] = __ldg(s.air_top + i);
     // sky / UNORM tables (sky.h:95-106 reads four texels per lookup)
     uchar4 *sky_s = nullptr;
     if (qp.sky_texels > 0) {

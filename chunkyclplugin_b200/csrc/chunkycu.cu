@@ -120,8 +120,8 @@ template <bool DEEP>
 static __device__ __noinline__ int first_hit_march(const DScene &s, LeanRay *ray, int st) {
     LeanRay r = *ray;
     while (__any_sync(0xffffffffu, st == 0)) {
-        if (!DEEP) st = lean_step_flat<false>(s, s.air_top, r, st == 0, st);
-        else if (st == 0) st = lean_probe<DEEP, false>(s, s.air_top, r);
+        if (!DEEP) st = lean_step_flat<false>(s, s.air_top, r, st == 0, st, s.draw_depth, ~0u << s.depth);
+        else if (st == 0) st = lean_probe<DEEP, false>(s, s.air_top, r, s.draw_depth);
     }
     ray->t = r.t;
     ray->steps = r.steps;
@@ -1661,14 +1661,12 @@ int ccu_debug_layout_lookup(const int32_t *tree, int64_t n, int32_t depth, const
             lvl -= 2;
             e = al.wide[(size_t)e * 64 + ((((bx >> lvl) & 3) << 4) | (((by >> lvl) & 3) << 2) | ((bz >> lvl) & 3))];
         }
-        int level;
-        if (e & CCU_WIDE_LEAF) {
+        int level;   // -1 = not air
+        if (e & CCU_WIDE_LEAF) {        // deep worlds only: shallow top entries are all brick offsets
             level = ((int)(e << 1)) >> 27;
         } else {
-            const unsigned wi = (unsigned)(((bx & 12) << 4) | ((by & 12) << 2) | (bz & 12) | (bx & 3));
-            const unsigned w = al.bricks[(size_t)e * 256 + wi];
-            const int code = (int)((w >> ((((by & 3) << 2) | (bz & 3)) * 2)) & 3u);
-            level = w >= CCU_BRICK_UNIFORM ? (int)(w & 31u) : code - 1;
+            const int code = air_brick_level(al.bricks[(size_t)e + air_brick_word(bx, by, bz)], bz);
+            level = code == CCU_AIR_SOLID ? -1 : code;
         }
         if (air_solid) air_solid[i] = level < 0 ? 1 : 0;
         if (air_level) air_level[i] = level;
