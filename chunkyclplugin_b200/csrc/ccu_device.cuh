@@ -117,12 +117,14 @@ __device__ __forceinline__ BiomeView &biome_smem() {
 // roughness bytes.  The other kernels keep the reference's record exactly.
 template <bool SPEC = false>
 struct SurfT {
+    static constexpr bool has_spec = false;
     float3 normal;
     float4 color;
     float emittance;
 };
 template <>
 struct SurfT<true> {
+    static constexpr bool has_spec = true;
     float3 normal;
     float4 color;
     float emittance;
@@ -295,9 +297,9 @@ __device__ __forceinline__ MatOut material_eval_core(const DScene &s, uint32_t f
     return out;
 }
 // rec.color / rec.emittance (and rec.spec) are written only on success (material.h:50-54 rejects before storing)
-template <bool SPEC, bool BIOME = false>
+template <bool BIOME, class Surface>
 __device__ __forceinline__ bool material_eval(const DScene &s, uint32_t flags, uint32_t tint, uint32_t tex_size, uint32_t col, uint32_t normal_emittance,
-                                              uint32_t spec, SurfT<SPEC> &rec, float u, float v, int bx = 0, int bz = 0) {
+                                              uint32_t spec, Surface &rec, float u, float v, int bx = 0, int bz = 0) {
     const MatOut m = material_eval_core<BIOME>(s, flags, tint, tex_size, col, normal_emittance, u, v, bx, bz);
     if (!m.ok) return false;
     rec.color = m.color;
@@ -307,17 +309,16 @@ __device__ __forceinline__ bool material_eval(const DScene &s, uint32_t flags, u
 }
 // Material_get + Material_sample for material pointer `material` (an int offset into matPalette, 6 words per material):
 // two 16-byte loads from the commit-time records, or the reference's own array for a pointer that is not on a record
-template <bool SPEC, bool BIOME = false>
-__device__ __forceinline__ bool material_sample(const DScene &s, int material, SurfT<SPEC> &rec, float u, float v, int bx = 0, int bz = 0) {
+template <bool BIOME = false, class Surface>
+__device__ __forceinline__ bool material_sample(const DScene &s, int material, Surface &rec, float u, float v, int bx = 0, int bz = 0) {
     const int idx = material / 6;
     if (material >= 0 && idx * 6 == material) {
         const int4 a = __ldg(s.mat_rec + 2 * idx), b = __ldg(s.mat_rec + 2 * idx + 1);
-        return material_eval<SPEC, BIOME>(s, (uint32_t)a.x, (uint32_t)a.y, (uint32_t)a.z, (uint32_t)a.w, (uint32_t)b.x, (uint32_t)b.y, rec, u, v,
-                                          bx, bz);
+        return material_eval<BIOME>(s, (uint32_t)a.x, (uint32_t)a.y, (uint32_t)a.z, (uint32_t)a.w, (uint32_t)b.x, (uint32_t)b.y, rec, u, v, bx, bz);
     }
     const int *m = s.mat_palette + material;
-    return material_eval<SPEC, BIOME>(s, __ldg(m), __ldg(m + 1), __ldg(m + 2), __ldg(m + 3), __ldg(m + 4), SPEC ? (uint32_t)__ldg(m + 5) : 0u,
-                                      rec, u, v, bx, bz);
+    return material_eval<BIOME>(s, __ldg(m), __ldg(m + 1), __ldg(m + 2), __ldg(m + 3), __ldg(m + 4), Surface::has_spec ? (uint32_t)__ldg(m + 5) : 0u,
+                                rec, u, v, bx, bz);
 }
 
 // ------------------------------------------------------------------------------------------------------
@@ -464,10 +465,10 @@ struct ModelHit {    // returned by value so that callers keep their state in re
 };
 
 // block.h:66-116: AABB models (type 2) and quad models (type 3).  Cold path, kept out of line (intersect_model_block).
-template <bool SPEC, bool BIOME>
-__device__ __forceinline__ ModelHit<SPEC> model_block_hit(const DScene &s, int model_type, int model_ptr, float3 norm_origin, float3 direction,
-                                                          float3 inv, int bx, int bz) {
-    ModelHit<SPEC> out;
+template <bool BIOME, class Hit>
+__device__ __forceinline__ Hit model_block_hit(const DScene &s, int model_type, int model_ptr, float3 norm_origin, float3 direction, float3 inv,
+                                               int bx, int bz) {
+    Hit out;
     out.surf.normal = f3(0, 0, 0);
     out.surf.color = make_float4(0, 0, 0, 0);
     out.surf.emittance = 0;
@@ -486,7 +487,7 @@ __device__ __forceinline__ ModelHit<SPEC> model_block_hit(const DScene &s, int m
             for (int k = 0; k < 4; k++) { const int4 t = __ldg(r + k); w[4 * k] = t.x; w[4 * k + 1] = t.y; w[4 * k + 2] = t.z; w[4 * k + 3] = t.w; }
             int material = 0;
             float t = textured_box(w, dist, norm_origin, direction, inv, normal, u, v, material);
-            if (!is_nan(t) && material_sample<SPEC, BIOME>(s, material, out.surf, u, v, bx, bz)) { out.surf.normal = normal; dist = t; hit = true; }
+            if (!is_nan(t) && material_sample<BIOME>(s, material, out.surf, u, v, bx, bz)) { out.surf.normal = normal; dist = t; hit = true; }
         }
     } else {
         const int quads = __ldg(s.quad_rec + model_ptr).x;
@@ -495,7 +496,7 @@ __device__ __forceinline__ ModelHit<SPEC> model_block_hit(const DScene &s, int m
 #pragma unroll
             for (int k = 0; k < 4; k++) { const int4 t = __ldg(r + k); w[4 * k] = t.x; w[4 * k + 1] = t.y; w[4 * k + 2] = t.z; w[4 * k + 3] = t.w; }
             float t = quad_hit(w, dist, norm_origin, direction, normal, u, v);
-            if (!is_nan(t) && material_sample<SPEC, BIOME>(s, w[13], out.surf, u, v, bx, bz)) { out.surf.normal = normal; dist = t; hit = true; }
+            if (!is_nan(t) && material_sample<BIOME>(s, w[13], out.surf, u, v, bx, bz)) { out.surf.normal = normal; dist = t; hit = true; }
         }
     }
     out.dist = hit ? dist : nanf_();
@@ -504,21 +505,21 @@ __device__ __forceinline__ ModelHit<SPEC> model_block_hit(const DScene &s, int m
 template <bool SPEC>
 static __device__ __noinline__ ModelHit<SPEC> intersect_model_block(const DScene &s, int model_type, int model_ptr, float3 norm_origin,
                                                        float3 direction, float3 inv) {
-    return model_block_hit<SPEC, false>(s, model_type, model_ptr, norm_origin, direction, inv, 0, 0);
+    return model_block_hit<false, ModelHit<SPEC>>(s, model_type, model_ptr, norm_origin, direction, inv, 0, 0);
 }
 // the same for the biome kernels: (bx, bz) is the model's voxel column
 template <bool SPEC>
 static __device__ __noinline__ ModelHit<SPEC> intersect_model_block_biome(const DScene &s, int model_type, int model_ptr, float3 norm_origin,
                                                              float3 direction, float3 inv, int bx, int bz) {
-    return model_block_hit<SPEC, true>(s, model_type, model_ptr, norm_origin, direction, inv, bx, bz);
+    return model_block_hit<true, ModelHit<SPEC>>(s, model_type, model_ptr, norm_origin, direction, inv, bx, bz);
 }
 
 // Returns the hit distance relative to the marched position (NaN = miss) and fills `surf` on a hit.
 // (The reference also overwrites record.normal when a full block fails its alpha test, block.h:59-60; that
 // value is never read before the next successful hit overwrites it, so it is not reproduced.)
 // BIOME: the biome colours of voxel column (bx, bz) tint the surface (DESIGN §13).
-template <bool SPEC, bool BIOME = false>
-__device__ __forceinline__ float intersect_block(const DScene &s, int block, int bx, int by, int bz, SurfT<SPEC> &surf, float3 pos,
+template <bool BIOME, class Surface>
+__device__ __forceinline__ float intersect_block(const DScene &s, int block, int bx, int by, int bz, Surface &surf, float3 pos,
                                                  float3 direction, float3 inv) {
     if (block == CCU_ANY_TYPE) return nanf_();
     if (block < 0 || block + 1 >= s.block_palette_len) return nanf_();   // out-of-palette leaf (undefined in the reference)
@@ -535,7 +536,7 @@ __device__ __forceinline__ float intersect_block(const DScene &s, int block, int
         Surf tmp;
         // the full cube's material travels with its palette entry
         const int4 r1 = __ldg(s.block_rec + 2 * block + 1);
-        if (!material_eval<false, BIOME>(s, (uint32_t)r0.z, (uint32_t)r0.w, (uint32_t)r1.x, (uint32_t)r1.y, (uint32_t)r1.z, 0u, tmp, u, v, bx, bz))
+        if (!material_eval<BIOME>(s, (uint32_t)r0.z, (uint32_t)r0.w, (uint32_t)r1.x, (uint32_t)r1.y, (uint32_t)r1.z, 0u, tmp, u, v, bx, bz))
             return nanf_();
         surf.color = tmp.color;
         surf.emittance = tmp.emittance;
@@ -544,8 +545,8 @@ __device__ __forceinline__ float intersect_block(const DScene &s, int block, int
         return dist - CCU_OFFSET;
     }
     if (model_type == 2 || model_type == 3) {
-        ModelHit<SPEC> m = BIOME ? intersect_model_block_biome<SPEC>(s, model_type, model_ptr, norm_origin, direction, inv, bx, bz)
-                                 : intersect_model_block<SPEC>(s, model_type, model_ptr, norm_origin, direction, inv);
+        const auto m = BIOME ? intersect_model_block_biome<Surface::has_spec>(s, model_type, model_ptr, norm_origin, direction, inv, bx, bz)
+                             : intersect_model_block<Surface::has_spec>(s, model_type, model_ptr, norm_origin, direction, inv);
         if (is_nan(m.dist)) return nanf_();
         surf = m.surf;
         return m.dist;
@@ -655,11 +656,10 @@ __device__ __forceinline__ void march_exit(March &m, const Cell &c, int level) {
 // otherwise the ray has been advanced past the leaf.
 // CUT (kernels built with CCU_RENDER_EMITTER_MODELS) and `cut` (the ray is an emitter sample's shadow ray): the hit counts only
 // when it lies before the ray's limit, so that a model's own voxel does not occlude the primitive sampled inside it (DESIGN §12).
-// BIOME: the kernels of CCU_RENDER_BIOME_TINT (intersect_block).
-template <bool SPEC, bool CUT = false, bool BIOME = false>
-__device__ __forceinline__ bool march_block(const DScene &s, March &m, int data, int level, SurfT<SPEC> &surf, float &hit_t, bool cut = false) {
+template <class V, bool CUT = false>
+__device__ __forceinline__ bool march_block(const DScene &s, March &m, int data, int level, SurfT<V::spec> &surf, float &hit_t, bool cut = false) {
     Cell c = march_cell(m);
-    float dist = intersect_block<SPEC, BIOME>(s, data, c.bx, c.by, c.bz, surf, c.pos, m.d, m.inv);
+    float dist = intersect_block<V::biome>(s, data, c.bx, c.by, c.bz, surf, c.pos, m.d, m.inv);
     if (!is_nan(dist) && !(CUT && cut && !(m.t + dist < m.limit))) {
         hit_t = m.t + dist;
         return true;
@@ -670,8 +670,8 @@ __device__ __forceinline__ bool march_block(const DScene &s, March &m, int data,
 
 // One whole iteration of octree.h:66-107 on the reference's own node array (root descent per step).
 // Returns 0 = keep marching, 1 = hit (hit_t / surf / block / node filled), 2 = ray left.
-template <bool SPEC, bool CUT = false, bool BIOME = false>
-__device__ __forceinline__ int march_step_ref(const DScene &s, March &m, SurfT<SPEC> &surf, float &hit_t, int &hit_block, int &hit_node, Cell &hit_cell) {
+template <class V, bool CUT = false>
+__device__ __forceinline__ int march_step_ref(const DScene &s, March &m, SurfT<V::spec> &surf, float &hit_t, int &hit_block, int &hit_node, Cell &hit_cell) {
     if (m.steps >= s.draw_depth || m.t > m.limit) return 2;
     const int depth = s.depth;
     const Cell c = march_cell(m);
@@ -682,7 +682,7 @@ __device__ __forceinline__ int march_step_ref(const DScene &s, March &m, SurfT<S
         march_exit(m, c, level);
         return 0;
     }
-    if (march_block<SPEC, CUT, BIOME>(s, m, data, level, surf, hit_t, CUT)) {
+    if (march_block<V, CUT>(s, m, data, level, surf, hit_t, CUT)) {
         hit_block = data;
         hit_node = node;
         hit_cell = c;
@@ -691,15 +691,15 @@ __device__ __forceinline__ int march_step_ref(const DScene &s, March &m, SurfT<S
     return 0;
 }
 
-template <bool SPEC, bool CUT = false, bool BIOME = false>
-__device__ __forceinline__ bool octree_intersect_ref(const DScene &s, float3 origin, float3 direction, RecordT<SPEC> &rec, HitInfo &hi) {
+template <class V, bool CUT = false>
+__device__ __forceinline__ bool octree_intersect_ref(const DScene &s, float3 origin, float3 direction, RecordT<V::spec> &rec, HitInfo &hi) {
     March m;
     if (!march_begin(s, m, origin, direction, rec.distance)) return false;
     for (;;) {
         float t;
         int block, node;
         Cell cell;
-        int r = march_step_ref<SPEC, CUT, BIOME>(s, m, rec.surf, t, block, node, cell);
+        int r = march_step_ref<V, CUT>(s, m, rec.surf, t, block, node, cell);
         if (r == 1) {
             rec.distance = t;
             rec.material = block;
@@ -798,9 +798,9 @@ __device__ __forceinline__ bool bvh_pair(const DScene &s, float3 origin, float3 
 }
 
 // kernel.h:14-24 on the reference's own node array
-template <bool SPEC, bool CUT = false, bool BIOME = false>
-__device__ __forceinline__ bool closest_intersect_ref(const DScene &s, float3 origin, float3 direction, RecordT<SPEC> &rec, HitInfo &hi) {
-    bool hit = octree_intersect_ref<SPEC, CUT, BIOME>(s, origin, direction, rec, hi);
+template <class V, bool CUT = false>
+__device__ __forceinline__ bool closest_intersect_ref(const DScene &s, float3 origin, float3 direction, RecordT<V::spec> &rec, HitInfo &hi) {
+    bool hit = octree_intersect_ref<V, CUT>(s, origin, direction, rec, hi);
     int kind = 0;
     if (bvh_pair(s, origin, direction, rec.distance, rec.surf, kind)) {
         hit = true;
@@ -979,6 +979,14 @@ __device__ __forceinline__ int emitter_list(const EmitView &g, int3 c, int &N) {
 enum NeeKind : int { NEE_NONE = 0, NEE_AREA = 1, NEE_NEAR = 2, NEE_AREA_MODELS = 3, NEE_NEAR_MODELS = 4 };
 __host__ __device__ constexpr bool nee_near_field(int kind) { return kind == NEE_NEAR || kind == NEE_NEAR_MODELS; }
 __host__ __device__ constexpr bool nee_models(int kind) { return kind == NEE_AREA_MODELS || kind == NEE_NEAR_MODELS; }
+// The shading variant a render kernel is built with, picked per launch by shade_variant (chunkycu.cu, DESIGN §5).
+template <bool S, NeeKind N, bool B>
+struct Shade {
+    static constexpr bool spec = S, biome = B;
+    static constexpr NeeKind nee = N;
+    static constexpr bool models = nee_models(N);   // the wider emitter table of CCU_RENDER_EMITTER_MODELS
+};
+using PlainShade = Shade<false, NEE_NONE, false>;   // the first-hit and preview kernels
 #define CCU_NEE_RHO2 0.015625f   // DESIGN §11: an emitter is near when its box distance² is below rho² = (1/8)²
 
 // The emission rule: an octree hit on voxel (bx, by, bz) of block palette position `block` that the previous hit's sample
@@ -1075,7 +1083,7 @@ __device__ __forceinline__ bool nee_model(const DScene &s, const EmitView &g, in
             const float3 inv = f3(1.0f / w.x, 1.0f / w.y, 1.0f / w.z);
             Surf hit;
             hit.emittance = 0.0f;
-            const float t = intersect_block<false, BIOME>(s, e.w, e.x, e.y, e.z, hit, x, w, inv);
+            const float t = intersect_block<BIOME>(s, e.w, e.x, e.y, e.z, hit, x, w, inv);
             if (is_nan(t) || !(hit.emittance > 0.0f)) return false;
             const float k = (hit.emittance * s.emitter_scale) * (float)N;
             c = f3((T.x * (hit.color.x * hit.color.x)) * k, (T.y * (hit.color.y * hit.color.y)) * k, (T.z * (hit.color.z * hit.color.z)) * k);

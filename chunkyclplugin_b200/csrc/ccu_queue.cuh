@@ -71,7 +71,7 @@ enum QField : int {
     QF_COUNT_BVH_SPEC,
     QF_HDIST = QF_LIMIT, QF_HEM = QF_T, QF_HNX = QF_STEPS
 };
-// NEE kernels only (CCU_RENDER_EMITTER_SAMPLING, DESIGN §10): two fields after all the others, q_nee_field(bvh, spec) + 0 / 1,
+// NEE kernels only (CCU_RENDER_EMITTER_SAMPLING, DESIGN §10): two fields after all the others, q_fields(bvh, spec) + 0 / 1,
 // hold the y / z of the emitter sample's contribution while its shadow ray is in flight (x sits in QF_SHW, free then).  The
 // surface normal waits in QF_SN* as for the sun's shadow ray; during the bounce segment that follows a sample, QF_SN* hold
 // the sampled cell (ints) for the emission rule.
@@ -95,7 +95,6 @@ constexpr int Q_STACK = CCU_Q_STACK;
 constexpr int Q_DEEP = 64 - Q_STACK;          // stack entries beyond the shared-memory part
 constexpr int Q_STACK_WORDS = Q_STACK * Q_SLOTS;
 __host__ __device__ constexpr int q_fields(bool bvh, bool spec) { return bvh ? (spec ? (int)QF_COUNT_BVH_SPEC : (int)QF_COUNT_BVH) : (int)QF_COUNT; }
-__host__ __device__ constexpr int q_nee_field(bool bvh, bool spec) { return q_fields(bvh, spec); }
 __host__ __device__ constexpr int q_fields(bool bvh, bool spec, bool nee) { return q_fields(bvh, spec) + (nee ? 2 : 0); }
 __host__ __device__ constexpr int q_stages(bool bvh) { return bvh ? (int)QS_COUNT_BVH : (int)QS_COUNT; }
 __host__ __device__ constexpr int q_mask_words(bool bvh) { return q_stages(bvh) * Q_MW * 32; }
@@ -314,17 +313,18 @@ __device__ __forceinline__ void q_stage_march(const DScene &s, const unsigned *_
 // What follows closestIntersect in rayTracer.cl:93-107 for a ray whose closest hit is known: sky for a miss
 // (kernel.h:26-31), otherwise the surface response (kernel.h:33-44) and the sun sampling ray (sky.h:68-93); when the ray
 // was the shadow ray (or sun sampling is off) the diffuse bounce (nextPath, kernel.h:46-98) follows right away.
-// SPEC: a specular event at the hit (DESIGN "Beyond the reference: specular materials") bounces right away, without a sun sample.
-// NEE (a NeeKind): after the sun sample (or in its place) and before the bounce, the emitter sample of DESIGN §10 (§11 for
-// NEE_NEAR) with its own shadow ray (NFI: index of the two NEE fields); `covered`: the hit is an emitter the previous hit's sample covered, whose emission is
-// left out.  BIOME: the emitter sample reads the biome colours of CCU_RENDER_BIOME_TINT (DESIGN §13).
-template <bool SPEC, int NEE, int NFI, bool BIOME>
+// V::spec: a specular event at the hit (DESIGN "Beyond the reference: specular materials") bounces right away, without a sun sample.
+// V::nee: after the sun sample (or in its place) and before the bounce, the emitter sample of DESIGN §10 (§11 for NEE_NEAR) with its
+// own shadow ray (NFI: index of the two NEE fields); `covered`: the hit is an emitter the previous hit's sample covered, whose
+// emission is left out.  V::biome: the emitter sample reads the biome colours of CCU_RENDER_BIOME_TINT (DESIGN §13).
+template <bool HAS_BVH, class V>
 __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint32_t *F, unsigned *mask, int lane, int row, float3 o,
-                                        float3 d, float distance, bool ray_hit, const SurfT<SPEC> &hit, bool covered) {
+                                        float3 d, float distance, bool ray_hit, const SurfT<V::spec> &hit, bool covered) {
+    constexpr int NFI = q_fields(HAS_BVH, V::spec);
     const int slot = row * 32 + lane;
-    uint32_t meta = QU(QF_META) & ~(NEE ? (QM_HIT | QM_COVERED) : QM_HIT);
+    uint32_t meta = QU(QF_META) & ~(V::nee ? (QM_HIT | QM_COVERED) : QM_HIT);
     const bool shadow = (meta & QM_SHADOW) != 0;
-    const bool nee_ray = NEE && (meta & QM_NEE_RAY) != 0;
+    const bool nee_ray = V::nee && (meta & QM_NEE_RAY) != 0;
     // What the path continues with: the sun-sampling shadow ray (sky.h:68-93), the diffuse bounce (nextPath, kernel.h:46-98), or
     // nothing (END).  Both continuations draw two random numbers, take the sine / cosine of 2 pi x2 and start a ray: that part is
     // written ONCE below the case analysis, so a batch that mixes the cases runs it once.
@@ -336,7 +336,7 @@ __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint
     bool specular = false;           // SPEC: the bounce is a specular event's (mirror direction blended by the roughness ro)
     float ro = 0;
     if (!ray_hit) {
-        if (NEE && nee_ray) {
+        if (V::nee && nee_ray) {
             // the emitter sample's shadow ray reached its limit: its contribution counts
             float3 color = f3(QFL(QF_COLX), QFL(QF_COLY), QFL(QF_COLZ));
             color = color + f3(QFL(QF_SHW), QFL(NFI), QFL(NFI + 1));
@@ -350,33 +350,33 @@ __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint
             float3 sky = sky_radiance(s, d);
             color = color + (sky * throughput) * (shadow ? QFL(QF_SHW) : 1.0f);
             QFL(QF_COLX) = color.x; QFL(QF_COLY) = color.y; QFL(QF_COLZ) = color.z;
-            if (shadow) { if (NEE) nee_step = true; else bounce = true; }
+            if (shadow) { if (V::nee) nee_step = true; else bounce = true; }
             else q_push(mask, QS_END, lane, row);
         }
     } else if (shadow) {
-        if (NEE) nee_step = true; else bounce = true;
-    } else if (NEE && nee_ray) {
+        if (V::nee) nee_step = true; else bounce = true;
+    } else if (V::nee && nee_ray) {
         bounce = true;               // the emitter sample is occluded
         nee_ran = true;
-    } else if (!SPEC) {
+    } else if (!V::spec) {
         // kernel.h:20-22 + applyRayColor kernel.h:33-44
         float3 throughput = f3(QFL(QF_THRX), QFL(QF_THRY), QFL(QF_THRZ));
         float3 color = f3(QFL(QF_COLX), QFL(QF_COLY), QFL(QF_COLZ));
         from = o + d * (distance - CCU_OFFSET);
         float3 col = f3(hit.color.x, hit.color.y, hit.color.z);
         throughput = throughput * col;
-        if (!(NEE && covered)) color = color + (col * (hit.emittance * s.emitter_scale)) * throughput;
+        if (!(V::nee && covered)) color = color + (col * (hit.emittance * s.emitter_scale)) * throughput;
         QFL(QF_THRX) = throughput.x; QFL(QF_THRY) = throughput.y; QFL(QF_THRZ) = throughput.z;
         QFL(QF_COLX) = color.x; QFL(QF_COLY) = color.y; QFL(QF_COLZ) = color.z;
         normal = hit.normal;
         if (s.sun_flags & 1) sun = true;
-        else if (NEE) nee_step = true;
+        else if (V::nee) nee_step = true;
         else bounce = true;
     } else {
         // the event draws come first; then applyRayColor (diffuse event) or its emission with the throughput tinted by a
         // metal only (specular event)
         bool metal = false;
-        if constexpr (SPEC) {
+        if constexpr (V::spec) {
             uint32_t rng = QU(QF_RNG);
             specular = specular_event(hit.spec, rng, metal, ro);
             QU(QF_RNG) = rng;
@@ -386,16 +386,16 @@ __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint
         from = o + d * (distance - CCU_OFFSET);
         float3 col = f3(hit.color.x, hit.color.y, hit.color.z);
         const float3 tinted = throughput * col;
-        if (!(NEE && covered)) color = color + (col * (hit.emittance * s.emitter_scale)) * tinted;
+        if (!(V::nee && covered)) color = color + (col * (hit.emittance * s.emitter_scale)) * tinted;
         if (!specular || metal) throughput = tinted;
         QFL(QF_THRX) = throughput.x; QFL(QF_THRY) = throughput.y; QFL(QF_THRZ) = throughput.z;
         QFL(QF_COLX) = color.x; QFL(QF_COLY) = color.y; QFL(QF_COLZ) = color.z;
         normal = hit.normal;
         if ((s.sun_flags & 1) && !specular) sun = true;
-        else if (NEE && !specular) nee_step = true;
+        else if (V::nee && !specular) nee_step = true;
         else bounce = true;
     }
-    if constexpr (NEE) {
+    if constexpr (V::nee) {
         if (nee_step) {
             // DESIGN §10: only where the bounce will be traced, and without a draw where L(cell) is empty
             if (shadow) normal = f3(QFL(QF_SNX), QFL(QF_SNY), QFL(QF_SNZ));
@@ -407,7 +407,7 @@ __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint
                 uint32_t rng = QU(QF_RNG);
                 float3 c, w;
                 float limit;
-                const bool ray = nee_sample<NEE, BIOME>(s, g, first, n_list, from, normal, f3(QFL(QF_THRX), QFL(QF_THRY), QFL(QF_THRZ)), rng, c, w, limit);
+                const bool ray = nee_sample<V::nee, V::biome>(s, g, first, n_list, from, normal, f3(QFL(QF_THRX), QFL(QF_THRY), QFL(QF_THRZ)), rng, c, w, limit);
                 QU(QF_RNG) = rng;
                 if (ray) {
                     QFL(QF_SNX) = normal.x; QFL(QF_SNY) = normal.y; QFL(QF_SNZ) = normal.z;
@@ -443,12 +443,12 @@ __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint
         next_limit = distance;
     } else {
         next_d = diffuse_direction_sc(normal, x1, sn, cs);
-        if (SPEC && specular) next_d = specular_direction(d, normal, next_d, ro);
+        if (V::spec && specular) next_d = specular_direction(d, normal, next_d, ro);
         next_o = from + next_d * CCU_OFFSET;
         next_limit = inff_();
         const int ray_depth = (int)((meta >> 16) & 0xFF) + 1;
         meta = (meta & ~(0xFFu << 16) & ~QM_SHADOW) | ((uint32_t)ray_depth << 16);
-        if constexpr (NEE) {
+        if constexpr (V::nee) {
             // the bounce segment carries the sampled cell for the emission rule at its hit
             meta &= ~(QM_NEE_RAY | QM_NEE_PREV);
             int3 cell;
@@ -481,8 +481,7 @@ __device__ __forceinline__ bool q_covered(const DScene &s, const EmitView &g, co
 
 // BLOCK (kind_block = true) and EXIT (false): the octree part of closestIntersect (kernel.h:14-16) is finished here;
 // without BVHs the ray is shaded right away, with BVHs it goes to the BVH stage.  kind_block is warp-uniform.
-// BIOME: block hits are tinted by the biome colours of CCU_RENDER_BIOME_TINT (DESIGN §13).
-template <bool HAS_BVH, bool SPEC, int NEE, bool BIOME>
+template <bool HAS_BVH, class V>
 __device__ __forceinline__ bool q_stage_resolve(const DScene &s, const EmitView &g, uint32_t *F, unsigned *mask, int lane, const bool kind_block,
                                                 int min_lanes) {
     const int row = q_pop_batch(mask, kind_block ? QS_BLOCK : QS_EXIT, lane, min_lanes);
@@ -498,7 +497,7 @@ __device__ __forceinline__ bool q_stage_resolve(const DScene &s, const EmitView 
     m.steps = QI(QF_STEPS);
     bool ray_hit = false;
     float hit_t = 0;
-    SurfT<SPEC> hit;
+    SurfT<V::spec> hit;
     hit.normal = f3(0, 0, 0); hit.color = make_float4(0, 0, 0, 0); hit.emittance = 0;
     surf_set_spec(hit, 0u);
     bool covered = false;   // NEE: the hit is an emitter the previous hit's sample covered
@@ -508,14 +507,14 @@ __device__ __forceinline__ bool q_stage_resolve(const DScene &s, const EmitView 
         int level;
         const int data = find_leaf_wide(s, c.bx, c.by, c.bz, level);   // the kernel is only launched on the commit-time layouts
         // NEE_*_MODELS: an emitter sample's shadow ray counts a block hit only before its limit (march_block)
-        const bool cut = nee_models(NEE) ? (QU(QF_META) & QM_NEE_RAY) != 0 : false;
-        if (!march_block<SPEC, nee_models(NEE), BIOME>(s, m, data, level, hit, hit_t, cut)) {
+        const bool cut = V::models ? (QU(QF_META) & QM_NEE_RAY) != 0 : false;
+        if (!march_block<V, V::models>(s, m, data, level, hit, hit_t, cut)) {
             QFL(QF_T) = m.t; QI(QF_STEPS) = m.steps;
             q_push(mask, QS_MARCH, lane, row);
             return true;
         }
         ray_hit = true;
-        if constexpr (NEE) covered = q_covered<NEE>(s, g, F, slot, QU(QF_META), data, c);
+        if constexpr (V::nee) covered = q_covered<V::nee>(s, g, F, slot, QU(QF_META), data, c);
     }
     const float distance = ray_hit ? hit_t : m.limit;
     if (HAS_BVH) {
@@ -525,15 +524,15 @@ __device__ __forceinline__ bool q_stage_resolve(const DScene &s, const EmitView 
             QFL(QF_HEM) = hit.emittance;
             QFL(QF_HNX) = hit.normal.x; QFL(QF_HNY) = hit.normal.y; QFL(QF_HNZ) = hit.normal.z;
             QFL(QF_HCX) = hit.color.x; QFL(QF_HCY) = hit.color.y; QFL(QF_HCZ) = hit.color.z;
-            if constexpr (SPEC) QU(QF_HSPEC) = hit.spec;
+            if constexpr (V::spec) QU(QF_HSPEC) = hit.spec;
         }
         uint32_t meta = QU(QF_META);
-        if constexpr (NEE) meta = covered ? (meta | QM_COVERED) : (meta & ~QM_COVERED);
+        if constexpr (V::nee) meta = covered ? (meta | QM_COVERED) : (meta & ~QM_COVERED);
         QU(QF_META) = ray_hit ? (meta | QM_HIT) : (meta & ~QM_HIT);
         // A shadow ray only asks WHETHER something lies between the surface and the sun (rayTracer.cl:101-106 uses nothing else
         // of its record): once the octree has answered yes, the BVHs - which can only find a closer hit - cannot change that.
         // The same holds for the emitter sample's shadow ray (NEE).
-        if (ray_hit && (meta & (NEE ? (QM_SHADOW | QM_NEE_RAY) : QM_SHADOW))) {
+        if (ray_hit && (meta & (V::nee ? (QM_SHADOW | QM_NEE_RAY) : QM_SHADOW))) {
             q_push(mask, QS_SHADE, lane, row);
             return true;
         }
@@ -544,13 +543,13 @@ __device__ __forceinline__ bool q_stage_resolve(const DScene &s, const EmitView 
         QI(QF_BSP) = phase << 8;
         q_push(mask, ref < 0 ? QS_LEAF : QS_BVH, lane, row);
     } else {
-        q_shade<SPEC, NEE, q_nee_field(HAS_BVH, SPEC), BIOME>(s, g, F, mask, lane, row, m.o, m.d, distance, ray_hit, hit, covered);
+        q_shade<HAS_BVH, V>(s, g, F, mask, lane, row, m.o, m.d, distance, ray_hit, hit, covered);
     }
     return true;
 }
 
 // SHADE (HAS_BVH kernels): closestIntersect is complete (kernel.h:17-22)
-template <bool SPEC, int NEE, bool BIOME>
+template <class V>
 __device__ __forceinline__ bool q_stage_shade(const DScene &s, const EmitView &g, uint32_t *F, unsigned *mask, int lane, int min_lanes) {
     const int row = q_pop_batch(mask, QS_SHADE, lane, min_lanes);
     if (row == -2) return false;
@@ -560,13 +559,12 @@ __device__ __forceinline__ bool q_stage_shade(const DScene &s, const EmitView &g
     const float3 o = f3(QFL(QF_OX), QFL(QF_OY), QFL(QF_OZ));
     const float3 d = f3(QFL(QF_DX), QFL(QF_DY), QFL(QF_DZ));
     const bool ray_hit = (QU(QF_META) & QM_HIT) != 0;
-    SurfT<SPEC> hit;
+    SurfT<V::spec> hit;
     hit.normal = f3(QFL(QF_HNX), QFL(QF_HNY), QFL(QF_HNZ));
     hit.color = make_float4(QFL(QF_HCX), QFL(QF_HCY), QFL(QF_HCZ), 0.0f);
     hit.emittance = QFL(QF_HEM);
-    if constexpr (SPEC) hit.spec = QU(QF_HSPEC);
-    q_shade<SPEC, NEE, q_nee_field(true, SPEC), BIOME>(s, g, F, mask, lane, row, o, d, QFL(QF_HDIST), ray_hit, hit,
-                                                       NEE && (QU(QF_META) & QM_COVERED) != 0);
+    if constexpr (V::spec) hit.spec = QU(QF_HSPEC);
+    q_shade<true, V>(s, g, F, mask, lane, row, o, d, QFL(QF_HDIST), ray_hit, hit, V::nee && (QU(QF_META) & QM_COVERED) != 0);
     return true;
 }
 
@@ -721,7 +719,7 @@ __device__ __forceinline__ void q_stage_bvh(const DScene &s, uint32_t *F, unsign
 }
 
 // QS_LEAF: the triangles of one leaf (bvh.h:52-67) for walks that sit at a leaf, then the walk's next node from its stack
-template <bool SPEC, int NEE>
+template <class V>
 __device__ __forceinline__ bool q_stage_leaf(const DScene &s, uint32_t *F, unsigned *mask, int *stk, int *deep, int lane, int min_lanes) {
     const int row = q_pop_batch(mask, QS_LEAF, lane, min_lanes);
     if (row == -2) return false;
@@ -734,7 +732,7 @@ __device__ __forceinline__ bool q_stage_leaf(const DScene &s, uint32_t *F, unsig
     int ref = QI(QF_BREF);
     const int bsp = QI(QF_BSP);
     int sp = bsp & 0xFF, phase = bsp >> 8;
-    SurfT<SPEC> hit;
+    SurfT<V::spec> hit;
     hit.normal = f3(0, 0, 0); hit.color = make_float4(0, 0, 0, 0); hit.emittance = 0;
     surf_set_spec(hit, 0u);
     bool any = false;
@@ -743,7 +741,7 @@ __device__ __forceinline__ bool q_stage_leaf(const DScene &s, uint32_t *F, unsig
     const uint32_t meta = QU(QF_META);
     // a shadow ray (the sun's or, NEE, the emitter sample's) is answered by its first accepted triangle (see q_stage_resolve):
     // the rest of the walk could only find a closer one
-    const bool first_hit_ends = (meta & (NEE ? (QM_SHADOW | QM_NEE_RAY) : QM_SHADOW)) != 0;
+    const bool first_hit_ends = (meta & (V::nee ? (QM_SHADOW | QM_NEE_RAY) : QM_SHADOW)) != 0;
     // the head of the first triangle is requested together with the count word (a leaf block holds at least one triangle; the
     // array is padded so that the read is in bounds even for an empty one), the head of triangle i + 1 while triangle i is tested
     Int8 q0 = ldg256(blk + 8);
@@ -767,8 +765,8 @@ __device__ __forceinline__ bool q_stage_leaf(const DScene &s, uint32_t *F, unsig
         QFL(QF_HEM) = hit.emittance;
         QFL(QF_HNX) = hit.normal.x; QFL(QF_HNY) = hit.normal.y; QFL(QF_HNZ) = hit.normal.z;
         QFL(QF_HCX) = hit.color.x; QFL(QF_HCY) = hit.color.y; QFL(QF_HCZ) = hit.color.z;
-        if constexpr (SPEC) QU(QF_HSPEC) = hit.spec;
-        QU(QF_META) = (NEE ? (meta & ~QM_COVERED) : meta) | QM_HIT;   // NEE: a triangle is no covered emitter
+        if constexpr (V::spec) QU(QF_HSPEC) = hit.spec;
+        QU(QF_META) = (V::nee ? (meta & ~QM_COVERED) : meta) | QM_HIT;   // NEE: a triangle is no covered emitter
     }
     if (any && first_hit_ends) { phase = 2; ref = 0; }
     else if (sp == 0) bvh_phase_done(s, ref, phase);
@@ -922,19 +920,16 @@ __device__ __forceinline__ bool q_stage_end(const DScene &s, const PassParams &w
 }
 
 // LAY 0: the top table of the air layout fits Q_TOP_WORDS and is staged in shared memory; 1: it is read from global memory;
-// 2: deep world (64-ary nodes between the top table and the bricks).  SPEC: CCU_RENDER_SPECULAR on a scene with specular words.
-// NEE: the emitter sampler (NeeKind) of CCU_RENDER_EMITTER_SAMPLING, with CCU_RENDER_EMITTER_NEAR_FIELD for NEE_NEAR(_MODELS) and
-// CCU_RENDER_EMITTER_MODELS for NEE_*_MODELS (the table `g` is then the wider one, DESIGN §12), on a scene
-// with emitters (table `g`, an argument after the others so that the kernels without it keep their parameter offsets).
-// BIOME: CCU_RENDER_BIOME_TINT on a scene with biome colours (`bv`, the last argument for the same reason; DESIGN §13).
-template <bool HAS_BVH, int LAY, bool SPEC, int NEE, bool BIOME>
+// 2: deep world (64-ary nodes between the top table and the bricks).  V: the launch's Shade.  The emitter table `g` and the biome
+// colours `bv` come after the other arguments, so that the kernels without them keep their parameter offsets.
+template <bool HAS_BVH, int LAY, class V>
 __global__ void __launch_bounds__(Q_WARPS * 32, 1) k_render_queue(const __grid_constant__ DScene s, const __grid_constant__ QueueParams qp,
                                                                  const __grid_constant__ EmitView g, const __grid_constant__ BiomeView bv) {
     constexpr int NST = q_stages(HAS_BVH);
     constexpr int MASK_WORDS = q_mask_words(HAS_BVH);
     extern __shared__ uint32_t q_mem[];
     uint32_t *F = q_mem;
-    unsigned *mask = q_mem + q_fields(HAS_BVH, SPEC, NEE) * Q_SLOTS;
+    unsigned *mask = q_mem + q_fields(HAS_BVH, V::spec, V::nee) * Q_SLOTS;
     int *live = reinterpret_cast<int *>(mask + MASK_WORDS);
     unsigned *top_s = mask + MASK_WORDS + 32;
     int *stk = reinterpret_cast<int *>(top_s + (LAY == 0 ? Q_TOP_WORDS : 0));   // HAS_BVH only: stacks by slot
@@ -956,7 +951,7 @@ __global__ void __launch_bounds__(Q_WARPS * 32, 1) k_render_queue(const __grid_c
         sky_s = reinterpret_cast<uchar4 *>(top_s + (LAY == 0 ? Q_TOP_WORDS : 0) + (HAS_BVH ? Q_STACK_WORDS : 0));
         for (int i = threadIdx.x; i < qp.sky_texels; i += blockDim.x) sky_s[i] = __ldg(s.sky + i);
     }
-    if constexpr (BIOME) {
+    if constexpr (V::biome) {
         if (threadIdx.x == 0) biome_smem() = bv;   // read after the barrier of stage_tables
     }
     stage_tables(s, sky_s);
@@ -1009,11 +1004,11 @@ __global__ void __launch_bounds__(Q_WARPS * 32, 1) k_render_queue(const __grid_c
         switch (best) {
             case QS_MARCH: QSTAT(0, 1); q_stage_march<NST, LAY>(s, top, F, mask, lane, qp.yield_below, qp.refill_min); break;
             case QS_BLOCK:
-            case QS_EXIT: ran = q_stage_resolve<HAS_BVH, SPEC, NEE, BIOME>(s, g, F, mask, lane, best == QS_BLOCK, min_lanes); break;
+            case QS_EXIT: ran = q_stage_resolve<HAS_BVH, V>(s, g, F, mask, lane, best == QS_BLOCK, min_lanes); break;
             case QS_END: ran = q_stage_end<!HAS_BVH>(s, qp.w, F, mask, live, lane, min_lanes); break;
             case QS_BVH: QSTAT(16, 1); if (HAS_BVH) q_stage_bvh<NST>(s, F, mask, stk, qp.bvh_deep, lane, qp.yield_below, qp.refill_min); break;
-            case QS_LEAF: if (HAS_BVH) ran = q_stage_leaf<SPEC, NEE>(s, F, mask, stk, qp.bvh_deep, lane, min_lanes); break;
-            default: if (HAS_BVH) ran = q_stage_shade<SPEC, NEE, BIOME>(s, g, F, mask, lane, min_lanes); break;
+            case QS_LEAF: if (HAS_BVH) ran = q_stage_leaf<V>(s, F, mask, stk, qp.bvh_deep, lane, min_lanes); break;
+            default: if (HAS_BVH) ran = q_stage_shade<V>(s, g, F, mask, lane, min_lanes); break;
         }
         sticky = (ran && best != QS_MARCH && best != QS_BVH) ? best : -1;
         if (ran) {

@@ -45,14 +45,13 @@ __global__ void k_sun_setup(const int *sun_words, float *out /* su sv sw radius_
 // Thread-per-pixel path tracer: all passes of the batch in one launch, the running mean of
 // rayTracer.cl:109-112 carried in registers between passes (identical arithmetic, no memory round trip).
 // MODE: 0 = the reference's own node array, 1 = commit-time layouts, 2 = commit-time layouts of a deep world.
-// SPEC: CCU_RENDER_SPECULAR on a scene with specular words; NEE: the emitter sampler (NeeKind) of CCU_RENDER_EMITTER_SAMPLING and
-// CCU_RENDER_EMITTER_NEAR_FIELD / CCU_RENDER_EMITTER_MODELS on a scene with emitters (sample_pixel).  BIOME: CCU_RENDER_BIOME_TINT
-// on a scene with biome colours (`bv`, after the others so that the other kernels keep their parameter offsets).
-template <int MODE, bool SPEC, int NEE, bool BIOME>
+// V: the Shade of the launch (sample_pixel, DESIGN §5).  The emitter table `g` and the biome colours `bv` come after the other
+// arguments, so that the kernels without them keep their parameter offsets.
+template <int MODE, class V>
 __global__ void __launch_bounds__(128) k_render_mega(const __grid_constant__ DScene s, const int *__restrict__ seeds, int n_passes,
                                                      int start_spp, float *res, const float *res_prev, int n_pixels,
                                                      const __grid_constant__ EmitView g, const __grid_constant__ BiomeView bv) {
-    if constexpr (BIOME) {
+    if constexpr (V::biome) {
         if (threadIdx.x == 0) biome_smem() = bv;   // read after the barrier of stage_tables
     }
     stage_tables(s, nullptr);
@@ -61,7 +60,7 @@ __global__ void __launch_bounds__(128) k_render_mega(const __grid_constant__ DSc
         const float *pp = res_prev + (size_t)gid * 3;    // what the reference's single buffer holds when the window starts
         float3 buf = f3(pp[0], pp[1], pp[2]);
         for (int pass = 0; pass < n_passes; pass++) {
-            float3 col = sample_pixel<MODE, SPEC, NEE, BIOME>(s, g, gid, __ldg(seeds + pass));
+            float3 col = sample_pixel<MODE, V>(s, g, gid, __ldg(seeds + pass));
             int spp = start_spp + pass;
             float fs = (float)spp, fs1 = (float)(spp + 1);
             buf.x = (buf.x * fs + col.x) / fs1;
@@ -147,7 +146,7 @@ __global__ void __launch_bounds__(CCU_FH_THREADS, CCU_FH_MIN_BLOCKS) k_first_hit
         rec.surf.color = make_float4(0, 0, 0, 0); rec.surf.emittance = 0;
         HitInfo hi = {-1, 0, 0, 0, 0};
         bool hit = false;
-        if (valid) hit = HAS_BVH ? closest_intersect_ref(s, o, d, rec, hi) : octree_intersect_ref(s, o, d, rec, hi);
+        if (valid) hit = HAS_BVH ? closest_intersect_ref<PlainShade>(s, o, d, rec, hi) : octree_intersect_ref<PlainShade>(s, o, d, rec, hi);
         if (valid) first_hit_store(out, gid, hit, rec.material, rec.surf.normal, hi.node, hi.kind, rec.distance, rec.surf.color);
         return;
     }
@@ -172,7 +171,7 @@ __global__ void __launch_bounds__(CCU_FH_THREADS, CCU_FH_MIN_BLOCKS) k_first_hit
             const int data = find_leaf_wide(s, c.bx, c.by, c.bz, level);
             float th;
             Surf hs;
-            if (march_block(s, m, data, level, hs, th)) {
+            if (march_block<PlainShade>(s, m, data, level, hs, th)) {
                 st = 3;
                 if (!HAS_BVH) {
                     int hnode = -1;
@@ -224,7 +223,7 @@ __global__ void __launch_bounds__(256) k_preview(const __grid_constant__ DScene 
     rec.surf.color = make_float4(0, 0, 0, 0); rec.surf.emittance = 0;
     HitInfo hi = {-1, 0, 0, 0, 0};
     float3 c;
-    if (closest_intersect_mode<MODE>(s, o, d, rec, hi)) {
+    if (closest_intersect_mode<MODE, PlainShade>(s, o, d, rec, hi)) {
         float shading = dot3(rec.surf.normal, f3(0.25f, 0.866f, 0.433f));
         shading = fmaxf(0.3f, shading);
         c = f3(rec.surf.color.x * shading, rec.surf.color.y * shading, rec.surf.color.z * shading);
@@ -483,40 +482,50 @@ void dispatch(bool v, F &&f) {
     else f(std::false_type{});
 }
 
-// the wavefront kernel (ccu_queue.cuh) for the scene's entity BVHs and air layout (air_layout_id), with or without specular events,
-// emitter sampler and biome colours
-auto queue_kernel(bool bvh, int lay, bool spec, int nee, bool biome) {
-    decltype(&k_render_queue<false, 0, false, NEE_NONE, false>) k = nullptr;
+// A launch's Shade (ccu_device.cuh) as runtime values
+struct ShadeKey {
+    bool spec;
+    int nee;   // a NeeKind
+    bool biome;
+};
+constexpr int N_SHADES = 2 * 5 * 2;
+ShadeKey nth_shade(int i) { return {i % 2 != 0, i / 2 % 5, i / 10 != 0}; }   // every ShadeKey for i in [0, N_SHADES)
+
+// Calls f(Shade<spec, nee, biome>{}) for the values of v.
+template <class F>
+void dispatch(const ShadeKey &v, F &&f) {
+    dispatch(v.spec, [&](auto S) {
+        dispatch<5>(v.nee, [&](auto N) { dispatch(v.biome, [&](auto B) { f(Shade<S, NeeKind(N.value), B>{}); }); });
+    });
+}
+
+// The Shade of a render launch (DESIGN §5).  Each flag picks its kernels only on a scene where they compute something the
+// others do not:
+// - CCU_RENDER_SPECULAR: the specular kernels, on a scene with a specular word;
+// - CCU_RENDER_EMITTER_SAMPLING: the NEE kernels, on a scene with emitters; CCU_RENDER_EMITTER_NEAR_FIELD picks the near-field
+//   sampler (NEE_NEAR) among them.  CCU_RENDER_EMITTER_MODELS picks the samplers of the wider table (NEE_*_MODELS, EmitView
+//   memit_view) when the scene has one; without a model emitter it changes nothing;
+// - CCU_RENDER_BIOME_TINT: the biome kernels, on a scene with biome colours.
+ShadeKey shade_variant(const ccu_ctx *c) {
+    const int f = c->params.flags;
+    const auto &info = c->scene.info;
+    const bool near_field = (f & CCU_RENDER_EMITTER_NEAR_FIELD) != 0;
+    int nee = NEE_NONE;
+    if (f & CCU_RENDER_EMITTER_SAMPLING) {
+        if ((f & CCU_RENDER_EMITTER_MODELS) && info.has_model_emitters) nee = near_field ? NEE_NEAR_MODELS : NEE_AREA_MODELS;
+        else if (info.has_emitters) nee = near_field ? NEE_NEAR : NEE_AREA;
+    }
+    return {(f & CCU_RENDER_SPECULAR) && info.has_specular, nee, (f & CCU_RENDER_BIOME_TINT) && info.has_biome};
+}
+
+// the wavefront kernel (ccu_queue.cuh) for the scene's entity BVHs, air layout (air_layout_id) and the launch's Shade
+auto queue_kernel(bool bvh, int lay, const ShadeKey &v) {
+    decltype(&k_render_queue<false, 0, PlainShade>) k = nullptr;
     dispatch(bvh, [&](auto B) {
-        dispatch<3>(lay, [&](auto L) {
-            dispatch(spec, [&](auto S) {
-                dispatch<5>(nee, [&](auto N) { dispatch(biome, [&](auto T) { k = k_render_queue<B, L, S, N, T>; }); });
-            });
-        });
+        dispatch<3>(lay, [&](auto L) { dispatch(v, [&](auto V) { k = k_render_queue<B, L, decltype(V)>; }); });
     });
     return k;
 }
-
-// CCU_RENDER_SPECULAR launches the specular kernels only on a scene that has a specular word: without one they compute exactly
-// what the other kernels compute
-bool specular_launch(const ccu_ctx *c) { return (c->params.flags & CCU_RENDER_SPECULAR) && c->scene.info.has_specular; }
-
-// CCU_RENDER_EMITTER_SAMPLING launches the NEE kernels only on a scene with emitters: without one they draw nothing and compute
-// exactly what the other kernels compute.  CCU_RENDER_EMITTER_NEAR_FIELD picks the near-field sampler (NEE_NEAR) among them.
-// CCU_RENDER_EMITTER_MODELS picks the samplers of the wider table (NEE_*_MODELS, EmitView memit_view) when the scene has one;
-// without a model emitter it changes nothing.
-int nee_launch(const ccu_ctx *c) {
-    const int f = c->params.flags;
-    if (!(f & CCU_RENDER_EMITTER_SAMPLING)) return NEE_NONE;
-    if ((f & CCU_RENDER_EMITTER_MODELS) && c->scene.info.has_model_emitters)
-        return (f & CCU_RENDER_EMITTER_NEAR_FIELD) ? NEE_NEAR_MODELS : NEE_AREA_MODELS;
-    if (!c->scene.info.has_emitters) return NEE_NONE;
-    return (f & CCU_RENDER_EMITTER_NEAR_FIELD) ? NEE_NEAR : NEE_AREA;
-}
-
-// CCU_RENDER_BIOME_TINT launches the biome kernels only on a scene with biome colours: without them they compute exactly what the
-// other kernels compute
-bool biome_launch(const ccu_ctx *c) { return (c->params.flags & CCU_RENDER_BIOME_TINT) && c->scene.info.has_biome; }
 
 }  // namespace
 
@@ -678,11 +687,9 @@ int ccu_ctx_create(int device_index, ccu_ctx **out) {
     for (Event &ev : c->chunk_ev) if (e == cudaSuccess) e = ev.create(cudaEventDisableTiming);
     for (Event &ev : c->rays_used) if (e == cudaSuccess) e = ev.create(cudaEventDisableTiming);
     for (bool bvh : {false, true})
-        for (bool spec : {false, true})
-            for (int nee : {NEE_NONE, NEE_AREA, NEE_NEAR, NEE_AREA_MODELS, NEE_NEAR_MODELS})
-                for (bool biome : {false, true})
-                    for (int lay = 0; lay < 3 && e == cudaSuccess; lay++)
-                        e = cudaFuncSetAttribute(queue_kernel(bvh, lay, spec, nee, biome), cudaFuncAttributeMaxDynamicSharedMemorySize, Q_SMEM_LIMIT);
+        for (int lay = 0; lay < 3; lay++)
+            for (int i = 0; i < N_SHADES && e == cudaSuccess; i++)
+                e = cudaFuncSetAttribute(queue_kernel(bvh, lay, nth_shade(i)), cudaFuncAttributeMaxDynamicSharedMemorySize, Q_SMEM_LIMIT);
     if (e == cudaSuccess) e = c->unorm.alloc(256);
     if (e == cudaSuccess) {
         k_unorm_table<<<1, 256, 0, c->stream>>>(c->unorm.p);
@@ -1099,10 +1106,8 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
     if (first_chunk) CU(cudaEventRecord(c->ev0, c->stream));
     const bool bvh = !(s.world_bvh_empty && s.actor_bvh_empty);
     const int mode = layout_mode(c);
-    const bool spec = specular_launch(c);
-    const int nee = nee_launch(c);
-    const EmitView &emit_view = nee_models(nee) ? c->scene.memit_view : c->scene.emit_view;
-    const bool biome = biome_launch(c);
+    const ShadeKey shade = shade_variant(c);
+    const EmitView &emit_view = nee_models(shade.nee) ? c->scene.memit_view : c->scene.emit_view;
     const BiomeView &biome_view = c->scene.biome_view;
     float *res = c->accum[c->accum_active].p;
     const float *res_prev = c->window_spp == 0 ? c->window_base : res;
@@ -1111,13 +1116,9 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
     if (kernel == 1) {
         const int threads = 128, blocks = (n_pixels + threads - 1) / threads;
         dispatch<3>(mode, [&](auto M) {
-            dispatch(spec, [&](auto S) {
-                dispatch<5>(nee, [&](auto N) {
-                    dispatch(biome, [&](auto T) {
-                        k_render_mega<M, S, N, T><<<blocks, threads, 0, c->stream>>>(s, seeds_dev, n_passes, c->window_spp, res, res_prev,
-                                                                                   n_pixels, emit_view, biome_view);
-                    });
-                });
+            dispatch(shade, [&](auto V) {
+                k_render_mega<M, decltype(V)><<<blocks, threads, 0, c->stream>>>(s, seeds_dev, n_passes, c->window_spp, res, res_prev, n_pixels,
+                                                                                emit_view, biome_view);
             });
         });
     } else {
@@ -1145,7 +1146,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
         // 128 x 128 table (64 KiB) taken from L1 costs more brick / atlas hits than the sky lookups gain (measured: +1.8 % per
         // pass on config 1).  CCU_SKY_SMEM_MAX (bytes, default 16 KiB = 64 x 64 texels) moves the threshold.
         const int sky_texels = c->scene.info.sky_res * c->scene.info.sky_res;
-        const int base_smem = q_smem_bytes(bvh, lay == 0, spec, nee != NEE_NONE);
+        const int base_smem = q_smem_bytes(bvh, lay == 0, shade.spec, shade.nee != NEE_NONE);
         const char *sky_env = getenv("CCU_SKY_SMEM_MAX");
         const int sky_max = sky_env ? atoi(sky_env) : 16384;
         const bool sky_smem = sky_texels * 4 <= sky_max && base_smem + sky_texels * 4 <= Q_SMEM_LIMIT;
@@ -1157,7 +1158,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
             qp.bvh_deep = c->bvh_deep.p;
         }
         const int smem = base_smem + qp.sky_texels * 4;
-        queue_kernel(bvh, lay, spec, nee, biome)<<<grid, block, smem, c->stream>>>(s, qp, emit_view, biome_view);
+        queue_kernel(bvh, lay, shade)<<<grid, block, smem, c->stream>>>(s, qp, emit_view, biome_view);
 #ifdef CCU_Q_STATS
         {
             cudaStreamSynchronize(c->stream);

@@ -1,6 +1,6 @@
 """Size of the octree march step of the default wavefront kernel, from its SASS (no GPU needed).
 
-Compiles k_render_queue<false, 0, false, NEE_NONE, false> (no BVHs, top table in shared memory, no render flags) from the
+Compiles k_render_queue<false, 0, PlainShade> (no BVHs, top table in shared memory, no render flags) from the
 headers under chunkyclplugin_b200/csrc with the library's nvcc flags, finds the inner march loop - the smallest loop,
 closed by a backward branch, whose body holds the brick load (LDG) and the three F2I.FLOOR of the voxel coordinates - and
 prints its instruction count with the kernel's registers and spill bytes.
@@ -24,7 +24,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from chunkyclplugin_b200.build import CSRC, NVCC_FLAGS  # noqa: E402
 
-KERNEL = "k_render_queue<false, 0, false, 0, false>"
+KERNEL = "k_render_queue<false, 0, PlainShade>"
 INSN = re.compile(r"^\s*/\*([0-9a-f]{4,})\*/\s+(.*?)\s*;")
 
 
@@ -33,7 +33,7 @@ def compile_kernel(tmp: str) -> tuple[str, str]:
     src = os.path.join(tmp, "march_step.cu")
     with open(src, "w") as f:
         f.write('#include "ccu_queue.cuh"\n'
-                f"void *march_step_kernel() {{ return (void *)&ccu::{KERNEL}; }}\n")
+                f"namespace ccu {{ void *march_step_kernel() {{ return (void *)&{KERNEL}; }} }}\n")
     flags = [f for f in NVCC_FLAGS if f not in ("-shared", "-cudart", "static", "--threads", "2", "-Xcompiler", "-fPIC")]
     cubin = os.path.join(tmp, "march_step.cubin")
     nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
