@@ -290,6 +290,7 @@ struct ccu_ctx {
     float last_ms = 0;
     bool timing_pending = false;
     int64_t launches = 0;
+    int32_t last_render[7] = {0, 0, 0, 0, 0, 0, 0};   // the last render launch's instance (ccu_debug_last_render)
 };
 
 namespace ccu_host {

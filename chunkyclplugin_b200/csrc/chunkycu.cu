@@ -1113,6 +1113,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
     const float *res_prev = c->window_spp == 0 ? c->window_base : res;
     int kernel = c->params.kernel;
     if (kernel == 0) kernel = (mode != 0 && (!bvh || c->scene.info.use_bvh2)) ? 4 : 1;   // layouts refused at commit: the reference's own arrays
+    int lay = 0, sky_staged = 0;   // kernel 4: its LAY, and the sky texels it stages in shared memory
     if (kernel == 1) {
         const int threads = 128, blocks = (n_pixels + threads - 1) / threads;
         dispatch<3>(mode, [&](auto M) {
@@ -1140,7 +1141,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
         qp.shade_min = c->q_shade_min;
         qp.sticky_min = c->q_sticky_min > 0 ? c->q_sticky_min : (bvh ? 16 : 33);   // measured: -3 % with BVH stages, +5 % without
         qp.march_warps = bvh ? 64 : c->q_march_warps;   // the cap applies to the BVH-less kernels; with BVH stages every warp may march
-        const int lay = air_layout_id(c);
+        lay = air_layout_id(c);
         const int grid = c->sm_count, block = Q_WARPS * 32;
         // The sky table is staged in shared memory when it is small: shared memory and L1 are one array on this chip, and a
         // 128 x 128 table (64 KiB) taken from L1 costs more brick / atlas hits than the sky lookups gain (measured: +1.8 % per
@@ -1150,7 +1151,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
         const char *sky_env = getenv("CCU_SKY_SMEM_MAX");
         const int sky_max = sky_env ? atoi(sky_env) : 16384;
         const bool sky_smem = sky_texels * 4 <= sky_max && base_smem + sky_texels * 4 <= Q_SMEM_LIMIT;
-        qp.sky_texels = sky_smem ? sky_texels : 0;
+        qp.sky_texels = sky_staged = sky_smem ? sky_texels : 0;
         qp.bvh_deep = nullptr;
         if (bvh) {
             // scratch for traversal-stack entries beyond the shared-memory part (bvh.h:38 allows 64 pending nodes)
@@ -1178,6 +1179,8 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
 #endif
     }
     c->launches++;
+    const int32_t last[7] = {kernel, bvh, kernel == 1 ? mode : lay, shade.spec, shade.nee, shade.biome, sky_staged};
+    std::copy(last, last + 7, c->last_render);
     CU(cudaGetLastError());
     CU(cudaEventRecord(c->ev1, c->stream));
     CU(cudaEventRecord(ring.ev[slot], c->stream));
@@ -1451,6 +1454,13 @@ int ccu_launch_count(ccu_ctx *c, int64_t *launches) {
     if (!c || !launches) return fail(CCU_EINVAL, "ccu_launch_count: null argument");
     std::lock_guard<std::mutex> lk(c->mu);
     *launches = c->launches;
+    return CCU_OK;
+}
+
+int ccu_debug_last_render(ccu_ctx *c, int32_t out[7]) {
+    if (!c || !out) return fail(CCU_EINVAL, "ccu_debug_last_render: null argument");
+    std::lock_guard<std::mutex> lk(c->mu);
+    std::copy(c->last_render, c->last_render + 7, out);
     return CCU_OK;
 }
 

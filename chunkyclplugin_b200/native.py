@@ -83,6 +83,7 @@ SYMBOLS = {
     "ccu_preview": (C.c_int, [_vp, _vp]),
     "ccu_last_kernel_ms": (C.c_int, [_vp, C.POINTER(_f)]),
     "ccu_launch_count": (C.c_int, [_vp, C.POINTER(_i64)]),
+    "ccu_debug_last_render": (C.c_int, [_vp, _vp]),
     "ccu_scene_device_bytes": (C.c_int, [_vp, C.POINTER(_i64)]),
     "ccu_scene_commit_ms": (C.c_int, [_vp, C.POINTER(C.c_double)]),
     "ccu_tonemap": (C.c_int, [_vp, _i32, _i32, _f, _vp, _i32, _vp]),
@@ -462,6 +463,13 @@ class Context:
         n = C.c_int64()
         check(self._lib.ccu_launch_count(self._h, C.byref(n)))
         return n.value
+
+    def last_render(self) -> tuple:
+        """The render kernel instance of the last render_passes launch: (kernel, has_bvh, lay or mode, spec, nee, biome,
+        staged sky texels), all zero before the first launch (ccu_debug_last_render)."""
+        out = np.zeros(7, np.int32)
+        check(self._lib.ccu_debug_last_render(self._h, _ptr(out)))
+        return tuple(int(v) for v in out)
 
     def scene_device_bytes(self) -> int:
         n = C.c_int64()

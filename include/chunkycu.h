@@ -195,6 +195,11 @@ int ccu_tonemap(ccu_ctx *ctx, int32_t width, int32_t height, float exposure, con
 /* ---- instrumentation ------------------------------------------------------------------------------------------ */
 int ccu_last_kernel_ms(ccu_ctx *ctx, float *ms);          /* CUDA-event time of the last render_passes / first_hit launch(es) */
 int ccu_launch_count(ccu_ctx *ctx, int64_t *launches);    /* kernels launched by this context so far */
+/* Test support: the render kernel instance of the context's last ccu_render_passes[_async] launch (all zero before the first).
+ * out = {kernel launched (1 or 4, after the choice for kernel 0), HAS_BVH, LAY (kernel 4) or MODE (kernel 1), spec, nee (a NeeKind:
+ * 0 none, 1 area, 2 near, 3 area + models, 4 near + models), biome, sky texels staged in shared memory (0 for kernel 1)};
+ * DESIGN.md §5.  A launch refused with an error leaves it as it was. */
+int ccu_debug_last_render(ccu_ctx *ctx, int32_t out[7]);
 int ccu_scene_device_bytes(ccu_ctx *ctx, int64_t *bytes); /* HBM held by the committed scene */
 int ccu_scene_commit_ms(ccu_ctx *ctx, double *ms);        /* host time the last ccu_scene_commit spent building + uploading the layouts */
 /* Memory-system denominators for this path's roofline (dependent 32-byte-sector gathers, SURVEY 8d): random 16-byte
