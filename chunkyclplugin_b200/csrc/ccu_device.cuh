@@ -76,6 +76,10 @@ struct DScene {   // what a launch reads: commit fills the scene's fields once (
     // launch parameters
     int draw_depth, max_depth;
     float emitter_scale;
+    // the scene's fog (ccu_scene_set_fog, DESIGN §14), read only by the fog kernels; kept last so that no other field moves
+    float fog_sigma, fog_sky;
+    float3 fog_color;
+    int fog_fast;
 };
 
 // The emitter table of CCU_RENDER_EMITTER_SAMPLING (DESIGN §10), built at commit and passed to the thread-per-pixel kernel as
@@ -980,11 +984,12 @@ enum NeeKind : int { NEE_NONE = 0, NEE_AREA = 1, NEE_NEAR = 2, NEE_AREA_MODELS =
 __host__ __device__ constexpr bool nee_near_field(int kind) { return kind == NEE_NEAR || kind == NEE_NEAR_MODELS; }
 __host__ __device__ constexpr bool nee_models(int kind) { return kind == NEE_AREA_MODELS || kind == NEE_NEAR_MODELS; }
 // The shading variant a render kernel is built with, picked per launch by shade_variant (chunkycu.cu, DESIGN §5).
-template <bool S, NeeKind N, bool B>
+template <bool S, NeeKind N, bool B, bool F = false>
 struct Shade {
     static constexpr bool spec = S, biome = B;
     static constexpr NeeKind nee = N;
     static constexpr bool models = nee_models(N);   // the wider emitter table of CCU_RENDER_EMITTER_MODELS
+    static constexpr bool fog = F;                  // the fog of CCU_RENDER_FOG (DESIGN §14; thread-per-pixel kernel only)
 };
 using PlainShade = Shade<false, NEE_NONE, false>;   // the first-hit and preview kernels
 #define CCU_NEE_RHO2 0.015625f   // DESIGN §11: an emitter is near when its box distance² is below rho² = (1/8)²

@@ -169,6 +169,16 @@ struct SceneInfo {
     int memit_g0[3] = {0, 0, 0}, memit_dim[3] = {0, 0, 0}, memit_shift = 3;   // its grid
     int has_biome = 0;      // biome colours were set: CCU_RENDER_BIOME_TINT launches the biome kernels
     int biome_box[4] = {0, 0, 0, 0};   // the biome grid's chunk box (BiomeView::x0, z0, gx, gz)
+    int has_fog = 0;        // ccu_scene_set_fog with sigma > 0: CCU_RENDER_FOG launches the fog kernels
+    float fog_sigma = 0, fog_sky = 0, fog_color[3] = {0, 0, 0};   // DScene::fog_*
+    int fog_fast = 0;
+    void set_fog(float sigma, float sky, const float *color, int fast) {   // color may be null for sigma = 0 (no fog)
+        has_fog = sigma > 0.0f;
+        fog_sigma = sigma;
+        fog_sky = sky;
+        for (int i = 0; i < 3; i++) fog_color[i] = color ? color[i] : 0.0f;
+        fog_fast = fast;
+    }
     float sky_intensity = 0;
     int sun_host[6] = {0, 0, 0, 0, 0, 0};
     bool have_sun = false, have_atlas = false, have_sky = false;
@@ -290,7 +300,7 @@ struct ccu_ctx {
     float last_ms = 0;
     bool timing_pending = false;
     int64_t launches = 0;
-    int32_t last_render[7] = {0, 0, 0, 0, 0, 0, 0};   // the last render launch's instance (ccu_debug_last_render)
+    int32_t last_render[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // the last render launch's instance (ccu_debug_last_render_n)
 };
 
 namespace ccu_host {

@@ -210,8 +210,21 @@ __device__ __forceinline__ bool closest_intersect_mode(const DScene &s, float3 o
     return closest_intersect_lean<MODE == 2, V, CUT>(s, origin, direction, rec, hi);
 }
 
+// The fog's sun sample at the end of a hit (DESIGN §14 step 3): the two draws, the sun direction as the surface sun sample
+// draws it, and a ray from the scattering point p without a limit; an escaped ray adds the pending weight w times the sky
+// (and sun disc) along it.  `rec` is a copy of the hit's record.
+template <int MODE, class V>
+__device__ __forceinline__ void fog_sun_sample(const DScene &s, uint32_t &rng, float3 p, float3 w, RecordT<V::spec> rec, float3 &color) {
+    const float x1 = rng_float(rng);
+    const float x2 = rng_float(rng);
+    const float3 d = sun_sample_direction(s, x1, x2);
+    rec.distance = inff_();
+    HitInfo hi;
+    if (!closest_intersect_mode<MODE, V>(s, p, d, rec, hi)) color = color + w * sky_radiance(s, d);
+}
+
 // one path sample for pixel gid, thread-sequential: rayTracer.cl:40-107 (+ kernel.h:33-98, sky.h:68-93), with the specular events,
-// emitter sampler and biome colours the Shade V switches on (DESIGN §5)
+// emitter sampler, biome colours and fog the Shade V switches on (DESIGN §5)
 template <int MODE, class V>
 __device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &g, int gid, int seed) {
     float3 color = f3(0, 0, 0), throughput = f3(1, 1, 1);
@@ -231,12 +244,30 @@ __device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &
     HitInfo hi = {-1, 0, 0, 0, 0};
     bool nee_prev = false;   // NEE: the hit this segment left sampled the list of cell nee_cell
     int3 nee_cell = make_int3(0, 0, 0);
+    float3 fog_p = f3(0, 0, 0), fog_w = f3(0, 0, 0);   // fog: the hit's scattering point and its pending weight (DESIGN §14)
     for (;;) {
         if (!closest_intersect_mode<MODE, V>(s, origin, direction, rec, hi)) {
             // miss: emittance = 1, sky (+ sun disc) added through the throughput (rayTracer.cl:95-97, kernel.h:26-31)
             float3 sky = sky_radiance(s, direction);
+            if constexpr (V::fog) {   // the sky blended towards the fog colour by elevation (§14.3)
+                const float y = direction.y / sqrtf(dot3(direction, direction));
+                const float f = s.fog_sky * (y > 0 ? (1 - y) * (1 - y) : 1.0f);
+                sky = sky * (1 - f) + s.fog_color * f;
+            }
             color = color + (sky * throughput) * 1.0f;
             break;
+        }
+        if constexpr (V::fog) {   // §14.2 steps 1-2: the scattering draw, then the segment's transmittance
+            const float a = rec.distance * sqrtf(dot3(direction, direction));
+            const float e = s.fog_sigma * a;
+            const float tau = dm_expf(-e);
+            if (s.sun_flags & 1) {
+                const float u = rng_float(rng);
+                fog_p = origin + direction * (u * rec.distance);
+                const float k = s.fog_fast ? 1 - tau : e * dm_expf(-(s.fog_sigma * (u * a)));
+                fog_w = (throughput * s.fog_color) * k;
+            }
+            throughput = throughput * tau;
         }
         bool emits = true;   // NEE: an emitter the previous hit's sample covered delivers no emission here
         if constexpr (V::nee) {
@@ -255,6 +286,9 @@ __device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &
             const float x1 = rng_float(rng);
             const float x2 = rng_float(rng);
             direction = specular_direction(direction, rec.surf.normal, diffuse_direction(rec.surf.normal, x1, x2), ro);
+            if constexpr (V::fog) {
+                if (s.sun_flags & 1) fog_sun_sample<MODE, V>(s, rng, fog_p, fog_w, rec, color);
+            }
             origin = rec.point + direction * CCU_OFFSET;
             ray_depth += 1;
             rec.distance = inff_();
@@ -301,6 +335,9 @@ __device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &
         float x1 = rng_float(rng);
         float x2 = rng_float(rng);
         direction = diffuse_direction(rec.surf.normal, x1, x2);
+        if constexpr (V::fog) {
+            if (s.sun_flags & 1) fog_sun_sample<MODE, V>(s, rng, fog_p, fog_w, rec, color);
+        }
         origin = rec.point + direction * CCU_OFFSET;
         ray_depth += 1;
         rec.distance = inff_();

@@ -120,6 +120,32 @@ __device__ __forceinline__ float dm_acos(float x) {
     return 1.5707963267948966f - as;
 }
 
+// e^x as a fixed kernel (the fog's transmittance, DESIGN §14), built like dm_powf (ccu_tonemap.cuh): an fp64 series from
+// + - * / only, rounded once to fp32, so that the CPU restatement evaluates the same bits.  exp(-inf) = 0, exp(NaN) = NaN.
+__device__ __forceinline__ float dm_expf(float x) {
+    if (x != x) return nanf_();
+    if (x > 89.0f) return inff_();
+    if (x < -104.0f) return 0.0f;                                   // e^-104 < 2^-150: rounds to 0
+    const double p = (double)x * 1.4426950408889634;                // log2 e
+    const double k = floor(p + 0.5);
+    const double f = (p - k) * 0.6931471805599453;                  // ln 2, |f| <= 0.3466
+    double r = 1.0 / 479001600.0;                                   // exp(f), Taylor to f^12
+    r = r * f + 1.0 / 39916800.0;
+    r = r * f + 1.0 / 3628800.0;
+    r = r * f + 1.0 / 362880.0;
+    r = r * f + 1.0 / 40320.0;
+    r = r * f + 1.0 / 5040.0;
+    r = r * f + 1.0 / 720.0;
+    r = r * f + 1.0 / 120.0;
+    r = r * f + 1.0 / 24.0;
+    r = r * f + 1.0 / 6.0;
+    r = r * f + 0.5;
+    r = r * f + 1.0;
+    r = r * f + 1.0;
+    const double scale = __longlong_as_double((long long)((int)k + 1023) << 52);   // 2^k, -151 <= k <= 129
+    return (float)(r * scale);
+}
+
 // 256-bit read-only global load (LDG.E.256 on sm_100a): one instruction and one L1 tag lookup per lane for a 32-byte record half
 struct __align__(32) Int8 { int v[8]; };
 __device__ __forceinline__ Int8 ldg256(const void *p) {

@@ -82,6 +82,10 @@ constexpr uint32_t QM_HIT = 1u << 26;        // BVH / SHADE stages: the ray has 
 constexpr uint32_t QM_NEE_RAY = 1u << 27;    // NEE: the ray in flight is the emitter sample's shadow ray
 constexpr uint32_t QM_NEE_PREV = 1u << 28;   // NEE: the segment in flight left a hit that sampled the list of cell QF_SN*
 constexpr uint32_t QM_COVERED = 1u << 29;    // NEE + BVH: the closest hit so far is an emitter voxel that list covered
+constexpr uint32_t QM_FOG_RAY = 1u << 30;    // FOG: the ray in flight is the fog's sun sample (DESIGN §14); the bounce waits
+// FOG kernels only (CCU_RENDER_FOG, DESIGN §14): 8 fields after all the others, q_fields(bvh, spec, nee) + 0 .. 7.  From a
+// path-segment hit to its bounce, + 0..2 hold the scattering point p and + 3..5 its weight W; while the fog ray flies, + 0..2
+// hold the origin of the bounce that follows it, and QF_SHW, + 6, + 7 its direction.
 
 constexpr int Q_TOP_WORDS = 4096;            // top tables up to 16^3 cells are staged in shared memory
 // BVH stage: the first Q_STACK entries of a walk's traversal stack (bvh.h:38 nodesToVisit[64]) live in shared memory, one
@@ -96,11 +100,12 @@ constexpr int Q_DEEP = 64 - Q_STACK;          // stack entries beyond the shared
 constexpr int Q_STACK_WORDS = Q_STACK * Q_SLOTS;
 __host__ __device__ constexpr int q_fields(bool bvh, bool spec) { return bvh ? (spec ? (int)QF_COUNT_BVH_SPEC : (int)QF_COUNT_BVH) : (int)QF_COUNT; }
 __host__ __device__ constexpr int q_fields(bool bvh, bool spec, bool nee) { return q_fields(bvh, spec) + (nee ? 2 : 0); }
+__host__ __device__ constexpr int q_fields(bool bvh, bool spec, bool nee, bool fog) { return q_fields(bvh, spec, nee) + (fog ? 8 : 0); }
 __host__ __device__ constexpr int q_stages(bool bvh) { return bvh ? (int)QS_COUNT_BVH : (int)QS_COUNT; }
 __host__ __device__ constexpr int q_mask_words(bool bvh) { return q_stages(bvh) * Q_MW * 32; }
 // slot fields + work masks + control words (live, tile lock / base / used) [+ the staged top table]
-__host__ __device__ constexpr int q_smem_bytes(bool bvh, bool tops, bool spec, bool nee) {
-    return (q_fields(bvh, spec, nee) * Q_SLOTS + q_mask_words(bvh) + 32 + (tops ? Q_TOP_WORDS : 0) + (bvh ? Q_STACK_WORDS : 0)) * 4;
+__host__ __device__ constexpr int q_smem_bytes(bool bvh, bool tops, bool spec, bool nee, bool fog = false) {
+    return (q_fields(bvh, spec, nee, fog) * Q_SLOTS + q_mask_words(bvh) + 32 + (tops ? Q_TOP_WORDS : 0) + (bvh ? Q_STACK_WORDS : 0)) * 4;
 }
 static_assert(q_smem_bytes(true, true, true, true) + 64 * 64 * 4 <= Q_SMEM_LIMIT, "the largest kernel still stages a 64 x 64 sky table");
 
@@ -108,7 +113,8 @@ static_assert(q_smem_bytes(true, true, true, true) + 64 * 64 * 4 <= Q_SMEM_LIMIT
 // debug counters (build with -DCCU_Q_STATS): [2*st] = executions of stage st, [2*st+1] = lanes that had a slot;
 // [10] march iterations, [11] lanes in flight summed over iterations, [12] scheduler rounds that found no work,
 // [13] march yields, [14] pop attempts, [15] pop retries, [24] march refills, [25] BVH refills
-__device__ unsigned long long g_qstats[32];   // [16] BVH stage entries, [18] BVH steps, [19] walking lanes, [20] leaf turns, [21] leaf lanes, [22] SHADE runs, [23] lanes
+// one copy per translation unit, read through queue_stats_take (ccu_render.cuh)
+static __device__ unsigned long long g_qstats[32];   // [16] BVH stage entries, [18] BVH steps, [19] walking lanes, [20] leaf turns, [21] leaf lanes, [22] SHADE runs, [23] lanes
 #define QSTAT(i, v) do { const unsigned long long v_ = (unsigned long long)(v); if ((threadIdx.x & 31) == 0) atomicAdd(&g_qstats[i], v_); } while (0)
 #define QSTAT_LANE(i, v) atomicAdd(&g_qstats[i], (unsigned long long)(v))
 #else
@@ -317,12 +323,55 @@ __device__ __forceinline__ void q_stage_march(const DScene &s, const unsigned *_
 // V::nee: after the sun sample (or in its place) and before the bounce, the emitter sample of DESIGN §10 (§11 for NEE_NEAR) with its
 // own shadow ray (NFI: index of the two NEE fields); `covered`: the hit is an emitter the previous hit's sample covered, whose
 // emission is left out.  V::biome: the emitter sample reads the biome colours of CCU_RENDER_BIOME_TINT (DESIGN §13).
+// FOG: §14.2 steps 1-2 at a path-segment hit from o along d at record distance `distance`: with the sun on the scattering draw,
+// p and W into the fog fields (FFI = the first), then the segment's transmittance on the slot's throughput.
+template <int FFI>
+__device__ __forceinline__ void q_fog_hit(const DScene &s, uint32_t *F, int slot, float3 o, float3 d, float distance) {
+    float3 throughput = f3(QFL(QF_THRX), QFL(QF_THRY), QFL(QF_THRZ));
+    const float a = distance * sqrtf(dot3(d, d));
+    const float e = s.fog_sigma * a;
+    const float tau = dm_expf(-e);
+    if (s.sun_flags & 1) {
+        uint32_t rng = QU(QF_RNG);
+        const float u = rng_float(rng);
+        QU(QF_RNG) = rng;
+        const float3 p = o + d * (u * distance);
+        const float k = s.fog_fast ? 1 - tau : e * dm_expf(-(s.fog_sigma * (u * a)));
+        const float3 w = (throughput * s.fog_color) * k;
+        QFL(FFI) = p.x; QFL(FFI + 1) = p.y; QFL(FFI + 2) = p.z;
+        QFL(FFI + 3) = w.x; QFL(FFI + 4) = w.y; QFL(FFI + 5) = w.z;
+    }
+    throughput = throughput * tau;
+    QFL(QF_THRX) = throughput.x; QFL(QF_THRY) = throughput.y; QFL(QF_THRZ) = throughput.z;
+}
+
 template <bool HAS_BVH, class V>
 __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint32_t *F, unsigned *mask, int lane, int row, float3 o,
                                         float3 d, float distance, bool ray_hit, const SurfT<V::spec> &hit, bool covered) {
     constexpr int NFI = q_fields(HAS_BVH, V::spec);
+    constexpr int FFI = q_fields(HAS_BVH, V::spec, V::nee);   // FOG: the first fog field
     const int slot = row * 32 + lane;
     uint32_t meta = QU(QF_META) & ~(V::nee ? (QM_HIT | QM_COVERED) : QM_HIT);
+    if constexpr (V::fog) {
+        if (meta & QM_FOG_RAY) {
+            // §14.2 step 3: an escaped fog ray adds W times the sky (and sun disc) along it; then the waiting bounce, or END
+            if (!ray_hit) {
+                float3 color = f3(QFL(QF_COLX), QFL(QF_COLY), QFL(QF_COLZ));
+                color = color + f3(QFL(FFI + 3), QFL(FFI + 4), QFL(FFI + 5)) * sky_radiance(s, d);
+                QFL(QF_COLX) = color.x; QFL(QF_COLY) = color.y; QFL(QF_COLZ) = color.z;
+            }
+            meta &= ~QM_FOG_RAY;
+            QU(QF_META) = meta;
+            if ((int)((meta >> 16) & 0xFF) < s.max_depth) {
+                March m;
+                const bool entered = march_begin(s, m, f3(QFL(FFI), QFL(FFI + 1), QFL(FFI + 2)), f3(QFL(QF_SHW), QFL(FFI + 6), QFL(FFI + 7)), inff_());
+                q_store_ray(F, mask, lane, row, m, entered);
+            } else {
+                q_push(mask, QS_END, lane, row);
+            }
+            return;
+        }
+    }
     const bool shadow = (meta & QM_SHADOW) != 0;
     const bool nee_ray = V::nee && (meta & QM_NEE_RAY) != 0;
     // What the path continues with: the sun-sampling shadow ray (sky.h:68-93), the diffuse bounce (nextPath, kernel.h:46-98), or
@@ -348,6 +397,13 @@ __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint
             float3 throughput = f3(QFL(QF_THRX), QFL(QF_THRY), QFL(QF_THRZ));
             float3 color = f3(QFL(QF_COLX), QFL(QF_COLY), QFL(QF_COLZ));
             float3 sky = sky_radiance(s, d);
+            if constexpr (V::fog) {   // §14.3: a path segment's sky blended towards the fog colour by elevation
+                if (!shadow) {
+                    const float y = d.y / sqrtf(dot3(d, d));
+                    const float f = s.fog_sky * (y > 0 ? (1 - y) * (1 - y) : 1.0f);
+                    sky = sky * (1 - f) + s.fog_color * f;
+                }
+            }
             color = color + (sky * throughput) * (shadow ? QFL(QF_SHW) : 1.0f);
             QFL(QF_COLX) = color.x; QFL(QF_COLY) = color.y; QFL(QF_COLZ) = color.z;
             if (shadow) { if (V::nee) nee_step = true; else bounce = true; }
@@ -360,6 +416,7 @@ __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint
         nee_ran = true;
     } else if (!V::spec) {
         // kernel.h:20-22 + applyRayColor kernel.h:33-44
+        if constexpr (V::fog) q_fog_hit<FFI>(s, F, slot, o, d, distance);
         float3 throughput = f3(QFL(QF_THRX), QFL(QF_THRY), QFL(QF_THRZ));
         float3 color = f3(QFL(QF_COLX), QFL(QF_COLY), QFL(QF_COLZ));
         from = o + d * (distance - CCU_OFFSET);
@@ -376,6 +433,7 @@ __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint
         // the event draws come first; then applyRayColor (diffuse event) or its emission with the throughput tinted by a
         // metal only (specular event)
         bool metal = false;
+        if constexpr (V::fog) q_fog_hit<FFI>(s, F, slot, o, d, distance);   // its draw comes before the event draws
         if constexpr (V::spec) {
             uint32_t rng = QU(QF_RNG);
             specular = specular_event(hit.spec, rng, metal, ro);
@@ -458,7 +516,24 @@ __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint
             }
         }
         QU(QF_META) = meta;
-        if (!(ray_depth < s.max_depth)) {
+        bool fog = false;
+        if constexpr (V::fog) {
+            if (s.sun_flags & 1) {
+                // §14.2 step 3: after the bounce's draws, the fog's sun sample from p; the bounce waits in the fog fields
+                uint32_t frng = QU(QF_RNG);
+                const float y1 = rng_float(frng);
+                const float y2 = rng_float(frng);
+                QU(QF_RNG) = frng;
+                const float3 p = f3(QFL(FFI), QFL(FFI + 1), QFL(FFI + 2));
+                QFL(FFI) = next_o.x; QFL(FFI + 1) = next_o.y; QFL(FFI + 2) = next_o.z;
+                QFL(QF_SHW) = next_d.x; QFL(FFI + 6) = next_d.y; QFL(FFI + 7) = next_d.z;
+                QU(QF_META) = meta | QM_FOG_RAY;
+                next_o = p;
+                next_d = sun_sample_direction(s, y1, y2);
+                fog = true;
+            }
+        }
+        if (!fog && !(ray_depth < s.max_depth)) {
             next_ray = false;
             q_push(mask, QS_END, lane, row);
         }
@@ -514,7 +589,7 @@ __device__ __forceinline__ bool q_stage_resolve(const DScene &s, const EmitView 
             return true;
         }
         ray_hit = true;
-        if constexpr (V::nee) covered = q_covered<V::nee>(s, g, F, slot, QU(QF_META), data, c);
+        if constexpr (V::nee) covered = !(V::fog && (QU(QF_META) & QM_FOG_RAY)) && q_covered<V::nee>(s, g, F, slot, QU(QF_META), data, c);
     }
     const float distance = ray_hit ? hit_t : m.limit;
     if (HAS_BVH) {
@@ -532,7 +607,8 @@ __device__ __forceinline__ bool q_stage_resolve(const DScene &s, const EmitView 
         // A shadow ray only asks WHETHER something lies between the surface and the sun (rayTracer.cl:101-106 uses nothing else
         // of its record): once the octree has answered yes, the BVHs - which can only find a closer hit - cannot change that.
         // The same holds for the emitter sample's shadow ray (NEE).
-        if (ray_hit && (meta & (V::nee ? (QM_SHADOW | QM_NEE_RAY) : QM_SHADOW))) {
+        // So does the fog's sun sample (FOG).
+        if (ray_hit && (meta & ((V::nee ? (QM_SHADOW | QM_NEE_RAY) : QM_SHADOW) | (V::fog ? QM_FOG_RAY : 0u)))) {
             q_push(mask, QS_SHADE, lane, row);
             return true;
         }
@@ -741,7 +817,7 @@ __device__ __forceinline__ bool q_stage_leaf(const DScene &s, uint32_t *F, unsig
     const uint32_t meta = QU(QF_META);
     // a shadow ray (the sun's or, NEE, the emitter sample's) is answered by its first accepted triangle (see q_stage_resolve):
     // the rest of the walk could only find a closer one
-    const bool first_hit_ends = (meta & (V::nee ? (QM_SHADOW | QM_NEE_RAY) : QM_SHADOW)) != 0;
+    const bool first_hit_ends = (meta & ((V::nee ? (QM_SHADOW | QM_NEE_RAY) : QM_SHADOW) | (V::fog ? QM_FOG_RAY : 0u))) != 0;
     // the head of the first triangle is requested together with the count word (a leaf block holds at least one triangle; the
     // array is padded so that the read is in bounds even for an empty one), the head of triangle i + 1 while triangle i is tested
     Int8 q0 = ldg256(blk + 8);
@@ -929,7 +1005,7 @@ __global__ void __launch_bounds__(Q_WARPS * 32, 1) k_render_queue(const __grid_c
     constexpr int MASK_WORDS = q_mask_words(HAS_BVH);
     extern __shared__ uint32_t q_mem[];
     uint32_t *F = q_mem;
-    unsigned *mask = q_mem + q_fields(HAS_BVH, V::spec, V::nee) * Q_SLOTS;
+    unsigned *mask = q_mem + q_fields(HAS_BVH, V::spec, V::nee, V::fog) * Q_SLOTS;
     int *live = reinterpret_cast<int *>(mask + MASK_WORDS);
     unsigned *top_s = mask + MASK_WORDS + 32;
     int *stk = reinterpret_cast<int *>(top_s + (LAY == 0 ? Q_TOP_WORDS : 0));   // HAS_BVH only: stacks by slot

@@ -19,6 +19,7 @@
 #include "ccu_host.h"
 #include "ccu_march.cuh"
 #include "ccu_queue.cuh"
+#include "ccu_render.cuh"
 #include "ccu_tonemap.cuh"
 #include "ccu_layout.h"
 
@@ -40,35 +41,6 @@ __global__ void k_sun_setup(const int *sun_words, float *out /* su sv sw radius_
     out[3] = sv.x; out[4] = sv.y; out[5] = sv.z;
     out[6] = sw.x; out[7] = sw.y; out[8] = sw.z;
     out[9] = dm_cos(0.03f);
-}
-
-// Thread-per-pixel path tracer: all passes of the batch in one launch, the running mean of
-// rayTracer.cl:109-112 carried in registers between passes (identical arithmetic, no memory round trip).
-// MODE: 0 = the reference's own node array, 1 = commit-time layouts, 2 = commit-time layouts of a deep world.
-// V: the Shade of the launch (sample_pixel, DESIGN §5).  The emitter table `g` and the biome colours `bv` come after the other
-// arguments, so that the kernels without them keep their parameter offsets.
-template <int MODE, class V>
-__global__ void __launch_bounds__(128) k_render_mega(const __grid_constant__ DScene s, const int *__restrict__ seeds, int n_passes,
-                                                     int start_spp, float *res, const float *res_prev, int n_pixels,
-                                                     const __grid_constant__ EmitView g, const __grid_constant__ BiomeView bv) {
-    if constexpr (V::biome) {
-        if (threadIdx.x == 0) biome_smem() = bv;   // read after the barrier of stage_tables
-    }
-    stage_tables(s, nullptr);
-    for (int gid = blockIdx.x * blockDim.x + threadIdx.x; gid < n_pixels; gid += gridDim.x * blockDim.x) {
-        float *px = res + (size_t)gid * 3;
-        const float *pp = res_prev + (size_t)gid * 3;    // what the reference's single buffer holds when the window starts
-        float3 buf = f3(pp[0], pp[1], pp[2]);
-        for (int pass = 0; pass < n_passes; pass++) {
-            float3 col = sample_pixel<MODE, V>(s, g, gid, __ldg(seeds + pass));
-            int spp = start_spp + pass;
-            float fs = (float)spp, fs1 = (float)(spp + 1);
-            buf.x = (buf.x * fs + col.x) / fs1;
-            buf.y = (buf.y * fs + col.y) / fs1;
-            buf.z = (buf.z * fs + col.z) / fs1;
-        }
-        px[0] = buf.x; px[1] = buf.y; px[2] = buf.z;
-    }
 }
 
 __device__ __forceinline__ int face_of(float3 n) {
@@ -352,6 +324,8 @@ void fill_view(ccu_host::Scene &sc) {
     s.su = in.su; s.sv = in.sv; s.sw = in.sw; s.sun_radius_cos = in.sun_radius_cos;
     s.sun_flags = in.sun_host[0]; s.sun_tex_size = in.sun_host[1]; s.sun_tex = in.sun_host[2];
     memcpy(&s.sun_intensity, &in.sun_host[3], 4);
+    s.fog_sigma = in.fog_sigma; s.fog_sky = in.fog_sky; s.fog_fast = in.fog_fast;
+    s.fog_color = make_float3(in.fog_color[0], in.fog_color[1], in.fog_color[2]);
     EmitView &g = sc.emit_view;
     g.emit = reinterpret_cast<const int4 *>(sc.emit.p); g.off = sc.emit_off.p; g.list = sc.emit_list.p;
     g.g0 = make_int3(in.emit_g0[0], in.emit_g0[1], in.emit_g0[2]);
@@ -467,45 +441,14 @@ void free_target(ccu_ctx *c) {
     c->accum_floats = 0;
 }
 
-// Calls f(std::integral_constant<int, v>{}) for v in [0, N) (N - 1 for anything larger), or f(std::bool_constant<v>{}):
-// picks the template instance of a kernel from a runtime value.
-template <int N, int I = 0, class F>
-void dispatch(int v, F &&f) {
-    if constexpr (I + 1 < N) {
-        if (v != I) return dispatch<N, I + 1>(v, f);
-    }
-    f(std::integral_constant<int, I>{});
-}
-template <class F>
-void dispatch(bool v, F &&f) {
-    if (v) f(std::true_type{});
-    else f(std::false_type{});
-}
-
-// A launch's Shade (ccu_device.cuh) as runtime values
-struct ShadeKey {
-    bool spec;
-    int nee;   // a NeeKind
-    bool biome;
-};
-constexpr int N_SHADES = 2 * 5 * 2;
-ShadeKey nth_shade(int i) { return {i % 2 != 0, i / 2 % 5, i / 10 != 0}; }   // every ShadeKey for i in [0, N_SHADES)
-
-// Calls f(Shade<spec, nee, biome>{}) for the values of v.
-template <class F>
-void dispatch(const ShadeKey &v, F &&f) {
-    dispatch(v.spec, [&](auto S) {
-        dispatch<5>(v.nee, [&](auto N) { dispatch(v.biome, [&](auto B) { f(Shade<S, NeeKind(N.value), B>{}); }); });
-    });
-}
-
 // The Shade of a render launch (DESIGN §5).  Each flag picks its kernels only on a scene where they compute something the
 // others do not:
 // - CCU_RENDER_SPECULAR: the specular kernels, on a scene with a specular word;
 // - CCU_RENDER_EMITTER_SAMPLING: the NEE kernels, on a scene with emitters; CCU_RENDER_EMITTER_NEAR_FIELD picks the near-field
 //   sampler (NEE_NEAR) among them.  CCU_RENDER_EMITTER_MODELS picks the samplers of the wider table (NEE_*_MODELS, EmitView
 //   memit_view) when the scene has one; without a model emitter it changes nothing;
-// - CCU_RENDER_BIOME_TINT: the biome kernels, on a scene with biome colours.
+// - CCU_RENDER_BIOME_TINT: the biome kernels, on a scene with biome colours;
+// - CCU_RENDER_FOG: the fog kernels, on a scene with fog (SceneInfo::has_fog).
 ShadeKey shade_variant(const ccu_ctx *c) {
     const int f = c->params.flags;
     const auto &info = c->scene.info;
@@ -515,16 +458,23 @@ ShadeKey shade_variant(const ccu_ctx *c) {
         if ((f & CCU_RENDER_EMITTER_MODELS) && info.has_model_emitters) nee = near_field ? NEE_NEAR_MODELS : NEE_AREA_MODELS;
         else if (info.has_emitters) nee = near_field ? NEE_NEAR : NEE_AREA;
     }
-    return {(f & CCU_RENDER_SPECULAR) && info.has_specular, nee, (f & CCU_RENDER_BIOME_TINT) && info.has_biome};
+    return {(f & CCU_RENDER_SPECULAR) && info.has_specular, nee, (f & CCU_RENDER_BIOME_TINT) && info.has_biome,
+            (f & CCU_RENDER_FOG) && info.has_fog};
 }
 
-// the wavefront kernel (ccu_queue.cuh) for the scene's entity BVHs, air layout (air_layout_id) and the launch's Shade
-auto queue_kernel(bool bvh, int lay, const ShadeKey &v) {
-    decltype(&k_render_queue<false, 0, PlainShade>) k = nullptr;
-    dispatch(bvh, [&](auto B) {
-        dispatch<3>(lay, [&](auto L) { dispatch(v, [&](auto V) { k = k_render_queue<B, L, decltype(V)>; }); });
-    });
+// the wavefront kernel (ccu_queue.cuh) for the scene's entity BVHs, air layout (queue_layout) and the launch's Shade
+QueueFn queue_kernel(bool bvh, int lay, const ShadeKey &v) {
+    QueueFn k = nullptr;
+    dispatch(bvh, [&](auto B) { dispatch<3>(lay, [&](auto L) { k = queue_kernel_of<B, L>(v); }); });
     return k;
+}
+
+// LAY of a wavefront launch (DESIGN §5): air_layout_id, except that a fog launch whose slot fields do not fit beside the staged
+// top table (entity BVHs with the specular or emitter-sampling fields) reads the same table from global memory (LAY 1).
+int queue_layout(const ccu_ctx *c, bool bvh, const ShadeKey &v) {
+    const int lay = air_layout_id(c);
+    if (lay == 0 && v.fog && q_smem_bytes(bvh, true, v.spec, v.nee != NEE_NONE, true) > Q_SMEM_LIMIT) return 1;
+    return lay;
 }
 
 }  // namespace
@@ -733,6 +683,7 @@ int ccu_scene_begin(ccu_ctx *c) {
     c->scene.biome.reset();
     c->scene.biome_grid.release();
     c->scene.biome_tiles.release();
+    c->scene.info.set_fog(0.0f, 0.0f, nullptr, 0);
     return CCU_OK;
 }
 
@@ -837,6 +788,21 @@ int ccu_scene_set_sun(ccu_ctx *c, const int32_t sun_words[6]) {
     c->committed = false;
     memcpy(c->scene.info.sun_host, sun_words, sizeof c->scene.info.sun_host);
     c->scene.info.have_sun = true;
+    return CCU_OK;
+}
+
+int ccu_scene_set_fog(ccu_ctx *c, float sigma, float sky_density, const float color[3], int32_t fast) {
+    if (!c) return fail(CCU_EINVAL, "ccu_scene_set_fog: null context");
+    if (!(sigma >= 0.0f) || !std::isfinite(sigma)) return fail(CCU_EINVAL, "ccu_scene_set_fog: sigma %g is negative or not finite", sigma);
+    if (!(sky_density >= 0.0f && sky_density <= 1.0f)) return fail(CCU_EINVAL, "ccu_scene_set_fog: sky density %g is not in [0, 1]", sky_density);
+    if (!color) return fail(CCU_EINVAL, "ccu_scene_set_fog: null colour");
+    for (int i = 0; i < 3; i++)
+        if (!(color[i] >= 0.0f) || !std::isfinite(color[i]))
+            return fail(CCU_EINVAL, "ccu_scene_set_fog: colour component %d (%g) is negative or not finite", i, color[i]);
+    if (fast != 0 && fast != 1) return fail(CCU_EINVAL, "ccu_scene_set_fog: fast must be 0 or 1 (got %d)", fast);
+    std::lock_guard<std::mutex> lk(c->mu);
+    c->committed = false;
+    c->scene.info.set_fog(sigma, sky_density, color, fast);
     return CCU_OK;
 }
 
@@ -1061,7 +1027,7 @@ int ccu_render_set_params(ccu_ctx *c, const ccu_render_params *p) {
     if (p->draw_depth < 0 || p->draw_depth >= (1 << 24) || p->max_depth < 1 || p->max_depth > 255) return fail(CCU_EINVAL, "bad render params");
     if (p->kernel != 0 && p->kernel != 1 && p->kernel != 4) return fail(CCU_EINVAL, "unknown kernel %d (0 auto, 1 thread-per-pixel, 4 wavefront)", p->kernel);
     if (p->flags & ~(CCU_RENDER_NO_ENTITIES | CCU_RENDER_NO_SUN | CCU_RENDER_SPECULAR | CCU_RENDER_EMITTER_SAMPLING | CCU_RENDER_EMITTER_NEAR_FIELD |
-                     CCU_RENDER_EMITTER_MODELS | CCU_RENDER_BIOME_TINT))
+                     CCU_RENDER_EMITTER_MODELS | CCU_RENDER_BIOME_TINT | CCU_RENDER_FOG))
         return fail(CCU_EINVAL, "unknown render flags 0x%x", p->flags);
     if ((p->flags & CCU_RENDER_EMITTER_NEAR_FIELD) && !(p->flags & CCU_RENDER_EMITTER_SAMPLING))
         return fail(CCU_EINVAL, "CCU_RENDER_EMITTER_NEAR_FIELD needs CCU_RENDER_EMITTER_SAMPLING");
@@ -1117,10 +1083,8 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
     if (kernel == 1) {
         const int threads = 128, blocks = (n_pixels + threads - 1) / threads;
         dispatch<3>(mode, [&](auto M) {
-            dispatch(shade, [&](auto V) {
-                k_render_mega<M, decltype(V)><<<blocks, threads, 0, c->stream>>>(s, seeds_dev, n_passes, c->window_spp, res, res_prev, n_pixels,
-                                                                                emit_view, biome_view);
-            });
+            mega_kernel<M>(shade)<<<blocks, threads, 0, c->stream>>>(s, seeds_dev, n_passes, c->window_spp, res, res_prev, n_pixels,
+                                                                     emit_view, biome_view);
         });
     } else {
         // persistent wavefront kernel (ccu_queue.cuh): one CTA per SM, pixels handed out through a counter
@@ -1141,13 +1105,13 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
         qp.shade_min = c->q_shade_min;
         qp.sticky_min = c->q_sticky_min > 0 ? c->q_sticky_min : (bvh ? 16 : 33);   // measured: -3 % with BVH stages, +5 % without
         qp.march_warps = bvh ? 64 : c->q_march_warps;   // the cap applies to the BVH-less kernels; with BVH stages every warp may march
-        lay = air_layout_id(c);
+        lay = queue_layout(c, bvh, shade);
         const int grid = c->sm_count, block = Q_WARPS * 32;
         // The sky table is staged in shared memory when it is small: shared memory and L1 are one array on this chip, and a
         // 128 x 128 table (64 KiB) taken from L1 costs more brick / atlas hits than the sky lookups gain (measured: +1.8 % per
         // pass on config 1).  CCU_SKY_SMEM_MAX (bytes, default 16 KiB = 64 x 64 texels) moves the threshold.
         const int sky_texels = c->scene.info.sky_res * c->scene.info.sky_res;
-        const int base_smem = q_smem_bytes(bvh, lay == 0, shade.spec, shade.nee != NEE_NONE);
+        const int base_smem = q_smem_bytes(bvh, lay == 0, shade.spec, shade.nee != NEE_NONE, shade.fog);
         const char *sky_env = getenv("CCU_SKY_SMEM_MAX");
         const int sky_max = sky_env ? atoi(sky_env) : 16384;
         const bool sky_smem = sky_texels * 4 <= sky_max && base_smem + sky_texels * 4 <= Q_SMEM_LIMIT;
@@ -1164,7 +1128,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
         {
             cudaStreamSynchronize(c->stream);
             unsigned long long st[32];
-            cudaMemcpyFromSymbol(st, g_qstats, sizeof st);
+            dispatch(bvh, [&](auto B) { dispatch<3>(lay, [&](auto L) { queue_stats_take<B, L>(st); }); });
             const char *names[4] = {"march", "block", "exit", "end"};
             fprintf(stderr, "[qstats] ");
             for (int i = 1; i < 4; i++) fprintf(stderr, "%s: %llu x %.1f lanes  ", names[i], st[2 * i], st[2 * i] ? (double)st[2 * i + 1] / st[2 * i] : 0.0);
@@ -1173,14 +1137,12 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
             fprintf(stderr, "[qstats] bvh stages %llu, steps %llu x %.1f walking lanes, leaf turns %llu x %.1f lanes, shade %llu x %.1f lanes\n", st[16], st[18],
                     st[18] ? (double)st[19] / st[18] : 0.0, st[20], st[20] ? (double)st[21] / st[20] : 0.0, st[22], st[22] ? (double)st[23] / st[22] : 0.0);
             fprintf(stderr, "[qstats] march refills %llu, bvh refills %llu\n", st[24], st[25]);
-            unsigned long long z[32] = {0};
-            cudaMemcpyToSymbol(g_qstats, z, sizeof z);
         }
 #endif
     }
     c->launches++;
-    const int32_t last[7] = {kernel, bvh, kernel == 1 ? mode : lay, shade.spec, shade.nee, shade.biome, sky_staged};
-    std::copy(last, last + 7, c->last_render);
+    const int32_t last[8] = {kernel, bvh, kernel == 1 ? mode : lay, shade.spec, shade.nee, shade.biome, sky_staged, shade.fog};
+    std::copy(last, last + 8, c->last_render);
     CU(cudaGetLastError());
     CU(cudaEventRecord(c->ev1, c->stream));
     CU(cudaEventRecord(ring.ev[slot], c->stream));
@@ -1461,6 +1423,13 @@ int ccu_debug_last_render(ccu_ctx *c, int32_t out[7]) {
     if (!c || !out) return fail(CCU_EINVAL, "ccu_debug_last_render: null argument");
     std::lock_guard<std::mutex> lk(c->mu);
     std::copy(c->last_render, c->last_render + 7, out);
+    return CCU_OK;
+}
+
+int ccu_debug_last_render_n(ccu_ctx *c, int32_t *out, int32_t n) {
+    if (!c || !out || n < 0) return fail(CCU_EINVAL, "ccu_debug_last_render_n: null argument or negative n");
+    std::lock_guard<std::mutex> lk(c->mu);
+    std::copy(c->last_render, c->last_render + std::min(n, 8), out);
     return CCU_OK;
 }
 

@@ -18,6 +18,7 @@ CCU_RENDER_NO_ENTITIES, CCU_RENDER_NO_SUN, CCU_RENDER_SPECULAR, CCU_RENDER_EMITT
 CCU_RENDER_EMITTER_NEAR_FIELD = 128
 CCU_RENDER_EMITTER_MODELS = 256
 CCU_RENDER_BIOME_TINT = 512
+CCU_RENDER_FOG = 1024
 CCU_UNIQUE_ID_BYTES = 128
 
 CCU_OK, CCU_ENODEVICE, CCU_EINVAL, CCU_ECUDA, CCU_ENOMEM, CCU_ESTATE = 0, -1, -2, -3, -4, -5
@@ -55,6 +56,7 @@ SYMBOLS = {
     "ccu_scene_set_world_bvh": (C.c_int, [_vp, _vp, _i64]),
     "ccu_scene_set_actor_bvh": (C.c_int, [_vp, _vp, _i64]),
     "ccu_scene_set_biome_colors": (C.c_int, [_vp, _vp, _vp, _i64]),
+    "ccu_scene_set_fog": (C.c_int, [_vp, _f, _f, _vp, _i32]),
     "ccu_scene_atlas_create": (C.c_int, [_vp, _i32, _i32, _i32]),
     "ccu_scene_atlas_write": (C.c_int, [_vp, _i32, _i32, _i32, _i32, _i32, _vp]),
     "ccu_scene_set_atlas": (C.c_int, [_vp, _vp, _i32, _i32, _i32]),
@@ -84,6 +86,7 @@ SYMBOLS = {
     "ccu_last_kernel_ms": (C.c_int, [_vp, C.POINTER(_f)]),
     "ccu_launch_count": (C.c_int, [_vp, C.POINTER(_i64)]),
     "ccu_debug_last_render": (C.c_int, [_vp, _vp]),
+    "ccu_debug_last_render_n": (C.c_int, [_vp, _vp, _i32]),
     "ccu_scene_device_bytes": (C.c_int, [_vp, C.POINTER(_i64)]),
     "ccu_scene_commit_ms": (C.c_int, [_vp, C.POINTER(C.c_double)]),
     "ccu_tonemap": (C.c_int, [_vp, _i32, _i32, _f, _vp, _i32, _vp]),
@@ -319,6 +322,14 @@ class Context:
         chunks, rgb = _biome_arrays(chunks, rgb)
         check(self._lib.ccu_scene_set_biome_colors(self._h, _ptr(chunks), _ptr(rgb), chunks.shape[0]))
 
+    def set_fog(self, sigma: float, sky_density: float, color, fast: bool):
+        """The scene's fog for CCU_RENDER_FOG (DESIGN.md §14): extinction per block, sky fog density in [0, 1], linear RGB
+        colour, fast fog; sigma = 0 removes it."""
+        col = np.ascontiguousarray(color, np.float32)
+        if col.shape != (3,):
+            raise ValueError("the fog colour needs 3 components")
+        check(self._lib.ccu_scene_set_fog(self._h, float(sigma), float(sky_density), _ptr(col), int(fast)))
+
     def atlas_create(self, width: int, height: int, layers: int):
         check(self._lib.ccu_scene_atlas_create(self._h, width, height, layers))
 
@@ -470,6 +481,12 @@ class Context:
         out = np.zeros(7, np.int32)
         check(self._lib.ccu_debug_last_render(self._h, _ptr(out)))
         return tuple(int(v) for v in out)
+
+    def last_render_n(self, n: int = 8) -> tuple:
+        """The first min(n, 8) entries of the last launch's instance: last_render()'s 7, then fog (ccu_debug_last_render_n)."""
+        out = np.zeros(max(n, 0), np.int32)
+        check(self._lib.ccu_debug_last_render_n(self._h, _ptr(out), n))
+        return tuple(int(v) for v in out[:min(n, 8)])
 
     def scene_device_bytes(self) -> int:
         n = C.c_int64()

@@ -365,6 +365,29 @@ def camera_from_json(json_path: str) -> np.ndarray:
     return S.pinhole_camera(pos, 270.0 + math.degrees(yaw), -(90.0 + math.degrees(pitch)), float(cam.get("fov", 70.0)))
 
 
+# Chunky's extinction per block for a fog density of 1 (Fog.EXTINCTION_FACTOR).  chunky-core is not available here, so the value
+# is unverified: 0.04 is what it is believed to be.
+FOG_EXTINCTION_FACTOR = 0.04
+
+
+def fog_from_json(json_path: str) -> Tuple[float, float, Tuple[float, float, float], bool]:
+    """The fog of a Chunky scene description as ccu_scene_set_fog takes it (DESIGN.md §14): (sigma, sky density, linear RGB
+    colour, fast).  sigma = fogDensity * FOG_EXTINCTION_FACTOR, the only place that converts Chunky's density; a density of 0
+    gives sigma = 0, no fog.  fogColor is taken as linear RGB, and a missing key takes a default (fogDensity 0, skyFogDensity 1,
+    a white fogColor, fastFog true); like the extinction factor, neither is checked against chunky-core, which is not
+    available here."""
+    import json
+    d = json.loads(open(json_path, "rb").read().decode("latin-1"))
+    c = d.get("fogColor", {"red": 1.0, "green": 1.0, "blue": 1.0})
+    color = (float(c["red"]), float(c["green"]), float(c["blue"]))
+    return (float(d.get("fogDensity", 0.0)) * FOG_EXTINCTION_FACTOR, float(d.get("skyFogDensity", 1.0)), color,
+            bool(d.get("fastFog", True)))
+
+
 def load_scene(octree_path: str, json_path: str = None, width: int = 1920, height: int = 1080) -> S.PackedScene:
+    """The scene of an .octree2 file, with the camera and fog of a Chunky scene description when one is given."""
     o = load(octree_path)
-    return to_scene(o, width, height, camera=camera_from_json(json_path) if json_path else None)
+    p = to_scene(o, width, height, camera=camera_from_json(json_path) if json_path else None)
+    if json_path:
+        p.fog = fog_from_json(json_path)
+    return p

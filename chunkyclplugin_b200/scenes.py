@@ -70,6 +70,8 @@ class PackedScene:
     # biome colours for CCU_RENDER_BIOME_TINT: (chunks int32[n, 2] {cx, cz}, rgb float32[n, 3, 256, 3]) as
     # ccu_scene_set_biome_colors takes them (planes foliage, grass, water; texel (z & 15) * 16 + (x & 15)), or None
     biome: Optional[Tuple[np.ndarray, np.ndarray]] = None
+    # fog for CCU_RENDER_FOG: (sigma, sky density, (r, g, b), fast) as ccu_scene_set_fog takes them (DESIGN.md §14), or None
+    fog: Optional[Tuple[float, float, Tuple[float, float, float], bool]] = None
 
     def arrays(self) -> Dict[str, np.ndarray]:
         return {k: getattr(self, k) for k in (

@@ -92,6 +92,12 @@ typedef struct ccu_render_params {
  * reference's behaviour, and a scene without biome colours renders exactly as without the flag.  Valid alone and with every
  * other flag; both render kernels implement it.  DESIGN.md §13 holds the exact contract. */
 #define CCU_RENDER_BIOME_TINT 512
+/* Fog (beyond the reference; Chunky's uniform fog with sunlit light shafts): on a scene with fog (ccu_scene_set_fog, sigma > 0),
+ * every path segment that hits is attenuated by exp(-sigma * length) and, with the sun on, gains one sun sample from a point
+ * drawn uniformly along it, traced towards the sun without a limit; a segment that misses sees the sky blended towards the fog
+ * colour by elevation.  Shadow and emitter-sample rays see neither.  A scene without fog renders exactly as without the flag.
+ * Valid alone and with every other flag; both render kernels implement it.  DESIGN.md §14 holds the exact contract. */
+#define CCU_RENDER_FOG 1024
 
 /* ---- device enumeration: RendererInstance.java:39-75,123-157 (clGetPlatformIDs/clGetDeviceIDs/clGetDeviceInfo),
  *      used by the GPU selector UI (ui/GpuSelector.java:24-87) -------------------------------------------------- */
@@ -125,6 +131,11 @@ int ccu_scene_set_actor_bvh(ccu_ctx *ctx, const int32_t *words, int64_t n);     
  * max(1, 2^depth / 16) chunks per axis, or when the chunks' bounding box holds more than 2^24 chunks (the lookup grid covers
  * that box: every chunk of a depth-16 octree fits). */
 int ccu_scene_set_biome_colors(ccu_ctx *ctx, const int32_t *chunks, const float *rgb, int64_t n);
+/* Fog for CCU_RENDER_FOG (optional; beyond the reference).  sigma = extinction per block (>= 0, finite; 0 removes the fog),
+ * sky_density = Chunky's sky fog density in [0, 1], color = linear RGB fog colour (3 floats, each >= 0 and finite), fast = Chunky's
+ * "fast fog" switch (0 or 1).  CCU_EINVAL otherwise.  Like the sun it belongs to the scene: ccu_scene_begin removes it, and it
+ * takes effect at the next ccu_scene_commit (ccu_group_replicate_scene carries it). */
+int ccu_scene_set_fog(ccu_ctx *ctx, float sigma, float sky_density, const float color[3], int32_t fast);
 /* texture atlas: ClTextureLoader.java:46-66 - clCreateImage(8192x8192xlayers RGBA8) then one clEnqueueWriteImage
  * per texture at (16*tileX, 16*tileY, layer) */
 int ccu_scene_atlas_create(ccu_ctx *ctx, int32_t width, int32_t height, int32_t layers);
@@ -198,8 +209,11 @@ int ccu_launch_count(ccu_ctx *ctx, int64_t *launches);    /* kernels launched by
 /* Test support: the render kernel instance of the context's last ccu_render_passes[_async] launch (all zero before the first).
  * out = {kernel launched (1 or 4, after the choice for kernel 0), HAS_BVH, LAY (kernel 4) or MODE (kernel 1), spec, nee (a NeeKind:
  * 0 none, 1 area, 2 near, 3 area + models, 4 near + models), biome, sky texels staged in shared memory (0 for kernel 1)};
+ * LAY is the one the launch ran (a fog launch may move from LAY 0 to LAY 1, DESIGN.md §5).
  * DESIGN.md §5.  A launch refused with an error leaves it as it was. */
 int ccu_debug_last_render(ccu_ctx *ctx, int32_t out[7]);
+/* The same report with the switches added since: writes the first min(n, 8) of {the 7 entries above, fog}. */
+int ccu_debug_last_render_n(ccu_ctx *ctx, int32_t *out, int32_t n);
 int ccu_scene_device_bytes(ccu_ctx *ctx, int64_t *bytes); /* HBM held by the committed scene */
 int ccu_scene_commit_ms(ccu_ctx *ctx, double *ms);        /* host time the last ccu_scene_commit spent building + uploading the layouts */
 /* Memory-system denominators for this path's roofline (dependent 32-byte-sector gathers, SURVEY 8d): random 16-byte

@@ -40,6 +40,7 @@ public final class ChunkyCu {
     private static final MethodHandle SET_WORLD_BVH = h("ccu_scene_set_world_bvh", WORDS);
     private static final MethodHandle SET_ACTOR_BVH = h("ccu_scene_set_actor_bvh", WORDS);
     private static final MethodHandle SET_BIOME_COLORS = h("ccu_scene_set_biome_colors", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG));
+    private static final MethodHandle SET_FOG = h("ccu_scene_set_fog", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_FLOAT, JAVA_FLOAT, ADDRESS, JAVA_INT));
     private static final MethodHandle DEBUG_BIOME_LAYOUT = h("ccu_debug_biome_layout", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, JAVA_INT, ADDRESS, ADDRESS, ADDRESS));
     private static final MethodHandle ATLAS_CREATE = h("ccu_scene_atlas_create", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT, JAVA_INT, JAVA_INT));
     private static final MethodHandle ATLAS_WRITE = h("ccu_scene_atlas_write", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, ADDRESS));
@@ -87,6 +88,8 @@ public final class ChunkyCu {
     public static final int RENDER_EMITTER_MODELS = 256;
     /** ccu_render_params.flags: grass, foliage and water tinted by the biome colours of {@link Context#setBiomeColors} (DESIGN §13). */
     public static final int RENDER_BIOME_TINT = 512;
+    /** ccu_render_params.flags: the scene's fog of {@link Context#setFog}, with sunlit light shafts (DESIGN §14). */
+    public static final int RENDER_FOG = 1024;
     private static final StructLayout RENDER_PARAMS = MemoryLayout.structLayout(JAVA_INT.withName("draw_depth"), JAVA_INT.withName("max_depth"),
             JAVA_FLOAT.withName("emitter_scale"), JAVA_INT.withName("kernel"), JAVA_INT.withName("flags"));
 
@@ -197,6 +200,13 @@ public final class ChunkyCu {
                 MemorySegment c = n > 0 ? a.allocateFrom(JAVA_INT, java.util.Arrays.copyOf(chunks, 2 * n)) : MemorySegment.NULL;
                 MemorySegment r = n > 0 ? a.allocateFrom(JAVA_FLOAT, java.util.Arrays.copyOf(rgb, BIOME_TILE_FLOATS * n)) : MemorySegment.NULL;
                 check(call(SET_BIOME_COLORS, handle, c, r, (long) n));
+            }
+        }
+        /** The scene's fog: extinction per block (0 removes it), Chunky's sky fog density in [0, 1], a linear RGB colour, fast fog. */
+        public void setFog(float sigma, float skyDensity, float[] color, boolean fast) {
+            if (color.length != 3) throw new IllegalArgumentException("the fog colour needs 3 components");
+            try (Arena a = Arena.ofConfined()) {
+                check(call(SET_FOG, handle, sigma, skyDensity, a.allocateFrom(JAVA_FLOAT, color), fast ? 1 : 0));
             }
         }
         public void atlasCreate(int width, int height, int layers) { check(call(ATLAS_CREATE, handle, width, height, layers)); }

@@ -37,12 +37,24 @@ def lib():
         assert _lib.oracle_scene_struct_size() == C.sizeof(oracle._Scene), "OracleScene layout mismatch"
         assert _lib.emitter_grid_struct_size() == C.sizeof(_Grid), "EmitterGrid layout mismatch"
         assert _lib.biome_tiles_struct_size() == C.sizeof(_Biome), "BiomeTiles layout mismatch"
+        assert _lib.fog_params_struct_size() == C.sizeof(_Fog), "FogParams layout mismatch"
+        _lib.fog_expf_test.restype = C.c_float
+        _lib.fog_expf_test.argtypes = [C.c_float]
     return _lib
 
 
 class _Grid(C.Structure):
     _fields_ = [("emit", C.c_void_p), ("off", C.c_void_p), ("list", C.c_void_p),
                 ("g0", C.c_int32 * 3), ("dim", C.c_int32 * 3), ("shift", C.c_int32), ("mhead", C.c_void_p), ("mprim", C.c_void_p)]
+
+
+class _Fog(C.Structure):
+    _fields_ = [("sigma", C.c_float), ("sky", C.c_float), ("color", C.c_float * 3), ("fast", C.c_int32)]
+
+
+def dm_expf(x: float) -> float:
+    """The fog's transmittance kernel (DESIGN.md section 14), as the restatement and the kernels evaluate it."""
+    return float(np.float32(lib().fog_expf_test(float(x))))
 
 
 class _Biome(C.Structure):
@@ -52,6 +64,7 @@ class _Biome(C.Structure):
 
 CCU_RENDER_SPECULAR, CCU_RENDER_EMITTER_SAMPLING, CCU_RENDER_EMITTER_NEAR_FIELD, CCU_RENDER_EMITTER_MODELS = 4, 8, 128, 256
 CCU_RENDER_BIOME_TINT = 512
+CCU_RENDER_FOG = 1024
 EMIT_SHIFT0, EMIT_CELL_BUDGET, EMIT_MAX = 3, 1 << 21, 1 << 18      # DESIGN.md section 10
 
 
@@ -244,11 +257,18 @@ class FlagsOracle(oracle.Oracle):
     CCU_RENDER_EMITTER_NEAR_FIELD / CCU_RENDER_EMITTER_MODELS / CCU_RENDER_BIOME_TINT bits (the other flags act on the scene:
     oracle.edge_rays.without_sun, or empty BVHs for CCU_RENDER_NO_ENTITIES).  With CCU_RENDER_EMITTER_MODELS the wider table
     of section 12 is sampled when the scene has one, else the table of section 10.  With CCU_RENDER_BIOME_TINT the biome
-    colours are `biome` = (chunks, rgb) as ccu_scene_set_biome_colors takes them, by default the scene's own (scene.biome)."""
+    colours are `biome` = (chunks, rgb) as ccu_scene_set_biome_colors takes them, by default the scene's own (scene.biome).
+    With CCU_RENDER_FOG the fog of section 14 is `fog` = (sigma, sky density, colour, fast) as ccu_scene_set_fog takes it,
+    by default the scene's own (scene.fog); sigma = 0 is no fog."""
 
-    def __init__(self, scene, flags: int = 0, biome=None, **kw):
+    def __init__(self, scene, flags: int = 0, biome=None, fog=None, **kw):
         super().__init__(scene, **kw)
         self.flags = flags
+        if fog is None:
+            fog = getattr(scene, "fog", None)
+        self._fog = None
+        if flags & CCU_RENDER_FOG and fog is not None and fog[0] > 0:
+            self._fog = _Fog(fog[0], fog[1], (C.c_float * 3)(*fog[2]), int(fog[3]))
         if biome is None:
             biome = getattr(scene, "biome", None)
         self._biome = None
@@ -289,6 +309,7 @@ class FlagsOracle(oracle.Oracle):
                            res.ctypes.data_as(C.c_void_p), gp, C.c_int64(gn), C.c_int(threads), C.byref(cnt),
                            C.c_int(1 if self.flags & CCU_RENDER_SPECULAR else 0), C.byref(self._grid) if nee else None,
                            C.c_int(1 if self.flags & CCU_RENDER_EMITTER_NEAR_FIELD else 0),
-                           C.byref(self._biome) if self._biome is not None else None)
+                           C.byref(self._biome) if self._biome is not None else None,
+                           C.byref(self._fog) if self._fog is not None else None)
         self._counters(cnt)
         return res

@@ -14,7 +14,8 @@
  * The octree march also reports the hit voxel, which the emission rule of emitter sampling needs.  The path loop knows
  * both flags; the emitter table it samples is built by the Python side of this package from the packed arrays.
  * CCU_RENDER_BIOME_TINT (section 13) restates the material evaluation with the biome colours of the hit voxel's column; the
- * block test, the octree march and the emitter samplers pass that voxel on.
+ * block test, the octree march and the emitter samplers pass that voxel on.  CCU_RENDER_FOG (section 14) restates the fog of
+ * the path loop.
  */
 #include "../oracle/chunky_oracle.c"
 
@@ -531,8 +532,66 @@ static int nee_sample(const Ctx *c, const EmitterGrid *g, int near, int b, int n
     return 1;
 }
 
-/* one path sample: rayTracer.cl:40-107 with the specular events (spec) and emitter sampling (g != NULL; near: section 11) */
-static v3 sample_pixel_ext(const Ctx *c, int gid, int32_t seed, int spec, const EmitterGrid *g, int near) {
+/* ---- fog (DESIGN.md section 14) ---- */
+typedef struct {
+    float sigma, sky, color[3];
+    int32_t fast;
+} FogParams;
+
+/* dm_expf of ccu_math.cuh, operation for operation: an fp64 series rounded once to fp32 */
+static float fog_expf(float x) {
+    if (x != x) return NAN;
+    if (x > 89.0f) return HUGE_VALF;
+    if (x < -104.0f) return 0.0f;
+    const double p = (double)x * 1.4426950408889634;
+    const double k = floor(p + 0.5);
+    const double f = (p - k) * 0.6931471805599453;
+    double r = 1.0 / 479001600.0;
+    r = r * f + 1.0 / 39916800.0;
+    r = r * f + 1.0 / 3628800.0;
+    r = r * f + 1.0 / 362880.0;
+    r = r * f + 1.0 / 40320.0;
+    r = r * f + 1.0 / 5040.0;
+    r = r * f + 1.0 / 720.0;
+    r = r * f + 1.0 / 120.0;
+    r = r * f + 1.0 / 24.0;
+    r = r * f + 1.0 / 6.0;
+    r = r * f + 0.5;
+    r = r * f + 1.0;
+    r = r * f + 1.0;
+    const int64_t bits = (int64_t)((int)k + 1023) << 52;
+    double scale;
+    memcpy(&scale, &bits, sizeof scale);
+    return (float)(r * scale);
+}
+
+/* section 14.3: a path segment that misses sees the sky blended towards the fog colour by elevation */
+static void fog_intersect_sky(const Ctx *c, const FogParams *fog, Path *p, Record *rec) {
+    sky_intersect(c, p->direction, rec);
+    sun_intersect(c, p->direction, rec);
+    v3 d = p->direction;
+    float y = d.y / sqrtf(vdot(d, d));
+    float f = fog->sky * (y > 0 ? (1 - y) * (1 - y) : 1.0f);
+    v3 col = vadd(vscale(V(rec->color[0], rec->color[1], rec->color[2]), 1 - f), vscale(V(fog->color[0], fog->color[1], fog->color[2]), f));
+    p->pix_color = vadd(p->pix_color, vscale(vmul(col, p->throughput), rec->emittance));
+}
+
+/* section 14.2 step 3: the sun sample from the scattering point x, traced without a limit; w = the pending weight */
+static void fog_sun_sample(const Ctx *c, v3 x, v3 w, const Record *rec, uint32_t *state, Path *p) {
+    Path q = *p;
+    Record r = *rec;
+    q.origin = x;
+    if (!sun_sample_direction(c, &q, &r, state)) return;
+    r.distance = HUGE_VALF;
+    if (closest_intersect(c, &q, &r)) return;
+    sky_intersect(c, q.direction, &r);
+    sun_intersect(c, q.direction, &r);
+    p->pix_color = vadd(p->pix_color, vmul(w, V(r.color[0], r.color[1], r.color[2])));
+}
+
+/* one path sample: rayTracer.cl:40-107 with the specular events (spec), emitter sampling (g != NULL; near: section 11) and
+ * fog (fog != NULL, section 14) */
+static v3 sample_pixel_ext(const Ctx *c, int gid, int32_t seed, int spec, const EmitterGrid *g, int near, const FogParams *fog) {
     Path p;
     Record rec;
     uint32_t w5 = 0;
@@ -546,12 +605,27 @@ static v3 sample_pixel_ext(const Ctx *c, int gid, int32_t seed, int spec, const 
     rng_next(&state);
     camera_ray(c, gid, &state, &p, 0);
     c->cnt->samples++;
+    v3 fog_p = V(0, 0, 0), fog_w = V(0, 0, 0);
+    const int fog_sun = fog && (c->sun.flags & 1);
     for (;;) {
         c->cnt->segments++;
         if (!closest_intersect_w5(c, &p, &rec, &w5, vox, 0)) {
             rec.emittance = 1;
-            intersect_sky(c, &p, &rec);
+            if (fog) fog_intersect_sky(c, fog, &p, &rec);
+            else intersect_sky(c, &p, &rec);
             break;
+        }
+        if (fog) {   /* section 14.2 steps 1-2 */
+            float a = rec.distance * sqrtf(vdot(p.direction, p.direction));
+            float e = fog->sigma * a;
+            float tau = fog_expf(-e);
+            if (fog_sun) {
+                float u = rng_float(&state);
+                fog_p = vadd(p.origin, vscale(p.direction, u * rec.distance));
+                float k = fog->fast ? 1 - tau : e * fog_expf(-(fog->sigma * (u * a)));
+                fog_w = vscale(vmul(p.throughput, V(fog->color[0], fog->color[1], fog->color[2])), k);
+            }
+            p.throughput = vscale(p.throughput, tau);
         }
         int emits = 1;
         if (g) {
@@ -560,6 +634,7 @@ static v3 sample_pixel_ext(const Ctx *c, int gid, int32_t seed, int spec, const 
         }
         int more;
         if (spec && specular_event(c, &p, &rec, w5, &state, &more, emits)) {
+            if (fog_sun) fog_sun_sample(c, fog_p, fog_w, &rec, &state, &p);
             if (!more) break;
             continue;
         }
@@ -598,14 +673,16 @@ static v3 sample_pixel_ext(const Ctx *c, int gid, int32_t seed, int spec, const 
                 }
             }
         }
-        if (!next_path(c, &p, &rec, &state, c->sc->max_depth)) break;
+        more = next_path(c, &p, &rec, &state, c->sc->max_depth);
+        if (fog_sun) fog_sun_sample(c, fog_p, fog_w, &rec, &state, &p);
+        if (!more) break;
     }
     return p.pix_color;
 }
 
 static int render_ext(const OracleScene *s, const int32_t *seeds, int n_passes, int start_spp, float *res, const int32_t *gids,
                       int64_t n_gids, int nthreads, OracleCounters *out_counters, int spec, const EmitterGrid *g, int near,
-                      const BiomeTiles *biome) {
+                      const BiomeTiles *biome, const FogParams *fog) {
     int64_t n = gids ? n_gids : (int64_t)s->width * s->height;
     OracleCounters total;
     memset(&total, 0, sizeof total);
@@ -626,7 +703,7 @@ static int render_ext(const OracleScene *s, const int32_t *seeds, int n_passes, 
             float *px = res + (size_t)gid * 3;
             v3 buf = V(px[0], px[1], px[2]);
             for (int pass = 0; pass < n_passes; pass++) {
-                v3 col = sample_pixel_ext(c, gid, seeds[pass], spec, g, near);
+                v3 col = sample_pixel_ext(c, gid, seeds[pass], spec, g, near, fog);
                 int spp = start_spp + pass;
                 buf.x = (buf.x * (float)spp + col.x) / (float)(spp + 1);
                 buf.y = (buf.y * (float)spp + col.y) / (float)(spp + 1);
@@ -644,16 +721,21 @@ static int render_ext(const OracleScene *s, const int32_t *seeds, int n_passes, 
 /* oracle_render with the specular events (same arguments, same running mean) */
 int specular_render(const OracleScene *s, const int32_t *seeds, int n_passes, int start_spp, float *res, const int32_t *gids,
                     int64_t n_gids, int nthreads, OracleCounters *out_counters) {
-    return render_ext(s, seeds, n_passes, start_spp, res, gids, n_gids, nthreads, out_counters, 1, NULL, 0, NULL);
+    return render_ext(s, seeds, n_passes, start_spp, res, gids, n_gids, nthreads, out_counters, 1, NULL, 0, NULL, NULL);
 }
 
 /* oracle_render with CCU_RENDER_SPECULAR (spec), CCU_RENDER_EMITTER_SAMPLING (g != NULL), CCU_RENDER_EMITTER_NEAR_FIELD
- * (near, with g) and CCU_RENDER_BIOME_TINT (biome != NULL) */
+ * (near, with g), CCU_RENDER_BIOME_TINT (biome != NULL) and CCU_RENDER_FOG (fog != NULL: the scene has fog) */
 int flags_render(const OracleScene *s, const int32_t *seeds, int n_passes, int start_spp, float *res, const int32_t *gids,
                  int64_t n_gids, int nthreads, OracleCounters *out_counters, int spec, const EmitterGrid *g, int near,
-                 const BiomeTiles *biome) {
-    return render_ext(s, seeds, n_passes, start_spp, res, gids, n_gids, nthreads, out_counters, spec, g, near, biome);
+                 const BiomeTiles *biome, const FogParams *fog) {
+    return render_ext(s, seeds, n_passes, start_spp, res, gids, n_gids, nthreads, out_counters, spec, g, near, biome, fog);
 }
+
+int fog_params_struct_size(void) { return (int)sizeof(FogParams); }
+
+/* the fog's transmittance kernel alone, for tests */
+float fog_expf_test(float x) { return fog_expf(x); }
 
 int biome_tiles_struct_size(void) { return (int)sizeof(BiomeTiles); }
 
