@@ -116,6 +116,15 @@ __device__ __forceinline__ BiomeView &biome_smem() {
     return b;
 }
 
+// The cloud layer of CCU_RENDER_CLOUDS (DESIGN §15), set by ccu_scene_set_clouds and passed to both render kernels as an argument
+// of their own after the others, like the emitter table and the biome colours.  mask: 256 x 256 bits, cell (i, k) at bit
+// (k & 255) * 256 + (i & 255) (8 KiB, read through the read-only path); the box of a set cell is i <= x * inv + u0 <= i + 1,
+// y0 <= y <= y1, k <= z * inv + v0 <= k + 1.
+struct CloudView {
+    const unsigned *__restrict__ mask;
+    float inv, y0, y1, u0, v0;
+};
+
 // What a successful intersection writes into the IntersectionRecord (wavefront.h:37-78).  The specular kernels (SPEC, DESIGN
 // "Beyond the reference: specular materials") also carry word 5 of the material the colour came from: specular, metalness and
 // roughness bytes.  The other kernels keep the reference's record exactly.
@@ -149,7 +158,7 @@ using Record = RecordT<false>;
 
 struct HitInfo {     // first-hit bookkeeping, not part of the reference's record
     int node;        // treeData index of the hit leaf (reference layout), -1 when unknown / BVH hit
-    int kind;        // 0 miss, 1 octree, 2 world BVH, 3 actor BVH
+    int kind;        // 0 miss, 1 octree, 2 world BVH, 3 actor BVH, 4 cloud (render kernels with CCU_RENDER_CLOUDS only)
     int bx, by, bz;  // voxel of the octree hit
 };
 
@@ -984,14 +993,96 @@ enum NeeKind : int { NEE_NONE = 0, NEE_AREA = 1, NEE_NEAR = 2, NEE_AREA_MODELS =
 __host__ __device__ constexpr bool nee_near_field(int kind) { return kind == NEE_NEAR || kind == NEE_NEAR_MODELS; }
 __host__ __device__ constexpr bool nee_models(int kind) { return kind == NEE_AREA_MODELS || kind == NEE_NEAR_MODELS; }
 // The shading variant a render kernel is built with, picked per launch by shade_variant (chunkycu.cu, DESIGN §5).
-template <bool S, NeeKind N, bool B, bool F = false>
+template <bool S, NeeKind N, bool B, bool F = false, bool C = false>
 struct Shade {
     static constexpr bool spec = S, biome = B;
     static constexpr NeeKind nee = N;
     static constexpr bool models = nee_models(N);   // the wider emitter table of CCU_RENDER_EMITTER_MODELS
-    static constexpr bool fog = F;                  // the fog of CCU_RENDER_FOG (DESIGN §14; thread-per-pixel kernel only)
+    static constexpr bool fog = F;                  // the fog of CCU_RENDER_FOG (DESIGN §14)
+    static constexpr bool clouds = C;               // the cloud layer of CCU_RENDER_CLOUDS (DESIGN §15)
 };
 using PlainShade = Shade<false, NEE_NONE, false>;   // the first-hit and preview kernels
+
+// ------------------------------------------------------------------------------------------------------
+// beyond the reference: the cloud layer (CCU_RENDER_CLOUDS, DESIGN §15)
+// ------------------------------------------------------------------------------------------------------
+#define CCU_CLOUD_CELLS 1024            // §15.2: the walk visits at most this many cells, then reports a miss
+#define CCU_CLOUD_COORD_MAX 8388608.0f  // §15.2: 2^23, the walk reports a miss where a cell coordinate reaches it
+
+// The ray's parameter interval in cell c (c <= o + d t <= c + 1) of one cell axis; d = 0: the whole line (the walk only visits
+// cells that contain o on such an axis, cloud_start).
+__device__ __forceinline__ void cloud_axis(float o, float d, int c, float &lo, float &hi) {
+    if (d == 0.0f) { lo = -inff_(); hi = inff_(); return; }
+    const float a = ((float)c - o) / d, b = ((float)(c + 1) - o) / d;
+    lo = d > 0.0f ? a : b;
+    hi = d > 0.0f ? b : a;
+}
+// The walk's first cell on one axis: the cell whose interval holds ts, or the one before it; false for a miss (d = 0 with o on a
+// cell boundary, a coordinate at or beyond 2^23, NaN).  step: +1, -1 or 0 for d = 0.
+__device__ __forceinline__ bool cloud_start(float o, float d, float ts, int &c, int &step) {
+    if (d == 0.0f) {
+        const float f = floorf(o);
+        if (!(o > f) || !(fabsf(o) < CCU_CLOUD_COORD_MAX)) return false;
+        c = (int)f;
+        step = 0;
+        return true;
+    }
+    const float x = o + d * ts;
+    if (!(fabsf(x) < CCU_CLOUD_COORD_MAX)) return false;
+    c = (int)floorf(x);
+    step = d > 0.0f ? 1 : -1;
+    float lo, hi;
+    cloud_axis(o, d, c, lo, hi);
+    if (lo > ts) c -= step;
+    return true;
+}
+// §15.2: the smallest t > 0 below `limit` at which the ray o + d t enters the box of a set cell from outside (the boxes are
+// open: a ray inside one or on its boundary leaves it without a hit), found by a 2-D walk over the cells inside the slab
+// y0 < y < y1; n = the outward normal of the face entered (ties: y, then x, then z).
+__device__ __forceinline__ bool cloud_hit(const CloudView &cv, float3 o, float3 d, float limit, float &t, float3 &n) {
+    float ylo, yhi;
+    if (d.y == 0.0f) {
+        if (!(cv.y0 < o.y && o.y < cv.y1)) return false;
+        ylo = -inff_();
+        yhi = inff_();
+    } else {
+        const float a = (cv.y0 - o.y) / d.y, b = (cv.y1 - o.y) / d.y;
+        if (!(a == a && b == b)) return false;
+        ylo = d.y > 0.0f ? a : b;
+        yhi = d.y > 0.0f ? b : a;
+    }
+    const float tend = yhi < limit ? yhi : limit;
+    const float ts = ylo > 0.0f ? ylo : 0.0f;
+    if (!(ts < tend)) return false;
+    const float ox = o.x * cv.inv + cv.u0, dx = d.x * cv.inv;
+    const float oz = o.z * cv.inv + cv.v0, dz = d.z * cv.inv;
+    int i, k, si, sk;
+    if (!cloud_start(ox, dx, ts, i, si) || !cloud_start(oz, dz, ts, k, sk)) return false;
+    for (int step = 0; step < CCU_CLOUD_CELLS; step++) {
+        float xlo, xhi, zlo, zhi;
+        cloud_axis(ox, dx, i, xlo, xhi);
+        cloud_axis(oz, dz, k, zlo, zhi);
+        const unsigned bit = ((unsigned)(k & 255) << 8) | (unsigned)(i & 255);
+        if ((__ldg(cv.mask + (bit >> 5)) >> (bit & 31u)) & 1u) {
+            float tn = ylo;
+            int axis = 1;
+            if (xlo > tn) { tn = xlo; axis = 0; }
+            if (zlo > tn) { tn = zlo; axis = 2; }
+            float tf = yhi < xhi ? yhi : xhi;
+            tf = tf < zhi ? tf : zhi;
+            if (tn > 0.0f && tn < tf && tn < limit) {
+                t = tn;
+                n = axis == 0 ? f3(dx > 0.0f ? -1.0f : 1.0f, 0, 0) : (axis == 1 ? f3(0, d.y > 0.0f ? -1.0f : 1.0f, 0) : f3(0, 0, dz > 0.0f ? -1.0f : 1.0f));
+                return true;
+            }
+        }
+        const float te = xhi < zhi ? xhi : zhi;
+        if (!(te < tend)) return false;
+        if (xhi == te) i += si;
+        if (zhi == te) k += sk;
+    }
+    return false;
+}
 #define CCU_NEE_RHO2 0.015625f   // DESIGN §11: an emitter is near when its box distance² is below rho² = (1/8)²
 
 // The emission rule: an octree hit on voxel (bx, by, bz) of block palette position `block` that the previous hit's sample

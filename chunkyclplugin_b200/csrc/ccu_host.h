@@ -172,6 +172,8 @@ struct SceneInfo {
     int has_fog = 0;        // ccu_scene_set_fog with sigma > 0: CCU_RENDER_FOG launches the fog kernels
     float fog_sigma = 0, fog_sky = 0, fog_color[3] = {0, 0, 0};   // DScene::fog_*
     int fog_fast = 0;
+    int has_clouds = 0;     // a cloud mask with a set cell: CCU_RENDER_CLOUDS launches the cloud kernels
+    float cloud_inv = 0, cloud_y0 = 0, cloud_y1 = 0, cloud_u0 = 0, cloud_v0 = 0;   // CloudView::inv ...
     void set_fog(float sigma, float sky, const float *color, int fast) {   // color may be null for sigma = 0 (no fog)
         has_fog = sigma > 0.0f;
         fog_sigma = sigma;
@@ -210,6 +212,15 @@ struct BiomeColors {
     std::vector<float> rgb;        // n x 3 planes x 256 texels x 3
 };
 
+// The cloud layer of ccu_scene_set_clouds (DESIGN §15): the mask bit-packed as the kernels read it (CloudView), and the
+// parameters; commit uploads the mask.
+constexpr int CLOUD_CELLS = 256 * 256, CLOUD_WORDS = CLOUD_CELLS / 32;
+struct CloudLayer {
+    unsigned bits[CLOUD_WORDS] = {};
+    bool any = false;   // a cell is set
+    float inv = 0, y0 = 0, y1 = 0, u0 = 0, v0 = 0;
+};
+
 // Everything a context knows about its scene: the uploads, the layouts commit builds from them, and the launch view.
 struct Scene {
     PackedArray arrays[N_ARRAYS];
@@ -222,12 +233,15 @@ struct Scene {
     DevBuf<int> biome_grid;                               // biome colours (BiomeView), only when set
     DevBuf<float4> biome_tiles;
     std::shared_ptr<const BiomeColors> biome;             // set while the scene has biome colours; shared by a replica
+    DevBuf<unsigned> cloud_mask;                          // the cloud mask (CloudView), only when set
+    std::shared_ptr<const CloudLayer> clouds;             // set while the scene has a cloud layer; shared by a replica
     DevBuf<uchar4> atlas, sky;
     SceneInfo info;
     ccu::DScene view{};   // every field that depends on the committed scene alone (commit, replicate_scene)
     ccu::EmitView emit_view{};   // the emitter table's launch view (fill_view, with `view`)
     ccu::EmitView memit_view{};  // the wider table's launch view (CCU_RENDER_EMITTER_MODELS)
     ccu::BiomeView biome_view{};  // the biome colours' launch view (CCU_RENDER_BIOME_TINT)
+    ccu::CloudView cloud_view{};  // the cloud layer's launch view (CCU_RENDER_CLOUDS)
 
     // Calls f(a's buffer, b's same buffer) for every device array of a scene (replicate_scene, ccu_scene_device_bytes).
     template <class F>
@@ -239,6 +253,7 @@ struct Scene {
         f(a.emit, b.emit); f(a.emit_off, b.emit_off); f(a.emit_list, b.emit_list);
         f(a.memit, b.memit); f(a.memit_off, b.memit_off); f(a.memit_list, b.memit_list); f(a.memit_head, b.memit_head);
         f(a.memit_prim, b.memit_prim); f(a.biome_grid, b.biome_grid); f(a.biome_tiles, b.biome_tiles);
+        f(a.cloud_mask, b.cloud_mask);
     }
 };
 
@@ -300,7 +315,7 @@ struct ccu_ctx {
     float last_ms = 0;
     bool timing_pending = false;
     int64_t launches = 0;
-    int32_t last_render[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // the last render launch's instance (ccu_debug_last_render_n)
+    int32_t last_render[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};   // the last render launch's instance (ccu_debug_last_render_n)
 };
 
 namespace ccu_host {

@@ -210,23 +210,59 @@ __device__ __forceinline__ bool closest_intersect_mode(const DScene &s, float3 o
     return closest_intersect_lean<MODE == 2, V, CUT>(s, origin, direction, rec, hi);
 }
 
+// DESIGN §15: whether a shadow, emitter-sample or fog ray that the octree and the BVHs let through is blocked by a cloud before
+// `extent` (unbounded, except for an emitter-sample ray: the distance of its target).  Always false without V::clouds.
+template <class V>
+__device__ __forceinline__ bool cloud_blocks(const CloudView &cv, float3 o, float3 d, float extent) {
+    if constexpr (V::clouds) {
+        float t;
+        float3 n;
+        return cloud_hit(cv, o, d, extent, t, n);
+    }
+    return false;
+}
+
+// closestIntersect of a path segment with the cloud layer (DESIGN §15.3): a cloud hit strictly nearer than the octree / BVH hit
+// (any, on a miss) replaces it by a white surface that emits nothing, hi.kind 4.
+template <int MODE, class V>
+__device__ __forceinline__ bool segment_intersect(const DScene &s, const CloudView &cv, float3 origin, float3 direction, RecordT<V::spec> &rec,
+                                                  HitInfo &hi) {
+    bool hit = closest_intersect_mode<MODE, V>(s, origin, direction, rec, hi);
+    float t;
+    float3 n;
+    if (cloud_hit(cv, origin, direction, hit ? rec.distance : inff_(), t, n)) {
+        rec.distance = t;
+        rec.material = 0;
+        rec.point = origin + direction * (t - CCU_OFFSET);
+        rec.surf.normal = n;
+        rec.surf.color = make_float4(1, 1, 1, 1);
+        rec.surf.emittance = 0;
+        surf_set_spec(rec.surf, 0u);
+        hi.node = -1;
+        hi.kind = 4;
+        hit = true;
+    }
+    return hit;
+}
+
 // The fog's sun sample at the end of a hit (DESIGN §14 step 3): the two draws, the sun direction as the surface sun sample
 // draws it, and a ray from the scattering point p without a limit; an escaped ray adds the pending weight w times the sky
 // (and sun disc) along it.  `rec` is a copy of the hit's record.
 template <int MODE, class V>
-__device__ __forceinline__ void fog_sun_sample(const DScene &s, uint32_t &rng, float3 p, float3 w, RecordT<V::spec> rec, float3 &color) {
+__device__ __forceinline__ void fog_sun_sample(const DScene &s, const CloudView &cv, uint32_t &rng, float3 p, float3 w, RecordT<V::spec> rec,
+                                               float3 &color) {
     const float x1 = rng_float(rng);
     const float x2 = rng_float(rng);
     const float3 d = sun_sample_direction(s, x1, x2);
     rec.distance = inff_();
     HitInfo hi;
-    if (!closest_intersect_mode<MODE, V>(s, p, d, rec, hi)) color = color + w * sky_radiance(s, d);
+    if (!closest_intersect_mode<MODE, V>(s, p, d, rec, hi) && !cloud_blocks<V>(cv, p, d, inff_())) color = color + w * sky_radiance(s, d);
 }
 
 // one path sample for pixel gid, thread-sequential: rayTracer.cl:40-107 (+ kernel.h:33-98, sky.h:68-93), with the specular events,
-// emitter sampler, biome colours and fog the Shade V switches on (DESIGN §5)
+// emitter sampler, biome colours, fog and clouds the Shade V switches on (DESIGN §5)
 template <int MODE, class V>
-__device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &g, int gid, int seed) {
+__device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &g, const CloudView &cv, int gid, int seed) {
     float3 color = f3(0, 0, 0), throughput = f3(1, 1, 1);
     int ray_depth = 0;
     uint32_t rng = (uint32_t)seed + (uint32_t)gid;
@@ -246,7 +282,10 @@ __device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &
     int3 nee_cell = make_int3(0, 0, 0);
     float3 fog_p = f3(0, 0, 0), fog_w = f3(0, 0, 0);   // fog: the hit's scattering point and its pending weight (DESIGN §14)
     for (;;) {
-        if (!closest_intersect_mode<MODE, V>(s, origin, direction, rec, hi)) {
+        bool hit;
+        if constexpr (V::clouds) hit = segment_intersect<MODE, V>(s, cv, origin, direction, rec, hi);
+        else hit = closest_intersect_mode<MODE, V>(s, origin, direction, rec, hi);
+        if (!hit) {
             // miss: emittance = 1, sky (+ sun disc) added through the throughput (rayTracer.cl:95-97, kernel.h:26-31)
             float3 sky = sky_radiance(s, direction);
             if constexpr (V::fog) {   // the sky blended towards the fog colour by elevation (§14.3)
@@ -287,7 +326,7 @@ __device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &
             const float x2 = rng_float(rng);
             direction = specular_direction(direction, rec.surf.normal, diffuse_direction(rec.surf.normal, x1, x2), ro);
             if constexpr (V::fog) {
-                if (s.sun_flags & 1) fog_sun_sample<MODE, V>(s, rng, fog_p, fog_w, rec, color);
+                if (s.sun_flags & 1) fog_sun_sample<MODE, V>(s, cv, rng, fog_p, fog_w, rec, color);
             }
             origin = rec.point + direction * CCU_OFFSET;
             ray_depth += 1;
@@ -308,7 +347,7 @@ __device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &
             float shadow_emittance = fabsf(dot3(d, rec.surf.normal));
             RecordT<V::spec> sh = rec;                // keeps the surface hit's distance as the ray limit (SURVEY Q4)
             HitInfo shi;
-            if (!closest_intersect_mode<MODE, V>(s, origin, d, sh, shi)) {
+            if (!closest_intersect_mode<MODE, V>(s, origin, d, sh, shi) && !cloud_blocks<V>(cv, origin, d, inff_())) {
                 float3 sky = sky_radiance(s, d);
                 color = color + (sky * throughput) * shadow_emittance;
             }
@@ -318,6 +357,9 @@ __device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &
             int3 cell;
             int n_list = 0, first = 0;
             if (ray_depth + 1 < s.max_depth && emitter_cell(g, origin, cell)) first = emitter_list(g, cell, n_list);
+            if constexpr (V::clouds) {
+                if (hi.kind == 4) n_list = 0;   // a cloud takes no emitter sample (DESIGN §15.4)
+            }
             if (n_list > 0) {
                 nee_prev = true;
                 nee_cell = cell;
@@ -327,7 +369,7 @@ __device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &
                     RecordT<V::spec> sh = rec;
                     sh.distance = limit;
                     HitInfo shi;
-                    if (!closest_intersect_mode<MODE, V, V::models>(s, origin, w, sh, shi)) color = color + c;
+                    if (!closest_intersect_mode<MODE, V, V::models>(s, origin, w, sh, shi) && !cloud_blocks<V>(cv, origin, w, limit)) color = color + c;
                 }
             }
         }
@@ -336,7 +378,7 @@ __device__ __forceinline__ float3 sample_pixel(const DScene &s, const EmitView &
         float x2 = rng_float(rng);
         direction = diffuse_direction(rec.surf.normal, x1, x2);
         if constexpr (V::fog) {
-            if (s.sun_flags & 1) fog_sun_sample<MODE, V>(s, rng, fog_p, fog_w, rec, color);
+            if (s.sun_flags & 1) fog_sun_sample<MODE, V>(s, cv, rng, fog_p, fog_w, rec, color);
         }
         origin = rec.point + direction * CCU_OFFSET;
         ray_depth += 1;

@@ -83,6 +83,7 @@ constexpr uint32_t QM_NEE_RAY = 1u << 27;    // NEE: the ray in flight is the em
 constexpr uint32_t QM_NEE_PREV = 1u << 28;   // NEE: the segment in flight left a hit that sampled the list of cell QF_SN*
 constexpr uint32_t QM_COVERED = 1u << 29;    // NEE + BVH: the closest hit so far is an emitter voxel that list covered
 constexpr uint32_t QM_FOG_RAY = 1u << 30;    // FOG: the ray in flight is the fog's sun sample (DESIGN §14); the bounce waits
+constexpr uint32_t QM_CLOUD = 1u << 31;      // CLOUDS: the surface the sun's shadow ray left is a cloud (DESIGN §15): no emitter sample
 // FOG kernels only (CCU_RENDER_FOG, DESIGN §14): 8 fields after all the others, q_fields(bvh, spec, nee) + 0 .. 7.  From a
 // path-segment hit to its bounce, + 0..2 hold the scattering point p and + 3..5 its weight W; while the fog ray flies, + 0..2
 // hold the origin of the bounce that follows it, and QF_SHW, + 6, + 7 its direction.
@@ -345,9 +346,10 @@ __device__ __forceinline__ void q_fog_hit(const DScene &s, uint32_t *F, int slot
     QFL(QF_THRX) = throughput.x; QFL(QF_THRY) = throughput.y; QFL(QF_THRZ) = throughput.z;
 }
 
+// CLOUDS (DESIGN §15): `cloud`: the path segment hit a cloud (q_resolve_clouds), which takes no emitter sample.
 template <bool HAS_BVH, class V>
 __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint32_t *F, unsigned *mask, int lane, int row, float3 o,
-                                        float3 d, float distance, bool ray_hit, const SurfT<V::spec> &hit, bool covered) {
+                                        float3 d, float distance, bool ray_hit, const SurfT<V::spec> &hit, bool covered, bool cloud) {
     constexpr int NFI = q_fields(HAS_BVH, V::spec);
     constexpr int FFI = q_fields(HAS_BVH, V::spec, V::nee);   // FOG: the first fog field
     const int slot = row * 32 + lane;
@@ -453,6 +455,10 @@ __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint
         else if (V::nee && !specular) nee_step = true;
         else bounce = true;
     }
+    if constexpr (V::clouds) {
+        // a cloud takes no emitter sample (DESIGN §15.4): at the hit, nor when the sun's shadow ray it sent returns
+        if (nee_step && (cloud || (shadow && (meta & QM_CLOUD)))) { nee_step = false; bounce = true; }
+    }
     if constexpr (V::nee) {
         if (nee_step) {
             // DESIGN §10: only where the bounce will be traced, and without a draw where L(cell) is empty
@@ -496,6 +502,9 @@ __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint
         next_d = sun_sample_direction_sc(s, x1, sn, cs);
         QFL(QF_SHW) = fabsf(dot3(next_d, normal));
         QU(QF_META) = meta | QM_SHADOW;
+        if constexpr (V::clouds) {
+            if (cloud) QU(QF_META) = meta | QM_SHADOW | QM_CLOUD;
+        }
         // the shadow ray starts at the surface point and inherits the surface hit's distance as its limit (SURVEY Q4)
         next_o = from;
         next_limit = distance;
@@ -506,6 +515,7 @@ __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint
         next_limit = inff_();
         const int ray_depth = (int)((meta >> 16) & 0xFF) + 1;
         meta = (meta & ~(0xFFu << 16) & ~QM_SHADOW) | ((uint32_t)ray_depth << 16);
+        if constexpr (V::clouds) meta &= ~QM_CLOUD;
         if constexpr (V::nee) {
             // the bounce segment carries the sampled cell for the emission rule at its hit
             meta &= ~(QM_NEE_RAY | QM_NEE_PREV);
@@ -545,6 +555,38 @@ __device__ __forceinline__ void q_shade(const DScene &s, const EmitView &g, uint
     }
 }
 
+// CLOUDS (DESIGN §15.3): the cloud layer on a ray whose octree / BVH result is known, then q_shade.  A path segment that meets a
+// cloud strictly before its octree / BVH hit (anywhere, on a miss) hits the cloud: a white surface that emits nothing.  A shadow
+// or fog ray that got through is blocked by a cloud anywhere along it, an emitter sample's ray by one before its limit.
+template <bool HAS_BVH, class V>
+__device__ __forceinline__ void q_resolve_clouds(const DScene &s, const EmitView &g, const CloudView &cv, uint32_t *F, unsigned *mask, int lane,
+                                                 int row, float3 o, float3 d, float distance, bool ray_hit, const SurfT<V::spec> &hit,
+                                                 bool covered) {
+    if constexpr (V::clouds) {
+        const int slot = row * 32 + lane;
+        const uint32_t meta = QU(QF_META);
+        SurfT<V::spec> h = hit;
+        bool cloud = false;
+        float t;
+        float3 n;
+        if (!(meta & (QM_SHADOW | QM_NEE_RAY | QM_FOG_RAY))) {
+            cloud = cloud_hit(cv, o, d, ray_hit ? distance : inff_(), t, n);
+            if (cloud) {
+                h.normal = n; h.color = make_float4(1, 1, 1, 1); h.emittance = 0;
+                surf_set_spec(h, 0u);
+                distance = t;
+                ray_hit = true;
+                covered = false;
+            }
+        } else if (!ray_hit) {
+            ray_hit = cloud_hit(cv, o, d, (meta & QM_NEE_RAY) ? distance : inff_(), t, n);
+        }
+        q_shade<HAS_BVH, V>(s, g, F, mask, lane, row, o, d, distance, ray_hit, h, covered, cloud);
+    } else {
+        q_shade<HAS_BVH, V>(s, g, F, mask, lane, row, o, d, distance, ray_hit, hit, covered, false);
+    }
+}
+
 // NEE: whether an octree hit on voxel c of block `data` is an emitter the sample of the previous hit covered (a path-segment
 // ray whose meta carries QM_NEE_PREV; the cell waits in QF_SN*)
 template <int NEE>
@@ -557,7 +599,7 @@ __device__ __forceinline__ bool q_covered(const DScene &s, const EmitView &g, co
 // BLOCK (kind_block = true) and EXIT (false): the octree part of closestIntersect (kernel.h:14-16) is finished here;
 // without BVHs the ray is shaded right away, with BVHs it goes to the BVH stage.  kind_block is warp-uniform.
 template <bool HAS_BVH, class V>
-__device__ __forceinline__ bool q_stage_resolve(const DScene &s, const EmitView &g, uint32_t *F, unsigned *mask, int lane, const bool kind_block,
+__device__ __forceinline__ bool q_stage_resolve(const DScene &s, const EmitView &g, const CloudView &cv, uint32_t *F, unsigned *mask, int lane, const bool kind_block,
                                                 int min_lanes) {
     const int row = q_pop_batch(mask, kind_block ? QS_BLOCK : QS_EXIT, lane, min_lanes);
     if (row == -2) return false;
@@ -619,14 +661,14 @@ __device__ __forceinline__ bool q_stage_resolve(const DScene &s, const EmitView 
         QI(QF_BSP) = phase << 8;
         q_push(mask, ref < 0 ? QS_LEAF : QS_BVH, lane, row);
     } else {
-        q_shade<HAS_BVH, V>(s, g, F, mask, lane, row, m.o, m.d, distance, ray_hit, hit, covered);
+        q_resolve_clouds<HAS_BVH, V>(s, g, cv, F, mask, lane, row, m.o, m.d, distance, ray_hit, hit, covered);
     }
     return true;
 }
 
 // SHADE (HAS_BVH kernels): closestIntersect is complete (kernel.h:17-22)
 template <class V>
-__device__ __forceinline__ bool q_stage_shade(const DScene &s, const EmitView &g, uint32_t *F, unsigned *mask, int lane, int min_lanes) {
+__device__ __forceinline__ bool q_stage_shade(const DScene &s, const EmitView &g, const CloudView &cv, uint32_t *F, unsigned *mask, int lane, int min_lanes) {
     const int row = q_pop_batch(mask, QS_SHADE, lane, min_lanes);
     if (row == -2) return false;
     QSTAT(22, 1); QSTAT(23, __popc(__ballot_sync(0xffffffffu, row >= 0)));
@@ -640,7 +682,7 @@ __device__ __forceinline__ bool q_stage_shade(const DScene &s, const EmitView &g
     hit.color = make_float4(QFL(QF_HCX), QFL(QF_HCY), QFL(QF_HCZ), 0.0f);
     hit.emittance = QFL(QF_HEM);
     if constexpr (V::spec) hit.spec = QU(QF_HSPEC);
-    q_shade<true, V>(s, g, F, mask, lane, row, o, d, QFL(QF_HDIST), ray_hit, hit, V::nee && (QU(QF_META) & QM_COVERED) != 0);
+    q_resolve_clouds<true, V>(s, g, cv, F, mask, lane, row, o, d, QFL(QF_HDIST), ray_hit, hit, V::nee && (QU(QF_META) & QM_COVERED) != 0);
     return true;
 }
 
@@ -996,11 +1038,13 @@ __device__ __forceinline__ bool q_stage_end(const DScene &s, const PassParams &w
 }
 
 // LAY 0: the top table of the air layout fits Q_TOP_WORDS and is staged in shared memory; 1: it is read from global memory;
-// 2: deep world (64-ary nodes between the top table and the bricks).  V: the launch's Shade.  The emitter table `g` and the biome
-// colours `bv` come after the other arguments, so that the kernels without them keep their parameter offsets.
+// 2: deep world (64-ary nodes between the top table and the bricks).  V: the launch's Shade.  The emitter table `g`, the biome
+// colours `bv` and the cloud layer `cv` come after the other arguments, so that the kernels without them keep their parameter
+// offsets.
 template <bool HAS_BVH, int LAY, class V>
 __global__ void __launch_bounds__(Q_WARPS * 32, 1) k_render_queue(const __grid_constant__ DScene s, const __grid_constant__ QueueParams qp,
-                                                                 const __grid_constant__ EmitView g, const __grid_constant__ BiomeView bv) {
+                                                                 const __grid_constant__ EmitView g, const __grid_constant__ BiomeView bv,
+                                                                 const __grid_constant__ CloudView cv) {
     constexpr int NST = q_stages(HAS_BVH);
     constexpr int MASK_WORDS = q_mask_words(HAS_BVH);
     extern __shared__ uint32_t q_mem[];
@@ -1080,11 +1124,11 @@ __global__ void __launch_bounds__(Q_WARPS * 32, 1) k_render_queue(const __grid_c
         switch (best) {
             case QS_MARCH: QSTAT(0, 1); q_stage_march<NST, LAY>(s, top, F, mask, lane, qp.yield_below, qp.refill_min); break;
             case QS_BLOCK:
-            case QS_EXIT: ran = q_stage_resolve<HAS_BVH, V>(s, g, F, mask, lane, best == QS_BLOCK, min_lanes); break;
+            case QS_EXIT: ran = q_stage_resolve<HAS_BVH, V>(s, g, cv, F, mask, lane, best == QS_BLOCK, min_lanes); break;
             case QS_END: ran = q_stage_end<!HAS_BVH>(s, qp.w, F, mask, live, lane, min_lanes); break;
             case QS_BVH: QSTAT(16, 1); if (HAS_BVH) q_stage_bvh<NST>(s, F, mask, stk, qp.bvh_deep, lane, qp.yield_below, qp.refill_min); break;
             case QS_LEAF: if (HAS_BVH) ran = q_stage_leaf<V>(s, F, mask, stk, qp.bvh_deep, lane, min_lanes); break;
-            default: if (HAS_BVH) ran = q_stage_shade<V>(s, g, F, mask, lane, min_lanes); break;
+            default: if (HAS_BVH) ran = q_stage_shade<V>(s, g, cv, F, mask, lane, min_lanes); break;
         }
         sticky = (ran && best != QS_MARCH && best != QS_BVH) ? best : -1;
         if (ran) {

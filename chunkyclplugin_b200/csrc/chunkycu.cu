@@ -340,6 +340,9 @@ void fill_view(ccu_host::Scene &sc) {
     BiomeView &bv = sc.biome_view;
     bv.grid = sc.biome_grid.p; bv.tiles = sc.biome_tiles.p;
     bv.x0 = in.biome_box[0]; bv.z0 = in.biome_box[1]; bv.gx = in.biome_box[2]; bv.gz = in.biome_box[3];
+    CloudView &cv = sc.cloud_view;
+    cv.mask = sc.cloud_mask.p;
+    cv.inv = in.cloud_inv; cv.y0 = in.cloud_y0; cv.y1 = in.cloud_y1; cv.u0 = in.cloud_u0; cv.v0 = in.cloud_v0;
 }
 
 // build_biome_layout with its failures as CCU_* codes; `what` names the entry point
@@ -448,7 +451,8 @@ void free_target(ccu_ctx *c) {
 //   sampler (NEE_NEAR) among them.  CCU_RENDER_EMITTER_MODELS picks the samplers of the wider table (NEE_*_MODELS, EmitView
 //   memit_view) when the scene has one; without a model emitter it changes nothing;
 // - CCU_RENDER_BIOME_TINT: the biome kernels, on a scene with biome colours;
-// - CCU_RENDER_FOG: the fog kernels, on a scene with fog (SceneInfo::has_fog).
+// - CCU_RENDER_FOG: the fog kernels, on a scene with fog (SceneInfo::has_fog);
+// - CCU_RENDER_CLOUDS: the cloud kernels, on a scene with a cloud mask that has a set cell (SceneInfo::has_clouds).
 ShadeKey shade_variant(const ccu_ctx *c) {
     const int f = c->params.flags;
     const auto &info = c->scene.info;
@@ -459,13 +463,15 @@ ShadeKey shade_variant(const ccu_ctx *c) {
         else if (info.has_emitters) nee = near_field ? NEE_NEAR : NEE_AREA;
     }
     return {(f & CCU_RENDER_SPECULAR) && info.has_specular, nee, (f & CCU_RENDER_BIOME_TINT) && info.has_biome,
-            (f & CCU_RENDER_FOG) && info.has_fog};
+            (f & CCU_RENDER_FOG) && info.has_fog, (f & CCU_RENDER_CLOUDS) && info.has_clouds};
 }
 
 // the wavefront kernel (ccu_queue.cuh) for the scene's entity BVHs, air layout (queue_layout) and the launch's Shade
 QueueFn queue_kernel(bool bvh, int lay, const ShadeKey &v) {
     QueueFn k = nullptr;
-    dispatch(bvh, [&](auto B) { dispatch<3>(lay, [&](auto L) { k = queue_kernel_of<B, L>(v); }); });
+    dispatch(bvh, [&](auto B) {
+        dispatch<3>(lay, [&](auto L) { k = v.clouds ? queue_kernel_of<B, L, true>(v) : queue_kernel_of<B, L, false>(v); });
+    });
     return k;
 }
 
@@ -554,12 +560,14 @@ int replicate_scene(ccu_ctx *src, ccu_ctx *dst) {
     b.info = SceneInfo();
     for (PackedArray &p : b.arrays) p.host.reset();
     b.biome.reset();
+    b.clouds.reset();
     int rc = CCU_OK;
     Scene::each_buf(a, b, [&](auto &x, auto &y) { if (rc == CCU_OK) rc = copy_buf(src, dst, x, y); });
     if (rc != CCU_OK) return rc;
     CU(cudaStreamSynchronize(dst->stream));
     for (int i = 0; i < N_ARRAYS; i++) b.arrays[i].host = a.arrays[i].host;
     b.biome = a.biome;
+    b.clouds = a.clouds;
     b.info = a.info;
     fill_view(b);
     dst->committed = true;
@@ -684,6 +692,8 @@ int ccu_scene_begin(ccu_ctx *c) {
     c->scene.biome_grid.release();
     c->scene.biome_tiles.release();
     c->scene.info.set_fog(0.0f, 0.0f, nullptr, 0);
+    c->scene.clouds.reset();
+    c->scene.cloud_mask.release();
     return CCU_OK;
 }
 
@@ -806,6 +816,35 @@ int ccu_scene_set_fog(ccu_ctx *c, float sigma, float sky_density, const float co
     return CCU_OK;
 }
 
+// Kept on the host, bit-packed, until commit uploads it.
+int ccu_scene_set_clouds(ccu_ctx *c, const uint8_t *mask, float size, float y0, float y1, float u0, float v0) {
+    if (!c) return fail(CCU_EINVAL, "ccu_scene_set_clouds: null context");
+    std::shared_ptr<ccu_host::CloudLayer> cl;
+    if (mask) {
+        if (!(size > 0.0f) || !std::isfinite(size)) return fail(CCU_EINVAL, "ccu_scene_set_clouds: size %g is not positive and finite", size);
+        if (!std::isfinite(y0) || !std::isfinite(y1) || !std::isfinite(u0) || !std::isfinite(v0))
+            return fail(CCU_EINVAL, "ccu_scene_set_clouds: y0 %g, y1 %g, u0 %g, v0 %g: each must be finite", y0, y1, u0, v0);
+        if (!(y0 < y1)) return fail(CCU_EINVAL, "ccu_scene_set_clouds: y0 %g is not below y1 %g", y0, y1);
+        try {
+            cl = std::make_shared<ccu_host::CloudLayer>();
+        } catch (const std::bad_alloc &) {
+            return fail(CCU_ENOMEM, "ccu_scene_set_clouds: no host memory for the mask");
+        }
+        for (int b = 0; b < ccu_host::CLOUD_CELLS; b++) {
+            if (mask[b]) {
+                cl->bits[b >> 5] |= 1u << (b & 31);
+                cl->any = true;
+            }
+        }
+        cl->inv = 1.0f / size;
+        cl->y0 = y0; cl->y1 = y1; cl->u0 = u0; cl->v0 = v0;
+    }
+    std::lock_guard<std::mutex> lk(c->mu);
+    c->committed = false;
+    c->scene.clouds = std::move(cl);
+    return CCU_OK;
+}
+
 // Builds the layouts and the launch view from the uploads.  The context stays uncommitted until every step has succeeded.
 int ccu_scene_commit(ccu_ctx *c) {
     if (!c) return fail(CCU_EINVAL, "ccu_scene_commit: null context");
@@ -914,6 +953,16 @@ int ccu_scene_commit(ccu_ctx *c) {
         CU(sc.biome_tiles.upload(reinterpret_cast<const float4 *>(bl.tiles.data()), bl.tiles.size() / 4, c->stream));
         in.has_biome = 1;
         in.biome_box[0] = bl.x0; in.biome_box[1] = bl.z0; in.biome_box[2] = bl.gx; in.biome_box[3] = bl.gz;
+    }
+    // cloud layer (CCU_RENDER_CLOUDS), only when set
+    in.has_clouds = 0;
+    in.cloud_inv = in.cloud_y0 = in.cloud_y1 = in.cloud_u0 = in.cloud_v0 = 0.0f;
+    sc.cloud_mask.release();
+    if (sc.clouds) {
+        const ccu_host::CloudLayer &cl = *sc.clouds;
+        CU(sc.cloud_mask.upload(cl.bits, ccu_host::CLOUD_WORDS, c->stream));
+        in.has_clouds = cl.any ? 1 : 0;
+        in.cloud_inv = cl.inv; in.cloud_y0 = cl.y0; in.cloud_y1 = cl.y1; in.cloud_u0 = cl.u0; in.cloud_v0 = cl.v0;
     }
     // sun basis, computed on the device
     {
@@ -1027,7 +1076,7 @@ int ccu_render_set_params(ccu_ctx *c, const ccu_render_params *p) {
     if (p->draw_depth < 0 || p->draw_depth >= (1 << 24) || p->max_depth < 1 || p->max_depth > 255) return fail(CCU_EINVAL, "bad render params");
     if (p->kernel != 0 && p->kernel != 1 && p->kernel != 4) return fail(CCU_EINVAL, "unknown kernel %d (0 auto, 1 thread-per-pixel, 4 wavefront)", p->kernel);
     if (p->flags & ~(CCU_RENDER_NO_ENTITIES | CCU_RENDER_NO_SUN | CCU_RENDER_SPECULAR | CCU_RENDER_EMITTER_SAMPLING | CCU_RENDER_EMITTER_NEAR_FIELD |
-                     CCU_RENDER_EMITTER_MODELS | CCU_RENDER_BIOME_TINT | CCU_RENDER_FOG))
+                     CCU_RENDER_EMITTER_MODELS | CCU_RENDER_BIOME_TINT | CCU_RENDER_FOG | CCU_RENDER_CLOUDS))
         return fail(CCU_EINVAL, "unknown render flags 0x%x", p->flags);
     if ((p->flags & CCU_RENDER_EMITTER_NEAR_FIELD) && !(p->flags & CCU_RENDER_EMITTER_SAMPLING))
         return fail(CCU_EINVAL, "CCU_RENDER_EMITTER_NEAR_FIELD needs CCU_RENDER_EMITTER_SAMPLING");
@@ -1075,6 +1124,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
     const ShadeKey shade = shade_variant(c);
     const EmitView &emit_view = nee_models(shade.nee) ? c->scene.memit_view : c->scene.emit_view;
     const BiomeView &biome_view = c->scene.biome_view;
+    const CloudView &cloud_view = c->scene.cloud_view;
     float *res = c->accum[c->accum_active].p;
     const float *res_prev = c->window_spp == 0 ? c->window_base : res;
     int kernel = c->params.kernel;
@@ -1084,7 +1134,7 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
         const int threads = 128, blocks = (n_pixels + threads - 1) / threads;
         dispatch<3>(mode, [&](auto M) {
             mega_kernel<M>(shade)<<<blocks, threads, 0, c->stream>>>(s, seeds_dev, n_passes, c->window_spp, res, res_prev, n_pixels,
-                                                                     emit_view, biome_view);
+                                                                     emit_view, biome_view, cloud_view);
         });
     } else {
         // persistent wavefront kernel (ccu_queue.cuh): one CTA per SM, pixels handed out through a counter
@@ -1123,12 +1173,14 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
             qp.bvh_deep = c->bvh_deep.p;
         }
         const int smem = base_smem + qp.sky_texels * 4;
-        queue_kernel(bvh, lay, shade)<<<grid, block, smem, c->stream>>>(s, qp, emit_view, biome_view);
+        queue_kernel(bvh, lay, shade)<<<grid, block, smem, c->stream>>>(s, qp, emit_view, biome_view, cloud_view);
 #ifdef CCU_Q_STATS
         {
             cudaStreamSynchronize(c->stream);
             unsigned long long st[32];
-            dispatch(bvh, [&](auto B) { dispatch<3>(lay, [&](auto L) { queue_stats_take<B, L>(st); }); });
+            dispatch(bvh, [&](auto B) {
+                dispatch<3>(lay, [&](auto L) { dispatch(shade.clouds, [&](auto C) { queue_stats_take<B, L, C>(st); }); });
+            });
             const char *names[4] = {"march", "block", "exit", "end"};
             fprintf(stderr, "[qstats] ");
             for (int i = 1; i < 4; i++) fprintf(stderr, "%s: %llu x %.1f lanes  ", names[i], st[2 * i], st[2 * i] ? (double)st[2 * i + 1] / st[2 * i] : 0.0);
@@ -1141,8 +1193,8 @@ static int render_passes_locked(ccu_ctx *c, const int32_t *seeds, int32_t n_pass
 #endif
     }
     c->launches++;
-    const int32_t last[8] = {kernel, bvh, kernel == 1 ? mode : lay, shade.spec, shade.nee, shade.biome, sky_staged, shade.fog};
-    std::copy(last, last + 8, c->last_render);
+    const int32_t last[9] = {kernel, bvh, kernel == 1 ? mode : lay, shade.spec, shade.nee, shade.biome, sky_staged, shade.fog, shade.clouds};
+    std::copy(last, last + 9, c->last_render);
     CU(cudaGetLastError());
     CU(cudaEventRecord(c->ev1, c->stream));
     CU(cudaEventRecord(ring.ev[slot], c->stream));
@@ -1429,7 +1481,7 @@ int ccu_debug_last_render(ccu_ctx *c, int32_t out[7]) {
 int ccu_debug_last_render_n(ccu_ctx *c, int32_t *out, int32_t n) {
     if (!c || !out || n < 0) return fail(CCU_EINVAL, "ccu_debug_last_render_n: null argument or negative n");
     std::lock_guard<std::mutex> lk(c->mu);
-    std::copy(c->last_render, c->last_render + std::min(n, 8), out);
+    std::copy(c->last_render, c->last_render + std::min(n, 9), out);
     return CCU_OK;
 }
 

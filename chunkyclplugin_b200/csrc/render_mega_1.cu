@@ -1,4 +1,4 @@
 // render_mega_1.cu - the k_render_mega<1, V> instances (ccu_mega.cuh), compiled in parallel with the rest of the library.
 #include "ccu_mega.cuh"
 
-template ccu::MegaFn ccu::mega_kernel<1>(const ccu::ShadeKey &);
+template ccu::MegaFn ccu::mega_kernel_of<1, false>(const ccu::ShadeKey &);

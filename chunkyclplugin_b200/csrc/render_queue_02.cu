@@ -1,7 +1,7 @@
 // render_queue_02.cu - the k_render_queue<false, 2, V> instances (ccu_queue_units.cuh), compiled in parallel with the rest of the library.
 #include "ccu_queue_units.cuh"
 
-template ccu::QueueFn ccu::queue_kernel_of<false, 2>(const ccu::ShadeKey &);
+template ccu::QueueFn ccu::queue_kernel_of<false, 2, false>(const ccu::ShadeKey &);
 #ifdef CCU_Q_STATS
-template void ccu::queue_stats_take<false, 2>(unsigned long long *);
+template void ccu::queue_stats_take<false, 2, false>(unsigned long long *);
 #endif

@@ -19,6 +19,7 @@ CCU_RENDER_EMITTER_NEAR_FIELD = 128
 CCU_RENDER_EMITTER_MODELS = 256
 CCU_RENDER_BIOME_TINT = 512
 CCU_RENDER_FOG = 1024
+CCU_RENDER_CLOUDS = 2048
 CCU_UNIQUE_ID_BYTES = 128
 
 CCU_OK, CCU_ENODEVICE, CCU_EINVAL, CCU_ECUDA, CCU_ENOMEM, CCU_ESTATE = 0, -1, -2, -3, -4, -5
@@ -57,6 +58,7 @@ SYMBOLS = {
     "ccu_scene_set_actor_bvh": (C.c_int, [_vp, _vp, _i64]),
     "ccu_scene_set_biome_colors": (C.c_int, [_vp, _vp, _vp, _i64]),
     "ccu_scene_set_fog": (C.c_int, [_vp, _f, _f, _vp, _i32]),
+    "ccu_scene_set_clouds": (C.c_int, [_vp, _vp, _f, _f, _f, _f, _f]),
     "ccu_scene_atlas_create": (C.c_int, [_vp, _i32, _i32, _i32]),
     "ccu_scene_atlas_write": (C.c_int, [_vp, _i32, _i32, _i32, _i32, _i32, _vp]),
     "ccu_scene_set_atlas": (C.c_int, [_vp, _vp, _i32, _i32, _i32]),
@@ -330,6 +332,17 @@ class Context:
             raise ValueError("the fog colour needs 3 components")
         check(self._lib.ccu_scene_set_fog(self._h, float(sigma), float(sky_density), _ptr(col), int(fast)))
 
+    def set_clouds(self, mask, size: float = 1.0, y0: float = 0.0, y1: float = 1.0, u0: float = 0.0, v0: float = 0.0):
+        """The scene's cloud layer for CCU_RENDER_CLOUDS (DESIGN.md §15): mask uint8[256, 256] indexed [k, i] (non-zero = cloud),
+        cell size, slab y0 < y1 and cell offsets, in the plugin's frame; mask None removes it."""
+        if mask is None:
+            check(self._lib.ccu_scene_set_clouds(self._h, None, float(size), float(y0), float(y1), float(u0), float(v0)))
+            return
+        m = np.ascontiguousarray(mask, np.uint8)
+        if m.size != 256 * 256:
+            raise ValueError("the cloud mask needs 256 x 256 cells")
+        check(self._lib.ccu_scene_set_clouds(self._h, _ptr(m), float(size), float(y0), float(y1), float(u0), float(v0)))
+
     def atlas_create(self, width: int, height: int, layers: int):
         check(self._lib.ccu_scene_atlas_create(self._h, width, height, layers))
 
@@ -482,11 +495,12 @@ class Context:
         check(self._lib.ccu_debug_last_render(self._h, _ptr(out)))
         return tuple(int(v) for v in out)
 
-    def last_render_n(self, n: int = 8) -> tuple:
-        """The first min(n, 8) entries of the last launch's instance: last_render()'s 7, then fog (ccu_debug_last_render_n)."""
+    def last_render_n(self, n: int = 9) -> tuple:
+        """The first min(n, 9) entries of the last launch's instance: last_render()'s 7, then fog and clouds
+        (ccu_debug_last_render_n)."""
         out = np.zeros(max(n, 0), np.int32)
         check(self._lib.ccu_debug_last_render_n(self._h, _ptr(out), n))
-        return tuple(int(v) for v in out[:min(n, 8)])
+        return tuple(int(v) for v in out[:min(n, 9)])
 
     def scene_device_bytes(self) -> int:
         n = C.c_int64()

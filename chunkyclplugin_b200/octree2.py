@@ -346,6 +346,13 @@ def to_scene(o: Octree2, width: int = 1920, height: int = 1080, camera=None, sun
     return p
 
 
+def scene_origin(d: dict) -> Tuple[int, int, int]:
+    """The world position of the octree origin in a parsed Chunky scene description: the low corner of the loaded chunk
+    rectangle in x and z, yMin in y (see camera_from_json).  The plugin's frame is world minus this."""
+    chunks = np.asarray(d["chunkList"], dtype=np.int64)
+    return int(chunks[:, 0].min()) * 16, int(d.get("yMin", 0)), int(chunks[:, 1].min()) * 16
+
+
 def camera_from_json(json_path: str) -> np.ndarray:
     """float[15] camera settings (ClCamera.java:39-52) from a Chunky scene description.
 
@@ -357,10 +364,9 @@ def camera_from_json(json_path: str) -> np.ndarray:
     import json
     import math
     d = json.loads(open(json_path, "rb").read().decode("latin-1"))
-    chunks = np.asarray(d["chunkList"], dtype=np.int64)
-    ox, oz = int(chunks[:, 0].min()) * 16, int(chunks[:, 1].min()) * 16
+    ox, oy, oz = scene_origin(d)
     cam = d["camera"]
-    pos = (cam["position"]["x"] - ox, cam["position"]["y"] - int(d.get("yMin", 0)), cam["position"]["z"] - oz)
+    pos = (cam["position"]["x"] - ox, cam["position"]["y"] - oy, cam["position"]["z"] - oz)
     yaw, pitch = cam["orientation"]["yaw"], cam["orientation"]["pitch"]
     return S.pinhole_camera(pos, 270.0 + math.degrees(yaw), -(90.0 + math.degrees(pitch)), float(cam.get("fov", 70.0)))
 
@@ -384,10 +390,46 @@ def fog_from_json(json_path: str) -> Tuple[float, float, Tuple[float, float, flo
             bool(d.get("fastFog", True)))
 
 
-def load_scene(octree_path: str, json_path: str = None, width: int = 1920, height: int = 1080) -> S.PackedScene:
-    """The scene of an .octree2 file, with the camera and fog of a Chunky scene description when one is given."""
+# The cloud layer's thickness in blocks.  chunky-core is not available here, so the value is unverified: Minecraft's fancy clouds
+# are 4 blocks thick, and that is what Chunky's layer is believed to be.
+CLOUD_THICKNESS = 4.0
+# How cloudOffset x / z move the cells: +1 = the mask cell of world point (x, z) is floor((x + offset.x) / cloudSize),
+# floor((z + offset.z) / cloudSize), and the layer starts at y = offset.y.  Like the thickness it is not checked against
+# chunky-core.
+CLOUD_OFFSET_SIGN = 1.0
+
+
+def clouds_from_json(json_path: str, mask) -> Optional[Tuple[np.ndarray, float, float, float, float, float]]:
+    """The cloud layer of a Chunky scene description as ccu_scene_set_clouds takes it (DESIGN.md §15): (mask, size, y0, y1, u0, v0)
+    in the plugin's frame (world minus the scene origin of camera_from_json), or None when sky.cloudsEnabled is false or missing.
+    `mask` is Minecraft's cloud texture as uint8[256, 256] indexed [k, i] (non-zero = cloud): it is not part of the scene
+    description.  The layer spans CLOUD_THICKNESS blocks from cloudOffset.y; cloudOffset x / z shift the cells by
+    CLOUD_OFFSET_SIGN."""
+    import json
+    d = json.loads(open(json_path, "rb").read().decode("latin-1"))
+    sky = d.get("sky", {})
+    if not sky.get("cloudsEnabled", False):
+        return None
+    m = np.ascontiguousarray(mask, np.uint8)
+    if m.shape != (256, 256):
+        raise ValueError("the cloud mask needs 256 x 256 cells")
+    ox, oy, oz = scene_origin(d)
+    size = float(sky.get("cloudSize", 64.0))
+    off = sky.get("cloudOffset", {})
+    y0 = float(off.get("y", 128.0)) - oy
+    u0 = (ox + CLOUD_OFFSET_SIGN * float(off.get("x", 0.0))) / size
+    v0 = (oz + CLOUD_OFFSET_SIGN * float(off.get("z", 0.0))) / size
+    return m, size, y0, y0 + CLOUD_THICKNESS, u0, v0
+
+
+def load_scene(octree_path: str, json_path: str = None, width: int = 1920, height: int = 1080,
+               cloud_mask=None) -> S.PackedScene:
+    """The scene of an .octree2 file, with the camera and fog of a Chunky scene description when one is given, and its clouds
+    when a cloud mask is given too (clouds_from_json)."""
     o = load(octree_path)
     p = to_scene(o, width, height, camera=camera_from_json(json_path) if json_path else None)
     if json_path:
         p.fog = fog_from_json(json_path)
+        if cloud_mask is not None:
+            p.clouds = clouds_from_json(json_path, cloud_mask)
     return p

@@ -115,7 +115,7 @@ class RendererInstance:
 # ----------------------------------------------------------------------------------------------------
 def upload_scene(ctx, p) -> None:
     """Upload and commit a PackedScene through the C ABI in the order of the reference's loader (AbstractSceneLoader.java:60-162),
-    with its biome colours and fog when it has them."""
+    with its biome colours, fog and clouds when it has them."""
     ctx.scene_begin()
     ctx.set_atlas(p.atlas)                      # ClTextureLoader.buildTextures
     ctx.set_block_palette(p.block_palette)
@@ -131,6 +131,8 @@ def upload_scene(ctx, p) -> None:
         ctx.set_biome_colors(*p.biome)          # CCU_RENDER_BIOME_TINT's colours (beyond the reference)
     if p.fog is not None:
         ctx.set_fog(*p.fog)                     # CCU_RENDER_FOG's fog (beyond the reference)
+    if p.clouds is not None:
+        ctx.set_clouds(*p.clouds)               # CCU_RENDER_CLOUDS's cloud layer (beyond the reference)
     ctx.set_octree(p.octree, p.octree_depth)    # loadOctree, ClSceneLoader.java:52-63
     ctx.scene_commit()
 

@@ -72,6 +72,9 @@ class PackedScene:
     biome: Optional[Tuple[np.ndarray, np.ndarray]] = None
     # fog for CCU_RENDER_FOG: (sigma, sky density, (r, g, b), fast) as ccu_scene_set_fog takes them (DESIGN.md §14), or None
     fog: Optional[Tuple[float, float, Tuple[float, float, float], bool]] = None
+    # cloud layer for CCU_RENDER_CLOUDS: (mask uint8[256, 256] indexed [k, i], size, y0, y1, u0, v0) as ccu_scene_set_clouds takes
+    # them (DESIGN.md §15), or None
+    clouds: Optional[Tuple[np.ndarray, float, float, float, float, float]] = None
 
     def arrays(self) -> Dict[str, np.ndarray]:
         return {k: getattr(self, k) for k in (
@@ -973,3 +976,24 @@ def water_tinted(p: PackedScene) -> PackedScene:
     for m in mats[::2]:
         mp[m + 1] = 3 << 24
     return dataclasses.replace(p, mat_palette=mp, name=p.name + "_water")
+
+
+# --------------------------------------------------------------------------------------
+# cloud layer (CCU_RENDER_CLOUDS, DESIGN.md §15)
+# --------------------------------------------------------------------------------------
+def cloud_mask(seed: int = 1, cover: float = 0.5) -> np.ndarray:
+    """uint8[256, 256] (indexed [k, i]): cell (i, k) is set where a hash of the cell falls below `cover`."""
+    k, i = np.meshgrid(np.arange(256), np.arange(256), indexing="ij")
+    h = hash_u32(i.reshape(-1), k.reshape(-1), seed, 11).astype(np.float64) / 2.0 ** 32
+    return (h < cover).astype(np.uint8).reshape(256, 256)
+
+
+def with_clouds(p: PackedScene, mask: np.ndarray, size: float = 4.0, y0: float = None, y1: float = None, u0: float = 0.0,
+                v0: float = 0.0) -> PackedScene:
+    """p with a cloud layer of `mask` (uint8[256, 256] indexed [k, i]), cells of `size` blocks; the slab defaults to
+    [3/4, 7/8] of the octree's height."""
+    h = float(1 << p.octree_depth)
+    y0 = 0.75 * h if y0 is None else y0
+    y1 = 0.875 * h if y1 is None else y1
+    m = np.ascontiguousarray(mask, np.uint8).reshape(256, 256)
+    return dataclasses.replace(p, clouds=(m, float(size), float(y0), float(y1), float(u0), float(v0)), name=p.name + "_clouds")

@@ -98,6 +98,13 @@ typedef struct ccu_render_params {
  * colour by elevation.  Shadow and emitter-sample rays see neither.  A scene without fog renders exactly as without the flag.
  * Valid alone and with every other flag; both render kernels implement it.  DESIGN.md §14 holds the exact contract. */
 #define CCU_RENDER_FOG 1024
+/* Clouds (beyond the reference; Chunky's flat cloud layer): on a scene with a cloud layer (ccu_scene_set_clouds, a mask with a set
+ * cell), every ray the render kernels trace also meets the cloud boxes: a path segment that enters one before its octree / BVH hit
+ * hits a white diffuse surface that emits nothing, takes the sun sample and the diffuse bounce and no specular event or emitter
+ * sample; sun shadow rays, emitter-sample rays and fog rays that meet a cloud are blocked, so clouds cast shadows.  A scene
+ * without clouds renders exactly as without the flag.  First hit and preview do not see clouds.  Valid alone and with every
+ * other flag; both render kernels implement it.  DESIGN.md §15 holds the exact contract. */
+#define CCU_RENDER_CLOUDS 2048
 
 /* ---- device enumeration: RendererInstance.java:39-75,123-157 (clGetPlatformIDs/clGetDeviceIDs/clGetDeviceInfo),
  *      used by the GPU selector UI (ui/GpuSelector.java:24-87) -------------------------------------------------- */
@@ -136,6 +143,14 @@ int ccu_scene_set_biome_colors(ccu_ctx *ctx, const int32_t *chunks, const float 
  * "fast fog" switch (0 or 1).  CCU_EINVAL otherwise.  Like the sun it belongs to the scene: ccu_scene_begin removes it, and it
  * takes effect at the next ccu_scene_commit (ccu_group_replicate_scene carries it). */
 int ccu_scene_set_fog(ccu_ctx *ctx, float sigma, float sky_density, const float color[3], int32_t fast);
+/* Cloud layer for CCU_RENDER_CLOUDS (optional; beyond the reference).  mask = 256 x 256 bytes, non-zero = cloud; cell (i, k) is
+ * mask[(k & 255) * 256 + (i & 255)].  A point (x, y, z) of the plugin's frame (world minus scene origin, as for camera rays) is in a
+ * cloud when y0 <= y <= y1 and cell (floor(x / size + u0), floor(z / size + v0)) is set (1 / size is computed once, in fp32).
+ * CCU_EINVAL for a size that is not positive and finite, a y0, y1, u0 or v0 that is not finite, or y0 >= y1; mask = NULL removes
+ * the clouds (the other arguments are then ignored).  Like the fog it belongs to the scene: ccu_scene_begin removes it, and it
+ * takes effect at the next ccu_scene_commit (ccu_group_replicate_scene carries it).  The committed scene holds the mask
+ * bit-packed (8 KiB, counted by ccu_scene_device_bytes). */
+int ccu_scene_set_clouds(ccu_ctx *ctx, const uint8_t *mask, float size, float y0, float y1, float u0, float v0);
 /* texture atlas: ClTextureLoader.java:46-66 - clCreateImage(8192x8192xlayers RGBA8) then one clEnqueueWriteImage
  * per texture at (16*tileX, 16*tileY, layer) */
 int ccu_scene_atlas_create(ccu_ctx *ctx, int32_t width, int32_t height, int32_t layers);
@@ -212,7 +227,7 @@ int ccu_launch_count(ccu_ctx *ctx, int64_t *launches);    /* kernels launched by
  * LAY is the one the launch ran (a fog launch may move from LAY 0 to LAY 1, DESIGN.md §5).
  * DESIGN.md §5.  A launch refused with an error leaves it as it was. */
 int ccu_debug_last_render(ccu_ctx *ctx, int32_t out[7]);
-/* The same report with the switches added since: writes the first min(n, 8) of {the 7 entries above, fog}. */
+/* The same report with the switches added since: writes the first min(n, 9) of {the 7 entries above, fog, clouds}. */
 int ccu_debug_last_render_n(ccu_ctx *ctx, int32_t *out, int32_t n);
 int ccu_scene_device_bytes(ccu_ctx *ctx, int64_t *bytes); /* HBM held by the committed scene */
 int ccu_scene_commit_ms(ccu_ctx *ctx, double *ms);        /* host time the last ccu_scene_commit spent building + uploading the layouts */

@@ -41,6 +41,7 @@ public final class ChunkyCu {
     private static final MethodHandle SET_ACTOR_BVH = h("ccu_scene_set_actor_bvh", WORDS);
     private static final MethodHandle SET_BIOME_COLORS = h("ccu_scene_set_biome_colors", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG));
     private static final MethodHandle SET_FOG = h("ccu_scene_set_fog", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_FLOAT, JAVA_FLOAT, ADDRESS, JAVA_INT));
+    private static final MethodHandle SET_CLOUDS = h("ccu_scene_set_clouds", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_FLOAT, JAVA_FLOAT, JAVA_FLOAT, JAVA_FLOAT, JAVA_FLOAT));
     private static final MethodHandle DEBUG_BIOME_LAYOUT = h("ccu_debug_biome_layout", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, JAVA_INT, ADDRESS, ADDRESS, ADDRESS));
     private static final MethodHandle ATLAS_CREATE = h("ccu_scene_atlas_create", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT, JAVA_INT, JAVA_INT));
     private static final MethodHandle ATLAS_WRITE = h("ccu_scene_atlas_write", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, JAVA_INT, ADDRESS));
@@ -90,6 +91,8 @@ public final class ChunkyCu {
     public static final int RENDER_BIOME_TINT = 512;
     /** ccu_render_params.flags: the scene's fog of {@link Context#setFog}, with sunlit light shafts (DESIGN §14). */
     public static final int RENDER_FOG = 1024;
+    /** ccu_render_params.flags: the scene's cloud layer of {@link Context#setClouds}, which also shadows the scene (DESIGN §15). */
+    public static final int RENDER_CLOUDS = 2048;
     private static final StructLayout RENDER_PARAMS = MemoryLayout.structLayout(JAVA_INT.withName("draw_depth"), JAVA_INT.withName("max_depth"),
             JAVA_FLOAT.withName("emitter_scale"), JAVA_INT.withName("kernel"), JAVA_INT.withName("flags"));
 
@@ -207,6 +210,15 @@ public final class ChunkyCu {
             if (color.length != 3) throw new IllegalArgumentException("the fog colour needs 3 components");
             try (Arena a = Arena.ofConfined()) {
                 check(call(SET_FOG, handle, sigma, skyDensity, a.allocateFrom(JAVA_FLOAT, color), fast ? 1 : 0));
+            }
+        }
+        /** The scene's cloud layer: mask = 256 x 256 bytes (cell (i, k) at (k &amp; 255) * 256 + (i &amp; 255), non-zero = cloud; null removes
+         *  the layer), cell size, the slab y0 &lt; y1 and the cell offsets u0, v0, in the plugin's frame (DESIGN §15). */
+        public void setClouds(byte[] mask, float size, float y0, float y1, float u0, float v0) {
+            if (mask != null && mask.length != 256 * 256) throw new IllegalArgumentException("the cloud mask needs 256 x 256 cells");
+            try (Arena a = Arena.ofConfined()) {
+                MemorySegment m = mask != null ? a.allocateFrom(JAVA_BYTE, mask) : MemorySegment.NULL;
+                check(call(SET_CLOUDS, handle, m, size, y0, y1, u0, v0));
             }
         }
         public void atlasCreate(int width, int height, int layers) { check(call(ATLAS_CREATE, handle, width, height, layers)); }

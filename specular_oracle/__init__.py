@@ -1,5 +1,6 @@
 """ctypes binding of the CPU restatement of CCU_RENDER_SPECULAR, CCU_RENDER_EMITTER_SAMPLING, CCU_RENDER_EMITTER_NEAR_FIELD,
-CCU_RENDER_EMITTER_MODELS and CCU_RENDER_BIOME_TINT (specular_oracle.c).  TEST INFRASTRUCTURE ONLY.
+CCU_RENDER_EMITTER_MODELS, CCU_RENDER_BIOME_TINT, CCU_RENDER_FOG and CCU_RENDER_CLOUDS (specular_oracle.c).  TEST INFRASTRUCTURE
+ONLY.
 
 ``SpecularOracle`` is the parity oracle (``oracle.Oracle``) with the specular events of DESIGN.md section 9 in its path
 loop; ``FlagsOracle`` takes the render flags and adds the emitter sampling of sections 10 to 12, with the emitter table that
@@ -38,6 +39,7 @@ def lib():
         assert _lib.emitter_grid_struct_size() == C.sizeof(_Grid), "EmitterGrid layout mismatch"
         assert _lib.biome_tiles_struct_size() == C.sizeof(_Biome), "BiomeTiles layout mismatch"
         assert _lib.fog_params_struct_size() == C.sizeof(_Fog), "FogParams layout mismatch"
+        assert _lib.cloud_layer_struct_size() == C.sizeof(_Clouds), "CloudLayer layout mismatch"
         _lib.fog_expf_test.restype = C.c_float
         _lib.fog_expf_test.argtypes = [C.c_float]
     return _lib
@@ -50,6 +52,43 @@ class _Grid(C.Structure):
 
 class _Fog(C.Structure):
     _fields_ = [("sigma", C.c_float), ("sky", C.c_float), ("color", C.c_float * 3), ("fast", C.c_int32)]
+
+
+class _Clouds(C.Structure):
+    _fields_ = [("bits", C.c_void_p), ("inv", C.c_float), ("y0", C.c_float), ("y1", C.c_float), ("u0", C.c_float),
+                ("v0", C.c_float)]
+
+
+def cloud_bits(mask) -> np.ndarray:
+    """The mask uint8[256, 256] (indexed [k, i]) bit-packed as the library holds it: uint32[2048], cell (i, k) at bit
+    (k & 255) * 256 + (i & 255)."""
+    m = np.ascontiguousarray(mask, np.uint8).reshape(-1) != 0
+    return np.packbits(m, bitorder="little").view("<u4").astype(np.uint32)
+
+
+def _cloud_layer(clouds, keep: dict) -> "_Clouds":
+    mask, size, y0, y1, u0, v0 = clouds
+    bits = cloud_bits(mask)
+    keep["cloud_bits"] = bits
+    inv = np.float32(1.0) / np.float32(size)    # ccu_scene_set_clouds: 1.0f / size
+    return _Clouds(bits.ctypes.data, float(inv), float(np.float32(y0)), float(np.float32(y1)), float(np.float32(u0)),
+                   float(np.float32(v0)))
+
+
+def cloud_hit(clouds, o, d, limit=None):
+    """DESIGN.md section 15.2 for N rays (o, d float32[N, 3], limit float32[N], default unbounded) against the cloud layer
+    clouds = (mask, size, y0, y1, u0, v0): (t float32[N], NaN for a miss; normal float32[N, 3]; cells the walk tested int32[N])."""
+    keep = {}
+    cl = _cloud_layer(clouds, keep)
+    o = np.ascontiguousarray(o, np.float32).reshape(-1, 3)
+    d = np.ascontiguousarray(d, np.float32).reshape(-1, 3)
+    n = o.shape[0]
+    lim = np.full(n, np.inf, np.float32) if limit is None else np.ascontiguousarray(np.broadcast_to(limit, (n,)), np.float32)
+    out = np.zeros((n, 4), np.float32)
+    visited = np.zeros(n, np.int32)
+    lib().cloud_hit_batch(C.byref(cl), C.c_int64(n), o.ctypes.data_as(C.c_void_p), d.ctypes.data_as(C.c_void_p),
+                          lim.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p), visited.ctypes.data_as(C.c_void_p))
+    return out[:, 0], out[:, 1:], visited
 
 
 def dm_expf(x: float) -> float:
@@ -65,6 +104,7 @@ class _Biome(C.Structure):
 CCU_RENDER_SPECULAR, CCU_RENDER_EMITTER_SAMPLING, CCU_RENDER_EMITTER_NEAR_FIELD, CCU_RENDER_EMITTER_MODELS = 4, 8, 128, 256
 CCU_RENDER_BIOME_TINT = 512
 CCU_RENDER_FOG = 1024
+CCU_RENDER_CLOUDS = 2048
 EMIT_SHIFT0, EMIT_CELL_BUDGET, EMIT_MAX = 3, 1 << 21, 1 << 18      # DESIGN.md section 10
 
 
@@ -259,11 +299,18 @@ class FlagsOracle(oracle.Oracle):
     of section 12 is sampled when the scene has one, else the table of section 10.  With CCU_RENDER_BIOME_TINT the biome
     colours are `biome` = (chunks, rgb) as ccu_scene_set_biome_colors takes them, by default the scene's own (scene.biome).
     With CCU_RENDER_FOG the fog of section 14 is `fog` = (sigma, sky density, colour, fast) as ccu_scene_set_fog takes it,
-    by default the scene's own (scene.fog); sigma = 0 is no fog."""
+    by default the scene's own (scene.fog); sigma = 0 is no fog.  With CCU_RENDER_CLOUDS the cloud layer of section 15 is `clouds`
+    = (mask, size, y0, y1, u0, v0) as ccu_scene_set_clouds takes it, by default the scene's own (scene.clouds); a mask without a
+    set cell is no cloud layer."""
 
-    def __init__(self, scene, flags: int = 0, biome=None, fog=None, **kw):
+    def __init__(self, scene, flags: int = 0, biome=None, fog=None, clouds=None, **kw):
         super().__init__(scene, **kw)
         self.flags = flags
+        if clouds is None:
+            clouds = getattr(scene, "clouds", None)
+        self._clouds = None
+        if flags & CCU_RENDER_CLOUDS and clouds is not None and np.asarray(clouds[0]).any():
+            self._clouds = _cloud_layer(clouds, self._keep)
         if fog is None:
             fog = getattr(scene, "fog", None)
         self._fog = None
@@ -310,6 +357,7 @@ class FlagsOracle(oracle.Oracle):
                            C.c_int(1 if self.flags & CCU_RENDER_SPECULAR else 0), C.byref(self._grid) if nee else None,
                            C.c_int(1 if self.flags & CCU_RENDER_EMITTER_NEAR_FIELD else 0),
                            C.byref(self._biome) if self._biome is not None else None,
-                           C.byref(self._fog) if self._fog is not None else None)
+                           C.byref(self._fog) if self._fog is not None else None,
+                           C.byref(self._clouds) if self._clouds is not None else None)
         self._counters(cnt)
         return res

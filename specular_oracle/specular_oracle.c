@@ -15,7 +15,8 @@
  * both flags; the emitter table it samples is built by the Python side of this package from the packed arrays.
  * CCU_RENDER_BIOME_TINT (section 13) restates the material evaluation with the biome colours of the hit voxel's column; the
  * block test, the octree march and the emitter samplers pass that voxel on.  CCU_RENDER_FOG (section 14) restates the fog of
- * the path loop.
+ * the path loop.  CCU_RENDER_CLOUDS (section 15) restates the cloud walk and where the path loop, the shadow rays, the emitter
+ * sample's ray and the fog's sun sample meet it.
  */
 #include "../oracle/chunky_oracle.c"
 
@@ -532,6 +533,98 @@ static int nee_sample(const Ctx *c, const EmitterGrid *g, int near, int b, int n
     return 1;
 }
 
+/* ---- clouds (DESIGN.md section 15) ---- */
+#define CLOUD_CELLS 1024            /* section 15.2: the walk visits at most this many cells, then reports a miss */
+#define CLOUD_COORD_MAX 8388608.0f  /* section 15.2: 2^23, the walk reports a miss where a cell coordinate reaches it */
+
+typedef struct {
+    const uint32_t *bits;   /* 256 x 256 bits, cell (i, k) at bit (k & 255) * 256 + (i & 255) */
+    float inv, y0, y1, u0, v0;
+} CloudLayer;
+
+/* the ray's parameter interval in cell c of one cell axis; d = 0: the whole line */
+static void cloud_axis(float o, float d, int c, float *lo, float *hi) {
+    if (d == 0.0f) { *lo = -HUGE_VALF; *hi = HUGE_VALF; return; }
+    float a = ((float)c - o) / d, b = ((float)(c + 1) - o) / d;
+    *lo = d > 0.0f ? a : b;
+    *hi = d > 0.0f ? b : a;
+}
+
+/* the walk's first cell on one axis: the cell whose interval holds ts, or the one before it; 0 for a miss */
+static int cloud_start(float o, float d, float ts, int *c, int *step) {
+    if (d == 0.0f) {
+        float f = floorf(o);
+        if (!(o > f) || !(fabsf(o) < CLOUD_COORD_MAX)) return 0;
+        *c = (int)f;
+        *step = 0;
+        return 1;
+    }
+    float x = o + d * ts;
+    if (!(fabsf(x) < CLOUD_COORD_MAX)) return 0;
+    *c = (int)floorf(x);
+    *step = d > 0.0f ? 1 : -1;
+    float lo, hi;
+    cloud_axis(o, d, *c, &lo, &hi);
+    if (lo > ts) *c -= *step;
+    return 1;
+}
+
+/* section 15.2: the smallest t > 0 below limit at which o + d t enters the (open) box of a set cell; n = the outward normal of
+ * the face entered (ties: y, then x, then z).  visited (may be NULL): the cells the walk tested. */
+static int cloud_hit(const CloudLayer *cl, v3 o, v3 d, float limit, float *t, v3 *n, int *visited) {
+    float ylo, yhi;
+    if (visited) *visited = 0;
+    if (d.y == 0.0f) {
+        if (!(cl->y0 < o.y && o.y < cl->y1)) return 0;
+        ylo = -HUGE_VALF;
+        yhi = HUGE_VALF;
+    } else {
+        float a = (cl->y0 - o.y) / d.y, b = (cl->y1 - o.y) / d.y;
+        if (!(a == a && b == b)) return 0;
+        ylo = d.y > 0.0f ? a : b;
+        yhi = d.y > 0.0f ? b : a;
+    }
+    float tend = yhi < limit ? yhi : limit;
+    float ts = ylo > 0.0f ? ylo : 0.0f;
+    if (!(ts < tend)) return 0;
+    float ox = o.x * cl->inv + cl->u0, dx = d.x * cl->inv;
+    float oz = o.z * cl->inv + cl->v0, dz = d.z * cl->inv;
+    int i, k, si, sk;
+    if (!cloud_start(ox, dx, ts, &i, &si) || !cloud_start(oz, dz, ts, &k, &sk)) return 0;
+    for (int step = 0; step < CLOUD_CELLS; step++) {
+        float xlo, xhi, zlo, zhi;
+        if (visited) *visited = step + 1;
+        cloud_axis(ox, dx, i, &xlo, &xhi);
+        cloud_axis(oz, dz, k, &zlo, &zhi);
+        uint32_t bit = ((uint32_t)(k & 255) << 8) | (uint32_t)(i & 255);
+        if ((cl->bits[bit >> 5] >> (bit & 31u)) & 1u) {
+            float tn = ylo;
+            int axis = 1;
+            if (xlo > tn) { tn = xlo; axis = 0; }
+            if (zlo > tn) { tn = zlo; axis = 2; }
+            float tf = yhi < xhi ? yhi : xhi;
+            tf = tf < zhi ? tf : zhi;
+            if (tn > 0.0f && tn < tf && tn < limit) {
+                *t = tn;
+                *n = axis == 0 ? V(dx > 0.0f ? -1.0f : 1.0f, 0, 0) : (axis == 1 ? V(0, d.y > 0.0f ? -1.0f : 1.0f, 0) : V(0, 0, dz > 0.0f ? -1.0f : 1.0f));
+                return 1;
+            }
+        }
+        float te = xhi < zhi ? xhi : zhi;
+        if (!(te < tend)) return 0;
+        if (xhi == te) i += si;
+        if (zhi == te) k += sk;
+    }
+    return 0;
+}
+
+/* section 15.3: a shadow, emitter-sample or fog ray that got through is blocked by a cloud before extent; 0 without clouds */
+static int cloud_blocks(const CloudLayer *cl, v3 o, v3 d, float extent) {
+    float t;
+    v3 n;
+    return cl && cloud_hit(cl, o, d, extent, &t, &n, NULL);
+}
+
 /* ---- fog (DESIGN.md section 14) ---- */
 typedef struct {
     float sigma, sky, color[3];
@@ -577,21 +670,23 @@ static void fog_intersect_sky(const Ctx *c, const FogParams *fog, Path *p, Recor
 }
 
 /* section 14.2 step 3: the sun sample from the scattering point x, traced without a limit; w = the pending weight */
-static void fog_sun_sample(const Ctx *c, v3 x, v3 w, const Record *rec, uint32_t *state, Path *p) {
+static void fog_sun_sample(const Ctx *c, const CloudLayer *cl, v3 x, v3 w, const Record *rec, uint32_t *state, Path *p) {
     Path q = *p;
     Record r = *rec;
     q.origin = x;
     if (!sun_sample_direction(c, &q, &r, state)) return;
     r.distance = HUGE_VALF;
     if (closest_intersect(c, &q, &r)) return;
+    if (cloud_blocks(cl, q.origin, q.direction, HUGE_VALF)) return;
     sky_intersect(c, q.direction, &r);
     sun_intersect(c, q.direction, &r);
     p->pix_color = vadd(p->pix_color, vmul(w, V(r.color[0], r.color[1], r.color[2])));
 }
 
-/* one path sample: rayTracer.cl:40-107 with the specular events (spec), emitter sampling (g != NULL; near: section 11) and
- * fog (fog != NULL, section 14) */
-static v3 sample_pixel_ext(const Ctx *c, int gid, int32_t seed, int spec, const EmitterGrid *g, int near, const FogParams *fog) {
+/* one path sample: rayTracer.cl:40-107 with the specular events (spec), emitter sampling (g != NULL; near: section 11), fog
+ * (fog != NULL, section 14) and clouds (cl != NULL, section 15) */
+static v3 sample_pixel_ext(const Ctx *c, int gid, int32_t seed, int spec, const EmitterGrid *g, int near, const FogParams *fog,
+                           const CloudLayer *cl) {
     Path p;
     Record rec;
     uint32_t w5 = 0;
@@ -609,7 +704,26 @@ static v3 sample_pixel_ext(const Ctx *c, int gid, int32_t seed, int spec, const 
     const int fog_sun = fog && (c->sun.flags & 1);
     for (;;) {
         c->cnt->segments++;
-        if (!closest_intersect_w5(c, &p, &rec, &w5, vox, 0)) {
+        int hit = closest_intersect_w5(c, &p, &rec, &w5, vox, 0);
+        int cloud = 0;   /* section 15.3: the segment hit a cloud */
+        if (cl) {
+            float t;
+            v3 n;
+            cloud = cloud_hit(cl, p.origin, p.direction, hit ? rec.distance : HUGE_VALF, &t, &n, NULL);
+            if (cloud) {
+                rec.distance = t;
+                rec.material = 0;
+                rec.point = vadd(p.origin, vscale(p.direction, t - OFFSET));
+                rec.normal = n;
+                rec.color[0] = rec.color[1] = rec.color[2] = rec.color[3] = 1.0f;
+                rec.emittance = 0;
+                rec.hit_kind = 4;
+                rec.hit_node = -1;
+                w5 = 0;
+                hit = 1;
+            }
+        }
+        if (!hit) {
             rec.emittance = 1;
             if (fog) fog_intersect_sky(c, fog, &p, &rec);
             else intersect_sky(c, &p, &rec);
@@ -634,7 +748,7 @@ static v3 sample_pixel_ext(const Ctx *c, int gid, int32_t seed, int spec, const 
         }
         int more;
         if (spec && specular_event(c, &p, &rec, w5, &state, &more, emits)) {
-            if (fog_sun) fog_sun_sample(c, fog_p, fog_w, &rec, &state, &p);
+            if (fog_sun) fog_sun_sample(c, cl, fog_p, fog_w, &rec, &state, &p);
             if (!more) break;
             continue;
         }
@@ -647,10 +761,11 @@ static v3 sample_pixel_ext(const Ctx *c, int gid, int32_t seed, int spec, const 
         if (sun_sample_direction(c, &p, &rec, &state)) {
             Record s = rec; /* IntersectionRecord_copy keeps distance: SURVEY Q4 */
             s.point = rec.normal;
-            if (!closest_intersect(c, &p, &s)) intersect_sky(c, &p, &s);   /* the shadow ray needs no word 5 */
+            /* the shadow ray needs no word 5 */
+            if (!closest_intersect(c, &p, &s) && !cloud_blocks(cl, p.origin, p.direction, HUGE_VALF)) intersect_sky(c, &p, &s);
         }
         int cell[3];
-        if (g && p.ray_depth + 1 < c->sc->max_depth && point_cell(g, p.origin, cell)) {
+        if (g && !cloud && p.ray_depth + 1 < c->sc->max_depth && point_cell(g, p.origin, cell)) {
             int ci = (cell[0] * g->dim[1] + cell[1]) * g->dim[2] + cell[2];
             int b = g->off[ci], n = g->off[ci + 1] - b;
             if (n > 0) {
@@ -666,15 +781,16 @@ static v3 sample_pixel_ext(const Ctx *c, int gid, int32_t seed, int spec, const 
                     if (g->mhead) {   /* section 12: the shadow ray counts a block hit only before its limit */
                         uint32_t sw5;
                         int svox[3];
-                        if (!closest_intersect_w5(c, &q, &s, &sw5, svox, 1)) p.pix_color = vadd(p.pix_color, contrib);
-                    } else if (!closest_intersect(c, &q, &s)) {
+                        if (!closest_intersect_w5(c, &q, &s, &sw5, svox, 1) && !cloud_blocks(cl, q.origin, w, limit))
+                            p.pix_color = vadd(p.pix_color, contrib);
+                    } else if (!closest_intersect(c, &q, &s) && !cloud_blocks(cl, q.origin, w, limit)) {
                         p.pix_color = vadd(p.pix_color, contrib);
                     }
                 }
             }
         }
         more = next_path(c, &p, &rec, &state, c->sc->max_depth);
-        if (fog_sun) fog_sun_sample(c, fog_p, fog_w, &rec, &state, &p);
+        if (fog_sun) fog_sun_sample(c, cl, fog_p, fog_w, &rec, &state, &p);
         if (!more) break;
     }
     return p.pix_color;
@@ -682,7 +798,7 @@ static v3 sample_pixel_ext(const Ctx *c, int gid, int32_t seed, int spec, const 
 
 static int render_ext(const OracleScene *s, const int32_t *seeds, int n_passes, int start_spp, float *res, const int32_t *gids,
                       int64_t n_gids, int nthreads, OracleCounters *out_counters, int spec, const EmitterGrid *g, int near,
-                      const BiomeTiles *biome, const FogParams *fog) {
+                      const BiomeTiles *biome, const FogParams *fog, const CloudLayer *cl) {
     int64_t n = gids ? n_gids : (int64_t)s->width * s->height;
     OracleCounters total;
     memset(&total, 0, sizeof total);
@@ -703,7 +819,7 @@ static int render_ext(const OracleScene *s, const int32_t *seeds, int n_passes, 
             float *px = res + (size_t)gid * 3;
             v3 buf = V(px[0], px[1], px[2]);
             for (int pass = 0; pass < n_passes; pass++) {
-                v3 col = sample_pixel_ext(c, gid, seeds[pass], spec, g, near, fog);
+                v3 col = sample_pixel_ext(c, gid, seeds[pass], spec, g, near, fog, cl);
                 int spp = start_spp + pass;
                 buf.x = (buf.x * (float)spp + col.x) / (float)(spp + 1);
                 buf.y = (buf.y * (float)spp + col.y) / (float)(spp + 1);
@@ -721,15 +837,32 @@ static int render_ext(const OracleScene *s, const int32_t *seeds, int n_passes, 
 /* oracle_render with the specular events (same arguments, same running mean) */
 int specular_render(const OracleScene *s, const int32_t *seeds, int n_passes, int start_spp, float *res, const int32_t *gids,
                     int64_t n_gids, int nthreads, OracleCounters *out_counters) {
-    return render_ext(s, seeds, n_passes, start_spp, res, gids, n_gids, nthreads, out_counters, 1, NULL, 0, NULL, NULL);
+    return render_ext(s, seeds, n_passes, start_spp, res, gids, n_gids, nthreads, out_counters, 1, NULL, 0, NULL, NULL, NULL);
 }
 
 /* oracle_render with CCU_RENDER_SPECULAR (spec), CCU_RENDER_EMITTER_SAMPLING (g != NULL), CCU_RENDER_EMITTER_NEAR_FIELD
- * (near, with g), CCU_RENDER_BIOME_TINT (biome != NULL) and CCU_RENDER_FOG (fog != NULL: the scene has fog) */
+ * (near, with g), CCU_RENDER_BIOME_TINT (biome != NULL), CCU_RENDER_FOG (fog != NULL: the scene has fog) and CCU_RENDER_CLOUDS
+ * (cl != NULL: the scene has a cloud mask with a set cell) */
 int flags_render(const OracleScene *s, const int32_t *seeds, int n_passes, int start_spp, float *res, const int32_t *gids,
                  int64_t n_gids, int nthreads, OracleCounters *out_counters, int spec, const EmitterGrid *g, int near,
-                 const BiomeTiles *biome, const FogParams *fog) {
-    return render_ext(s, seeds, n_passes, start_spp, res, gids, n_gids, nthreads, out_counters, spec, g, near, biome, fog);
+                 const BiomeTiles *biome, const FogParams *fog, const CloudLayer *cl) {
+    return render_ext(s, seeds, n_passes, start_spp, res, gids, n_gids, nthreads, out_counters, spec, g, near, biome, fog, cl);
+}
+
+int cloud_layer_struct_size(void) { return (int)sizeof(CloudLayer); }
+
+/* the cloud walk alone, for tests: ray r = o[3 r .. 3 r + 2] + d[3 r .. 3 r + 2] t below limit[r]; out[4 r] = t (NaN for a miss),
+ * out[4 r + 1 .. 3] = the normal; visited[r] = the cells the walk tested (0 when it did not start) */
+void cloud_hit_batch(const CloudLayer *cl, int64_t n, const float *o, const float *d, const float *limit, float *out, int32_t *visited) {
+    for (int64_t r = 0; r < n; r++) {
+        float t;
+        v3 nrm = V(0, 0, 0);
+        int cells = 0;
+        int hit = cloud_hit(cl, V(o[3 * r], o[3 * r + 1], o[3 * r + 2]), V(d[3 * r], d[3 * r + 1], d[3 * r + 2]), limit[r], &t, &nrm, &cells);
+        out[4 * r] = hit ? t : NAN;
+        out[4 * r + 1] = nrm.x; out[4 * r + 2] = nrm.y; out[4 * r + 3] = nrm.z;
+        visited[r] = cells;
+    }
 }
 
 int fog_params_struct_size(void) { return (int)sizeof(FogParams); }
