@@ -298,6 +298,8 @@ struct ccu_ctx {
     ccu_host::HostBuf<float> pinned;        // host staging float[accum_floats]
     ccu_host::SeedRing seeds;
     ccu_host::DevBuf<int> fh_scratch;       // first-hit planes (kept between calls)
+    ccu_host::DevBuf<float> feat_scratch;   // feature buffers: albedo and normal, float[3*W*H] each (kept between calls)
+    ccu_host::DevBuf<int> feat_seeds;       // feature buffers: the pass seeds (CCU_FEATURES_MAX_PASSES)
     ccu_host::DevBuf<unsigned> work_counter;
     ccu_host::DevBuf<int> bvh_deep;         // wavefront kernel, BVH scenes: traversal-stack entries beyond the shared-memory part
     int yield_below = 20;
@@ -316,6 +318,7 @@ struct ccu_ctx {
     bool timing_pending = false;
     int64_t launches = 0;
     int32_t last_render[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};   // the last render launch's instance (ccu_debug_last_render_n)
+    int32_t last_features[4] = {0, 0, 0, 0};                // the last feature launch's instance (ccu_debug_last_features)
 };
 
 namespace ccu_host {

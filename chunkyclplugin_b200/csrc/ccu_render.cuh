@@ -3,7 +3,8 @@
 // The instances of k_render_mega and k_render_queue are compiled in translation units of their own, one per MODE or
 // (HAS_BVH, LAY) and value of the clouds switch (render_mega_<MODE>.cu, render_queue_<HAS_BVH><LAY>.cu, and the same names with
 // _c for the cloud kernels), which the build compiles in parallel with chunkycu.cu and links into the same library; each unit
-// returns its kernels through mega_kernel_of<MODE, CLOUDS> / queue_kernel_of<HAS_BVH, LAY, CLOUDS>.  chunkycu.cu sees only the
+// returns its kernels through mega_kernel_of<MODE, CLOUDS> / queue_kernel_of<HAS_BVH, LAY, CLOUDS>.  The feature-buffer kernel
+// (DESIGN §16) has one unit per MODE (render_features_<MODE>.cu, features_kernel_of<MODE>).  chunkycu.cu sees only the
 // declarations.
 #pragma once
 #include <type_traits>
@@ -62,6 +63,12 @@ using QueueFn = void (*)(DScene, QueueParams, EmitView, BiomeView, CloudView);
 // (render_queue_<HAS_BVH><LAY>[_c].cu)
 template <bool HAS_BVH, int LAY, bool CLOUDS>
 QueueFn queue_kernel_of(const ShadeKey &v);
+using FeaturesFn = void (*)(DScene, const int *, int, int, float *, float *, BiomeView, CloudView);
+// k_features<MODE, bvh, Shade with the biome and clouds switches> of the feature buffers (DESIGN §16, render_features_<MODE>.cu)
+template <int MODE>
+FeaturesFn features_kernel_of(bool bvh, bool biome, bool clouds);
+#define CCU_FEAT_THREADS 128   // threads per block of k_features
+
 #ifdef CCU_Q_STATS
 // the debug counters of the unit render_queue_<HAS_BVH><LAY>[_c].cu (_c: CLOUDS): copied to st[32], then cleared
 template <bool HAS_BVH, int LAY, bool CLOUDS>

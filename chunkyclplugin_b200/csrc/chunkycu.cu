@@ -83,21 +83,7 @@ __device__ __forceinline__ void first_hit_store(const FirstHitOut &out, int gid,
     if (out.color) reinterpret_cast<float4 *>(out.color)[gid] = hit ? color : make_float4(0, 0, 0, 0);
 }
 
-// The warp-synchronous march loop of the thread-per-ray kernels: every lane steps its ray until no lane of the warp is marching
-// any more.  Kept out of line so that the loop is register-allocated by itself - inlined into the 64-register kernel, next to the
-// block test, the ray was spilled and re-loaded inside the loop.  The ray travels through local memory once per call.
-// st: 0 marching, anything else: not marching (returned unchanged).
-template <bool DEEP>
-static __device__ __noinline__ int first_hit_march(const DScene &s, LeanRay *ray, int st) {
-    LeanRay r = *ray;
-    while (__any_sync(0xffffffffu, st == 0)) {
-        if (!DEEP) st = lean_step_flat<false>(s, s.air_top, r, st == 0, st, s.draw_depth, ~0u << s.depth);
-        else if (st == 0) st = lean_probe<DEEP, false>(s, s.air_top, r, s.draw_depth);
-    }
-    ray->t = r.t;
-    ray->steps = r.steps;
-    return st;
-}
+#include "ccu_first_hit.cuh"   // first_hit_march
 
 template <int MODE, bool HAS_BVH>
 __global__ void __launch_bounds__(CCU_FH_THREADS, CCU_FH_MIN_BLOCKS) k_first_hit(const __grid_constant__ DScene s, int seed, int n_pixels, const __grid_constant__ FirstHitOut out) {
@@ -1427,6 +1413,54 @@ int ccu_first_hit(ccu_ctx *c, int32_t seed, int32_t *block, int32_t *face, int32
     return CCU_OK;
 }
 
+// DESIGN §16: the running means of the first-hit albedo and normal over n_passes passes, in one launch of k_features.  Launched
+// on the render stream after whatever is queued there; it reads the launch view and writes only its own scratch, so the
+// accumulation window, its pass count and the render-instance record stay as they were.
+int ccu_render_features(ccu_ctx *c, const int32_t *seeds, int32_t n_passes, float *albedo, float *normal) {
+    if (!c) return fail(CCU_EINVAL, "ccu_render_features: null context");
+    if (!seeds) return fail(CCU_EINVAL, "ccu_render_features: null seeds");
+    if (n_passes < 1 || n_passes > CCU_FEATURES_MAX_PASSES)
+        return fail(CCU_EINVAL, "ccu_render_features: %d passes (1 to %d)", n_passes, CCU_FEATURES_MAX_PASSES);
+    if (!albedo && !normal) return fail(CCU_EINVAL, "ccu_render_features: no output (albedo and normal are both null)");
+    std::lock_guard<std::mutex> lk(c->mu);
+    int rc = render_ready(c, "ccu_render_features");
+    if (rc != CCU_OK) return rc;
+    DeviceGuard g(c->device);
+    const size_t n = (size_t)c->width * c->height;
+    if (c->feat_scratch.n < n * 6 || !c->feat_seeds.p) {
+        cudaStreamSynchronize(c->stream);
+        if (c->feat_scratch.n < n * 6) CU(c->feat_scratch.alloc(n * 6));
+        if (!c->feat_seeds.p) CU(c->feat_seeds.alloc(CCU_FEATURES_MAX_PASSES));
+    }
+    float *d_albedo = albedo ? c->feat_scratch.p : nullptr, *d_normal = normal ? c->feat_scratch.p + n * 3 : nullptr;
+    DScene s = launch_view(c);
+    s.sun_flags = c->scene.view.sun_flags;   // the sky of a miss keeps the scene's sun disc under CCU_RENDER_NO_SUN (§16)
+    const int mode = layout_mode(c);
+    const bool bvh = !(s.world_bvh_empty && s.actor_bvh_empty);
+    const ShadeKey shade = shade_variant(c);
+    cudaError_t e = cudaMemcpyAsync(c->feat_seeds.p, seeds, (size_t)n_passes * sizeof(int), cudaMemcpyHostToDevice, c->stream);
+    if (e != cudaSuccess) return fail(CCU_ECUDA, "ccu_render_features: %s", cudaGetErrorString(e));
+    const unsigned blocks = (unsigned)((n + CCU_FEAT_THREADS - 1) / CCU_FEAT_THREADS);
+    cudaEventRecord(c->ev0, c->stream);
+    FeaturesFn k = nullptr;
+    dispatch<3>(mode, [&](auto M) { k = features_kernel_of<M>(bvh, shade.biome, shade.clouds); });
+    k<<<blocks, CCU_FEAT_THREADS, 0, c->stream>>>(s, c->feat_seeds.p, n_passes, (int)n, d_albedo, d_normal, c->scene.biome_view,
+                                                  c->scene.cloud_view);
+    c->launches++;
+    cudaEventRecord(c->ev1, c->stream);
+    if (c->projector_type == -1) cudaEventRecord(c->rays_used[c->rays_active], c->stream);
+    c->timing_pending = true;
+    const int32_t last[4] = {mode, bvh, shade.biome, shade.clouds};
+    std::copy(last, last + 4, c->last_features);
+    e = cudaGetLastError();
+    if (albedo && e == cudaSuccess) e = cudaMemcpyAsync(albedo, d_albedo, n * 12, cudaMemcpyDeviceToHost, c->stream);
+    if (normal && e == cudaSuccess) e = cudaMemcpyAsync(normal, d_normal, n * 12, cudaMemcpyDeviceToHost, c->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+    if (e != cudaSuccess) return fail(CCU_ECUDA, "ccu_render_features: %s", cudaGetErrorString(e));
+    stop_timer(c);
+    return CCU_OK;
+}
+
 int ccu_preview(ccu_ctx *c, int32_t *argb) {
     if (!c || !argb) return fail(CCU_EINVAL, "ccu_preview: null argument");
     std::lock_guard<std::mutex> lk(c->mu);
@@ -1482,6 +1516,13 @@ int ccu_debug_last_render_n(ccu_ctx *c, int32_t *out, int32_t n) {
     if (!c || !out || n < 0) return fail(CCU_EINVAL, "ccu_debug_last_render_n: null argument or negative n");
     std::lock_guard<std::mutex> lk(c->mu);
     std::copy(c->last_render, c->last_render + std::min(n, 9), out);
+    return CCU_OK;
+}
+
+int ccu_debug_last_features(ccu_ctx *c, int32_t out[4]) {
+    if (!c || !out) return fail(CCU_EINVAL, "ccu_debug_last_features: null argument");
+    std::lock_guard<std::mutex> lk(c->mu);
+    std::copy(c->last_features, c->last_features + 4, out);
     return CCU_OK;
 }
 

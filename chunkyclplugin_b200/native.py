@@ -20,6 +20,7 @@ CCU_RENDER_EMITTER_MODELS = 256
 CCU_RENDER_BIOME_TINT = 512
 CCU_RENDER_FOG = 1024
 CCU_RENDER_CLOUDS = 2048
+CCU_FEATURES_MAX_PASSES = 1024    # passes of one ccu_render_features call (DESIGN.md §16)
 CCU_UNIQUE_ID_BYTES = 128
 
 CCU_OK, CCU_ENODEVICE, CCU_EINVAL, CCU_ECUDA, CCU_ENOMEM, CCU_ESTATE = 0, -1, -2, -3, -4, -5
@@ -85,10 +86,12 @@ SYMBOLS = {
     "ccu_stream_handle": (C.c_int, [_vp, C.POINTER(_vp)]),
     "ccu_first_hit": (C.c_int, [_vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "ccu_preview": (C.c_int, [_vp, _vp]),
+    "ccu_render_features": (C.c_int, [_vp, _vp, _i32, _vp, _vp]),
     "ccu_last_kernel_ms": (C.c_int, [_vp, C.POINTER(_f)]),
     "ccu_launch_count": (C.c_int, [_vp, C.POINTER(_i64)]),
     "ccu_debug_last_render": (C.c_int, [_vp, _vp]),
     "ccu_debug_last_render_n": (C.c_int, [_vp, _vp, _i32]),
+    "ccu_debug_last_features": (C.c_int, [_vp, _vp]),
     "ccu_scene_device_bytes": (C.c_int, [_vp, C.POINTER(_i64)]),
     "ccu_scene_commit_ms": (C.c_int, [_vp, C.POINTER(C.c_double)]),
     "ccu_tonemap": (C.c_int, [_vp, _i32, _i32, _f, _vp, _i32, _vp]),
@@ -456,6 +459,26 @@ class Context:
         check(self._lib.ccu_first_hit(self._h, seed, _ptr(out["block"]), _ptr(out["face"]), _ptr(out["node"]),
                                       _ptr(out["kind"]), _ptr(out["t"]), _ptr(out["normal"]), _ptr(out["color"])))
         return out
+
+    def render_features(self, seeds, albedo: bool = True, normal: bool = True):
+        """The denoiser's feature buffers (DESIGN.md §16): (albedo, normal), float32[H*W*3] each (None where not asked for),
+        averaged over the passes with these seeds (ccu_render_features).  The canvas size comes from the library's render
+        target (a group member's context learns it from ccu_group_render_begin); without one this raises CCU_ESTATE before the
+        call."""
+        _, n_floats = self.render_device_buffer()       # 3 * W * H of the live render target
+        sd = np.ascontiguousarray(seeds, np.int32).reshape(-1)
+        a = np.empty(n_floats, np.float32) if albedo else None
+        n = np.empty(n_floats, np.float32) if normal else None
+        check(self._lib.ccu_render_features(self._h, _ptr(sd) if sd.size else None, int(sd.size),
+                                            _ptr(a) if a is not None else None, _ptr(n) if n is not None else None))
+        return a, n
+
+    def last_features(self) -> tuple:
+        """The feature kernel instance of the last render_features launch: (MODE, HAS_BVH, biome, clouds), all zero before the
+        first (ccu_debug_last_features)."""
+        out = np.zeros(4, np.int32)
+        check(self._lib.ccu_debug_last_features(self._h, _ptr(out)))
+        return tuple(int(v) for v in out)
 
     def preview(self) -> np.ndarray:
         w, h = self._wh

@@ -321,6 +321,41 @@ class CudaPathTracingRenderer:
         if cameraErrors:
             raise cameraErrors[0]
 
+    def render_features(self, manager: DefaultRenderManager, spp: int):
+        """The denoiser's feature buffers of the buffered scene (DESIGN.md §16): (albedo, normal), Chunky-layout float64[3*W*H]
+        each, the first-hit means over `spp` passes whose seeds are drawn as render() draws them (JavaRandom(0), one nextInt per
+        pass).  With a projector the library generates the rays, so these are the camera rays of the first `spp` passes of
+        render().  With pre-generated rays (projector -1) one freshly jittered ray set serves every pass, whereas render()
+        switches to a new set every `camera_regen_passes` passes (whenever the background upload lands), so the jitter differs
+        from render()'s.  A render of more than CCU_FEATURES_MAX_PASSES passes is split into calls of at most that many, whose
+        means are combined in double."""
+        if spp < 1:
+            raise ValueError("render_features needs at least one pass")
+        ctx = self.sceneLoader.instance.context
+        scene = manager.bufferedScene
+        self.sceneLoader.ensureLoad(scene)
+        camera = CudaCamera(scene, self.sceneLoader.instance)
+        ctx.render_begin(scene.width, scene.height)
+        try:
+            camera.generate(None, True)
+            rand = JavaRandom(0)
+            seeds = np.array([rand.next_int() for _ in range(spp)], dtype=np.int32)
+            albedo = normal = None
+            done = 0
+            for off in range(0, spp, native.CCU_FEATURES_MAX_PASSES):
+                part = seeds[off:off + native.CCU_FEATURES_MAX_PASSES]
+                a, n = ctx.render_features(part)
+                if albedo is None:
+                    albedo, normal = a.astype(np.float64), n.astype(np.float64)
+                else:
+                    albedo = (albedo * done + a.astype(np.float64) * part.size) / (done + part.size)
+                    normal = (normal * done + n.astype(np.float64) * part.size) / (done + part.size)
+                done += part.size
+        finally:
+            camera.close()
+            ctx.render_end()
+        return albedo, normal
+
     @staticmethod
     def _isSaveEvent(control: SnapshotControl, scene: Scene, spp: int) -> bool:           # :193-195
         return control.saveSnapshot(scene, spp) or control.saveRenderDump(scene, spp)

@@ -210,6 +210,20 @@ int ccu_stream_handle(ccu_ctx *ctx, void **cuda_stream);
 int ccu_first_hit(ccu_ctx *ctx, int32_t seed, int32_t *block, int32_t *face, int32_t *node, int32_t *kind, float *t,
                   float *normal, float *color);
 
+/* ---- feature buffers for a denoiser (beyond the reference; DESIGN.md §16) -------------------------------------------
+ * The first-hit albedo and normal of the camera rays the render kernels trace for the passes with seeds[0 .. n_passes-1],
+ * averaged over the passes with the render kernels' running mean: what Open Image Denoise and the Chunky denoiser plugin take
+ * next to the beauty image.  Per pass, an octree or BVH hit gives albedo = the material colour (biome-tinted when
+ * CCU_RENDER_BIOME_TINT selects the biome colours) and normal = the surface normal; a cloud of CCU_RENDER_CLOUDS gives (1, 1, 1)
+ * and the normal of the face entered; a miss gives the sky radiance clamped to 1 per component and a zero normal.
+ * CCU_RENDER_NO_ENTITIES and draw_depth apply; the other render flags, max_depth and emitter_scale do not change the buffers.
+ * albedo, normal = float[3*W*H] (RGB / xyz interleaved, row-major like the accumulation buffer); either may be NULL, not both.
+ * Blocking; needs ccu_render_begin like ccu_first_hit.  Leaves the accumulation window, its pass count and
+ * ccu_debug_last_render[_n] as they were.  CCU_EINVAL for a NULL context or seeds, n_passes outside
+ * [1, CCU_FEATURES_MAX_PASSES], or both outputs NULL. */
+#define CCU_FEATURES_MAX_PASSES 1024
+int ccu_render_features(ccu_ctx *ctx, const int32_t *seeds, int32_t n_passes, float *albedo, float *normal);
+
 /* ---- preview: OpenClPreviewRenderer.java:47-115 (kernel rayTracer.cl:115-217), ARGB int[W*H] ----------------- */
 int ccu_preview(ccu_ctx *ctx, int32_t *argb);
 
@@ -219,7 +233,7 @@ int ccu_preview(ccu_ctx *ctx, int32_t *argb);
 int ccu_tonemap(ccu_ctx *ctx, int32_t width, int32_t height, float exposure, const double *input, int32_t type, int32_t *argb);
 
 /* ---- instrumentation ------------------------------------------------------------------------------------------ */
-int ccu_last_kernel_ms(ccu_ctx *ctx, float *ms);          /* CUDA-event time of the last render_passes / first_hit launch(es) */
+int ccu_last_kernel_ms(ccu_ctx *ctx, float *ms);          /* CUDA-event time of the last render_passes / first_hit / features launch(es) */
 int ccu_launch_count(ccu_ctx *ctx, int64_t *launches);    /* kernels launched by this context so far */
 /* Test support: the render kernel instance of the context's last ccu_render_passes[_async] launch (all zero before the first).
  * out = {kernel launched (1 or 4, after the choice for kernel 0), HAS_BVH, LAY (kernel 4) or MODE (kernel 1), spec, nee (a NeeKind:
@@ -229,6 +243,9 @@ int ccu_launch_count(ccu_ctx *ctx, int64_t *launches);    /* kernels launched by
 int ccu_debug_last_render(ccu_ctx *ctx, int32_t out[7]);
 /* The same report with the switches added since: writes the first min(n, 9) of {the 7 entries above, fog, clouds}. */
 int ccu_debug_last_render_n(ccu_ctx *ctx, int32_t *out, int32_t n);
+/* Test support: the feature kernel instance of the last ccu_render_features launch, {MODE, HAS_BVH, biome, clouds} (all zero
+ * before the first). */
+int ccu_debug_last_features(ccu_ctx *ctx, int32_t out[4]);
 int ccu_scene_device_bytes(ccu_ctx *ctx, int64_t *bytes); /* HBM held by the committed scene */
 int ccu_scene_commit_ms(ccu_ctx *ctx, double *ms);        /* host time the last ccu_scene_commit spent building + uploading the layouts */
 /* Memory-system denominators for this path's roofline (dependent 32-byte-sector gathers, SURVEY 8d): random 16-byte

@@ -64,6 +64,7 @@ public final class ChunkyCu {
             FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, ADDRESS), Linker.Option.critical(true));
     private static final MethodHandle RENDER_END = h("ccu_render_end", FunctionDescriptor.of(JAVA_INT, ADDRESS));
     private static final MethodHandle PREVIEW = h("ccu_preview", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS));
+    private static final MethodHandle RENDER_FEATURES = h("ccu_render_features", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, ADDRESS, ADDRESS));
     private static final MethodHandle TONEMAP = h("ccu_tonemap", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT, JAVA_INT, JAVA_FLOAT, ADDRESS, JAVA_INT, ADDRESS));
     // multi-GPU group (include/chunkycu.h "multi-GPU"): one JVM drives all GPUs of the box
     private static final MethodHandle GROUP_CREATE = h("ccu_group_create", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT, ADDRESS));
@@ -299,6 +300,19 @@ public final class ChunkyCu {
                 MemorySegment out = a.allocate(JAVA_INT, argb.length);
                 check(call(PREVIEW, handle, out));
                 MemorySegment.copy(out, JAVA_INT, 0, argb, 0, argb.length);
+            }
+        }
+
+        /** The denoiser's feature buffers (DESIGN §16): the first-hit albedo and normal averaged over the passes with these seeds,
+         *  3 floats per pixel each; either array may be null, not both (include/chunkycu.h, ccu_render_features). */
+        public void renderFeatures(int[] seeds, float[] albedo, float[] normal) {
+            try (Arena a = Arena.ofConfined()) {
+                MemorySegment s = a.allocateFrom(JAVA_INT, seeds);
+                MemorySegment al = albedo != null ? a.allocate(JAVA_FLOAT, albedo.length) : MemorySegment.NULL;
+                MemorySegment no = normal != null ? a.allocate(JAVA_FLOAT, normal.length) : MemorySegment.NULL;
+                check((int) RENDER_FEATURES.invokeExact(handle, s, seeds.length, al, no));
+                if (albedo != null) MemorySegment.copy(al, JAVA_FLOAT, 0, albedo, 0, albedo.length);
+                if (normal != null) MemorySegment.copy(no, JAVA_FLOAT, 0, normal, 0, normal.length);
             }
         }
 

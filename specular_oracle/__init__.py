@@ -4,7 +4,8 @@ ONLY.
 
 ``SpecularOracle`` is the parity oracle (``oracle.Oracle``) with the specular events of DESIGN.md section 9 in its path
 loop; ``FlagsOracle`` takes the render flags and adds the emitter sampling of sections 10 to 12, with the emitter table that
-``emitter_grid`` builds from the packed arrays (``model_emitters`` adds the model emitters of section 12).  Everything else - first hit, preview, counters - is the oracle's.  Like the
+``emitter_grid`` builds from the packed arrays (``model_emitters`` adds the model emitters of section 12), and its ``features``
+restates the denoiser's feature buffers of section 16.  Everything else - first hit, preview, counters - is the oracle's.  Like the
 oracle, only tests/ and scripts use it.
 """
 from __future__ import annotations
@@ -361,3 +362,25 @@ class FlagsOracle(oracle.Oracle):
                            C.byref(self._clouds) if self._clouds is not None else None)
         self._counters(cnt)
         return res
+
+    def features(self, seeds: Sequence[int], rays: Optional[np.ndarray] = None, threads: int = 0):
+        """DESIGN.md section 16: the feature buffers (albedo, normal), float32[H*W*3] each, of the passes with these seeds under
+        this oracle's flags: of them only CCU_RENDER_BIOME_TINT and CCU_RENDER_CLOUDS act (with the scene's biome colours and
+        cloud layer); CCU_RENDER_NO_ENTITIES acts on the scene (empty BVHs).  rays: pre-generated camera rays (float32[H*W*6])
+        in place of the scene's camera, as ccu_camera_set with projector -1 takes them."""
+        n = self._s.width * self._s.height
+        s = self._s
+        keep = None
+        if rays is not None:
+            keep = np.ascontiguousarray(rays, np.float32).reshape(-1)
+            assert keep.size == n * 6
+            s = oracle._Scene.from_buffer_copy(self._s)
+            s.projector_type = -1
+            s.camera = keep.ctypes.data
+        sd = np.ascontiguousarray(seeds, dtype=np.int32)
+        albedo = np.zeros(n * 3, np.float32)
+        normal = np.zeros(n * 3, np.float32)
+        lib().features_render(C.byref(s), sd.ctypes.data_as(C.c_void_p), C.c_int(sd.size), albedo.ctypes.data_as(C.c_void_p),
+                              normal.ctypes.data_as(C.c_void_p), C.byref(self._biome) if self._biome is not None else None,
+                              C.byref(self._clouds) if self._clouds is not None else None, C.c_int(threads))
+        return albedo, normal

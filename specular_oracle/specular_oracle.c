@@ -16,7 +16,8 @@
  * CCU_RENDER_BIOME_TINT (section 13) restates the material evaluation with the biome colours of the hit voxel's column; the
  * block test, the octree march and the emitter samplers pass that voxel on.  CCU_RENDER_FOG (section 14) restates the fog of
  * the path loop.  CCU_RENDER_CLOUDS (section 15) restates the cloud walk and where the path loop, the shadow rays, the emitter
- * sample's ray and the fog's sun sample meet it.
+ * sample's ray and the fog's sun sample meet it.  The feature buffers of a denoiser (section 16) take the first segment of the path
+ * loop with the biome colours and the clouds.
  */
 #include "../oracle/chunky_oracle.c"
 
@@ -847,6 +848,72 @@ int flags_render(const OracleScene *s, const int32_t *seeds, int n_passes, int s
                  int64_t n_gids, int nthreads, OracleCounters *out_counters, int spec, const EmitterGrid *g, int near,
                  const BiomeTiles *biome, const FogParams *fog, const CloudLayer *cl) {
     return render_ext(s, seeds, n_passes, start_spp, res, gids, n_gids, nthreads, out_counters, spec, g, near, biome, fog, cl);
+}
+
+/* DESIGN.md section 16: the feature buffers (albedo, normal; float[3 * W * H] each, either may be NULL) of n_passes passes.  Pass p
+ * traces the camera ray of sample_pixel_ext's pass with seed seeds[p] as its first path segment: closest_intersect with the biome
+ * colours (biome != NULL), then the cloud layer (cl != NULL) before the hit.  An octree / BVH hit gives the record's colour and
+ * normal, a cloud (1, 1, 1) and its face normal, a miss the sky and sun disc of intersect_sky clamped to 1 and a zero normal.
+ * The passes are folded in the running mean of the render loop, from zero. */
+int features_render(const OracleScene *s, const int32_t *seeds, int n_passes, float *albedo, float *normal, const BiomeTiles *biome,
+                    const CloudLayer *cl, int nthreads) {
+    int64_t n = (int64_t)s->width * s->height;
+#ifdef _OPENMP
+    if (nthreads > 0) omp_set_num_threads(nthreads);
+#endif
+#pragma omp parallel
+    {
+        OracleCounters local;
+        memset(&local, 0, sizeof local);
+        ExtCtx ec;
+        ctx_init(&ec.base, s, &local);
+        ec.biome = biome;
+        const Ctx *c = &ec.base;
+#pragma omp for schedule(dynamic, 64)
+        for (int64_t gid = 0; gid < n; gid++) {
+            v3 ab = V(0, 0, 0), nb = V(0, 0, 0);
+            for (int pass = 0; pass < n_passes; pass++) {
+                Path p;
+                Record rec;
+                uint32_t w5 = 0;
+                int vox[3] = {0, 0, 0};
+                p.pix_color = V(0, 0, 0);
+                p.throughput = V(1, 1, 1);
+                p.ray_depth = 0;
+                record_new(&rec);
+                uint32_t state = (uint32_t)seeds[pass] + (uint32_t)gid;
+                rng_next(&state);
+                camera_ray(c, (int)gid, &state, &p, 0);
+                int hit = closest_intersect_w5(c, &p, &rec, &w5, vox, 0);
+                float t;
+                v3 a, nrm, cn;
+                if (cl && cloud_hit(cl, p.origin, p.direction, hit ? rec.distance : HUGE_VALF, &t, &cn, NULL)) {
+                    a = V(1, 1, 1);
+                    nrm = cn;
+                } else if (hit) {
+                    a = V(rec.color[0], rec.color[1], rec.color[2]);
+                    nrm = rec.normal;
+                } else {
+                    Record sky;
+                    record_new(&sky);
+                    sky_intersect(c, p.direction, &sky);
+                    sun_intersect(c, p.direction, &sky);
+                    a = V(fminf(sky.color[0], 1.0f), fminf(sky.color[1], 1.0f), fminf(sky.color[2], 1.0f));
+                    nrm = V(0, 0, 0);
+                }
+                const float fs = (float)pass, fs1 = (float)(pass + 1);
+                ab.x = (ab.x * fs + a.x) / fs1;
+                ab.y = (ab.y * fs + a.y) / fs1;
+                ab.z = (ab.z * fs + a.z) / fs1;
+                nb.x = (nb.x * fs + nrm.x) / fs1;
+                nb.y = (nb.y * fs + nrm.y) / fs1;
+                nb.z = (nb.z * fs + nrm.z) / fs1;
+            }
+            if (albedo) { albedo[gid * 3] = ab.x; albedo[gid * 3 + 1] = ab.y; albedo[gid * 3 + 2] = ab.z; }
+            if (normal) { normal[gid * 3] = nb.x; normal[gid * 3 + 1] = nb.y; normal[gid * 3 + 2] = nb.z; }
+        }
+    }
+    return 0;
 }
 
 int cloud_layer_struct_size(void) { return (int)sizeof(CloudLayer); }
