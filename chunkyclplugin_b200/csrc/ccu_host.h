@@ -300,6 +300,8 @@ struct ccu_ctx {
     ccu_host::DevBuf<int> fh_scratch;       // first-hit planes (kept between calls)
     ccu_host::DevBuf<float> feat_scratch;   // feature buffers: albedo and normal, float[3*W*H] each (kept between calls)
     ccu_host::DevBuf<int> feat_seeds;       // feature buffers: the pass seeds (CCU_FEATURES_MAX_PASSES)
+    ccu_host::DevBuf<float4> dn_scratch;    // denoiser: working records, 4 per pixel (kept between calls)
+    ccu_host::DevBuf<double> dn_io;         // denoiser: the colour in and the result out, double[3*W*H], then albedo and normal float[3*W*H]
     ccu_host::DevBuf<unsigned> work_counter;
     ccu_host::DevBuf<int> bvh_deep;         // wavefront kernel, BVH scenes: traversal-stack entries beyond the shared-memory part
     int yield_below = 20;

@@ -145,6 +145,8 @@ __device__ __forceinline__ float dm_expf(float x) {
     const double scale = __longlong_as_double((long long)((int)k + 1023) << 52);   // 2^k, -151 <= k <= 129
     return (float)(r * scale);
 }
+// The denoiser's edge-stopping exp (DESIGN §17): dm_expf, with 0 below -87, where e^x leaves the normal fp32 range.
+__device__ __forceinline__ float dm_expf_weight(float x) { return x < -87.0f ? 0.0f : dm_expf(x); }
 
 // 256-bit read-only global load (LDG.E.256 on sm_100a): one instruction and one L1 tag lookup per lane for a 32-byte record half
 struct __align__(32) Int8 { int v[8]; };

@@ -23,6 +23,12 @@
 #include "ccu_tonemap.cuh"
 #include "ccu_layout.h"
 
+namespace ccu {
+// ccu_denoise.cuh, compiled in denoise.cu (DESIGN §17)
+int denoise_launch(cudaStream_t st, int w, int h, int iterations, float sigma_l, double *io, const float *albedo, const float *normal,
+                   float4 *rec);
+}
+
 using namespace ccu;
 
 // ======================================================================================================
@@ -399,7 +405,7 @@ int set_array(ccu_ctx *c, ccu_host::SceneArray a, const int32_t *words, int64_t 
     return CCU_OK;
 }
 
-// device time of the last render / first-hit / preview / tonemap launch(es); waits for them (caller holds c->mu)
+// device time of the last render / first-hit / preview / tonemap / denoise launch(es); waits for them (caller holds c->mu)
 void stop_timer(ccu_ctx *c) {
     if (c->timing_pending) {
         cudaEventSynchronize(c->ev1);
@@ -1457,6 +1463,47 @@ int ccu_render_features(ccu_ctx *c, const int32_t *seeds, int32_t n_passes, floa
     if (normal && e == cudaSuccess) e = cudaMemcpyAsync(normal, d_normal, n * 12, cudaMemcpyDeviceToHost, c->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
     if (e != cudaSuccess) return fail(CCU_ECUDA, "ccu_render_features: %s", cudaGetErrorString(e));
+    stop_timer(c);
+    return CCU_OK;
+}
+
+// DESIGN §17: the guided a-trous filter of a sample buffer, on the render stream after whatever is queued there.  It reads
+// only the caller's buffers and writes only its own scratch, so neither the render target nor the scene is needed, and the
+// accumulation window, its pass count and the render-instance record stay as they were.
+int ccu_denoise(ccu_ctx *c, int32_t width, int32_t height, const double *color, const float *albedo, const float *normal,
+                int32_t iterations, float sigma_luminance, double *out) {
+    if (!c) return fail(CCU_EINVAL, "ccu_denoise: null context");
+    if (!color || !albedo || !normal || !out) return fail(CCU_EINVAL, "ccu_denoise: null buffer");
+    if (width < 1 || height < 1 || (int64_t)width * height > INT64_MAX / 3)
+        return fail(CCU_EINVAL, "ccu_denoise: bad canvas %dx%d", width, height);
+    if (iterations < 0 || iterations > CCU_DENOISE_MAX_ITERATIONS)
+        return fail(CCU_EINVAL, "ccu_denoise: %d iterations (0 to %d)", iterations, CCU_DENOISE_MAX_ITERATIONS);
+    if (!(sigma_luminance > 0.0f) || !std::isfinite(sigma_luminance))
+        return fail(CCU_EINVAL, "ccu_denoise: sigma_luminance %g is not positive and finite", (double)sigma_luminance);
+    const size_t n = (size_t)width * height;
+    if (n > ((size_t)1 << 34)) return fail(CCU_ENOMEM, "ccu_denoise: %dx%d needs more device memory than there is", width, height);
+    std::lock_guard<std::mutex> lk(c->mu);
+    DeviceGuard g(c->device);
+    if (c->dn_scratch.n < n * 4 || c->dn_io.n < n * 6) {
+        cudaStreamSynchronize(c->stream);
+        if (c->dn_scratch.n < n * 4) CU(c->dn_scratch.alloc(n * 4));
+        if (c->dn_io.n < n * 6) CU(c->dn_io.alloc(n * 6));
+    }
+    double *d_io = c->dn_io.p;
+    float *d_albedo = reinterpret_cast<float *>(d_io + n * 3), *d_normal = d_albedo + n * 3;
+    cudaError_t e = cudaMemcpyAsync(d_io, color, n * 3 * sizeof(double), cudaMemcpyHostToDevice, c->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_albedo, albedo, n * 3 * sizeof(float), cudaMemcpyHostToDevice, c->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_normal, normal, n * 3 * sizeof(float), cudaMemcpyHostToDevice, c->stream);
+    if (e == cudaSuccess) {
+        cudaEventRecord(c->ev0, c->stream);
+        c->launches += denoise_launch(c->stream, width, height, iterations, sigma_luminance, d_io, d_albedo, d_normal, c->dn_scratch.p);
+        cudaEventRecord(c->ev1, c->stream);
+        c->timing_pending = true;
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out, d_io, n * 3 * sizeof(double), cudaMemcpyDeviceToHost, c->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+    if (e != cudaSuccess) return fail(CCU_ECUDA, "ccu_denoise: %s", cudaGetErrorString(e));
     stop_timer(c);
     return CCU_OK;
 }

@@ -21,6 +21,7 @@ CCU_RENDER_BIOME_TINT = 512
 CCU_RENDER_FOG = 1024
 CCU_RENDER_CLOUDS = 2048
 CCU_FEATURES_MAX_PASSES = 1024    # passes of one ccu_render_features call (DESIGN.md §16)
+CCU_DENOISE_MAX_ITERATIONS = 8    # a-trous iterations of one ccu_denoise call (DESIGN.md §17)
 CCU_UNIQUE_ID_BYTES = 128
 
 CCU_OK, CCU_ENODEVICE, CCU_EINVAL, CCU_ECUDA, CCU_ENOMEM, CCU_ESTATE = 0, -1, -2, -3, -4, -5
@@ -95,6 +96,7 @@ SYMBOLS = {
     "ccu_scene_device_bytes": (C.c_int, [_vp, C.POINTER(_i64)]),
     "ccu_scene_commit_ms": (C.c_int, [_vp, C.POINTER(C.c_double)]),
     "ccu_tonemap": (C.c_int, [_vp, _i32, _i32, _f, _vp, _i32, _vp]),
+    "ccu_denoise": (C.c_int, [_vp, _i32, _i32, _vp, _vp, _vp, _i32, _f, _vp]),
     "ccu_bench_gather": (C.c_int, [_vp, _i64, _i32, C.POINTER(_f), C.POINTER(_f)]),
     "ccu_debug_layout_lookup": (C.c_int, [_vp, _i64, _i32, _vp, _i64, _vp, _vp, _vp, _vp]),
     "ccu_debug_bvh_layout": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _i64, _vp, _i64, C.POINTER(_i64), C.POINTER(_i64), _pi32, _pi32]),
@@ -493,6 +495,29 @@ class Context:
             raise ValueError("sample buffer must hold 3 doubles per pixel")
         out = np.empty(width * height, dtype=np.int32)
         check(self._lib.ccu_tonemap(self._h, width, height, C.c_float(exposure), _ptr(inp), filter_type, _ptr(out)))
+        return out
+
+    def denoise(self, color, albedo, normal, iterations: int = 5, sigma_luminance: float = 4.0,
+                width: Optional[int] = None, height: Optional[int] = None) -> np.ndarray:
+        """The guided a-trous denoiser (DESIGN.md §17, ccu_denoise): a new float64[3*W*H] from the sample buffer `color`
+        (float64) and the feature buffers `albedo` and `normal` (float32, as render_features returns them).  The canvas is
+        (width, height) when given, else the (H, W, 3) shape of `color`; every buffer must hold 3 * W * H values, which is
+        checked before the call."""
+        c = np.ascontiguousarray(color, dtype=np.float64)
+        if width is None or height is None:
+            if c.ndim != 3 or c.shape[2] != 3:
+                raise ValueError("denoise: give width and height, or a colour buffer of shape (H, W, 3)")
+            height, width = c.shape[0], c.shape[1]
+        n = 3 * int(width) * int(height)
+        c = c.reshape(-1)
+        a = np.ascontiguousarray(albedo, dtype=np.float32).reshape(-1)
+        nrm = np.ascontiguousarray(normal, dtype=np.float32).reshape(-1)
+        for name, buf in (("color", c), ("albedo", a), ("normal", nrm)):
+            if buf.size != n:
+                raise ValueError(f"denoise: {name} holds {buf.size} values, not 3 * {width} * {height} = {n}")
+        out = np.empty(n, dtype=np.float64)
+        check(self._lib.ccu_denoise(self._h, int(width), int(height), _ptr(c), _ptr(a), _ptr(nrm), int(iterations),
+                                    C.c_float(sigma_luminance), _ptr(out)))
         return out
 
     def bench_gather(self, array_bytes: int, dependent: bool = False):

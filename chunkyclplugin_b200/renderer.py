@@ -356,6 +356,17 @@ class CudaPathTracingRenderer:
             ctx.render_end()
         return albedo, normal
 
+    def denoise(self, manager: DefaultRenderManager, feature_spp: int = 16, iterations: int = 5,
+                sigma_luminance: float = 4.0) -> np.ndarray:
+        """The buffered scene's sample buffer denoised on the GPU (DESIGN.md §17): render_features(manager, feature_spp), then
+        the guided a-trous filter of the sample buffer with those albedo and normal buffers.  Returns a new Chunky-layout
+        float64[3*W*H], ready for GpuPostProcessingFilter.processFrame or pfm.write_pfm; the sample buffer stays as it was."""
+        scene = manager.bufferedScene
+        albedo, normal = self.render_features(manager, feature_spp)
+        ctx = self.sceneLoader.instance.context
+        return ctx.denoise(scene.sample_buffer, albedo.astype(np.float32), normal.astype(np.float32), iterations,
+                           sigma_luminance, width=scene.width, height=scene.height)
+
     @staticmethod
     def _isSaveEvent(control: SnapshotControl, scene: Scene, spp: int) -> bool:           # :193-195
         return control.saveSnapshot(scene, spp) or control.saveRenderDump(scene, spp)

@@ -232,8 +232,23 @@ int ccu_preview(ccu_ctx *ctx, int32_t *argb);
  *      type: 0 GAMMA, 1 TONEMAP1, 2 ACES ("TONEMAP2"), 3 HABLE ("TONEMAP3") (ImposterCombinationGpuPostProcessingFilter.java:11-16) */
 int ccu_tonemap(ccu_ctx *ctx, int32_t width, int32_t height, float exposure, const double *input, int32_t type, int32_t *argb);
 
+/* ---- guided denoiser (beyond the reference; DESIGN.md §17) --------------------------------------------------------
+ * An edge-avoiding a-trous wavelet filter of Chunky's sample buffer, guided by the feature buffers of ccu_render_features.
+ * color = double[3*W*H] (the layout ccu_tonemap takes), albedo and normal = float[3*W*H]; the result goes to
+ * out = double[3*W*H], which may alias color.  The filter divides the colour by max(albedo, 2^-8), runs `iterations` 5x5
+ * passes with steps 1, 2, 4, ... whose weights stop at albedo, normal and luminance edges (the luminance stop scaled by
+ * sigma_luminance times the local standard deviation, from a 7x7 variance estimate), and multiplies the albedo back in, all in
+ * fp32.  Two pixels with zero normals (sky) blend with each other, not with geometry; a pixel with a non-finite input
+ * component keeps its value and is left out of its neighbours'.  Defaults: iterations 5, sigma_luminance 4.
+ * Blocking; needs a context but not ccu_render_begin, and leaves the accumulation window, its pass count and
+ * ccu_debug_last_render[_n] as they were.  CCU_EINVAL for a NULL context or buffer, width or height below 1, 3*W*H beyond
+ * int64, iterations outside [0, CCU_DENOISE_MAX_ITERATIONS], or a sigma_luminance that is not positive and finite. */
+#define CCU_DENOISE_MAX_ITERATIONS 8
+int ccu_denoise(ccu_ctx *ctx, int32_t width, int32_t height, const double *color, const float *albedo, const float *normal,
+                int32_t iterations, float sigma_luminance, double *out);
+
 /* ---- instrumentation ------------------------------------------------------------------------------------------ */
-int ccu_last_kernel_ms(ccu_ctx *ctx, float *ms);          /* CUDA-event time of the last render_passes / first_hit / features launch(es) */
+int ccu_last_kernel_ms(ccu_ctx *ctx, float *ms);          /* CUDA-event time of the last render_passes / first_hit / features / denoise launch(es) */
 int ccu_launch_count(ccu_ctx *ctx, int64_t *launches);    /* kernels launched by this context so far */
 /* Test support: the render kernel instance of the context's last ccu_render_passes[_async] launch (all zero before the first).
  * out = {kernel launched (1 or 4, after the choice for kernel 0), HAS_BVH, LAY (kernel 4) or MODE (kernel 1), spec, nee (a NeeKind:

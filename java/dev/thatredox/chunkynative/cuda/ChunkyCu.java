@@ -66,6 +66,7 @@ public final class ChunkyCu {
     private static final MethodHandle PREVIEW = h("ccu_preview", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS));
     private static final MethodHandle RENDER_FEATURES = h("ccu_render_features", FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, ADDRESS, ADDRESS));
     private static final MethodHandle TONEMAP = h("ccu_tonemap", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT, JAVA_INT, JAVA_FLOAT, ADDRESS, JAVA_INT, ADDRESS));
+    private static final MethodHandle DENOISE = h("ccu_denoise", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT, JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_INT, JAVA_FLOAT, ADDRESS));
     // multi-GPU group (include/chunkycu.h "multi-GPU"): one JVM drives all GPUs of the box
     private static final MethodHandle GROUP_CREATE = h("ccu_group_create", FunctionDescriptor.of(JAVA_INT, ADDRESS, JAVA_INT, ADDRESS));
     private static final MethodHandle GROUP_DESTROY = h("ccu_group_destroy", FunctionDescriptor.of(JAVA_INT, ADDRESS));
@@ -323,6 +324,21 @@ public final class ChunkyCu {
                 MemorySegment out = a.allocate(JAVA_INT, argb.length);
                 check(call(TONEMAP, handle, width, height, (float) exposure, in, filter, out));
                 MemorySegment.copy(out, JAVA_INT, 0, argb, 0, argb.length);
+            }
+        }
+
+        /** The guided a-trous denoiser (DESIGN §17): color = the double[3*W*H] sample buffer, albedo and normal = the float
+         *  feature buffers of renderFeatures, out = double[3*W*H] (may be color itself); defaults iterations 5,
+         *  sigmaLuminance 4 (include/chunkycu.h, ccu_denoise). */
+        public void denoise(int width, int height, double[] color, float[] albedo, float[] normal, int iterations,
+                            float sigmaLuminance, double[] out) {
+            try (Arena a = Arena.ofConfined()) {
+                MemorySegment c = a.allocateFrom(JAVA_DOUBLE, color);
+                MemorySegment al = a.allocateFrom(JAVA_FLOAT, albedo);
+                MemorySegment no = a.allocateFrom(JAVA_FLOAT, normal);
+                MemorySegment o = a.allocate(JAVA_DOUBLE, out.length);
+                check(call(DENOISE, handle, width, height, c, al, no, iterations, sigmaLuminance, o));
+                MemorySegment.copy(o, JAVA_DOUBLE, 0, out, 0, out.length);
             }
         }
 

@@ -5,7 +5,7 @@ ONLY.
 ``SpecularOracle`` is the parity oracle (``oracle.Oracle``) with the specular events of DESIGN.md section 9 in its path
 loop; ``FlagsOracle`` takes the render flags and adds the emitter sampling of sections 10 to 12, with the emitter table that
 ``emitter_grid`` builds from the packed arrays (``model_emitters`` adds the model emitters of section 12), and its ``features``
-restates the denoiser's feature buffers of section 16.  Everything else - first hit, preview, counters - is the oracle's.  Like the
+restates the denoiser's feature buffers of section 16; ``denoise`` restates the denoiser of section 17.  Everything else - first hit, preview, counters - is the oracle's.  Like the
 oracle, only tests/ and scripts use it.
 """
 from __future__ import annotations
@@ -95,6 +95,25 @@ def cloud_hit(clouds, o, d, limit=None):
 def dm_expf(x: float) -> float:
     """The fog's transmittance kernel (DESIGN.md section 14), as the restatement and the kernels evaluate it."""
     return float(np.float32(lib().fog_expf_test(float(x))))
+
+
+def denoise(color, albedo, normal, iterations: int, sigma_l: float, width: Optional[int] = None,
+            height: Optional[int] = None) -> np.ndarray:
+    """DESIGN.md section 17: the guided a-trous filter of a sample buffer, as the restatement evaluates it.  color: float64
+    (H, W, 3) or flat with width and height given; albedo, normal: float32 of the same layout.  Returns float64[3*W*H]."""
+    c = np.ascontiguousarray(color, np.float64)
+    if width is None or height is None:
+        height, width = c.shape[0], c.shape[1]
+    c = c.reshape(-1)
+    a = np.ascontiguousarray(albedo, np.float32).reshape(-1)
+    nrm = np.ascontiguousarray(normal, np.float32).reshape(-1)
+    assert c.size == a.size == nrm.size == 3 * width * height
+    out = np.empty_like(c)
+    rc = lib().denoise(C.c_int32(width), C.c_int32(height), c.ctypes.data_as(C.c_void_p), a.ctypes.data_as(C.c_void_p),
+                       nrm.ctypes.data_as(C.c_void_p), C.c_int32(iterations), C.c_float(sigma_l), out.ctypes.data_as(C.c_void_p))
+    if rc != 0:
+        raise MemoryError("specular_oracle.denoise: out of memory")
+    return out
 
 
 class _Biome(C.Structure):

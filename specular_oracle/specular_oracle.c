@@ -17,7 +17,8 @@
  * block test, the octree march and the emitter samplers pass that voxel on.  CCU_RENDER_FOG (section 14) restates the fog of
  * the path loop.  CCU_RENDER_CLOUDS (section 15) restates the cloud walk and where the path loop, the shadow rays, the emitter
  * sample's ray and the fog's sun sample meet it.  The feature buffers of a denoiser (section 16) take the first segment of the path
- * loop with the biome colours and the clouds.
+ * loop with the biome colours and the clouds.  The guided denoiser (section 17) is restated whole: it reads only the buffers
+ * it is given.
  */
 #include "../oracle/chunky_oracle.c"
 
@@ -936,6 +937,115 @@ int fog_params_struct_size(void) { return (int)sizeof(FogParams); }
 
 /* the fog's transmittance kernel alone, for tests */
 float fog_expf_test(float x) { return fog_expf(x); }
+
+/* ---- the guided denoiser (DESIGN.md section 17) ---- */
+
+/* dm_expf_weight of ccu_math.cuh: fog_expf, with 0 below -87 */
+static float denoise_expf(float x) { return x < -87.0f ? 0.0f : fog_expf(x); }
+
+static float denoise_lum(float x, float y, float z) { return 0.2126f * x + 0.7152f * y + 0.0722f * z; }
+
+/* section 2 rule 2: dot(u, v) = fma(u.z, v.z, fma(u.x, v.x, u.y * v.y)) */
+static float denoise_dot(const float *u, const float *v) { return fmaf(u[2], v[2], fmaf(u[0], v[0], u[1] * v[1])); }
+
+/* The edge-avoiding a-trous filter of section 17.1 on W x H pixels: color double[3WH] (Chunky's sample buffer), albedo and
+ * normal float[3WH], iterations in [0, 8], sigma_l > 0; out double[3WH] may alias color.  Returns -1 without memory. */
+int denoise(int32_t w, int32_t h, const double *color, const float *albedo, const float *normal, int32_t iterations, float sigma_l,
+            double *out) {
+    static const float K[5] = {1.0f / 16, 1.0f / 4, 3.0f / 8, 1.0f / 4, 1.0f / 16};
+    const int64_t n = (int64_t)w * h;
+    float *e = malloc((size_t)n * 4 * sizeof(float)), *f = malloc((size_t)n * 4 * sizeof(float));   /* (e.rgb, var) */
+    float *lum = malloc((size_t)n * sizeof(float));
+    unsigned char *valid = malloc((size_t)n);
+    if (!e || !f || !lum || !valid) { free(e); free(f); free(lum); free(valid); return -1; }
+    /* 1. per-pixel setup */
+    for (int64_t i = 0; i < n; i++) {
+        int ok = 1;
+        for (int k = 0; k < 3; k++) {
+            const float c = (float)color[3 * i + k], d = fmaxf(albedo[3 * i + k], 0x1p-8f);
+            ok &= isfinite(c) && isfinite(albedo[3 * i + k]) && isfinite(normal[3 * i + k]);
+            e[4 * i + k] = c / d;
+        }
+        e[4 * i + 3] = 0.0f;
+        valid[i] = (unsigned char)ok;
+        lum[i] = denoise_lum(e[4 * i], e[4 * i + 1], e[4 * i + 2]);
+    }
+    /* 2. the initial variance: luminance moments over the valid pixels of the 7x7 window inside the image */
+    if (iterations > 0) {
+#pragma omp parallel for schedule(static)
+        for (int64_t i = 0; i < n; i++) {
+            if (!valid[i]) continue;
+            const int x = (int)(i % w), y = (int)(i / w);
+            float s1 = 0.0f, s2 = 0.0f, m = 0.0f;
+            for (int dy = -3; dy <= 3; dy++)
+                for (int dx = -3; dx <= 3; dx++) {
+                    const int qx = x + dx, qy = y + dy;
+                    if (qx < 0 || qx >= w || qy < 0 || qy >= h) continue;
+                    const int64_t q = (int64_t)qy * w + qx;
+                    if (!valid[q]) continue;
+                    s1 = s1 + lum[q];
+                    s2 = s2 + lum[q] * lum[q];
+                    m = m + 1.0f;
+                }
+            const float mu = s1 / m;
+            e[4 * i + 3] = fmaxf(0.0f, s2 / m - mu * mu);
+        }
+    }
+    /* 3. the iterations, step 2^it */
+    for (int it = 0; it < iterations; it++) {
+        const int step = 1 << it;
+#pragma omp parallel for schedule(static)
+        for (int64_t i = 0; i < n; i++) {
+            const float *ep = e + 4 * i;
+            float *fp = f + 4 * i;
+            if (!valid[i]) { memcpy(fp, ep, 4 * sizeof(float)); continue; }
+            const int x = (int)(i % w), y = (int)(i / w);
+            const float *ap = albedo + 3 * i, *np_ = normal + 3 * i;
+            const float lp = denoise_lum(ep[0], ep[1], ep[2]);
+            const float dl_den = sigma_l * sqrtf(ep[3]) + 1e-4f;
+            const int sky_p = np_[0] == 0.0f && np_[1] == 0.0f && np_[2] == 0.0f;
+            float sw = 0.0f, sv = 0.0f, s[3] = {0.0f, 0.0f, 0.0f};
+            for (int dy = -2; dy <= 2; dy++)
+                for (int dx = -2; dx <= 2; dx++) {
+                    const int qx = x + dx * step, qy = y + dy * step;
+                    if (qx < 0 || qx >= w || qy < 0 || qy >= h) continue;
+                    const int64_t q = (int64_t)qy * w + qx;
+                    if (!valid[q]) continue;
+                    const float *eq = e + 4 * q;
+                    float wt;
+                    if (dx == 0 && dy == 0) {
+                        wt = 9.0f / 64.0f;
+                    } else {
+                        const float *aq = albedo + 3 * q, *nq = normal + 3 * q;
+                        const float dl = fabsf(lp - denoise_lum(eq[0], eq[1], eq[2])) / dl_den;
+                        const float da3[3] = {ap[0] - aq[0], ap[1] - aq[1], ap[2] - aq[2]};
+                        const float da = denoise_dot(da3, da3) / 0.01f;
+                        float wn = 1.0f;
+                        if (!(sky_p && nq[0] == 0.0f && nq[1] == 0.0f && nq[2] == 0.0f)) {
+                            wn = fmaxf(0.0f, denoise_dot(np_, nq));
+                            for (int r = 0; r < 7; r++) wn = wn * wn;
+                        }
+                        wt = K[dx + 2] * K[dy + 2] * wn * denoise_expf(-(dl + da));
+                    }
+                    s[0] = s[0] + wt * eq[0];
+                    s[1] = s[1] + wt * eq[1];
+                    s[2] = s[2] + wt * eq[2];
+                    sv = sv + wt * wt * eq[3];
+                    sw = sw + wt;
+                }
+            fp[0] = s[0] / sw;
+            fp[1] = s[1] / sw;
+            fp[2] = s[2] / sw;
+            fp[3] = sv / (sw * sw);
+        }
+        float *t = e; e = f; f = t;
+    }
+    /* 4. remodulation */
+    for (int64_t i = 0; i < n; i++)
+        for (int k = 0; k < 3; k++) out[3 * i + k] = (double)(e[4 * i + k] * fmaxf(albedo[3 * i + k], 0x1p-8f));
+    free(e); free(f); free(lum); free(valid);
+    return 0;
+}
 
 int biome_tiles_struct_size(void) { return (int)sizeof(BiomeTiles); }
 
